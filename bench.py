@@ -11,7 +11,7 @@ Workload (BASELINE.json configs[2], the one the metric is quoted on; fits one GP
   over N ranks (BASELINE configs[2] as stated: "strong" scaling, 16 / N frequencies per GPU); with N > 1 the line also
   carries `weak_scaling`: the rate with 16 frequencies kept on every GPU (a 16*N-frequency objective over the same band).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   (N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 `value`  : device-resident inputs, CUDA events, max over ranks.
@@ -74,7 +74,12 @@ def parse():
     ap.add_argument("--engine", default="auto", choices=["auto", "simt", "tc2"])
     ap.add_argument("--cpu-cols", type=int, default=24, help="columns of the CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the (loss, grad) of the last timed step as DIR/loss.npy and DIR/grad.npy, for comparing two builds "
+                         "output for output (the inputs are the same from run to run)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if a.config == "cfg2":
         a.n, a.nsrc, a.nfreq = 256, 256, 1
     elif a.config == "cfg4":
@@ -349,6 +354,8 @@ def main():
         clk.start()
     ms_dev, (loss, grad) = H.timed(H.step_dev, a.steps)
     clocks = clk.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, loss, grad)
     launches = int(L.ust_launch_count())
     ms_step = ms_dev / a.steps
     value = units_per_step / (ms_step / 1e3)
@@ -517,6 +524,22 @@ def main():
     H.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, loss, grad):
+    """What the timed step hands its caller: the all-reduced loss (float64) and gradient (float32 for complex64, float64 for
+    complex128).  A gradient larger than DUMP_BYTES is replaced by the entries at a fixed, seeded, sorted set of flat indices."""
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "loss.npy"), loss.detach().cpu().numpy().astype(np.float64))
+    g = grad.detach().cpu().numpy().ravel()
+    if g.nbytes > DUMP_BYTES - 4096:
+        g = g[np.sort(np.random.default_rng(0).choice(g.size, (DUMP_BYTES - 4096) // g.itemsize, replace=False))]
+    else:
+        g = g.reshape(grad.shape)
+    np.save(os.path.join(d, "grad.npy"), g)
 
 
 def plan_np(geom):

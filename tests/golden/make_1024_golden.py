@@ -3,9 +3,11 @@
 The oracle is too slow at this size to run inside the GPU test suite, so its wavefields for 8 of the 1024 sources (forward and
 adjoint) are sampled -- every ring-element node, three full grid rows, the field norms -- and committed; tests/test_gpu_parity.py
 holds the CUDA path (complex64 and complex128) to them."""
+import io
 import os
 import sys
 import time
+import zipfile
 
 import numpy as np
 
@@ -38,6 +40,11 @@ if __name__ == "__main__":
         out["norm_" + key] = np.linalg.norm(u.reshape(-1, u.shape[2]), axis=0)
         out["norm_interior_" + key] = np.linalg.norm(u[1:-1, 1:-1].reshape(-1, u.shape[2]), axis=0)
         print(key, out["norm_" + key], flush=True)
-    np.savez_compressed(os.path.join(HERE, "cfg4_1024_wavefields.npz"), n=n, nelem=nelem, stride=stride, f=f, bde=np.array(bde),
-                        rows=np.array(ROWS), **out)
+    out.update(n=n, nelem=nelem, stride=stride, f=f, bde=np.array(bde), rows=np.array(ROWS))
+    # an .npz with LZMA members (np.load reads them): deflate leaves the complex128 samples just over 1 MB
+    with zipfile.ZipFile(os.path.join(HERE, "cfg4_1024_wavefields.npz"), "w", compression=zipfile.ZIP_LZMA) as zf:
+        for k, v in out.items():
+            buf = io.BytesIO()
+            np.lib.format.write_array(buf, np.asanyarray(v))
+            zf.writestr(k + ".npy", buf.getvalue())
     print("done %.0f s" % (time.time() - t0))

@@ -32,7 +32,8 @@ def test_library_exports_every_declared_symbol():
 def test_library_is_built_for_sm100a_only():
     from waveforminversionust_b200 import build
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", build.LIBPATH], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(os.path.realpath(build._nvcc())), "cuobjdump")  # the toolkit that built the library, on PATH or not
+    out = subprocess.run([cuobjdump, "-lelf", build.LIBPATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
