@@ -124,6 +124,15 @@ int ust_fwi_loss_grad_host(ust_plan* plan, const void* slow_host, const void* re
  * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles. */
 int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, void* stream);
 
+/* Gauss-Newton Hessian-vector product of the joint objective on the factors, forward fields and source estimates of the last
+ * ust_fwi_loss_grad on this plan (no assembly, no factorisation): hv = Re(J^H J v) with J the linearisation of
+ * nonlinearcg.py:258,279 (alpha fixed).  v_dev, hv_dev: (ny, nx) real.  jv2_dev: one double, sum |J v|^2 (= <v, hv>).
+ * jv_dev: (nfreq, nt, nm) complex J v at the kept receivers (mask order), or NULL.  Overwrites the adjoint wavefield.
+ * J is the linearisation the gradient uses (virtual source 2 w^2 s alpha u without the stencil's mass weights and the PML
+ * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).
+ * Fails if ust_factor or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad. */
+int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream);
+
 /* Introspection for parity tests and callers that want the intermediate fields (device pointers into
  * plan-owned buffers, valid until the next ust_fwi_* call on the plan). */
 int ust_get_bde(ust_plan* plan, double* bde_host /* max_freq*3 */);

@@ -7,7 +7,9 @@ from .api import (  # noqa: F401
     clear_plans,
     continuation_stages,
     frequency_continuation,
+    fwi_gauss_newton_product,
     fwi_loss_function,
+    gauss_newton_fwi,
     hanning,
     idtft,
     nonlinear_conjugate_gradient,

@@ -18,6 +18,7 @@ or "c128"), ``engine`` ("auto" | "simt" | "tc2": block-GEMM engine; tcgen05 is c
 from __future__ import annotations
 
 import hashlib
+import math
 
 import numpy as np
 
@@ -166,10 +167,65 @@ def fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, i
         rec = REC_DATA.to(plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
         slow = params.to(plan.treal).reshape(plan.ny, plan.nx).contiguous()
         loss, grad = plan.fwi_loss_grad(slow, rec, freqs, bde=bde)
+        plan._eval_key = _eval_key(params, REC_DATA, freqs, bde)
         return loss[0], grad.reshape(params.shape)
     p = _to_np(params)
     loss, grad = plan.fwi_loss_grad_host(p.reshape(plan.ny, plan.nx), _to_np(REC_DATA), freqs, bde=bde)
+    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde)
     return loss, grad.reshape(p.shape)
+
+
+def _eval_key(params, REC_DATA, freqs, bde):
+    """What identifies an evaluation's state on the plan: device inputs are kept as copies (compared on the device), host
+    inputs as a hash."""
+    b = None if bde is None else np.asarray(bde, dtype=np.float64)
+    if _is_torch(params) and params.is_cuda:
+        rec = REC_DATA.detach().clone() if _is_torch(REC_DATA) else _fingerprint(np.asarray(REC_DATA))
+        return ("dev", params.detach().clone(), rec, _fingerprint(freqs, b))
+    return ("host", _fingerprint(np.asarray(_to_np(params)), np.asarray(_to_np(REC_DATA)), freqs, b))
+
+
+def _same_eval(a, b):
+    import torch
+    if a is None or b is None or a[0] != b[0] or len(a) != len(b):
+        return False
+    for x, y in zip(a[1:], b[1:]):
+        if _is_torch(x) != _is_torch(y):
+            return False
+        if _is_torch(x):
+            if x.shape != y.shape or x.dtype != y.dtype or x.device != y.device or not torch.equal(x, y):
+                return False
+        elif x != y:
+            return False
+    return True
+
+
+def fwi_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
+                             *, dtype="c64", bde=None, stencil="python", engine="auto"):
+    """Gauss-Newton Hessian-vector product ``H_GN v = Re(J^H J v)`` of the objective of ``fwi_loss_function`` at slowness
+    ``params``, returned with ``params``' shape (NumPy in, NumPy out; a CUDA tensor ``v`` gives a CUDA tensor).
+
+    ``J`` is the linearisation the gradient is built from (``nonlinearcg.py:258,279``): the perturbation solve with virtual
+    source ``-2 w^2 s alpha u v``, gathered at the kept receivers, with the source estimates ``alpha`` held fixed, so that the
+    gradient is ``Re(J^H residual)``.  The virtual source leaves out the stencil's mass weights and the PML factor, as the
+    reference does: ``J`` is not the exact derivative of the discrete forward map (DESIGN.md section 7c).
+
+    A product costs two all-source sweeps on the factorisation the last evaluation left on the plan; when the last
+    ``fwi_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)``, the evaluation runs first.
+    """
+    import torch
+    dev = _device_of(params, REC_DATA, v)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
+    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde)):
+        fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
+                          dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+    shape = tuple(params.shape) if hasattr(params, "shape") else np.shape(params)
+    if _is_torch(v) and v.is_cuda:
+        hv, _ = plan.gn_hvp(v.detach().to(plan.treal).reshape(plan.ny, plan.nx).contiguous())
+        return hv.reshape(shape)
+    vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real).reshape(plan.ny, plan.nx))).to(f"cuda:{plan.device}")
+    hv, _ = plan.gn_hvp(vt)
+    return hv.cpu().numpy().reshape(shape)
 
 
 def nonlinear_conjugate_gradient(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter,
@@ -270,6 +326,103 @@ def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, 
     return 1.0 / final_slow
 
 
+def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
+                     cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, dtype="c64", bde=None, stencil="python", device=0,
+                     engine="auto", history=None, loss_grad=None, hvp=None):
+    """Truncated Gauss-Newton FWI on the slowness, with the arguments of ``nonlinear_conjugate_gradient``; returns the sound
+    speed (Ny, Nx) as a NumPy array.
+
+    Per outer iteration: conjugate gradients from ``p = 0`` on ``(H_GN + mu I) p = -g`` with at most ``cg_iters`` Gauss-Newton
+    products (``fwi_gauss_newton_product``), stopped early when ``|r| <= cg_tol |g|`` or the curvature is not positive;
+    ``mu = damping * <g, H_GN g> / <g, g>`` comes from the first product.  Then ``s + p`` is tried and the step halved up to
+    ``max_backtracks`` times until the loss decreases; without a decrease the driver stops.  One evaluation (one
+    factorisation) per trial; the products reuse the factorisation of the accepted trial.  With ``cg_iters=1`` and
+    ``damping=0`` the first iteration is the reference NCG's first iteration (steepest descent with the linearised exact step,
+    ``nonlinearcg.py:268-301``).
+
+    ``loss_grad(slow) -> (loss, grad)`` and ``hvp(v) -> hv`` (products at the point of the last ``loss_grad`` call) replace
+    the GPU objective; they receive (Ny, Nx) float64 torch tensors and may return tensors or NumPy arrays.  The vector
+    algebra is float64 torch on the device of the first gradient.  ``history`` (a list) receives one dict per outer
+    iteration: loss, CG iterations, the quadratic-model value ``q(p_k) = <g,p_k>/2 - <p_k,r_k>/2`` of every CG iterate, mu,
+    the accepted step, cumulative evaluation and product counts, the velocity range, and ``stop`` when the driver stops.
+    """
+    import torch
+    ny, nx = _to_np(yi).size, _to_np(xi).size
+    if loss_grad is None or hvp is None:
+        freqs = np.atleast_1d(np.asarray(_to_np(f), dtype=np.float64)).ravel()
+        dv = torch.device(f"cuda:{device}")
+        real = torch.float32 if dtype == "c64" else torch.float64
+        rec = torch.as_tensor(_to_np(REC_DATA)).to(dv).reshape(freqs.size, len(_to_np(tx_include)), -1).contiguous()
+        state = {}
+        fargs = (xi, yi, rec, SRC, freqs, a0, L_PML, tx_include, ind_matlab, mask_indices, numElements)
+        kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+
+        def loss_grad(slow):
+            state["slow"] = slow.to(dv, real).contiguous()
+            loss, grad = fwi_loss_function(state["slow"], *fargs, **kw)
+            return float(loss), grad
+
+        def hvp(v):
+            return fwi_gauss_newton_product(state["slow"], v.to(dv, real).contiguous(), *fargs, **kw)
+
+    def f64(a, dv):
+        return a.detach().to(dv, torch.float64) if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, dtype=np.float64)).to(dv)
+
+    c0 = np.asarray(_to_np(c_init), dtype=np.float64) * np.ones((ny, nx))
+    s = torch.as_tensor(1.0 / c0)
+    loss, g = loss_grad(s)
+    dv = g.device if torch.is_tensor(g) else torch.device("cpu")
+    s, g, loss = s.to(dv), f64(g, dv).reshape(ny, nx), float(loss)
+    nevals, nprods = 1, 0
+    dot = lambda a, b: float(torch.sum(a * b))
+    for it in range(int(Niter)):
+        rec = dict(it=it, loss=loss)
+        gg = dot(g, g)
+        p = torch.zeros_like(g)
+        r, d, rr = -g, -g, gg
+        qs, mu, k = [], 0.0, 0
+        while k < int(cg_iters):
+            Hd = f64(hvp(d), dv).reshape(ny, nx)
+            nprods += 1
+            if k == 0:
+                mu = float(damping) * dot(d, Hd) / gg  # d = -g
+            Ad = Hd + mu * d
+            curv = dot(d, Ad)
+            if not curv > 0:
+                break
+            a = rr / curv
+            p = p + a * d
+            r = r - a * Ad
+            k += 1
+            qs.append(0.5 * dot(g, p) - 0.5 * dot(p, r))
+            rr_new = dot(r, r)
+            if math.sqrt(rr_new) <= float(cg_tol) * math.sqrt(gg):
+                break
+            d = r + (rr_new / rr) * d
+            rr = rr_new
+        rec.update(cg_iters=k, q=qs, mu=mu)
+        step, accepted = 1.0, False
+        if k > 0:
+            for _ in range(int(max_backtracks) + 1):
+                trial = s + step * p
+                lt, gt = loss_grad(trial)
+                nevals += 1
+                if float(lt) < loss:
+                    s, loss, g, accepted = trial, float(lt), f64(gt, dv).reshape(ny, nx), True
+                    break
+                step *= 0.5
+        rec.update(step=step if accepted else 0.0, evals=nevals, products=nprods, vel_min=float(1.0 / s.max()),
+                   vel_max=float(1.0 / s.min()))
+        if not accepted:
+            rec["stop"] = ("no positive curvature along -g" if k == 0 else
+                           f"no loss decrease after {int(max_backtracks)} step halvings")
+        if history is not None:
+            history.append(rec)
+        if not accepted:
+            break
+    return (1.0 / s).cpu().numpy()
+
+
 # -------------------------------------------------------------------------------------------------
 # SURVEY section 8(f) rank 4: time-domain synthesis and the low-to-high frequency schedule
 # -------------------------------------------------------------------------------------------------
@@ -360,13 +513,16 @@ def continuation_stages(f, nstages):
 
 
 def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, stages, Niter,
-                           a0, L_PML, mask_indices, *, dtype="c64", stencil="python", device=0, engine="auto", history=None):
+                           a0, L_PML, mask_indices, *, dtype="c64", stencil="python", device=0, engine="auto", history=None,
+                           method="ncg"):
     """Multi-frequency FWI by frequency continuation: for every stage (an index array into ``f``, see
-    ``continuation_stages``) ``Niter`` NCG iterations (``nonlinear_conjugate_gradient``) on the joint objective of that
-    stage's frequencies, each stage starting from the sound speed the previous one ended with.  ``REC_DATA`` is
-    (Nf, Nt, E).  Returns the final sound speed (Ny, Nx); ``history`` (a list) receives one list of per-iteration
-    records per stage.
+    ``continuation_stages``) ``Niter`` NCG iterations (``nonlinear_conjugate_gradient``; ``method="gn"``: ``Niter`` outer
+    iterations of ``gauss_newton_fwi`` with its default settings) on the joint objective of that stage's frequencies, each
+    stage starting from the sound speed the previous one ended with.  ``REC_DATA`` is (Nf, Nt, E).  Returns the final sound
+    speed (Ny, Nx); ``history`` (a list) receives one list of per-iteration records per stage.
     """
+    if method not in ("ncg", "gn"):
+        raise ValueError("method must be 'ncg' or 'gn'")
     f = np.asarray(_to_np(f), dtype=np.float64).ravel()
     rec = _to_np(REC_DATA)
     if rec.ndim != 3 or rec.shape[0] != f.size:
@@ -379,9 +535,13 @@ def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
             clear_plans()  # a plan is sized for its number of frequencies; do not keep two factor stores alive
         prev = idx.size
         h = [] if history is not None else None
-        vel, _, _, _, _ = nonlinear_conjugate_gradient(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter,
-                                                       a0, L_PML, mask_indices, dtype=dtype, stencil=stencil, device=device,
-                                                       history=h, return_fields=False, engine=engine)
+        if method == "gn":
+            vel = gauss_newton_fwi(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter, a0, L_PML,
+                                   mask_indices, dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+        else:
+            vel, _, _, _, _ = nonlinear_conjugate_gradient(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter,
+                                                           a0, L_PML, mask_indices, dtype=dtype, stencil=stencil, device=device,
+                                                           history=h, return_fields=False, engine=engine)
         if history is not None:
             history.append(h)
     return vel

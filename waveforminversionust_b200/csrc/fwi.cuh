@@ -6,6 +6,8 @@
 //                           one warp per pixel, warp-shuffle reduction     (nonlinearcg.py:258,264-265)
 //   pert_rhs_kernel       : RHS of the perturbation solve  -VIRT * sd      (nonlinearcg.py:279-281)
 //   linesearch_kernel     : dREC gather and the two step-size scalars      (nonlinearcg.py:22-28,284-298)
+//   gn_receiver_kernel    : Gauss-Newton product: J v = perturbation field at the kept receivers, and sum |J v|^2
+//   gn_scatter_kernel     : Gauss-Newton product: J v back at the receiver nodes as the adjoint source of J^H (J v)
 // Algorithmic bytes of gradient_kernel: 2 complex reads per (pixel, source, frequency) = 16 B (c64).
 #pragma once
 #include "common.cuh"
@@ -230,6 +232,48 @@ __global__ void __launch_bounds__(256) linesearch_kernel(LineArgs<R> a) {
         atomicAdd(a.out2 + 0, s[0]);
         atomicAdd(a.out2 + 1, s[1]);
     }
+}
+
+// Gauss-Newton product H_GN v = Re(J^H J v) (ustfwi.cu gn_hvp_enqueue).  After the perturbation solve Pert = H^-1(-VIRT v),
+// J v of transmitter t is Pert at its kept receivers: gathered into drec [nfreq][nt][nm] (mask order, what linesearch_kernel
+// reads as dREC) with sum |J v|^2 -> *jv2.  One CTA per (transmitter, frequency).
+template <typename R>
+struct GnRecvArgs {
+    const cx<R>* Pert;  // perturbation fields [nfreq][N*nt]
+    cx<R>* Lam;         // adjoint right-hand side [nfreq][N*nt], zeroed between the two kernels (gn_scatter_kernel)
+    size_t stride_f;
+    const int* rx_lin;
+    const int* mask;
+    cx<R>* drec;        // [nfreq][nt][nm]
+    double* jv2;
+    int nt, nm;
+};
+
+template <typename R>
+__global__ void __launch_bounds__(256) gn_receiver_kernel(GnRecvArgs<R> a) {
+    __shared__ double sh[1 * 32];
+    const int t = blockIdx.x, f = blockIdx.y;
+    const cx<R>* Pf = a.Pert + (size_t)f * a.stride_f;
+    const int* mk = a.mask + (size_t)t * a.nm;
+    cx<R>* d_out = a.drec + ((size_t)f * a.nt + t) * a.nm;
+    double s[1] = {0};
+    for (int j = threadIdx.x; j < a.nm; j += blockDim.x) {
+        const cx<R> d = Pf[(size_t)a.rx_lin[mk[j]] * a.nt + t];
+        d_out[j] = d;
+        s[0] += (double)d.re * d.re + (double)d.im * d.im;
+    }
+    block_sum<1>(s, sh);
+    if (threadIdx.x == 0) atomicAdd(a.jv2, s[0]);
+}
+
+// J v as the adjoint source: the same stores as receiver_kernel's Lf[o] = d, so that J^H is the adjoint the gradient uses
+template <typename R>
+__global__ void __launch_bounds__(256) gn_scatter_kernel(GnRecvArgs<R> a) {
+    const int t = blockIdx.x, f = blockIdx.y;
+    cx<R>* Lf = a.Lam + (size_t)f * a.stride_f;
+    const int* mk = a.mask + (size_t)t * a.nm;
+    const cx<R>* d_in = a.drec + ((size_t)f * a.nt + t) * a.nm;
+    for (int j = threadIdx.x; j < a.nm; j += blockDim.x) Lf[(size_t)a.rx_lin[mk[j]] * a.nt + t] = d_in[j];
 }
 
 // Residual of one forward column: r = H u_t - e_src(t) on the interior nodes, from the nine coefficient planes (what

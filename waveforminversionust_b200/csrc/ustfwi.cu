@@ -79,7 +79,9 @@ struct ust_plan {
     short first_row[8], last_row[8];   // per 128-column tile: smallest / largest interior block row holding a source
     // plan-owned copies of the FWI inputs / outputs (stable addresses for graph replay)
     void *slow_in = nullptr, *rec_in = nullptr, *grad_out = nullptr, *sd_in = nullptr;
+    void *v_in = nullptr, *hv_out = nullptr, *drec = nullptr;  // Gauss-Newton product: v, H_GN v, J v at the kept receivers
     bool fwi_done = false;
+    bool gn_ok = false;  // the factors, fields and source estimates are those of the last ust_fwi_loss_grad (ust_fwi_gn_hvp)
     bool use_graphs = true;  // UST_NO_GRAPHS=1 disables
     struct GraphEntry { cudaGraphExec_t exec = nullptr; long long launches = 0; };
     std::map<long long, GraphEntry> graphs;
@@ -464,6 +466,7 @@ static int factor_enqueue(ust_plan* p, const void* vel_dev, int nfreq, bool has_
 
 template <typename R>
 static int factor_impl(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs, const double* bde, cudaStream_t st) {
+    p->gn_ok = false;  // the factors no longer belong to the forward fields of the last evaluation
     UST_TRY(upload_params(p, nfreq, freqs, bde, st));
     return factor_enqueue<R>(p, vel_dev, nfreq, bde != nullptr, st);
 }
@@ -724,6 +727,61 @@ static int linesearch_enqueue(ust_plan* p, cudaStream_t st) {
     return 0;
 }
 
+// Gauss-Newton Hessian-vector product hv = Re(J^H J v) on the factors, forward fields and source estimates of the last
+// evaluation, device work only: reads p->v_in, writes p->hv_out, p->drec (J v) and p->d_scal[6] (sum |J v|^2).  Per group:
+// perturbation solve with RHS -VIRT*v (as linesearch_enqueue), J v gathered at the kept receivers, scattered back as the
+// adjoint source, adjoint sweeps (as fwi_enqueue); the groups meet at gradient_kernel, which forms sum_f -Re(conj(VIRT) * adj).
+template <typename R>
+static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st) {
+    const Geom& g = p->g;
+    const int nt = p->nt, nfreq = p->nfreq_cur;
+    const size_t stride = (size_t)g.N * nt;
+    double* jv2 = p->d_scal + 6;
+    UST_CUDA(cudaMemsetAsync(jv2, 0, sizeof(double), st));
+    const std::vector<Group> gs = make_groups(p, 0, nfreq, st);
+    UST_TRY(fork_groups(p, gs));
+    for (const Group& q : gs) {
+        PertArgs<R> pa;
+        pa.U = (const cx<R>*)p->U + (size_t)q.f0 * stride; pa.Out = (cx<R>*)p->Lam + (size_t)q.f0 * stride; pa.stride_f = stride;
+        pa.src_est = (const cx<R>*)p->src_est + (size_t)q.f0 * nt;
+        pa.freqs = p->d_freqs + q.f0; pa.slow = (const R*)p->slow_in; pa.sd = (const R*)p->v_in; pa.N = g.N; pa.nt = nt; pa.nfreq = q.nf;
+        pert_rhs_kernel<R><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+        UST_LAUNCH_CHECK();
+    }
+    UST_TRY(sweeps_groups<R>(p, gs, (cx<R>*)p->Lam, stride, nt, 0));
+    for (const Group& q : gs) {
+        GnRecvArgs<R> ra;
+        ra.Pert = (const cx<R>*)p->Lam + (size_t)q.f0 * stride; ra.Lam = (cx<R>*)p->Lam + (size_t)q.f0 * stride; ra.stride_f = stride;
+        ra.rx_lin = p->rx_lin; ra.mask = p->mask; ra.drec = (cx<R>*)p->drec + (size_t)q.f0 * nt * p->nm; ra.jv2 = jv2;
+        ra.nt = nt; ra.nm = p->nm;
+        {
+            ProfScope ps(p, PC_RECEIVER, q.st);
+            gn_receiver_kernel<R><<<dim3(nt, q.nf), 256, 0, q.st>>>(ra);
+        }
+        UST_LAUNCH_CHECK();
+        UST_CUDA(cudaMemsetAsync((cx<R>*)p->Lam + (size_t)q.f0 * stride, 0, stride * q.nf * sizeof(cx<R>), q.st));
+        {
+            ProfScope ps(p, PC_RECEIVER, q.st);
+            gn_scatter_kernel<R><<<dim3(nt, q.nf), 256, 0, q.st>>>(ra);
+        }
+        UST_LAUNCH_CHECK();
+    }
+    UST_TRY(sweeps_groups<R>(p, gs, (cx<R>*)p->Lam, stride, nt, 1));
+    for (const Group& q : gs)
+        for (int f = q.f0; f < q.f0 + q.nf; ++f) UST_TRY(ring_fix<R>(p, f, (cx<R>*)p->Lam + (size_t)f * stride, nt, 1, false, q.st));
+    UST_TRY(join_groups(p, gs));
+    GradArgs<R> ga;
+    ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
+    ga.freqs = p->d_freqs; ga.slow = (const R*)p->slow_in; ga.grad = (R*)p->hv_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
+    const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
+    {
+        ProfScope ps(p, PC_GRADIENT, st);
+        gradient_kernel<R><<<blocks, 256, 0, st>>>(ga);
+    }
+    UST_LAUNCH_CHECK();
+    return 0;
+}
+
 // Run `enqueue` on the caller's stream directly, or -- the normal case -- as a CUDA graph captured once per key and
 // replayed: a step is ~2e4 dependent launches of 5-100 us each, and at ~10 us of host time per launch the CPU, not
 // the GPU, sets the pace as soon as the per-GPU batch is small.  Graphs run on the plan's own stream (the caller's may
@@ -775,12 +833,14 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     if (rec != p->rec_in) UST_CUDA(cudaMemcpyAsync(p->rec_in, rec, (size_t)nfreq * p->nt * p->nelem * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
     const bool has_bde = bde != nullptr;
     const long long key = 1000LL * nfreq + (has_bde ? 1 : 0);
+    p->gn_ok = false;
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_); }));
     p->nfreq_cur = nfreq;
     p->factored = true;
     UST_CUDA(cudaMemcpyAsync(loss_dev, p->d_scal, sizeof(double), cudaMemcpyDeviceToDevice, st));
     UST_CUDA(cudaMemcpyAsync(grad_dev, p->grad_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     p->fwi_done = true;
+    p->gn_ok = true;
     if (p->trace) return dump_update_trace(p, st);
     return 0;
 }
@@ -793,6 +853,25 @@ static int linesearch_impl(ust_plan* p, const void* sd, double* out2, cudaStream
     const long long key = 1000LL * p->nfreq_cur + 500;
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_); }));
     UST_CUDA(cudaMemcpyAsync(out2, p->d_scal + 2, 2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+template <typename R>
+static int gn_hvp_impl(ust_plan* p, const void* v, void* hv, double* jv2, void* jv, cudaStream_t st) {
+    const Geom& g = p->g;
+    if (!p->v_in) { set_error("ust_fwi_gn_hvp: plan was created with fwi_buffers=0"); return 1; }
+    if (!p->factored || !p->fwi_done) { set_error("ust_fwi_gn_hvp: call ust_fwi_loss_grad first"); return 1; }
+    if (!p->gn_ok) {
+        set_error("ust_fwi_gn_hvp: the factors were replaced (ust_factor / ust_solve_helmholtz_host) after the last ust_fwi_loss_grad; "
+                  "call ust_fwi_loss_grad again");
+        return 1;
+    }
+    UST_CUDA(cudaMemcpyAsync(p->v_in, v, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    const long long key = 1000LL * p->nfreq_cur + 600;
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_); }));
+    UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    UST_CUDA(cudaMemcpyAsync(jv2, p->d_scal + 6, sizeof(double), cudaMemcpyDeviceToDevice, st));
+    if (jv) UST_CUDA(cudaMemcpyAsync(jv, p->drec, (size_t)p->nfreq_cur * p->nt * p->nm * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
     return 0;
 }
 
@@ -991,6 +1070,8 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
         rc |= dev_alloc(p, &p->slow_in, g.N * p->rsz);
         rc |= dev_alloc(p, &p->grad_out, g.N * p->rsz);
         rc |= dev_alloc(p, &p->sd_in, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->v_in, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->hv_out, g.N * p->rsz);
     }
     if (const char* e = getenv("UST_NO_GRAPHS")) p->use_graphs = atoi(e) == 0;
     if (const char* e = getenv("UST_NO_PDL")) ust::g_use_pdl = atoi(e) == 0;
@@ -1057,7 +1138,7 @@ int ust_plan_destroy(ust_plan* p) {
     for (void* q : ptrs)
         if (q) cudaFree(q);
     drop_graphs(p);
-    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in})
+    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in, p->v_in, p->hv_out, p->drec})
         if (q) cudaFree(q);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
     if (p->ev_out) cudaEventDestroy(p->ev_out);
@@ -1119,11 +1200,14 @@ int ust_plan_set_acquisition(ust_plan* p, int nt, const int32_t* src_lin, int ne
     UST_CUDA(cudaDeviceSynchronize());
     drop_graphs(p);
     p->fwi_done = false;
+    p->gn_ok = false;
     for (int** q : {&p->src_lin, &p->rx_lin, &p->mask})
         if (*q) { cudaFree(*q); *q = nullptr; }
     if (p->rec_in) { cudaFree(p->rec_in); p->rec_in = nullptr; }
     if (p->rec_h2d) { cudaFree(p->rec_h2d); p->rec_h2d = nullptr; }  // sized by nt * nelem: regrown by the next host call
+    if (p->drec) { cudaFree(p->drec); p->drec = nullptr; }
     if (p->d.fwi_buffers) UST_CUDA(cudaMalloc(&p->rec_in, (size_t)p->d.max_freq * nt * nelem * p->csz));
+    if (p->d.fwi_buffers) UST_CUDA(cudaMalloc(&p->drec, (size_t)p->d.max_freq * nt * nm * p->csz));
     UST_CUDA(cudaMalloc((void**)&p->src_lin, nt * sizeof(int)));
     UST_CUDA(cudaMalloc((void**)&p->rx_lin, nelem * sizeof(int)));
     UST_CUDA(cudaMalloc((void**)&p->mask, (size_t)nt * nm * sizeof(int)));
@@ -1224,6 +1308,13 @@ int ust_ncg_linesearch(ust_plan* p, const void* sd_dev, double* out2_dev, void* 
     if (!sd_dev || !out2_dev) { set_error("ust_ncg_linesearch: null argument"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
     return DISPATCH(p, linesearch_impl, p, sd_dev, out2_dev, (cudaStream_t)stream);
+}
+
+int ust_fwi_gn_hvp(ust_plan* p, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream) {
+    UST_TRY(check_plan(p));
+    if (!v_dev || !hv_dev || !jv2_dev) { set_error("ust_fwi_gn_hvp: null argument"); return 1; }
+    UST_CUDA(cudaSetDevice(p->d.device));
+    return DISPATCH(p, gn_hvp_impl, p, v_dev, hv_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
 }
 
 int ust_get_bde(ust_plan* p, double* out) {

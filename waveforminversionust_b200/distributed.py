@@ -103,6 +103,19 @@ class ShardedFWI:
             grad = self.torch.zeros_like(slow_dev)
         return allreduce_loss_grad(loss, grad, self.group)
 
+    def gn_hvp_device(self, v_dev):
+        """Gauss-Newton product of the joint objective at the point of the last ``loss_grad_device``: this rank's part
+        (``HelmholtzPlan.gn_hvp``: its frequencies or its transmitters) and one all-reduce of the packed ``[hv, jv2]``.
+        Returns ``(hv, jv2)`` with ``jv2 = sum |J v|^2`` (0-d float64 tensor)."""
+        if len(self.local) and len(self.local_tx):
+            hv, jv2 = self.plan.gn_hvp(v_dev)
+            jv2 = jv2[0]
+        else:
+            jv2 = self.torch.zeros((), dtype=self.torch.float64, device=v_dev.device)
+            hv = self.torch.zeros_like(v_dev)
+        jv2, hv = allreduce_loss_grad(jv2, hv, self.group)
+        return hv, jv2
+
     def local_rec(self, rec_all):
         """This rank's part of the full observed data ``rec_all`` (nfreq, Nt, E): its frequencies (all transmitters) or its
         transmitters (all frequencies)."""
@@ -157,3 +170,25 @@ def run_lbfgs_sharded(eng, rec_local_dev, c_init, maxiter=1, tol=1e-5, history_s
     return api.run_lbfgs_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0, geom.L_PML,
                              geom.mask_indices, maxiter=maxiter, tol=tol, history_size=history_size, dtype=plan.dtype,
                              history=history, loss_grad=loss_grad, pert_scale=pert_scale)
+
+
+def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None):
+    """``api.gauss_newton_fwi`` on a sharded engine: every rank runs the same driver on the all-reduced (loss, grad) and
+    products, which NCCL delivers bit-identically to all ranks, so the ranks take identical steps.  ``rec_local_dev``: this
+    rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound speed (Ny, Nx)."""
+    import torch
+    from . import api
+    geom, plan = eng.geom, eng.plan
+    dv = torch.device(f"cuda:{eng.device}")
+
+    def loss_grad(slow):
+        loss, grad = eng.loss_grad_device(slow.to(dv, plan.treal).contiguous(), rec_local_dev)
+        return float(loss), grad
+
+    def hvp(v):
+        return eng.gn_hvp_device(v.to(dv, plan.treal).contiguous())[0]
+
+    return api.gauss_newton_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs,
+                                Niter, geom.a0, geom.L_PML, geom.mask_indices, cg_iters=cg_iters, cg_tol=cg_tol, damping=damping,
+                                max_backtracks=max_backtracks, dtype=plan.dtype, device=eng.device, history=history,
+                                loss_grad=loss_grad, hvp=hvp)

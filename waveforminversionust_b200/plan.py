@@ -54,6 +54,7 @@ class HelmholtzPlan:
         self._grid_key = None
         self._acq_key = None
         self._factor_key = None
+        self._eval_key = None  # inputs of the last fwi_loss_function on this plan (api.fwi_gauss_newton_product)
 
     def close(self):
         if getattr(self, "h", None):
@@ -131,6 +132,7 @@ class HelmholtzPlan:
                    "ust_factor")
         self.nfreq = fr.size
         self._factor_key = None  # api.solve_helmholtz's cached factorisation is gone (it re-sets the key itself)
+        self._eval_key = None  # the factors of the last fwi_loss_grad are gone too (api.fwi_gauss_newton_product)
 
     def solve(self, rhs, ifreq=0, adjoint=False):
         """In-place solve; ``rhs`` is an (ny*nx, nrhs) (or (ny, nx, nrhs)) complex CUDA tensor."""
@@ -154,6 +156,7 @@ class HelmholtzPlan:
                                             _stream_ptr(self.device)), "ust_fwi_loss_grad")
         self.nfreq = fr.size
         self._factor_key = None  # the plan now holds the factors of (slow, freqs), not api.solve_helmholtz's
+        self._eval_key = None  # api.fwi_loss_function records its inputs after this call
         self._keep = (slow, rec)  # ust_ncg_linesearch reads them again
         return loss, grad
 
@@ -165,6 +168,19 @@ class HelmholtzPlan:
                                              _stream_ptr(self.device)), "ust_ncg_linesearch")
         return out
 
+    def gn_hvp(self, v, jv=False):
+        """Gauss-Newton product on the state of the last ``fwi_loss_grad`` (no factorisation): ``v`` (ny, nx) real CUDA
+        tensor -> ``(hv, jv2[, jv])`` with ``hv = Re(J^H J v)`` (ny, nx), ``jv2 = sum |J v|^2`` (1-element float64 tensor)
+        and, when ``jv``, ``J v`` at the kept receivers (nfreq, nt, nm) complex (``ust_fwi_gn_hvp``)."""
+        torch = _torch()
+        self._check_tensor(v, self.treal, self.nx * self.ny)
+        hv = torch.empty((self.ny, self.nx), dtype=self.treal, device=v.device)
+        jv2 = torch.empty(1, dtype=torch.float64, device=v.device)
+        jvt = torch.empty((getattr(self, "nfreq", 1), self.nt, getattr(self, "nm", 0)), dtype=self.tcplx, device=v.device) if jv else None
+        _lib.check(self.L.ust_fwi_gn_hvp(self.h, C.c_void_p(v.data_ptr()), C.c_void_p(hv.data_ptr()), C.c_void_p(jv2.data_ptr()),
+                                         C.c_void_p(jvt.data_ptr()) if jv else None, _stream_ptr(self.device)), "ust_fwi_gn_hvp")
+        return (hv, jv2, jvt) if jv else (hv, jv2)
+
     # -- host-buffer entry points (NumPy; no torch needed) ------------------------------------
     def solve_helmholtz_host(self, vel, src, f, adjoint=False, bde=None, refactor=True):
         vel = None if vel is None else np.ascontiguousarray(np.asarray(vel, dtype=self.real))
@@ -172,6 +188,8 @@ class HelmholtzPlan:
         nrhs = src.size // (self.nx * self.ny)
         out = np.empty((self.ny, self.nx, nrhs), dtype=self.cplx)
         b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(3))
+        if refactor:
+            self._eval_key = None
         _lib.check(self.L.ust_solve_helmholtz_host(
             self.h, None if vel is None else vel.ctypes.data_as(C.c_void_p), src.ctypes.data_as(C.c_void_p),
             out.ctypes.data_as(C.c_void_p), nrhs, float(f), _pd(b), int(bool(adjoint)), int(bool(refactor))),
@@ -193,6 +211,7 @@ class HelmholtzPlan:
                    "ust_fwi_loss_grad_host")
         self.nfreq = fr.size
         self._factor_key = None
+        self._eval_key = None
         return loss.value, grad
 
     # -- introspection ---------------------------------------------------------------------
