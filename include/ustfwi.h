@@ -89,6 +89,13 @@ int ust_plan_set_acquisition(ust_plan* plan, int nt, const int32_t* src_lin_host
 int ust_factor(ust_plan* plan, const void* vel_dev, int nfreq, const double* freqs_host,
                const double* bde_host, void* stream);
 
+/* Same for a lossy medium: complex slowness sigma = 1/vel - i kappa per node, wavenumber k = 2 pi f sigma, so the amplitude
+ * attenuation is 2 pi f kappa Np/m (linear in frequency, no dispersion; alpha0 [dB/(cm MHz)] = 5.458e5 * kappa [s/m]).
+ * kappa_dev: (ny, nx) real, >= 0 for a decaying wave; required (NULL is an error, not the lossless operator).  The stencil
+ * weights come from min/max(vel) as in ust_factor.  ust_solve then solves the lossy operator. */
+int ust_factor_lossy(ust_plan* plan, const void* vel_dev, const void* kappa_dev, int nfreq, const double* freqs_host,
+                     const double* bde_host, void* stream);
+
 /* In-place multi-RHS solve on the current factors of frequency slot ifreq:
  *   rhs_inout_dev (ny*nx, nrhs) complex, row-major; adjoint!=0 solves conj(H)^T u = rhs
  *   (solve_helmholtz.py:66-73) on the same factors.
@@ -118,10 +125,27 @@ int ust_fwi_loss_grad_host(ust_plan* plan, const void* slow_host, const void* re
                            const double* freqs_host, const double* bde_host, double* loss_host,
                            void* grad_host);
 
+/* Joint (loss, grad) for a lossy medium (the complex slowness of ust_factor_lossy): the evaluation of ust_fwi_loss_grad with
+ * the sigma^2 assembly, and the gradients with respect to both maps, alpha held fixed as in ust_fwi_loss_grad.  With
+ * z_f = sum_t conj(alpha_t u_t) lambda_t, A = sum_f -2 w_f^2 Re z_f and B = sum_f -2 w_f^2 Im z_f per node:
+ *   grad_s = s A - kappa B,   grad_kappa = -s B - kappa A      (kappa = 0: grad_s is ust_fwi_loss_grad's gradient, bit for bit)
+ *   slow_dev, kappa_dev (ny, nx) real; kappa_dev is required.  grad_s_dev, grad_kappa_dev (ny, nx) real, overwritten.
+ * After it, ust_ncg_linesearch and ust_fwi_gn_hvp refuse (their virtual source assumes a real slowness) until the next
+ * ust_fwi_loss_grad. */
+int ust_fwi_loss_grad_lossy(ust_plan* plan, const void* slow_dev, const void* kappa_dev, const void* rec_dev, int nfreq,
+                            const double* freqs_host, const double* bde_host, double* loss_dev, void* grad_s_dev,
+                            void* grad_kappa_dev, void* stream);
+
+/* Same, HOST buffers in and out (the twin of ust_fwi_loss_grad_host). */
+int ust_fwi_loss_grad_lossy_host(ust_plan* plan, const void* slow_host, const void* kappa_host, const void* rec_host, int nfreq,
+                                 const double* freqs_host, const double* bde_host, double* loss_host, void* grad_s_host,
+                                 void* grad_kappa_host);
+
 /* NCG caller support (nonlinearcg.py:268-301), valid after ust_fwi_loss_grad on the same plan:
  * perturbation solve with RHS -VIRT*sd on the existing factors, gather at the receivers and return
  * the two line-search scalars  num = Re<dREC, REC_DATA-REC_SIM>, den = Re<dREC,dREC>
- * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles. */
+ * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles.
+ * Fails while the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad). */
 int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, void* stream);
 
 /* Gauss-Newton Hessian-vector product of the joint objective on the factors, forward fields and source estimates of the last
@@ -130,7 +154,8 @@ int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, voi
  * jv_dev: (nfreq, nt, nm) complex J v at the kept receivers (mask order), or NULL.  Overwrites the adjoint wavefield.
  * J is the linearisation the gradient uses (virtual source 2 w^2 s alpha u without the stencil's mass weights and the PML
  * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).
- * Fails if ust_factor or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad. */
+ * Fails if ust_factor or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and while the plan holds
+ * a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad). */
 int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream);
 
 /* Introspection for parity tests and callers that want the intermediate fields (device pointers into

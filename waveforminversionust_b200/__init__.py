@@ -8,6 +8,7 @@ from .api import (  # noqa: F401
     continuation_stages,
     frequency_continuation,
     fwi_gauss_newton_product,
+    fwi_joint_loss_function,
     fwi_loss_function,
     gauss_newton_fwi,
     hanning,
@@ -15,7 +16,9 @@ from .api import (  # noqa: F401
     nonlinear_conjugate_gradient,
     nonlinear_conjugate_gradient_vectorized,
     run_lbfgs_fwi,
+    run_lbfgs_joint_fwi,
     solve_helmholtz,
     time_domain_simulation,
 )
+from .geometry import attenuation_blob_model, db_cm_mhz_to_kappa, kappa_to_db_cm_mhz  # noqa: F401
 from .plan import HelmholtzPlan  # noqa: F401

@@ -14,6 +14,10 @@ Inputs may be NumPy arrays (host buffers: copies happen inside the C call) or to
 Extensions over the reference (keyword-only): ``dtype`` ("c64" default = the reference's precision,
 or "c128"), ``engine`` ("auto" | "simt" | "tc2": block-GEMM engine; tcgen05 is complex64 only), ``bde`` (inject the stencil weights), ``stencil`` ("python" | "matlab"), and ``f`` /
 ``REC_DATA`` may carry a leading frequency axis for the joint multi-frequency objective.
+
+Attenuation (not in the reference): ``kappa`` (attenuation slowness, s/m) makes the medium lossy with complex slowness
+``1/c - i kappa`` (``solve_helmholtz``, ``time_domain_simulation``); ``fwi_joint_loss_function`` and ``run_lbfgs_joint_fwi``
+invert sound speed and attenuation together (DESIGN.md section 7d).
 """
 from __future__ import annotations
 
@@ -77,33 +81,47 @@ def _fingerprint(*parts):
     return h.digest()
 
 
-def solve_helmholtz(x, y, vel, src, f, a0, L_PML, adjoint, *, dtype="c64", bde=None, stencil="python", engine="auto"):
+def solve_helmholtz(x, y, vel, src, f, a0, L_PML, adjoint, *, dtype="c64", bde=None, stencil="python", engine="auto",
+                    kappa=None):
     """Solve H(vel, f) u = src (or conj(H)^T u = src when ``adjoint``) for every column of ``src``.
 
     ``src`` is (Ny, Nx, nrhs) (anything that reshapes C-order to (Ny*Nx, nrhs), solve_helmholtz.py:78);
     returns (Ny, Nx, nrhs) complex (solve_helmholtz.py:101).  The factorisation is cached and reused
-    while (vel, f, grid, PML, weights) stay the same, so the forward / adjoint / perturbation solves of
+    while (vel, f, grid, PML, weights, kappa) stay the same, so the forward / adjoint / perturbation solves of
     one iteration (nonlinearcg.py:213,263,279) factorise once instead of three times.
+
+    ``kappa`` ((Ny, Nx) attenuation slowness, s/m, >= 0): lossy medium with complex slowness ``1/vel - i kappa``, amplitude
+    attenuation ``2 pi f kappa`` Np/m (``geometry.db_cm_mhz_to_kappa`` converts from dB/(cm MHz)).  NumPy inputs then go
+    through device tensors; the result is NumPy as for the lossless call.
     """
     xh, yh = _to_np(x).astype(np.float64).ravel(), _to_np(y).astype(np.float64).ravel()
     nx, ny = xh.size, yh.size
     f = float(np.asarray(_to_np(f)).reshape(-1)[0])
     adjoint = bool(np.asarray(_to_np(adjoint)).reshape(-1)[0]) if not isinstance(adjoint, bool) else adjoint
     nrhs = int(np.prod(src.shape)) // (nx * ny)
-    dev = _device_of(src, vel)
+    dev = _device_of(src, vel, kappa)
     plan = get_plan(nx, ny, dtype, dev, 1, nrhs, stencil, False, engine)
     plan.set_grid(xh, yh, float(a0), float(L_PML))
-    if _is_torch(src) and src.is_cuda:
+    on_dev = _is_torch(src) and src.is_cuda
+    if on_dev or kappa is not None:
         import torch
+        dv = src.device if on_dev else torch.device(f"cuda:{dev}")
         velt = vel if _is_torch(vel) else torch.as_tensor(_to_np(vel))
-        velt = velt.to(device=src.device, dtype=plan.treal).contiguous()
-        key = _fingerprint(velt.cpu().numpy(), f, None if bde is None else np.asarray(bde, dtype=np.float64))
+        velt = velt.to(device=dv, dtype=plan.treal).reshape(ny, nx).contiguous()
+        parts = (velt.cpu().numpy(), f, None if bde is None else np.asarray(bde, dtype=np.float64))
+        kapt = None
+        if kappa is not None:
+            kapt = (kappa if _is_torch(kappa) else torch.as_tensor(_to_np(kappa))).to(device=dv, dtype=plan.treal).reshape(ny, nx).contiguous()
+            parts += ("kappa", kapt.cpu().numpy())
+        key = _fingerprint(*parts)
         if plan._factor_key != key:
-            plan.factor(velt, [f], bde=None if bde is None else [bde])
+            plan.factor(velt, [f], bde=None if bde is None else [bde], kappa=kapt)
             plan._factor_key = key
-        out = src.to(plan.tcplx).reshape(ny * nx, nrhs).contiguous().clone()
+        srct = src if _is_torch(src) else torch.as_tensor(_to_np(src))
+        out = srct.to(device=dv, dtype=plan.tcplx).reshape(ny * nx, nrhs).contiguous().clone()
         plan.solve(out, 0, adjoint)
-        return out.reshape(ny, nx, nrhs)
+        out = out.reshape(ny, nx, nrhs)
+        return out if on_dev else out.cpu().numpy()
     velh = _to_np(vel).astype(plan.real)
     key = _fingerprint(velh, f, None if bde is None else np.asarray(bde, dtype=np.float64))
     refactor = plan._factor_key != key
@@ -173,6 +191,28 @@ def fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, i
     loss, grad = plan.fwi_loss_grad_host(p.reshape(plan.ny, plan.nx), _to_np(REC_DATA), freqs, bde=bde)
     plan._eval_key = _eval_key(params, REC_DATA, freqs, bde)
     return loss, grad.reshape(p.shape)
+
+
+def fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
+                            *, dtype="c64", bde=None, stencil="python", engine="auto"):
+    """(loss, grad) of the joint sound-speed and attenuation problem: ``params`` is (2, Ny, Nx) = [slowness s (s/m),
+    attenuation slowness kappa (s/m)] of the complex slowness ``s - i kappa``, and ``grad`` has ``params``' shape
+    ([dloss/ds, dloss/dkappa]).  The other arguments and the loss are those of ``fwi_loss_function``; the gradients use the
+    same linearisation (source estimates held fixed, DESIGN.md section 7d).  The ``value_and_grad`` contract of
+    ``fwi_loss_function``: torch CUDA in -> torch out (device buffers), NumPy in -> NumPy out (host buffers)."""
+    dev = _device_of(params, REC_DATA)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
+    if tuple(params.shape) != (2, plan.ny, plan.nx):
+        raise ValueError(f"params must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa]")
+    if _is_torch(params) and params.is_cuda:
+        import torch
+        rec = REC_DATA.to(plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
+        p = params.to(plan.treal)
+        loss, gs, gk = plan.fwi_loss_grad_lossy(p[0].contiguous(), p[1].contiguous(), rec, freqs, bde=bde)
+        return loss[0], torch.stack([gs, gk])
+    p = np.asarray(_to_np(params), dtype=plan.real)
+    loss, gs, gk = plan.fwi_loss_grad_lossy_host(p[0], p[1], _to_np(REC_DATA), freqs, bde=bde)
+    return loss, np.stack([gs, gk])
 
 
 def _eval_key(params, REC_DATA, freqs, bde):
@@ -326,6 +366,59 @@ def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, 
     return 1.0 / final_slow
 
 
+def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, L_PML, mask_indices, *, kappa_init=0.0,
+                        kappa_scale=None, maxiter=1, tol=1e-5, history_size=10, dtype="c64", bde=None, stencil="python",
+                        engine="auto", history=None, loss_grad=None, pert_scale=1e-2):
+    """L-BFGS on sound speed and attenuation together (``fwi_joint_loss_function``); returns ``(c, kappa)``, both (Ny, Nx).
+
+    SciPy's L-BFGS-B with the bound ``kappa >= 0``, on the problem non-dimensionalised per block: the slowness as in
+    ``run_lbfgs_fwi`` (``p_s = (s / s0 - 1) / pert_scale``), the attenuation as ``p_kappa = kappa / kappa_scale`` (default
+    ``kappa_scale``: the kappa of 0.5 dB/(cm MHz), ``geometry.db_cm_mhz_to_kappa(0.5)``), and the objective
+    ``loss / loss(start)``; ``tol`` applies to the projected gradient of that scaled problem.  ``kappa_init`` is a scalar or an
+    (Ny, Nx) map.
+
+    ``loss_grad(params) -> (loss, grad)`` with ``params`` (2, Ny, Nx) float64 = [slowness, kappa] replaces the objective (the
+    parity test drives the same optimiser with the oracle's); ``history`` receives ``(loss, params.copy())`` of every
+    evaluation.
+    """
+    from scipy.optimize import minimize
+    from .geometry import db_cm_mhz_to_kappa
+    ny, nx = _to_np(yi).size, _to_np(xi).size
+    num_elements = int(SRC.shape[2]) if SRC is not None else 0  # unused when ``loss_grad`` is injected
+    c0 = np.asarray(_to_np(c_init), dtype=np.float64)
+    s0 = 1.0 / float(c0.mean())
+    ks = float(db_cm_mhz_to_kappa(0.5) if kappa_scale is None else kappa_scale)
+    real = np.float32 if dtype == "c64" else np.float64
+    state = {"loss0": None}
+    if loss_grad is None:
+        def loss_grad(params):
+            return fwi_joint_loss_function(params.astype(real), xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab,
+                                           mask_indices, num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+
+    n = ny * nx
+
+    def fun(p):
+        params = np.stack([(1.0 + pert_scale * p[:n].reshape(ny, nx)) * s0, ks * p[n:].reshape(ny, nx)])
+        loss, grad = loss_grad(params)
+        if np.shape(grad) != params.shape:
+            raise ValueError("loss_grad must return a gradient with the shape of its argument (2, Ny, Nx)")
+        if state["loss0"] is None:
+            state["loss0"] = float(loss)
+        if history is not None:
+            history.append((float(loss), params.copy()))
+        scale = 1.0 / state["loss0"]
+        g = np.asarray(grad, dtype=np.float64)
+        return float(loss) * scale, np.concatenate([g[0].ravel() * (s0 * pert_scale * scale), g[1].ravel() * (ks * scale)])
+
+    p0 = np.concatenate([((np.ones((ny, nx)) / (c0 * s0) - 1.0) / pert_scale).ravel(),
+                         (np.asarray(_to_np(kappa_init), dtype=np.float64) * np.ones((ny, nx)) / ks).ravel()])
+    bounds = [(None, None)] * n + [(0.0, None)] * n
+    res = minimize(fun, p0, jac=True, method="L-BFGS-B", bounds=bounds,
+                   options=dict(maxiter=int(maxiter), maxcor=int(history_size), gtol=float(tol)))
+    final_slow = (1.0 + pert_scale * res.x[:n].reshape(ny, nx)) * s0
+    return 1.0 / final_slow, ks * res.x[n:].reshape(ny, nx)
+
+
 def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
                      cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, dtype="c64", bde=None, stencil="python", device=0,
                      engine="auto", history=None, loss_grad=None, hvp=None):
@@ -470,10 +563,11 @@ def idtft(WVFIELD_F, f, resp_freq, time, df=None, *, device=0):
 
 
 def time_domain_simulation(xi, yi, C_map, src, f, resp_freq, time, a0, L_PML, *, dtype="c64", stencil="python",
-                           engine="auto", device=0, batch=16):
+                           engine="auto", device=0, batch=16, kappa=None):
     """``Lecture19_Fwi/TimeDomainSimulation.m:36-56`` on the GPU path: one forward solve per frequency for the source
     ``src`` (Ny, Nx) of one transmitting element, ``batch`` frequencies factorised per launch sequence, then the inverse
     discrete-time Fourier transform to the time axis ``time``.  Returns NumPy ``(WVFIELD_F (Ny, Nx, Nf), WVFIELD_T (Ny, Nx, Nt))``.
+    ``kappa`` ((Ny, Nx) attenuation slowness, s/m): lossy medium, attenuation linear in frequency (``solve_helmholtz``).
     """
     import torch
     xh, yh = _to_np(xi).astype(np.float64).ravel(), _to_np(yi).astype(np.float64).ravel()
@@ -485,11 +579,12 @@ def time_domain_simulation(xi, yi, C_map, src, f, resp_freq, time, a0, L_PML, *,
     plan._factor_key = None
     dv = torch.device(f"cuda:{device}")
     vel = torch.as_tensor(_to_np(C_map)).to(device=dv, dtype=plan.treal).reshape(ny, nx).contiguous()
+    kap = None if kappa is None else torch.as_tensor(_to_np(kappa)).to(device=dv, dtype=plan.treal).reshape(ny, nx).contiguous()
     rhs0 = torch.as_tensor(_to_np(src)).to(device=dv, dtype=plan.tcplx).reshape(ny * nx, 1).contiguous()
     U = torch.empty((f.size, ny * nx), dtype=plan.tcplx, device=dv)
     for k0 in range(0, f.size, batch):
         fb = f[k0:k0 + batch]
-        plan.factor(vel, fb)
+        plan.factor(vel, fb, kappa=kap)
         for i in range(fb.size):
             X = rhs0.clone()
             plan.solve(X, i, False)

@@ -3,6 +3,7 @@
 //   stencil_params_kernel: optimal 9-point weights (b,d,e)           (solve_helmholtz.py:104-154)
 //   assemble_kernel      : nine coefficient planes of the mixed-grid (solve_helmholtz.py:158-260)
 //                          PML Helmholtz operator, one thread per grid node, coalesced plane stores.
+//                          LOSSY = true: complex slowness sigma = s - i kappa, k^2 = w^2 sigma^2 (DESIGN.md section 7d).
 // Algorithmic bytes per node and frequency: read vel (sizeof R) + write 9 complex coefficients
 // (9 * 2 * sizeof R) = 76 B (c64) / 152 B (c128).
 #pragma once
@@ -102,12 +103,24 @@ __global__ void __launch_bounds__(256) inv_v2_kernel(const R* __restrict__ vel, 
     if (i < n) { const double v = (double)vel[i]; out[i] = 1.0 / (v * v); }
 }
 
+// Lossy models: sigma^2 = (s - i kappa)^2 per node in float64, interleaved (re, im).  Re is formed as 1/v^2 - kappa^2 with 1/v^2
+// exactly as inv_v2_kernel forms it, so that kappa = 0 gives the lossless operator's doubles; Im = -2 kappa / v.
+template <typename R>
+__global__ void __launch_bounds__(256) sig2_kernel(const R* __restrict__ vel, const R* __restrict__ kappa, double2* __restrict__ out, long long n) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        const double v = (double)vel[i], k = (double)kappa[i];
+        out[i] = make_double2(1.0 / (v * v) - k * k, -2.0 * k / v);
+    }
+}
+
 constexpr int ASM_MAXF = 32;  // frequencies per assemble_kernel launch (the host loops over chunks)
 
 // General (absorbing-layer) node: complex FP64 products.  Kept out of line: it needs ~100 registers, and inlined it made EVERY
 // thread of assemble_kernel pay for local-memory spills although ~90 % of the nodes of a benchmark grid take the real-arithmetic
-// path.  fc = the per-frequency constants staged by the kernel ([nfreq][12] doubles in shared memory).
-template <typename R>
+// path.  fc = the per-frequency constants staged by the kernel ([nfreq][12] doubles in shared memory).  LOSSY: `inv_v2` holds the
+// complex sigma^2 (sig2_kernel, double2 per node) instead of the real 1/v^2.
+template <typename R, bool LOSSY>
 __device__ __noinline__ void assemble_pml_node(const AsmArgs& a, int x, int y, const double* __restrict__ inv_v2, const cx<R>* __restrict__ exn,
                                                const cx<R>* __restrict__ rexh, const cx<R>* __restrict__ eyn, const cx<R>* __restrict__ reyh,
                                                const double* fcp, cx<R>* __restrict__ out0, int f_lo, int f_hi) {
@@ -117,10 +130,18 @@ __device__ __noinline__ void assemble_pml_node(const AsmArgs& a, int x, int y, c
     const double ih2 = 1.0 / (a.h * a.h), ig2 = 1.0 / (a.gr * a.gr);
     const double (*fc)[12] = reinterpret_cast<const double (*)[12]>(fcp);
     double iv2[3][3];  // 1 / v^2 on the 3x3 neighbourhood (re-read here: passing the caller's copy by reference would pin it in local memory)
+    Z s2[3][3];        // LOSSY: sigma^2 on the 3x3 neighbourhood
 #pragma unroll
     for (int j = 0; j < 3; ++j)
 #pragma unroll
-        for (int i = 0; i < 3; ++i) iv2[j][i] = inv_v2[(size_t)(y - 1 + j) * Nx + (x - 1 + i)];
+        for (int i = 0; i < 3; ++i) {
+            if constexpr (LOSSY) {
+                const double2 t = reinterpret_cast<const double2*>(inv_v2)[(size_t)(y - 1 + j) * Nx + (x - 1 + i)];
+                s2[j][i] = Z(t.x, t.y);
+            } else {
+                iv2[j][i] = inv_v2[(size_t)(y - 1 + j) * Nx + (x - 1 + i)];
+            }
+        }
     // PML factors around the node
     Z ex_[3], ey_[3], rxh[3], ryh[3];
 #pragma unroll
@@ -144,12 +165,15 @@ __device__ __noinline__ void assemble_pml_node(const AsmArgs& a, int x, int y, c
     for (int fi = f_lo; fi < f_hi; ++fi) {
         const double w2 = fc[fi][0], b = fc[fi][1], beta = fc[fi][2], cc = fc[fi][6], d4 = fc[fi][7], e4 = fc[fi][8];
         const double bih2 = fc[fi][10], betaih2 = fc[fi][11];
-        // q = C k^2 on the 3x3 neighbourhood, k^2 = w^2 / v^2
+        // q = C k^2 on the 3x3 neighbourhood, k^2 = w^2 / v^2 (LOSSY: w^2 sigma^2)
         Z q[3][3];
 #pragma unroll
         for (int j = 0; j < 3; ++j)
 #pragma unroll
-            for (int i = 0; i < 3; ++i) q[j][i] = (w2 * iv2[j][i]) * (ex_[i] * ey_[j]);
+            for (int i = 0; i < 3; ++i) {
+                if constexpr (LOSSY) q[j][i] = Z(w2 * s2[j][i].re, w2 * s2[j][i].im) * (ex_[i] * ey_[j]);
+                else q[j][i] = (w2 * iv2[j][i]) * (ex_[i] * ey_[j]);
+            }
         Z v[9];
         v[PL_C] = cc * q[1][1] - bih2 * (A(1, 1) + A(1, 0) + ig2 * (B(1, 1) + B(0, 1)));
         v[PL_L] = ih2 * (b * A(1, 0) - (beta * ig2) * (B(1, 0) + B(0, 0))) + d4 * q[1][0];
@@ -170,8 +194,9 @@ __device__ __noinline__ void assemble_pml_node(const AsmArgs& a, int x, int y, c
 // PML vectors (complex R): exn[x]=e_x(node x), rexh[x]=1/e_x(x+1/2) (x<=Nx-2), eyn[y], reyh[y].
 // One thread per grid node, looping over the launch's frequencies: the stretch factors around the node and the nine 1/v^2
 // values are loaded once and serve every frequency; each store instruction of a warp writes 256 contiguous bytes of one plane.
-// grid = (ceil(Nx/256), Ny), 256 threads.
-template <typename R>
+// grid = (ceil(Nx/256), Ny), 256 threads.  LOSSY: `inv_v2` is the double2 sigma^2 of sig2_kernel; the flat nodes keep their real
+// stencil part and gain an imaginary mass term (the stretch factors are 1 there, so only k^2 is complex).
+template <typename R, bool LOSSY>
 __global__ void __launch_bounds__(256, 4) assemble_kernel(AsmArgs a, const double* __restrict__ inv_v2, const cx<R>* __restrict__ exn,
                                                         const cx<R>* __restrict__ rexh, const cx<R>* __restrict__ eyn,
                                                         const cx<R>* __restrict__ reyh, const double* __restrict__ freqs,
@@ -232,7 +257,36 @@ __global__ void __launch_bounds__(256, 4) assemble_kernel(AsmArgs a, const doubl
         flat = flat && t0.re == R(1) && t0.im == R(0) && t1.re == R(1) && t1.im == R(0) &&
                t2.re == R(1) && t2.im == R(0) && t3.re == R(1) && t3.im == R(0);
     }
-    if (flat) {
+    if (LOSSY && flat) {
+        const double2* s2 = reinterpret_cast<const double2*>(inv_v2);
+        double sr[3][3], si[3][3];  // sigma^2 on the 3x3 neighbourhood
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+                const double2 t = s2[(size_t)(y - 1 + j) * Nx + (x - 1 + i)];
+                sr[j][i] = t.x; si[j][i] = t.y;
+            }
+        for (int fi = 0; fi < a.nfreq; ++fi) {
+            const double w2 = fc[fi][0], edge_x = fc[fi][3], edge_y = fc[fi][4], corner = fc[fi][5];
+            const double cc = fc[fi][6], d4 = fc[fi][7], e4 = fc[fi][8], ctr = fc[fi][9];
+            double r[9], m[9];
+            r[PL_C] = cc * (w2 * sr[1][1]) - ctr;          m[PL_C] = cc * (w2 * si[1][1]);
+            r[PL_L] = edge_x + d4 * (w2 * sr[1][0]);       m[PL_L] = d4 * (w2 * si[1][0]);
+            r[PL_R] = edge_x + d4 * (w2 * sr[1][2]);       m[PL_R] = d4 * (w2 * si[1][2]);
+            r[PL_D] = edge_y + d4 * (w2 * sr[0][1]);       m[PL_D] = d4 * (w2 * si[0][1]);
+            r[PL_U] = edge_y + d4 * (w2 * sr[2][1]);       m[PL_U] = d4 * (w2 * si[2][1]);
+            r[PL_DL] = corner + e4 * (w2 * sr[0][0]);      m[PL_DL] = e4 * (w2 * si[0][0]);
+            r[PL_DR] = corner + e4 * (w2 * sr[0][2]);      m[PL_DR] = e4 * (w2 * si[0][2]);
+            r[PL_UL] = corner + e4 * (w2 * sr[2][0]);      m[PL_UL] = e4 * (w2 * si[2][0]);
+            r[PL_UR] = corner + e4 * (w2 * sr[2][2]);      m[PL_UR] = e4 * (w2 * si[2][2]);
+            cx<R>* out = out0 + (size_t)fi * 9 * pl;
+#pragma unroll
+            for (int p = 0; p < 9; ++p) out[p * pl] = cx<R>((R)r[p], (R)m[p]);
+        }
+        return;
+    }
+    if (!LOSSY && flat) {
         double iv2[3][3];  // 1 / v^2 on the 3x3 neighbourhood
 #pragma unroll
         for (int j = 0; j < 3; ++j)
@@ -257,7 +311,7 @@ __global__ void __launch_bounds__(256, 4) assemble_kernel(AsmArgs a, const doubl
         }
         return;
     }
-    assemble_pml_node<R>(a, x, y, inv_v2, exn, rexh, eyn, reyh, &fc[0][0], out0, 0, a.nfreq);
+    assemble_pml_node<R, LOSSY>(a, x, y, inv_v2, exn, rexh, eyn, reyh, &fc[0][0], out0, 0, a.nfreq);
 }
 
 }  // namespace ust

@@ -4,6 +4,7 @@
 //                           scatter, one CTA per (transmitter, frequency)  (nonlinearcg.py:220-254)
 //   gradient_kernel       : grad = sum_f sum_t -Re(conj(VIRT) * ADJ_WV),  VIRT = 2 w^2 s alpha_t u_t
 //                           one warp per pixel, warp-shuffle reduction     (nonlinearcg.py:258,264-265)
+//                           LOSSY: gradients w.r.t. s and kappa of the complex slowness s - i kappa (DESIGN.md section 7d)
 //   pert_rhs_kernel       : RHS of the perturbation solve  -VIRT * sd      (nonlinearcg.py:279-281)
 //   linesearch_kernel     : dREC gather and the two step-size scalars      (nonlinearcg.py:22-28,284-298)
 //   gn_receiver_kernel    : Gauss-Newton product: J v = perturbation field at the kept receivers, and sum |J v|^2
@@ -105,6 +106,8 @@ struct GradArgs {
     R* grad;               // [N]
     long long N;
     int nt, nfreq;
+    const R* kappa;        // [N] LOSSY only: attenuation slowness
+    R* grad_kappa;         // [N] LOSSY only
 };
 
 // One warp per pixel.  The nt sources of a (pixel, frequency) are contiguous: complex64 lanes read 16 bytes (two sources)
@@ -113,7 +116,10 @@ struct GradArgs {
 // rounding stays at the level of the complex64 inputs while the dependent chain is four times shorter than one FP64
 // accumulator's); complex128 keeps the FP64 path.  Loads of consecutive iterations are independent: the unrolled loop keeps
 // several 16-byte requests per lane in flight.
-template <typename R>
+// LOSSY: with z_f = sum_t conj(alpha_t u_t) lambda_t the kernel also accumulates Im z_f, in four more FP32 partials beside the
+// four of Re z_f (which keep the lossless kernel's exact structure, so kappa = 0 reproduces its grad_s bit for bit), and writes
+//   A = sum_f -2 w^2 Re z_f,  B = sum_f -2 w^2 Im z_f,  grad_s = s A - kappa B,  grad_kappa = -s B - kappa A.
+template <typename R, bool LOSSY>
 __global__ void __launch_bounds__(256) gradient_kernel(GradArgs<R> a) {
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -121,18 +127,19 @@ __global__ void __launch_bounds__(256) gradient_kernel(GradArgs<R> a) {
     const double PI = 3.14159265358979323846;
     const bool vec = sizeof(R) == 4 && (a.nt & 1) == 0 && (a.stride_f & 1) == 0;
     for (long long p = warp; p < a.N; p += nwarps) {
-        double tot = 0.0;
+        double tot = 0.0, tot_im = 0.0;
         for (int f = 0; f < a.nfreq; ++f) {
             const cx<R>* u = a.U + (size_t)f * a.stride_f + (size_t)p * a.nt;
             const cx<R>* l = a.Lam + (size_t)f * a.stride_f + (size_t)p * a.nt;
             const cx<R>* al = a.src_est + (size_t)f * a.nt;
-            double acc = 0.0;
+            double acc = 0.0, acc_im = 0.0;
             if constexpr (sizeof(R) == 4) {
                 if (vec) {
                     const float4* u4 = reinterpret_cast<const float4*>(u);
                     const float4* l4 = reinterpret_cast<const float4*>(l);
                     const float4* a4 = reinterpret_cast<const float4*>(al);
                     float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+                    float q0 = 0.f, q1 = 0.f, q2 = 0.f, q3 = 0.f;
                     const int n2 = a.nt >> 1;
 #pragma unroll 4
                     for (int t = lane; t < n2; t += 32) {
@@ -142,13 +149,19 @@ __global__ void __launch_bounds__(256) gradient_kernel(GradArgs<R> a) {
                         const float br = aa.z * uu.z - aa.w * uu.w, bi = aa.z * uu.w + aa.w * uu.z;
                         s0 = fmaf(ar, ll.x, s0); s1 = fmaf(ai, ll.y, s1);  // Re(conj(alpha u) lambda)
                         s2 = fmaf(br, ll.z, s2); s3 = fmaf(bi, ll.w, s3);
+                        if constexpr (LOSSY) {  // Im(conj(alpha u) lambda)
+                            q0 = fmaf(ar, ll.y, q0); q1 = fmaf(-ai, ll.x, q1);
+                            q2 = fmaf(br, ll.w, q2); q3 = fmaf(-bi, ll.z, q3);
+                        }
                     }
                     acc = ((double)s0 + (double)s1) + ((double)s2 + (double)s3);
+                    if constexpr (LOSSY) acc_im = ((double)q0 + (double)q1) + ((double)q2 + (double)q3);
                 } else {
                     for (int t = lane; t < a.nt; t += 32) {
                         cx<R> uu = al[t] * u[t];
                         cx<R> ll = l[t];
                         acc += (double)uu.re * ll.re + (double)uu.im * ll.im;
+                        if constexpr (LOSSY) acc_im += (double)uu.re * ll.im - (double)uu.im * ll.re;
                     }
                 }
             } else {
@@ -156,13 +169,24 @@ __global__ void __launch_bounds__(256) gradient_kernel(GradArgs<R> a) {
                     cx<R> uu = al[t] * u[t];   // alpha_t u_t
                     cx<R> ll = l[t];
                     acc += (double)uu.re * ll.re + (double)uu.im * ll.im;  // Re(conj(uu) * ll)
+                    if constexpr (LOSSY) acc_im += (double)uu.re * ll.im - (double)uu.im * ll.re;  // Im(conj(uu) * ll)
                 }
             }
             double w = 2.0 * PI * a.freqs[f];
             tot += -2.0 * w * w * acc;
+            if constexpr (LOSSY) tot_im += -2.0 * w * w * acc_im;
         }
         tot = warp_sum(tot);
-        if (lane == 0) a.grad[p] = (R)(tot * (double)a.slow[p]);
+        if constexpr (LOSSY) {
+            tot_im = warp_sum(tot_im);
+            if (lane == 0) {
+                const double s = (double)a.slow[p], k = (double)a.kappa[p];
+                a.grad[p] = (R)(tot * s - tot_im * k);
+                a.grad_kappa[p] = (R)(-s * tot_im - k * tot);
+            }
+        } else {
+            if (lane == 0) a.grad[p] = (R)(tot * (double)a.slow[p]);
+        }
     }
 }
 

@@ -69,6 +69,7 @@ struct ust_plan {
     // device buffers
     void *exn = nullptr, *rexh = nullptr, *eyn = nullptr, *reyh = nullptr;
     double *d_vminmax = nullptr, *d_freqs = nullptr, *d_bde = nullptr, *d_scal = nullptr, *d_invv2 = nullptr;
+    double* d_sig2 = nullptr;  // lossy models: complex sigma^2 per node (2N doubles, sig2_kernel)
     int* d_status = nullptr;
     void *planes = nullptr, *T = nullptr, *scratch = nullptr, *W = nullptr, *pbuf = nullptr;
     void *vel = nullptr, *U = nullptr, *Lam = nullptr, *src_est = nullptr, *Xh = nullptr;
@@ -80,7 +81,12 @@ struct ust_plan {
     // plan-owned copies of the FWI inputs / outputs (stable addresses for graph replay)
     void *slow_in = nullptr, *rec_in = nullptr, *grad_out = nullptr, *sd_in = nullptr;
     void *v_in = nullptr, *hv_out = nullptr, *drec = nullptr;  // Gauss-Newton product: v, H_GN v, J v at the kept receivers
+    void *kappa_in = nullptr, *grad_kappa_out = nullptr;       // lossy evaluation: attenuation slowness, its gradient
+    void *kappa_h2d = nullptr, *grad_kappa_d2h = nullptr;      // staging of ust_fwi_loss_grad_lossy_host
     bool fwi_done = false;
+    // the factors and fields are those of a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy): the line search and the
+    // Gauss-Newton product, whose virtual source assumes a real slowness, refuse until a lossless ust_fwi_loss_grad
+    bool lossy = false;
     bool gn_ok = false;  // the factors, fields and source estimates are those of the last ust_fwi_loss_grad (ust_fwi_gn_hvp)
     bool use_graphs = true;  // UST_NO_GRAPHS=1 disables
     struct GraphEntry { cudaGraphExec_t exec = nullptr; long long launches = 0; };
@@ -412,8 +418,9 @@ static int join_groups(ust_plan* p, const std::vector<Group>& gs) {
 }
 
 // stencil weights (when not injected) + status reset: once per evaluation, before the groups fork
+// kappa_dev != nullptr: lossy model, sigma^2 (sig2_kernel) instead of 1/v^2
 template <typename R>
-static int factor_prologue(ust_plan* p, const void* vel_dev, int nfreq, bool has_bde, cudaStream_t st) {
+static int factor_prologue(ust_plan* p, const void* vel_dev, int nfreq, bool has_bde, cudaStream_t st, const void* kappa_dev = nullptr) {
     const Geom& g = p->g;
     if (!has_bde) {
         minmax_kernel<R><<<1, 1024, 0, st>>>((const R*)vel_dev, g.N, p->d_vminmax);
@@ -422,7 +429,8 @@ static int factor_prologue(ust_plan* p, const void* vel_dev, int nfreq, bool has
         UST_LAUNCH_CHECK();
     }
     UST_CUDA(cudaMemsetAsync(p->d_status, 0, sizeof(int), st));
-    inv_v2_kernel<R><<<(unsigned)((g.N + 255) / 256), 256, 0, st>>>((const R*)vel_dev, p->d_invv2, g.N);
+    if (kappa_dev) sig2_kernel<R><<<(unsigned)((g.N + 255) / 256), 256, 0, st>>>((const R*)vel_dev, (const R*)kappa_dev, (double2*)p->d_sig2, g.N);
+    else inv_v2_kernel<R><<<(unsigned)((g.N + 255) / 256), 256, 0, st>>>((const R*)vel_dev, p->d_invv2, g.N);
     UST_LAUNCH_CHECK();
     return 0;
 }
@@ -431,7 +439,7 @@ static int factor_prologue(ust_plan* p, const void* vel_dev, int nfreq, bool has
 // already be on the device.  Launches are enqueued step by step across the groups so that the streams fill evenly
 // when the launches are not replayed from a graph.
 template <typename R>
-static int factor_groups(ust_plan* p, const void* vel_dev, const std::vector<Group>& gs) {
+static int factor_groups(ust_plan* p, const void* vel_dev, const std::vector<Group>& gs, bool lossy = false) {
     const Geom& g = p->g;
     AsmArgs aa;
     aa.g = g; aa.h = p->h; aa.gr = p->gr; aa.stencil = p->d.stencil; aa.exp = (p->exp & 8) ? 1 : 0;
@@ -440,9 +448,15 @@ static int factor_groups(ust_plan* p, const void* vel_dev, const std::vector<Gro
             const int f0 = q.f0 + c0;
             aa.nfreq = std::min(q.nf - c0, (int)ASM_MAXF);
             ProfScope ps(p, PC_ASSEMBLE, q.st);
-            assemble_kernel<R><<<dim3(cdiv_i(g.Nx, 256), g.Ny), 256, 0, q.st>>>(
-                aa, p->d_invv2, (const cx<R>*)p->exn, (const cx<R>*)p->rexh, (const cx<R>*)p->eyn, (const cx<R>*)p->reyh,
-                p->d_freqs + f0, p->d_bde + 3 * f0, (cx<R>*)p->planes + (size_t)f0 * 9 * g.N);
+            const dim3 grid(cdiv_i(g.Nx, 256), g.Ny);
+            if (lossy)
+                assemble_kernel<R, true><<<grid, 256, 0, q.st>>>(
+                    aa, p->d_sig2, (const cx<R>*)p->exn, (const cx<R>*)p->rexh, (const cx<R>*)p->eyn, (const cx<R>*)p->reyh,
+                    p->d_freqs + f0, p->d_bde + 3 * f0, (cx<R>*)p->planes + (size_t)f0 * 9 * g.N);
+            else
+                assemble_kernel<R, false><<<grid, 256, 0, q.st>>>(
+                    aa, p->d_invv2, (const cx<R>*)p->exn, (const cx<R>*)p->rexh, (const cx<R>*)p->eyn, (const cx<R>*)p->reyh,
+                    p->d_freqs + f0, p->d_bde + 3 * f0, (cx<R>*)p->planes + (size_t)f0 * 9 * g.N);
             UST_LAUNCH_CHECK();
         }
     const int len = std::max(g.mid, g.M - 1 - g.mid);
@@ -453,22 +467,25 @@ static int factor_groups(ust_plan* p, const void* vel_dev, const std::vector<Gro
 }
 
 template <typename R>
-static int factor_enqueue(ust_plan* p, const void* vel_dev, int nfreq, bool has_bde, cudaStream_t st) {
-    UST_TRY(factor_prologue<R>(p, vel_dev, nfreq, has_bde, st));
+static int factor_enqueue(ust_plan* p, const void* vel_dev, int nfreq, bool has_bde, cudaStream_t st, const void* kappa_dev) {
+    UST_TRY(factor_prologue<R>(p, vel_dev, nfreq, has_bde, st, kappa_dev));
     const std::vector<Group> gs = make_groups(p, 0, nfreq, st);
     UST_TRY(fork_groups(p, gs));
-    UST_TRY(factor_groups<R>(p, vel_dev, gs));
+    UST_TRY(factor_groups<R>(p, vel_dev, gs, kappa_dev != nullptr));
     UST_TRY(join_groups(p, gs));
     p->nfreq_cur = nfreq;
     p->factored = true;
     return 0;
 }
 
+// kappa_dev != nullptr: the lossy operator of the complex slowness 1/vel - i kappa (ust_factor_lossy)
 template <typename R>
-static int factor_impl(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs, const double* bde, cudaStream_t st) {
+static int factor_impl(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs, const double* bde, cudaStream_t st,
+                       const void* kappa_dev = nullptr) {
     p->gn_ok = false;  // the factors no longer belong to the forward fields of the last evaluation
     UST_TRY(upload_params(p, nfreq, freqs, bde, st));
-    return factor_enqueue<R>(p, vel_dev, nfreq, bde != nullptr, st);
+    if (kappa_dev) p->lossy = true;
+    return factor_enqueue<R>(p, vel_dev, nfreq, bde != nullptr, st, kappa_dev);
 }
 
 template <typename R, int BM, int BN>
@@ -643,8 +660,9 @@ __global__ void recip_kernel(const R* __restrict__ in, R* __restrict__ out, long
 // One joint (loss, grad) evaluation, device work only (CUDA-graph capturable): reads p->slow_in / p->rec_in, writes
 // p->d_scal[0] (loss) and p->grad_out.  Each frequency group runs assemble -> factor -> forward sweeps -> receivers ->
 // adjoint sweeps as its own chain; the groups meet again at the gradient, which sums over all frequencies.
+// lossy: also reads p->kappa_in (sigma^2 assembly) and writes p->grad_kappa_out; everything between assembly and gradient is the same.
 template <typename R>
-static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st) {
+static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bool lossy = false) {
     const Geom& g = p->g;
     const int nt = p->nt;
     const size_t stride = (size_t)g.N * nt;
@@ -652,11 +670,11 @@ static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st) {
     double* loss_dev = p->d_scal;
     recip_kernel<R><<<(unsigned)((g.N + 255) / 256), 256, 0, st>>>((const R*)slow, (R*)p->vel, g.N);  // VEL = 1/SLOW (fwi_loss_function.py:50)
     UST_LAUNCH_CHECK();
-    UST_TRY(factor_prologue<R>(p, p->vel, nfreq, has_bde, st));
+    UST_TRY(factor_prologue<R>(p, p->vel, nfreq, has_bde, st, lossy ? p->kappa_in : nullptr));
     UST_CUDA(cudaMemsetAsync(loss_dev, 0, sizeof(double), st));
     const std::vector<Group> gs = make_groups(p, 0, nfreq, st);
     UST_TRY(fork_groups(p, gs));
-    UST_TRY(factor_groups<R>(p, p->vel, gs));
+    UST_TRY(factor_groups<R>(p, p->vel, gs, lossy));
     // forward: one-hot sources
     for (const Group& q : gs) {
         cx<R>* Uq = (cx<R>*)p->U + (size_t)q.f0 * stride;
@@ -686,10 +704,12 @@ static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st) {
     GradArgs<R> ga;
     ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
     ga.freqs = p->d_freqs; ga.slow = (const R*)slow; ga.grad = (R*)p->grad_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
+    ga.kappa = (const R*)p->kappa_in; ga.grad_kappa = (R*)p->grad_kappa_out;
     const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
     {
         ProfScope ps(p, PC_GRADIENT, st);
-        gradient_kernel<R><<<blocks, 256, 0, st>>>(ga);
+        if (lossy) gradient_kernel<R, true><<<blocks, 256, 0, st>>>(ga);
+        else gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
     }
     UST_LAUNCH_CHECK();
     return 0;
@@ -773,10 +793,11 @@ static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st) {
     GradArgs<R> ga;
     ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
     ga.freqs = p->d_freqs; ga.slow = (const R*)p->slow_in; ga.grad = (R*)p->hv_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
+    ga.kappa = nullptr; ga.grad_kappa = nullptr;
     const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
     {
         ProfScope ps(p, PC_GRADIENT, st);
-        gradient_kernel<R><<<blocks, 256, 0, st>>>(ga);
+        gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
     }
     UST_LAUNCH_CHECK();
     return 0;
@@ -820,10 +841,12 @@ static int run_graphed(ust_plan* p, long long key, cudaStream_t user, F enqueue)
     return 0;
 }
 
+// kappa != nullptr: lossy evaluation (ust_fwi_loss_grad_lossy), gradient w.r.t. kappa into grad_kappa_dev
 template <typename R>
 static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, const double* freqs, const double* bde,
-                    double* loss_dev, void* grad_dev, cudaStream_t st) {
+                    double* loss_dev, void* grad_dev, cudaStream_t st, const void* kappa = nullptr, void* grad_kappa_dev = nullptr) {
     const Geom& g = p->g;
+    const bool lossy = kappa != nullptr;
     if (!p->acq_set) { set_error("ust_fwi_loss_grad: ust_plan_set_acquisition has not been called"); return 1; }
     if (!p->U) { set_error("ust_fwi_loss_grad: plan was created with fwi_buffers=0"); return 1; }
     if (p->nt > p->d.max_nrhs) { set_error("ust_fwi_loss_grad: nt exceeds plan max_nrhs"); return 1; }
@@ -831,16 +854,20 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     // inputs -> plan-owned buffers (stable addresses for the captured graph; the line search reads them again)
     if (slow != p->slow_in) UST_CUDA(cudaMemcpyAsync(p->slow_in, slow, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     if (rec != p->rec_in) UST_CUDA(cudaMemcpyAsync(p->rec_in, rec, (size_t)nfreq * p->nt * p->nelem * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
+    if (lossy) UST_CUDA(cudaMemcpyAsync(p->kappa_in, kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     const bool has_bde = bde != nullptr;
-    const long long key = 1000LL * nfreq + (has_bde ? 1 : 0);
+    // lossless evaluation 0/1, line search 500, Gauss-Newton product 600, lossy evaluation 700/701
+    const long long key = 1000LL * nfreq + (lossy ? 700 : 0) + (has_bde ? 1 : 0);
     p->gn_ok = false;
-    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_); }));
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_, lossy); }));
     p->nfreq_cur = nfreq;
     p->factored = true;
     UST_CUDA(cudaMemcpyAsync(loss_dev, p->d_scal, sizeof(double), cudaMemcpyDeviceToDevice, st));
     UST_CUDA(cudaMemcpyAsync(grad_dev, p->grad_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    if (lossy) UST_CUDA(cudaMemcpyAsync(grad_kappa_dev, p->grad_kappa_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     p->fwi_done = true;
-    p->gn_ok = true;
+    p->lossy = lossy;
+    p->gn_ok = !lossy;
     if (p->trace) return dump_update_trace(p, st);
     return 0;
 }
@@ -849,6 +876,11 @@ template <typename R>
 static int linesearch_impl(ust_plan* p, const void* sd, double* out2, cudaStream_t st) {
     const Geom& g = p->g;
     if (!p->factored || !p->fwi_done) { set_error("ust_ncg_linesearch: call ust_fwi_loss_grad first"); return 1; }
+    if (p->lossy) {
+        set_error("ust_ncg_linesearch: the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy) and the line search "
+                  "assumes a real slowness; call ust_fwi_loss_grad first");
+        return 1;
+    }
     UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     const long long key = 1000LL * p->nfreq_cur + 500;
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_); }));
@@ -861,6 +893,11 @@ static int gn_hvp_impl(ust_plan* p, const void* v, void* hv, double* jv2, void* 
     const Geom& g = p->g;
     if (!p->v_in) { set_error("ust_fwi_gn_hvp: plan was created with fwi_buffers=0"); return 1; }
     if (!p->factored || !p->fwi_done) { set_error("ust_fwi_gn_hvp: call ust_fwi_loss_grad first"); return 1; }
+    if (p->lossy) {
+        set_error("ust_fwi_gn_hvp: the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy) and the product "
+                  "assumes a real slowness; call ust_fwi_loss_grad first");
+        return 1;
+    }
     if (!p->gn_ok) {
         set_error("ust_fwi_gn_hvp: the factors were replaced (ust_factor / ust_solve_helmholtz_host) after the last ust_fwi_loss_grad; "
                   "call ust_fwi_loss_grad again");
@@ -1032,6 +1069,7 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
     rc |= dev_alloc(p, (void**)&p->d_scal, 8 * sizeof(double));
     rc |= dev_alloc(p, (void**)&p->d_status, sizeof(int));
     rc |= dev_alloc(p, (void**)&p->d_invv2, g.N * sizeof(double));
+    rc |= dev_alloc(p, (void**)&p->d_sig2, 2 * g.N * sizeof(double));
     rc |= dev_alloc(p, &p->planes, (size_t)d->max_freq * 9 * g.N * p->csz);
     rc |= dev_alloc(p, &p->T, (size_t)d->max_freq * (p->t_ring ? 4 : g.M) * bs);
     if (!(d->dtype == UST_C64 && (d->engine == UST_ENGINE_TC2 || d->engine == UST_ENGINE_AUTO))) rc |= dev_alloc(p, &p->scratch, (size_t)2 * d->max_freq * bs);  // TC2 inverts in place
@@ -1072,6 +1110,8 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
         rc |= dev_alloc(p, &p->sd_in, g.N * p->rsz);
         rc |= dev_alloc(p, &p->v_in, g.N * p->rsz);
         rc |= dev_alloc(p, &p->hv_out, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->kappa_in, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->grad_kappa_out, g.N * p->rsz);
     }
     if (const char* e = getenv("UST_NO_GRAPHS")) p->use_graphs = atoi(e) == 0;
     if (const char* e = getenv("UST_NO_PDL")) ust::g_use_pdl = atoi(e) == 0;
@@ -1132,13 +1172,13 @@ int ust_plan_destroy(ust_plan* p) {
     if (!p) return 0;
     cudaSetDevice(p->d.device);
     cudaDeviceSynchronize();
-    void* ptrs[] = {p->exn, p->rexh, p->eyn, p->reyh, p->d_vminmax, p->d_freqs, p->d_bde, p->d_scal, p->d_status, p->d_invv2, p->planes,
+    void* ptrs[] = {p->exn, p->rexh, p->eyn, p->reyh, p->d_vminmax, p->d_freqs, p->d_bde, p->d_scal, p->d_status, p->d_invv2, p->d_sig2, p->planes,
                     p->T, p->scratch, p->W, p->pbuf, p->Tp, p->Wp, p->Rp, p->Cp, p->Xp, p->Pp, p->Rs, p->gj_flags, p->snap, p->vel, p->U, p->Lam, p->src_est, p->Xh, p->src_lin, p->rx_lin, p->mask,
-                    p->slow_h2d, p->rec_h2d, p->grad_d2h};
+                    p->slow_h2d, p->rec_h2d, p->grad_d2h, p->kappa_h2d, p->grad_kappa_d2h};
     for (void* q : ptrs)
         if (q) cudaFree(q);
     drop_graphs(p);
-    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in, p->v_in, p->hv_out, p->drec})
+    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in, p->v_in, p->hv_out, p->drec, p->kappa_in, p->grad_kappa_out})
         if (q) cudaFree(q);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
     if (p->ev_out) cudaEventDestroy(p->ev_out);
@@ -1235,6 +1275,13 @@ int ust_factor(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs,
     return rc;
 }
 
+int ust_factor_lossy(ust_plan* p, const void* vel_dev, const void* kappa_dev, int nfreq, const double* freqs, const double* bde, void* stream) {
+    UST_TRY(check_plan(p));
+    if (!vel_dev || !kappa_dev || !freqs) { set_error("ust_factor_lossy: null argument (kappa_dev is required)"); return 1; }
+    UST_CUDA(cudaSetDevice(p->d.device));
+    return DISPATCH(p, factor_impl, p, vel_dev, nfreq, freqs, bde, (cudaStream_t)stream, kappa_dev);
+}
+
 int ust_solve(ust_plan* p, int ifreq, void* X, int nrhs, int adjoint, void* stream) {
     UST_TRY(check_plan(p));
     if (!X) { set_error("ust_solve: null argument"); return 1; }
@@ -1275,32 +1322,65 @@ int ust_fwi_loss_grad(ust_plan* p, const void* slow, const void* rec, int nfreq,
     return DISPATCH(p, fwi_impl, p, slow, rec, nfreq, freqs, bde, loss_dev, grad_dev, (cudaStream_t)stream);
 }
 
-int ust_fwi_loss_grad_host(ust_plan* p, const void* slow_host, const void* rec_host, int nfreq, const double* freqs,
-                           const double* bde, double* loss_host, void* grad_host) {
-    UST_TRY(check_plan(p));
-    if (!slow_host || !rec_host || !freqs || !loss_host || !grad_host) { set_error("ust_fwi_loss_grad_host: null argument"); return 1; }
-    if (!p->acq_set) { set_error("ust_fwi_loss_grad_host: ust_plan_set_acquisition has not been called"); return 1; }
+// host twins of ust_fwi_loss_grad (kappa_host == nullptr) and ust_fwi_loss_grad_lossy: staging buffers allocated on first use
+static int fwi_host(ust_plan* p, const char* name, const void* slow_host, const void* kappa_host, const void* rec_host, int nfreq,
+                    const double* freqs, const double* bde, double* loss_host, void* grad_host, void* grad_kappa_host) {
+    if (!p->acq_set) { set_error(std::string(name) + ": ust_plan_set_acquisition has not been called"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
     const Geom& g = p->g;
     cudaStream_t st = p->own_stream;
-    if (nfreq < 1 || nfreq > p->d.max_freq) { set_error("ust_fwi_loss_grad_host: nfreq out of range"); return 1; }
+    if (nfreq < 1 || nfreq > p->d.max_freq) { set_error(std::string(name) + ": nfreq out of range"); return 1; }
     const size_t rec_bytes = (size_t)p->d.max_freq * p->nt * p->nelem * p->csz;
     if (!p->slow_h2d) UST_TRY(dev_alloc(p, &p->slow_h2d, g.N * p->rsz));
     if (!p->grad_d2h) UST_TRY(dev_alloc(p, &p->grad_d2h, g.N * p->rsz));
     if (!p->rec_h2d) UST_CUDA(cudaMalloc(&p->rec_h2d, rec_bytes));
+    if (kappa_host && !p->kappa_h2d) UST_TRY(dev_alloc(p, &p->kappa_h2d, g.N * p->rsz));
+    if (kappa_host && !p->grad_kappa_d2h) UST_TRY(dev_alloc(p, &p->grad_kappa_d2h, g.N * p->rsz));
     UST_CUDA(cudaMemcpyAsync(p->slow_h2d, slow_host, g.N * p->rsz, cudaMemcpyHostToDevice, st));
     UST_CUDA(cudaMemcpyAsync(p->rec_h2d, rec_host, (size_t)nfreq * p->nt * p->nelem * p->csz, cudaMemcpyHostToDevice, st));
-    UST_TRY(DISPATCH(p, fwi_impl, p, p->slow_h2d, p->rec_h2d, nfreq, freqs, bde, p->d_scal, p->grad_d2h, st));
+    if (kappa_host) UST_CUDA(cudaMemcpyAsync(p->kappa_h2d, kappa_host, g.N * p->rsz, cudaMemcpyHostToDevice, st));
+    UST_TRY(DISPATCH(p, fwi_impl, p, p->slow_h2d, p->rec_h2d, nfreq, freqs, bde, p->d_scal, p->grad_d2h, st,
+                     kappa_host ? p->kappa_h2d : nullptr, p->grad_kappa_d2h));
     UST_CUDA(cudaMemcpyAsync(loss_host, p->d_scal, sizeof(double), cudaMemcpyDeviceToHost, st));
     UST_CUDA(cudaMemcpyAsync(grad_host, p->grad_d2h, g.N * p->rsz, cudaMemcpyDeviceToHost, st));
+    if (kappa_host) UST_CUDA(cudaMemcpyAsync(grad_kappa_host, p->grad_kappa_d2h, g.N * p->rsz, cudaMemcpyDeviceToHost, st));
     int status = 0;
     UST_CUDA(cudaMemcpyAsync(&status, p->d_status, sizeof(int), cudaMemcpyDeviceToHost, st));
     UST_CUDA(cudaStreamSynchronize(st));
     if (status) {  // SciPy's analogue is MatrixRankWarning + NaN output; here it is an error, never a silent garbage gradient
-        set_error("ust_fwi_loss_grad_host: a block inversion met a zero / non-finite pivot (singular or ill-posed operator for this model and frequency)");
+        set_error(std::string(name) + ": a block inversion met a zero / non-finite pivot (singular or ill-posed operator for this model and frequency)");
         return 2;
     }
     return 0;
+}
+
+int ust_fwi_loss_grad_host(ust_plan* p, const void* slow_host, const void* rec_host, int nfreq, const double* freqs,
+                           const double* bde, double* loss_host, void* grad_host) {
+    UST_TRY(check_plan(p));
+    if (!slow_host || !rec_host || !freqs || !loss_host || !grad_host) { set_error("ust_fwi_loss_grad_host: null argument"); return 1; }
+    return fwi_host(p, "ust_fwi_loss_grad_host", slow_host, nullptr, rec_host, nfreq, freqs, bde, loss_host, grad_host, nullptr);
+}
+
+int ust_fwi_loss_grad_lossy(ust_plan* p, const void* slow, const void* kappa, const void* rec, int nfreq, const double* freqs,
+                            const double* bde, double* loss_dev, void* grad_s_dev, void* grad_kappa_dev, void* stream) {
+    UST_TRY(check_plan(p));
+    if (!slow || !kappa || !rec || !freqs || !loss_dev || !grad_s_dev || !grad_kappa_dev) {
+        set_error("ust_fwi_loss_grad_lossy: null argument (kappa_dev is required)");
+        return 1;
+    }
+    UST_CUDA(cudaSetDevice(p->d.device));
+    return DISPATCH(p, fwi_impl, p, slow, rec, nfreq, freqs, bde, loss_dev, grad_s_dev, (cudaStream_t)stream, kappa, grad_kappa_dev);
+}
+
+int ust_fwi_loss_grad_lossy_host(ust_plan* p, const void* slow_host, const void* kappa_host, const void* rec_host, int nfreq,
+                                 const double* freqs, const double* bde, double* loss_host, void* grad_s_host, void* grad_kappa_host) {
+    UST_TRY(check_plan(p));
+    if (!slow_host || !kappa_host || !rec_host || !freqs || !loss_host || !grad_s_host || !grad_kappa_host) {
+        set_error("ust_fwi_loss_grad_lossy_host: null argument (kappa_host is required)");
+        return 1;
+    }
+    return fwi_host(p, "ust_fwi_loss_grad_lossy_host", slow_host, kappa_host, rec_host, nfreq, freqs, bde, loss_host, grad_s_host,
+                    grad_kappa_host);
 }
 
 int ust_ncg_linesearch(ust_plan* p, const void* sd_dev, double* out2_dev, void* stream) {

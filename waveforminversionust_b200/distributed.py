@@ -116,6 +116,19 @@ class ShardedFWI:
         jv2, hv = allreduce_loss_grad(jv2, hv, self.group)
         return hv, jv2
 
+    def loss_grad_lossy_device(self, slow_dev, kappa_dev, rec_local_dev, bde=None):
+        """Joint sound-speed and attenuation evaluation (``HelmholtzPlan.fwi_loss_grad_lossy``) of this rank's frequencies or
+        transmitters, and one all-reduce of the packed ``[grad_s, grad_kappa, loss]``.  Returns (loss (0-d float64 tensor),
+        grad (2, Ny, Nx) = [grad_s, grad_kappa])."""
+        torch = self.torch
+        if len(self.local) and len(self.local_tx):
+            loss, gs, gk = self.plan.fwi_loss_grad_lossy(slow_dev, kappa_dev, rec_local_dev, self.local_freqs, bde=bde)
+            loss, grad = loss[0], torch.stack([gs, gk])
+        else:
+            loss = torch.zeros((), dtype=torch.float64, device=slow_dev.device)
+            grad = torch.zeros((2,) + tuple(slow_dev.shape), dtype=slow_dev.dtype, device=slow_dev.device)
+        return allreduce_loss_grad(loss, grad, self.group)
+
     def local_rec(self, rec_all):
         """This rank's part of the full observed data ``rec_all`` (nfreq, Nt, E): its frequencies (all transmitters) or its
         transmitters (all frequencies)."""
@@ -192,3 +205,24 @@ def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_t
                                 Niter, geom.a0, geom.L_PML, geom.mask_indices, cg_iters=cg_iters, cg_tol=cg_tol, damping=damping,
                                 max_backtracks=max_backtracks, dtype=plan.dtype, device=eng.device, history=history,
                                 loss_grad=loss_grad, hvp=hvp)
+
+
+def run_lbfgs_joint_sharded(eng, rec_local_dev, c_init, kappa_init=0.0, kappa_scale=None, maxiter=1, tol=1e-5, history_size=10,
+                            history=None, pert_scale=1e-2):
+    """``api.run_lbfgs_joint_fwi`` on a sharded engine: every rank runs the same joint L-BFGS driver on the all-reduced
+    ``(loss, [grad_s, grad_kappa])`` of ``ShardedFWI.loss_grad_lossy_device``, so the ranks take identical steps.  Returns
+    ``(c, kappa)`` (Ny, Nx) NumPy arrays (identical on every rank)."""
+    import torch
+    from . import api
+    geom, plan = eng.geom, eng.plan
+    dv = torch.device(f"cuda:{eng.device}")
+
+    def loss_grad(params):
+        p = torch.as_tensor(np.ascontiguousarray(params.astype(plan.real))).to(dv)
+        loss, grad = eng.loss_grad_lossy_device(p[0].contiguous(), p[1].contiguous(), rec_local_dev)
+        return float(loss), grad.to(torch.float64).cpu().numpy()
+
+    return api.run_lbfgs_joint_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0,
+                                   geom.L_PML, geom.mask_indices, kappa_init=kappa_init, kappa_scale=kappa_scale, maxiter=maxiter,
+                                   tol=tol, history_size=history_size, dtype=plan.dtype, history=history, loss_grad=loss_grad,
+                                   pert_scale=pert_scale)

@@ -98,6 +98,37 @@ def blob_model(geom, c0=1500.0, dc=60.0, nblobs=5, seed=1234, r_max=0.09):
     return c
 
 
+# alpha0 [dB/(cm MHz)] of the attenuation slowness kappa [s/m]: the amplitude attenuation is alpha(f) = 2 pi f kappa Np/m
+# (complex slowness s - i kappa), and 1 Np = 20/ln(10) dB, 1 m = 100 cm, f in MHz = f / 1e6
+DB_CM_MHZ_PER_KAPPA = 2.0 * np.pi * 1e6 * (20.0 / np.log(10.0)) / 100.0  # ~5.458e5
+
+
+def db_cm_mhz_to_kappa(alpha0):
+    """Attenuation slowness kappa (s/m) of an attenuation coefficient ``alpha0`` in dB/(cm MHz) (linear in frequency)."""
+    return np.asarray(alpha0, dtype=np.float64) / DB_CM_MHZ_PER_KAPPA
+
+
+def kappa_to_db_cm_mhz(kappa):
+    """Inverse of ``db_cm_mhz_to_kappa``."""
+    return np.asarray(kappa, dtype=np.float64) * DB_CM_MHZ_PER_KAPPA
+
+
+def attenuation_blob_model(geom, alpha0=0.0, dalpha=0.5, nblobs=5, seed=4321, r_max=0.09):
+    """Smooth synthetic attenuation map, built like ``blob_model``: attenuation slowness kappa (s/m) of a background
+    ``alpha0`` dB/(cm MHz) plus ``nblobs`` Gaussian inclusions of ``dalpha`` times U(0.5, 1) dB/(cm MHz) (non-negative, so
+    kappa >= 0 everywhere) inside radius r_max."""
+    rng = np.random.default_rng(seed)
+    X, Y = np.meshgrid(geom.xi.astype(np.float64), geom.yi.astype(np.float64), indexing="xy")
+    a = np.full(X.shape, float(alpha0))
+    for _ in range(nblobs):
+        r = 0.6 * r_max * np.sqrt(rng.uniform())
+        th = rng.uniform(0, 2 * np.pi)
+        sig = rng.uniform(5e-3, 15e-3)
+        amp = dalpha * rng.uniform(0.5, 1.0)
+        a += amp * np.exp(-((X - r * np.cos(th)) ** 2 + (Y - r * np.sin(th)) ** 2) / (2 * sig**2))
+    return db_cm_mhz_to_kappa(a)
+
+
 def source_amplitudes(nt, seed=1234):
     """Per-source random complex amplitude (``SimulateData.m:26``)."""
     rng = np.random.default_rng(seed)

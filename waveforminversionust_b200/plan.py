@@ -123,13 +123,20 @@ class HelmholtzPlan:
         torch = _torch()
         return torch.complex64 if self.dtype == "c64" else torch.complex128
 
-    def factor(self, vel, freqs, bde=None):
-        """Assemble + factorise for ``freqs`` (list) from a (ny, nx) CUDA tensor of sound speed."""
+    def factor(self, vel, freqs, bde=None, kappa=None):
+        """Assemble + factorise for ``freqs`` (list) from a (ny, nx) CUDA tensor of sound speed.  ``kappa`` (a (ny, nx) CUDA
+        tensor of attenuation slowness, s/m) factorises the lossy operator of the complex slowness ``1/vel - i kappa``
+        (``ust_factor_lossy``)."""
         self._check_tensor(vel, self.treal, self.nx * self.ny)
         fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
         b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
-        _lib.check(self.L.ust_factor(self.h, C.c_void_p(vel.data_ptr()), fr.size, _pd(fr), _pd(b), _stream_ptr(self.device)),
-                   "ust_factor")
+        if kappa is None:
+            _lib.check(self.L.ust_factor(self.h, C.c_void_p(vel.data_ptr()), fr.size, _pd(fr), _pd(b), _stream_ptr(self.device)),
+                       "ust_factor")
+        else:
+            self._check_tensor(kappa, self.treal, self.nx * self.ny)
+            _lib.check(self.L.ust_factor_lossy(self.h, C.c_void_p(vel.data_ptr()), C.c_void_p(kappa.data_ptr()), fr.size, _pd(fr),
+                                               _pd(b), _stream_ptr(self.device)), "ust_factor_lossy")
         self.nfreq = fr.size
         self._factor_key = None  # api.solve_helmholtz's cached factorisation is gone (it re-sets the key itself)
         self._eval_key = None  # the factors of the last fwi_loss_grad are gone too (api.fwi_gauss_newton_product)
@@ -159,6 +166,28 @@ class HelmholtzPlan:
         self._eval_key = None  # api.fwi_loss_function records its inputs after this call
         self._keep = (slow, rec)  # ust_ncg_linesearch reads them again
         return loss, grad
+
+    def fwi_loss_grad_lossy(self, slow, kappa, rec, freqs, bde=None):
+        """Fused (loss, grad_s, grad_kappa) of a lossy medium on device tensors (``ust_fwi_loss_grad_lossy``): slow and kappa
+        (ny, nx) real, rec (nfreq, nt, nelem) complex.  Afterwards ``ncg_linesearch`` and ``gn_hvp`` refuse until the next
+        ``fwi_loss_grad``."""
+        torch = _torch()
+        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
+        self._check_tensor(slow, self.treal, self.nx * self.ny)
+        self._check_tensor(kappa, self.treal, self.nx * self.ny)
+        self._check_tensor(rec, self.tcplx, fr.size * self.nt * self.nelem)
+        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
+        loss = torch.empty(1, dtype=torch.float64, device=slow.device)
+        grad_s = torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device)
+        grad_k = torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device)
+        _lib.check(self.L.ust_fwi_loss_grad_lossy(self.h, C.c_void_p(slow.data_ptr()), C.c_void_p(kappa.data_ptr()),
+                                                  C.c_void_p(rec.data_ptr()), fr.size, _pd(fr), _pd(b), C.c_void_p(loss.data_ptr()),
+                                                  C.c_void_p(grad_s.data_ptr()), C.c_void_p(grad_k.data_ptr()),
+                                                  _stream_ptr(self.device)), "ust_fwi_loss_grad_lossy")
+        self.nfreq = fr.size
+        self._factor_key = None
+        self._eval_key = None
+        return loss, grad_s, grad_k
 
     def ncg_linesearch(self, sd):
         torch = _torch()
@@ -213,6 +242,29 @@ class HelmholtzPlan:
         self._factor_key = None
         self._eval_key = None
         return loss.value, grad
+
+    def fwi_loss_grad_lossy_host(self, slow, kappa, rec, freqs, bde=None):
+        """Host twin of ``fwi_loss_grad_lossy`` (``ust_fwi_loss_grad_lossy_host``): NumPy in, ``(loss, grad_s, grad_kappa)`` out."""
+        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
+        slow = np.ascontiguousarray(np.asarray(slow, dtype=self.real))
+        kappa = np.ascontiguousarray(np.asarray(kappa, dtype=self.real))
+        rec = np.ascontiguousarray(np.asarray(rec).astype(self.cplx, copy=False))
+        if rec.size != fr.size * self.nt * self.nelem:
+            raise ValueError("REC_DATA has the wrong shape for (nfreq, nt, nelem)")
+        if slow.size != self.nx * self.ny or kappa.size != self.nx * self.ny:
+            raise ValueError("slowness and kappa must have ny * nx entries")
+        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
+        grad_s = np.empty((self.ny, self.nx), dtype=self.real)
+        grad_k = np.empty((self.ny, self.nx), dtype=self.real)
+        loss = C.c_double(0.0)
+        _lib.check(self.L.ust_fwi_loss_grad_lossy_host(self.h, slow.ctypes.data_as(C.c_void_p), kappa.ctypes.data_as(C.c_void_p),
+                                                       rec.ctypes.data_as(C.c_void_p), fr.size, _pd(fr), _pd(b), C.byref(loss),
+                                                       grad_s.ctypes.data_as(C.c_void_p), grad_k.ctypes.data_as(C.c_void_p)),
+                   "ust_fwi_loss_grad_lossy_host")
+        self.nfreq = fr.size
+        self._factor_key = None
+        self._eval_key = None
+        return loss.value, grad_s, grad_k
 
     # -- introspection ---------------------------------------------------------------------
     def bde(self):
