@@ -131,7 +131,7 @@ int ust_fwi_loss_grad_host(ust_plan* plan, const void* slow_host, const void* re
  *   grad_s = s A - kappa B,   grad_kappa = -s B - kappa A      (kappa = 0: grad_s is ust_fwi_loss_grad's gradient, bit for bit)
  *   slow_dev, kappa_dev (ny, nx) real; kappa_dev is required.  grad_s_dev, grad_kappa_dev (ny, nx) real, overwritten.
  * After it, ust_ncg_linesearch and ust_fwi_gn_hvp refuse (their virtual source assumes a real slowness) until the next
- * ust_fwi_loss_grad. */
+ * ust_fwi_loss_grad; their lossy twins ust_ncg_linesearch_lossy and ust_fwi_gn_hvp_lossy run on its state instead. */
 int ust_fwi_loss_grad_lossy(ust_plan* plan, const void* slow_dev, const void* kappa_dev, const void* rec_dev, int nfreq,
                             const double* freqs_host, const double* bde_host, double* loss_dev, void* grad_s_dev,
                             void* grad_kappa_dev, void* stream);
@@ -145,7 +145,8 @@ int ust_fwi_loss_grad_lossy_host(ust_plan* plan, const void* slow_host, const vo
  * perturbation solve with RHS -VIRT*sd on the existing factors, gather at the receivers and return
  * the two line-search scalars  num = Re<dREC, REC_DATA-REC_SIM>, den = Re<dREC,dREC>
  * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles.
- * Fails while the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad). */
+ * Fails while the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad);
+ * ust_ncg_linesearch_lossy is the line search of the lossy model. */
 int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, void* stream);
 
 /* Gauss-Newton Hessian-vector product of the joint objective on the factors, forward fields and source estimates of the last
@@ -155,8 +156,24 @@ int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, voi
  * J is the linearisation the gradient uses (virtual source 2 w^2 s alpha u without the stencil's mass weights and the PML
  * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).
  * Fails if ust_factor or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and while the plan holds
- * a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad). */
+ * a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad); ust_fwi_gn_hvp_lossy is the
+ * product of the lossy model. */
 int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream);
+
+/* Lossy twins of ust_ncg_linesearch and ust_fwi_gn_hvp for the joint (s, kappa) problem, valid only on the state of the last
+ * ust_fwi_loss_grad_lossy: they fail before any evaluation, after a lossless evaluation, and after any factorisation
+ * (ust_factor, ust_factor_lossy, ust_solve_helmholtz_host) or ust_plan_set_acquisition since that evaluation.  With the complex
+ * slowness sigma = s - i kappa and alpha held fixed, the linearisation of a joint direction [v_s; v_kappa] is
+ *   J [v_s; v_kappa] = P H^-1( -2 w^2 sigma alpha u (v_s - i v_kappa) )
+ * and J^H r = [s A - kappa B, -s B - kappa A], the two gradients of ust_fwi_loss_grad_lossy formed from the adjoint field of r.
+ * The kappa part of the direction (sd_kappa_dev, v_kappa_dev) is required.  At kappa = 0 and a zero kappa direction, out2 and
+ * hv_s / jv2 / jv equal those of the lossless entry points on the same slowness, bit for bit.
+ *   ust_ncg_linesearch_lossy: out2_dev = {num = Re<J sd, REC_DATA - REC_SIM>, den = |J sd|^2} (= -<sd, grad> and |J sd|^2).
+ *   ust_fwi_gn_hvp_lossy:     hv_s_dev, hv_kappa_dev (ny, nx) real = Re(J^H J v); jv2_dev = sum |J v|^2 (= <v, hv>);
+ *                             jv_dev (nfreq, nt, nm) complex J v at the kept receivers, or NULL. */
+int ust_ncg_linesearch_lossy(ust_plan* plan, const void* sd_s_dev, const void* sd_kappa_dev, double* out2_dev, void* stream);
+int ust_fwi_gn_hvp_lossy(ust_plan* plan, const void* v_s_dev, const void* v_kappa_dev, void* hv_s_dev, void* hv_kappa_dev,
+                         double* jv2_dev, void* jv_dev /* (nfreq, nt, nm) complex or NULL */, void* stream);
 
 /* Introspection for parity tests and callers that want the intermediate fields (device pointers into
  * plan-owned buffers, valid until the next ust_fwi_* call on the plan). */

@@ -8,12 +8,16 @@ from .api import (  # noqa: F401
     continuation_stages,
     frequency_continuation,
     fwi_gauss_newton_product,
+    fwi_joint_gauss_newton_product,
     fwi_joint_loss_function,
     fwi_loss_function,
     gauss_newton_fwi,
+    gauss_newton_joint_fwi,
     hanning,
     idtft,
+    joint_frequency_continuation,
     nonlinear_conjugate_gradient,
+    nonlinear_conjugate_gradient_joint,
     nonlinear_conjugate_gradient_vectorized,
     run_lbfgs_fwi,
     run_lbfgs_joint_fwi,

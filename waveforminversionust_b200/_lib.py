@@ -15,7 +15,8 @@ _LIB = None
 EXPORTS = [
     "ust_last_error", "ust_version", "ust_plan_create", "ust_plan_destroy", "ust_plan_device_bytes",
     "ust_plan_set_groups", "ust_plan_set_grid", "ust_plan_set_acquisition", "ust_factor", "ust_factor_lossy", "ust_solve",
-    "ust_solve_helmholtz_host", "ust_fwi_loss_grad", "ust_fwi_loss_grad_host", "ust_fwi_loss_grad_lossy", "ust_fwi_loss_grad_lossy_host", "ust_ncg_linesearch", "ust_fwi_gn_hvp", "ust_get_bde", "ust_get_planes",
+    "ust_solve_helmholtz_host", "ust_fwi_loss_grad", "ust_fwi_loss_grad_host", "ust_fwi_loss_grad_lossy", "ust_fwi_loss_grad_lossy_host", "ust_ncg_linesearch", "ust_fwi_gn_hvp",
+    "ust_ncg_linesearch_lossy", "ust_fwi_gn_hvp_lossy", "ust_get_bde", "ust_get_planes",
     "ust_get_src_est", "ust_get_wavefield", "ust_get_adjoint_wavefield", "ust_get_status",
     "ust_launch_count", "ust_launch_count_reset", "ust_profile", "ust_get_profile", "ust_test_cgemm", "ust_idtft", "ust_pack_f64_as_f32x2", "ust_residual_onehot",
 ]
@@ -63,6 +64,8 @@ def lib():
     L.ust_fwi_loss_grad_lossy_host.argtypes = [vp, vp, vp, vp, i, pd, pd, pd, vp, vp]
     L.ust_ncg_linesearch.argtypes = [vp, vp, vp, vp]
     L.ust_fwi_gn_hvp.argtypes = [vp, vp, vp, vp, vp, vp]
+    L.ust_ncg_linesearch_lossy.argtypes = [vp, vp, vp, vp, vp]
+    L.ust_fwi_gn_hvp_lossy.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
     L.ust_get_bde.argtypes = [vp, pd]
     L.ust_get_planes.argtypes = [vp, i, vp, vp]
     L.ust_get_src_est.argtypes = [vp, i, vp]

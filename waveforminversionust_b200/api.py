@@ -17,7 +17,9 @@ or "c128"), ``engine`` ("auto" | "simt" | "tc2": block-GEMM engine; tcgen05 is c
 
 Attenuation (not in the reference): ``kappa`` (attenuation slowness, s/m) makes the medium lossy with complex slowness
 ``1/c - i kappa`` (``solve_helmholtz``, ``time_domain_simulation``); ``fwi_joint_loss_function`` and ``run_lbfgs_joint_fwi``
-invert sound speed and attenuation together (DESIGN.md section 7d).
+invert sound speed and attenuation together (DESIGN.md section 7d); ``fwi_joint_gauss_newton_product``,
+``nonlinear_conjugate_gradient_joint``, ``gauss_newton_joint_fwi`` and ``joint_frequency_continuation`` add the joint
+Gauss-Newton product, NCG and truncated Gauss-Newton (section 7e).
 """
 from __future__ import annotations
 
@@ -209,20 +211,23 @@ def fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_incl
         rec = REC_DATA.to(plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
         p = params.to(plan.treal)
         loss, gs, gk = plan.fwi_loss_grad_lossy(p[0].contiguous(), p[1].contiguous(), rec, freqs, bde=bde)
+        plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy=True)
         return loss[0], torch.stack([gs, gk])
     p = np.asarray(_to_np(params), dtype=plan.real)
     loss, gs, gk = plan.fwi_loss_grad_lossy_host(p[0], p[1], _to_np(REC_DATA), freqs, bde=bde)
+    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy=True)
     return loss, np.stack([gs, gk])
 
 
-def _eval_key(params, REC_DATA, freqs, bde):
+def _eval_key(params, REC_DATA, freqs, bde, lossy=False):
     """What identifies an evaluation's state on the plan: device inputs are kept as copies (compared on the device), host
-    inputs as a hash."""
+    inputs as a hash.  The key of a lossy evaluation is tagged, so that it never matches a lossless one."""
     b = None if bde is None else np.asarray(bde, dtype=np.float64)
+    tag = "-lossy" if lossy else ""
     if _is_torch(params) and params.is_cuda:
         rec = REC_DATA.detach().clone() if _is_torch(REC_DATA) else _fingerprint(np.asarray(REC_DATA))
-        return ("dev", params.detach().clone(), rec, _fingerprint(freqs, b))
-    return ("host", _fingerprint(np.asarray(_to_np(params)), np.asarray(_to_np(REC_DATA)), freqs, b))
+        return ("dev" + tag, params.detach().clone(), rec, _fingerprint(freqs, b))
+    return ("host" + tag, _fingerprint(np.asarray(_to_np(params)), np.asarray(_to_np(REC_DATA)), freqs, b))
 
 
 def _same_eval(a, b):
@@ -266,6 +271,38 @@ def fwi_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_
     vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real).reshape(plan.ny, plan.nx))).to(f"cuda:{plan.device}")
     hv, _ = plan.gn_hvp(vt)
     return hv.cpu().numpy().reshape(shape)
+
+
+def fwi_joint_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
+                                   num_elements, *, dtype="c64", bde=None, stencil="python", engine="auto"):
+    """Gauss-Newton product ``H_GN v = Re(J^H J v)`` of the joint objective of ``fwi_joint_loss_function``: ``params`` and
+    ``v`` are (2, Ny, Nx) = [slowness, kappa] blocks, and so is the result (NumPy in, NumPy out; a CUDA tensor ``v`` gives a
+    CUDA tensor).
+
+    With the complex slowness ``sigma = s - i kappa`` and the source estimates held fixed, ``J [v_s; v_kappa]`` is the
+    perturbation solve with virtual source ``-2 w^2 sigma alpha u (v_s - i v_kappa)`` gathered at the kept receivers, the
+    linearisation the joint gradient is built from (DESIGN.md section 7e).  Because ``J_kappa = -i J_s``, the blocks satisfy
+    ``H_kk = H_ss`` and ``H_ks = -H_sk``.
+
+    A product costs two all-source sweeps on the factorisation the last evaluation left on the plan; when the last
+    ``fwi_joint_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)`` (or the last evaluation was lossless),
+    the evaluation runs first.
+    """
+    import torch
+    dev = _device_of(params, REC_DATA, v)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
+    if tuple(v.shape) != (2, plan.ny, plan.nx):
+        raise ValueError(f"v must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa] directions")
+    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde, lossy=True)):
+        fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
+                                dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+    if _is_torch(v) and v.is_cuda:
+        vt = v.detach().to(plan.treal)
+        hv, _ = plan.gn_hvp_lossy(vt[0].contiguous(), vt[1].contiguous())
+        return hv
+    vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real))).to(f"cuda:{plan.device}")
+    hv, _ = plan.gn_hvp_lossy(vt[0].contiguous(), vt[1].contiguous())
+    return hv.cpu().numpy()
 
 
 def nonlinear_conjugate_gradient(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter,
@@ -458,27 +495,45 @@ def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
         def hvp(v):
             return fwi_gauss_newton_product(state["slow"], v.to(dv, real).contiguous(), *fargs, **kw)
 
-    def f64(a, dv):
-        return a.detach().to(dv, torch.float64) if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, dtype=np.float64)).to(dv)
-
     c0 = np.asarray(_to_np(c_init), dtype=np.float64) * np.ones((ny, nx))
-    s = torch.as_tensor(1.0 / c0)
-    loss, g = loss_grad(s)
+    s = _gauss_newton_loop(torch.as_tensor(1.0 / c0), loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history,
+                           slow_of=lambda x: x)
+    return (1.0 / s).cpu().numpy()
+
+
+def _f64(a, dv):
+    import torch
+    return a.detach().to(dv, torch.float64) if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, dtype=np.float64)).to(dv)
+
+
+def _gauss_newton_loop(x, loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history, slow_of, scale=None,
+                       project=None):
+    """The outer loop of ``gauss_newton_fwi`` and ``gauss_newton_joint_fwi`` on the model ``x`` (float64 torch): CG on
+    ``(D H_GN D + mu I) p = -D g`` in the scaled variables, trial ``project(x + step D p)`` with step halving.  ``scale`` is
+    ``D`` (a tensor of ``x``'s shape; None: the identity, no arithmetic), ``project(x) -> (x, clipped node count)`` (None: no
+    projection), ``slow_of(x)`` the slowness map whose range the history reports.  Returns the final ``x``."""
+    import torch
+    shape = tuple(x.shape)
+    D = (lambda a: a) if scale is None else (lambda a: scale * a)
+    loss, g = loss_grad(x)
     dv = g.device if torch.is_tensor(g) else torch.device("cpu")
-    s, g, loss = s.to(dv), f64(g, dv).reshape(ny, nx), float(loss)
+    x, g, loss = x.to(dv), _f64(g, dv).reshape(shape), float(loss)
+    if scale is not None:
+        scale = scale.to(dv)
     nevals, nprods = 1, 0
     dot = lambda a, b: float(torch.sum(a * b))
     for it in range(int(Niter)):
         rec = dict(it=it, loss=loss)
-        gg = dot(g, g)
+        gs = D(g)
+        gg = dot(gs, gs)
         p = torch.zeros_like(g)
-        r, d, rr = -g, -g, gg
+        r, d, rr = -gs, -gs, gg
         qs, mu, k = [], 0.0, 0
         while k < int(cg_iters):
-            Hd = f64(hvp(d), dv).reshape(ny, nx)
+            Hd = D(_f64(hvp(D(d)), dv).reshape(shape))
             nprods += 1
             if k == 0:
-                mu = float(damping) * dot(d, Hd) / gg  # d = -g
+                mu = float(damping) * dot(d, Hd) / gg  # d = -D g
             Ad = Hd + mu * d
             curv = dot(d, Ad)
             if not curv > 0:
@@ -487,25 +542,31 @@ def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
             p = p + a * d
             r = r - a * Ad
             k += 1
-            qs.append(0.5 * dot(g, p) - 0.5 * dot(p, r))
+            qs.append(0.5 * dot(gs, p) - 0.5 * dot(p, r))
             rr_new = dot(r, r)
             if math.sqrt(rr_new) <= float(cg_tol) * math.sqrt(gg):
                 break
             d = r + (rr_new / rr) * d
             rr = rr_new
         rec.update(cg_iters=k, q=qs, mu=mu)
-        step, accepted = 1.0, False
+        step, accepted, clipped = 1.0, False, 0
         if k > 0:
+            dp = D(p)
             for _ in range(int(max_backtracks) + 1):
-                trial = s + step * p
+                trial = x + step * dp
+                if project is not None:
+                    trial, clipped = project(trial)
                 lt, gt = loss_grad(trial)
                 nevals += 1
                 if float(lt) < loss:
-                    s, loss, g, accepted = trial, float(lt), f64(gt, dv).reshape(ny, nx), True
+                    x, loss, g, accepted = trial, float(lt), _f64(gt, dv).reshape(shape), True
                     break
                 step *= 0.5
+        s = slow_of(x)
         rec.update(step=step if accepted else 0.0, evals=nevals, products=nprods, vel_min=float(1.0 / s.max()),
                    vel_max=float(1.0 / s.min()))
+        if project is not None:
+            rec["clipped"] = clipped
         if not accepted:
             rec["stop"] = ("no positive curvature along -g" if k == 0 else
                            f"no loss decrease after {int(max_backtracks)} step halvings")
@@ -513,7 +574,136 @@ def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
             history.append(rec)
         if not accepted:
             break
-    return (1.0 / s).cpu().numpy()
+    return x
+
+
+def _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale):
+    """Start model x0 (2, Ny, Nx) = [1/c_init, kappa_init] and the block scaling D = diag(s0 pert_scale, kappa_scale) of
+    ``run_lbfgs_joint_fwi``, both float64 torch (CPU)."""
+    import torch
+    from .geometry import db_cm_mhz_to_kappa
+    c0 = np.asarray(_to_np(c_init), dtype=np.float64) * np.ones((ny, nx))
+    s0 = 1.0 / float(c0.mean())
+    ks = float(db_cm_mhz_to_kappa(0.5) if kappa_scale is None else kappa_scale)
+    k0 = np.asarray(_to_np(kappa_init), dtype=np.float64) * np.ones((ny, nx))
+    x0 = torch.as_tensor(np.stack([1.0 / c0, k0]))
+    D = torch.as_tensor(np.stack([np.full((ny, nx), s0 * float(pert_scale)), np.full((ny, nx), ks)]))
+    return x0, D
+
+
+def _project_kappa(x):
+    """kappa <- max(kappa, 0) on a (2, Ny, Nx) model; returns (model, number of clipped nodes)."""
+    import torch
+    neg = x[1] < 0
+    return torch.stack([x[0], torch.clamp(x[1], min=0.0)]), int(neg.sum())
+
+
+def _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices, dtype, bde, stencil,
+                     device, engine):
+    """GPU objective of the joint drivers: loss_grad(x), the lossy line search and the lossy product at the point of the last
+    loss_grad call, on (2, Ny, Nx) float64 torch models."""
+    import torch
+    freqs = np.atleast_1d(np.asarray(_to_np(f), dtype=np.float64)).ravel()
+    dv = torch.device(f"cuda:{device}")
+    real = torch.float32 if dtype == "c64" else torch.float64
+    rec = torch.as_tensor(_to_np(REC_DATA)).to(dv).reshape(freqs.size, len(_to_np(tx_include)), -1).contiguous()
+    state = {}
+    fargs = (xi, yi, rec, SRC, freqs, a0, L_PML, tx_include, ind_matlab, mask_indices, numElements)
+    kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+
+    def loss_grad(x):
+        state["x"] = x.to(dv, real).contiguous()
+        loss, grad = fwi_joint_loss_function(state["x"], *fargs, **kw)
+        return float(loss), grad
+
+    def linesearch(sd):
+        plan, _ = _fwi_plan(xi, yi, rec, SRC, freqs, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine)
+        sdt = sd.to(dv, real)
+        nd = plan.ncg_linesearch_lossy(sdt[0].contiguous(), sdt[1].contiguous())
+        return float(nd[0]), float(nd[1])
+
+    def hvp(v):
+        return fwi_joint_gauss_newton_product(state["x"], v.to(dv, real).contiguous(), *fargs, **kw)
+
+    return loss_grad, linesearch, hvp
+
+
+def nonlinear_conjugate_gradient_joint(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML,
+                                       mask_indices, *, kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, dtype="c64", bde=None,
+                                       stencil="python", device=0, engine="auto", history=None, loss_grad=None,
+                                       linesearch=None):
+    """The reference's NCG loop (``nonlinear_conjugate_gradient``) on sound speed and attenuation together; returns ``(c,
+    kappa)`` as NumPy (Ny, Nx) arrays.
+
+    It works on the block-scaled variables of ``run_lbfgs_joint_fwi``, ``x = D x~`` with ``D = diag(s0 pert_scale,
+    kappa_scale)``: Hestenes-Stiefel on the scaled gradient ``g~ = D g`` (beta = 0 at the first iteration, as in the
+    reference), the physical direction ``sd = D d~``, the linearised exact step ``num / den`` of the joint line search
+    (``ust_ncg_linesearch_lossy``: ``num = -<sd, g>``, ``den = |J sd|^2``), and ``kappa <- max(kappa, 0)`` after every
+    step.  One evaluation (one factorisation) and one line search per iteration.
+
+    ``loss_grad(x) -> (loss, grad)`` and ``linesearch(sd) -> (num, den)`` (at the point of the last ``loss_grad`` call)
+    replace the GPU objective; they receive (2, Ny, Nx) float64 torch tensors = [slowness, kappa].  ``history`` (a list)
+    receives one dict per iteration: loss, gradient norm, beta, step, velocity range, largest kappa and clipped nodes.
+    """
+    import torch
+    ny, nx = _to_np(yi).size, _to_np(xi).size
+    if loss_grad is None or linesearch is None:
+        loss_grad, linesearch, _ = _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
+                                                    mask_indices, dtype, bde, stencil, device, engine)
+    x, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
+    dot = lambda a, b: float(torch.sum(a * b))
+    d = gprev = None
+    for it in range(int(Niter)):
+        loss, g = loss_grad(x)
+        if it == 0:
+            dv = g.device if torch.is_tensor(g) else torch.device("cpu")
+            x, D = x.to(dv), D.to(dv)
+        gt = D * _f64(g, dv).reshape(2, ny, nx)  # scaled gradient
+        if it == 0:
+            beta = 0.0
+        else:
+            dg = gt - gprev
+            beta = dot(gt, dg) / dot(d, dg)
+        d = -gt if it == 0 else beta * d - gt
+        sd = D * d
+        num, den = linesearch(sd)
+        step = float(num) / float(den)
+        x, clipped = _project_kappa(x + step * sd)
+        if history is not None:
+            history.append(dict(it=it, loss=float(loss), grad_norm=math.sqrt(dot(gt, gt)), beta=beta, step=step,
+                                vel_min=float(1.0 / x[0].max()), vel_max=float(1.0 / x[0].min()), kappa_max=float(x[1].max()),
+                                clipped=clipped))
+        gprev = gt
+    x = x.cpu().numpy()
+    return 1.0 / x[0], x[1]
+
+
+def gauss_newton_joint_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
+                           kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, cg_iters=8, cg_tol=1e-2, damping=0.0,
+                           max_backtracks=4, dtype="c64", bde=None, stencil="python", device=0, engine="auto", history=None,
+                           loss_grad=None, hvp=None):
+    """Truncated Gauss-Newton on sound speed and attenuation together; returns ``(c, kappa)`` as NumPy (Ny, Nx) arrays.
+
+    The outer loop of ``gauss_newton_fwi`` on the block-scaled variables of ``run_lbfgs_joint_fwi`` (``D = diag(s0 pert_scale,
+    kappa_scale)``): CG on ``(D H_GN D + mu I) p~ = -D g`` with the joint products (``fwi_joint_gauss_newton_product``), whose
+    off-diagonal blocks ``H_s,kappa`` couple the two maps from the first product; the trial ``x + step D p~`` has kappa
+    clipped at 0 and is backtracked as in ``gauss_newton_fwi``.  With ``cg_iters=1`` and ``damping=0`` an iteration is the
+    first iteration of ``nonlinear_conjugate_gradient_joint``.
+
+    ``loss_grad(x) -> (loss, grad)`` and ``hvp(v) -> hv`` (at the point of the last ``loss_grad`` call) replace the GPU
+    objective; they receive (2, Ny, Nx) float64 torch tensors = [slowness, kappa].  ``history`` receives the records of
+    ``gauss_newton_fwi`` plus ``clipped``, the number of kappa nodes clipped in the last trial.
+    """
+    import torch
+    ny, nx = _to_np(yi).size, _to_np(xi).size
+    if loss_grad is None or hvp is None:
+        loss_grad, _, hvp = _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices,
+                                             dtype, bde, stencil, device, engine)
+    x0, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
+    x = _gauss_newton_loop(x0, loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history, slow_of=lambda x: x[0],
+                           scale=D, project=_project_kappa)
+    x = x.cpu().numpy()
+    return 1.0 / x[0], x[1]
 
 
 # -------------------------------------------------------------------------------------------------
@@ -640,3 +830,38 @@ def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
         if history is not None:
             history.append(h)
     return vel
+
+
+def joint_frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, stages, Niter, a0, L_PML,
+                                 mask_indices, *, kappa_init=0.0, dtype="c64", stencil="python", device=0, engine="auto",
+                                 history=None, method="ncg"):
+    """``frequency_continuation`` for sound speed and attenuation together: per stage ``Niter`` iterations of
+    ``nonlinear_conjugate_gradient_joint`` (``method="ncg"``), outer iterations of ``gauss_newton_joint_fwi`` (``"gn"``) or
+    L-BFGS-B iterations of ``run_lbfgs_joint_fwi`` (``"lbfgs"``), each with its default settings and each stage starting
+    from the maps the previous one ended with.  Returns ``(c, kappa)``; ``history`` (a list) receives one list of records per
+    stage (for ``"lbfgs"``, ``(loss, params)`` of every evaluation).
+    """
+    if method not in ("ncg", "gn", "lbfgs"):
+        raise ValueError("method must be 'ncg', 'gn' or 'lbfgs'")
+    f = np.asarray(_to_np(f), dtype=np.float64).ravel()
+    rec = _to_np(REC_DATA)
+    if rec.ndim != 3 or rec.shape[0] != f.size:
+        raise ValueError("REC_DATA must be (Nf, Nt, E) with Nf == len(f)")
+    vel, kap = c_init, kappa_init
+    prev = None
+    for st in stages:
+        idx = np.asarray(st, dtype=np.int64).ravel()
+        if prev is not None and prev != idx.size:
+            clear_plans()  # a plan is sized for its number of frequencies; do not keep two factor stores alive
+        prev = idx.size
+        h = [] if history is not None else None
+        if method == "lbfgs":
+            vel, kap = run_lbfgs_joint_fwi(xi, yi, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], a0, L_PML, mask_indices,
+                                           kappa_init=kap, maxiter=Niter, dtype=dtype, stencil=stencil, engine=engine, history=h)
+        else:
+            drv = gauss_newton_joint_fwi if method == "gn" else nonlinear_conjugate_gradient_joint
+            vel, kap = drv(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter, a0, L_PML, mask_indices,
+                           kappa_init=kap, dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+        if history is not None:
+            history.append(h)
+    return vel, kap

@@ -202,9 +202,15 @@ struct PertArgs {
     const R* sd;
     long long N;
     int nt, nfreq;
+    const R* kappa;     // [N] LOSSY only: attenuation slowness
+    const R* sd_kappa;  // [N] LOSSY only: kappa part of the direction
 };
 
-template <typename R>
+// LOSSY (complex slowness sigma = s - i kappa, DESIGN.md section 7e): the RHS is -2 w^2 sigma alpha_t u_t (sd - i sd_kappa), with
+// the coefficient c = -2 w^2 (s - i kappa)(sd - i sd_kappa) formed in FP64 and cast once.  Its real part keeps the lossless
+// association ((-2 w w) s) sd and only adds terms that are zero at kappa = 0, sd_kappa = 0, so the lossy kernel then writes the
+// lossless RHS bit for bit (up to the sign of zero entries).
+template <typename R, bool LOSSY>
 __global__ void __launch_bounds__(256) pert_rhs_kernel(PertArgs<R> a) {
     const double PI = 3.14159265358979323846;
     const long long total = a.N * a.nt;
@@ -213,9 +219,18 @@ __global__ void __launch_bounds__(256) pert_rhs_kernel(PertArgs<R> a) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         long long p = i / a.nt;
         int t = (int)(i % a.nt);
-        R c = (R)(-2.0 * w * w * (double)a.slow[p] * (double)a.sd[p]);
-        cx<R> v = a.src_est[(size_t)f * a.nt + t] * a.U[(size_t)f * a.stride_f + i];
-        a.Out[(size_t)f * a.stride_f + i] = cx<R>(c * v.re, c * v.im);
+        if constexpr (LOSSY) {
+            const double s = (double)a.slow[p], k = (double)a.kappa[p], ds = (double)a.sd[p], dk = (double)a.sd_kappa[p];
+            const double m = -2.0 * w * w;
+            const R cr = (R)(m * s * ds - m * k * dk);  // Re c = -2 w^2 (s ds - kappa dk)
+            const R ci = (R)(-m * (s * dk + k * ds));    // Im c = +2 w^2 (s dk + kappa ds)
+            cx<R> v = a.src_est[(size_t)f * a.nt + t] * a.U[(size_t)f * a.stride_f + i];
+            a.Out[(size_t)f * a.stride_f + i] = cx<R>(cr * v.re - ci * v.im, cr * v.im + ci * v.re);
+        } else {
+            R c = (R)(-2.0 * w * w * (double)a.slow[p] * (double)a.sd[p]);
+            cx<R> v = a.src_est[(size_t)f * a.nt + t] * a.U[(size_t)f * a.stride_f + i];
+            a.Out[(size_t)f * a.stride_f + i] = cx<R>(c * v.re, c * v.im);
+        }
     }
 }
 

@@ -83,11 +83,13 @@ struct ust_plan {
     void *v_in = nullptr, *hv_out = nullptr, *drec = nullptr;  // Gauss-Newton product: v, H_GN v, J v at the kept receivers
     void *kappa_in = nullptr, *grad_kappa_out = nullptr;       // lossy evaluation: attenuation slowness, its gradient
     void *kappa_h2d = nullptr, *grad_kappa_d2h = nullptr;      // staging of ust_fwi_loss_grad_lossy_host
+    void *vk_in = nullptr, *hv_kappa_out = nullptr;  // lossy line search / product: kappa part of the direction, of H_GN v
     bool fwi_done = false;
     // the factors and fields are those of a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy): the line search and the
     // Gauss-Newton product, whose virtual source assumes a real slowness, refuse until a lossless ust_fwi_loss_grad
     bool lossy = false;
     bool gn_ok = false;  // the factors, fields and source estimates are those of the last ust_fwi_loss_grad (ust_fwi_gn_hvp)
+    bool gn_lossy_ok = false;  // ... of the last ust_fwi_loss_grad_lossy (ust_ncg_linesearch_lossy, ust_fwi_gn_hvp_lossy)
     bool use_graphs = true;  // UST_NO_GRAPHS=1 disables
     struct GraphEntry { cudaGraphExec_t exec = nullptr; long long launches = 0; };
     std::map<long long, GraphEntry> graphs;
@@ -482,7 +484,7 @@ static int factor_enqueue(ust_plan* p, const void* vel_dev, int nfreq, bool has_
 template <typename R>
 static int factor_impl(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs, const double* bde, cudaStream_t st,
                        const void* kappa_dev = nullptr) {
-    p->gn_ok = false;  // the factors no longer belong to the forward fields of the last evaluation
+    p->gn_ok = p->gn_lossy_ok = false;  // the factors no longer belong to the forward fields of the last evaluation
     UST_TRY(upload_params(p, nfreq, freqs, bde, st));
     if (kappa_dev) p->lossy = true;
     return factor_enqueue<R>(p, vel_dev, nfreq, bde != nullptr, st, kappa_dev);
@@ -715,9 +717,28 @@ static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bo
     return 0;
 }
 
-// perturbation solve + line-search scalars, device work only: reads p->sd_in, writes p->d_scal[2..3]
+// RHS of the perturbation solve for every group, from the direction `dir` (and, lossy, its kappa part p->vk_in)
 template <typename R>
-static int linesearch_enqueue(ust_plan* p, cudaStream_t st) {
+static int pert_rhs_groups(ust_plan* p, const std::vector<Group>& gs, const void* dir, bool lossy) {
+    const int nt = p->nt;
+    const size_t stride = (size_t)p->g.N * nt;
+    for (const Group& q : gs) {
+        PertArgs<R> pa;
+        pa.U = (const cx<R>*)p->U + (size_t)q.f0 * stride; pa.Out = (cx<R>*)p->Lam + (size_t)q.f0 * stride; pa.stride_f = stride;
+        pa.src_est = (const cx<R>*)p->src_est + (size_t)q.f0 * nt;
+        pa.freqs = p->d_freqs + q.f0; pa.slow = (const R*)p->slow_in; pa.sd = (const R*)dir; pa.N = p->g.N; pa.nt = nt; pa.nfreq = q.nf;
+        pa.kappa = (const R*)p->kappa_in; pa.sd_kappa = (const R*)p->vk_in;
+        if (lossy) pert_rhs_kernel<R, true><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+        else pert_rhs_kernel<R, false><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+        UST_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+// perturbation solve + line-search scalars, device work only: reads p->sd_in (lossy: also p->kappa_in and p->vk_in), writes
+// p->d_scal[2..3]
+template <typename R>
+static int linesearch_enqueue(ust_plan* p, cudaStream_t st, bool lossy = false) {
     const Geom& g = p->g;
     const int nt = p->nt, nfreq = p->nfreq_cur;
     const size_t stride = (size_t)g.N * nt;
@@ -725,14 +746,7 @@ static int linesearch_enqueue(ust_plan* p, cudaStream_t st) {
     UST_CUDA(cudaMemsetAsync(out2, 0, 2 * sizeof(double), st));
     const std::vector<Group> gs = make_groups(p, 0, nfreq, st);
     UST_TRY(fork_groups(p, gs));
-    for (const Group& q : gs) {
-        PertArgs<R> pa;
-        pa.U = (const cx<R>*)p->U + (size_t)q.f0 * stride; pa.Out = (cx<R>*)p->Lam + (size_t)q.f0 * stride; pa.stride_f = stride;
-        pa.src_est = (const cx<R>*)p->src_est + (size_t)q.f0 * nt;
-        pa.freqs = p->d_freqs + q.f0; pa.slow = (const R*)p->slow_in; pa.sd = (const R*)p->sd_in; pa.N = g.N; pa.nt = nt; pa.nfreq = q.nf;
-        pert_rhs_kernel<R><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
-        UST_LAUNCH_CHECK();
-    }
+    UST_TRY(pert_rhs_groups<R>(p, gs, p->sd_in, lossy));
     UST_TRY(sweeps_groups<R>(p, gs, (cx<R>*)p->Lam, stride, nt, 0));
     for (const Group& q : gs) {
         LineArgs<R> la;
@@ -751,8 +765,10 @@ static int linesearch_enqueue(ust_plan* p, cudaStream_t st) {
 // evaluation, device work only: reads p->v_in, writes p->hv_out, p->drec (J v) and p->d_scal[6] (sum |J v|^2).  Per group:
 // perturbation solve with RHS -VIRT*v (as linesearch_enqueue), J v gathered at the kept receivers, scattered back as the
 // adjoint source, adjoint sweeps (as fwi_enqueue); the groups meet at gradient_kernel, which forms sum_f -Re(conj(VIRT) * adj).
+// lossy: the complex-slowness RHS from v = [p->v_in, p->vk_in], and gradient_kernel<R, true> on p->slow_in / p->kappa_in writes
+// both halves of J^H (J v): p->hv_out and p->hv_kappa_out.
 template <typename R>
-static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st) {
+static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st, bool lossy = false) {
     const Geom& g = p->g;
     const int nt = p->nt, nfreq = p->nfreq_cur;
     const size_t stride = (size_t)g.N * nt;
@@ -760,14 +776,7 @@ static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st) {
     UST_CUDA(cudaMemsetAsync(jv2, 0, sizeof(double), st));
     const std::vector<Group> gs = make_groups(p, 0, nfreq, st);
     UST_TRY(fork_groups(p, gs));
-    for (const Group& q : gs) {
-        PertArgs<R> pa;
-        pa.U = (const cx<R>*)p->U + (size_t)q.f0 * stride; pa.Out = (cx<R>*)p->Lam + (size_t)q.f0 * stride; pa.stride_f = stride;
-        pa.src_est = (const cx<R>*)p->src_est + (size_t)q.f0 * nt;
-        pa.freqs = p->d_freqs + q.f0; pa.slow = (const R*)p->slow_in; pa.sd = (const R*)p->v_in; pa.N = g.N; pa.nt = nt; pa.nfreq = q.nf;
-        pert_rhs_kernel<R><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
-        UST_LAUNCH_CHECK();
-    }
+    UST_TRY(pert_rhs_groups<R>(p, gs, p->v_in, lossy));
     UST_TRY(sweeps_groups<R>(p, gs, (cx<R>*)p->Lam, stride, nt, 0));
     for (const Group& q : gs) {
         GnRecvArgs<R> ra;
@@ -793,11 +802,12 @@ static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st) {
     GradArgs<R> ga;
     ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
     ga.freqs = p->d_freqs; ga.slow = (const R*)p->slow_in; ga.grad = (R*)p->hv_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
-    ga.kappa = nullptr; ga.grad_kappa = nullptr;
+    ga.kappa = (const R*)p->kappa_in; ga.grad_kappa = (R*)p->hv_kappa_out;
     const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
     {
         ProfScope ps(p, PC_GRADIENT, st);
-        gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
+        if (lossy) gradient_kernel<R, true><<<blocks, 256, 0, st>>>(ga);
+        else gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
     }
     UST_LAUNCH_CHECK();
     return 0;
@@ -856,9 +866,10 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     if (rec != p->rec_in) UST_CUDA(cudaMemcpyAsync(p->rec_in, rec, (size_t)nfreq * p->nt * p->nelem * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(p->kappa_in, kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     const bool has_bde = bde != nullptr;
-    // lossless evaluation 0/1, line search 500, Gauss-Newton product 600, lossy evaluation 700/701
+    // lossless evaluation 0/1, line search 500, Gauss-Newton product 600, lossy evaluation 700/701, lossy line search 800,
+    // lossy Gauss-Newton product 900
     const long long key = 1000LL * nfreq + (lossy ? 700 : 0) + (has_bde ? 1 : 0);
-    p->gn_ok = false;
+    p->gn_ok = p->gn_lossy_ok = false;
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_, lossy); }));
     p->nfreq_cur = nfreq;
     p->factored = true;
@@ -868,6 +879,7 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     p->fwi_done = true;
     p->lossy = lossy;
     p->gn_ok = !lossy;
+    p->gn_lossy_ok = lossy;
     if (p->trace) return dump_update_trace(p, st);
     return 0;
 }
@@ -907,6 +919,51 @@ static int gn_hvp_impl(ust_plan* p, const void* v, void* hv, double* jv2, void* 
     const long long key = 1000LL * p->nfreq_cur + 600;
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_); }));
     UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    UST_CUDA(cudaMemcpyAsync(jv2, p->d_scal + 6, sizeof(double), cudaMemcpyDeviceToDevice, st));
+    if (jv) UST_CUDA(cudaMemcpyAsync(jv, p->drec, (size_t)p->nfreq_cur * p->nt * p->nm * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+// lossy twins of linesearch_impl / gn_hvp_impl: valid only on the state of the last ust_fwi_loss_grad_lossy
+static int check_lossy_state(ust_plan* p, const char* name) {
+    if (!p->vk_in) { set_error(std::string(name) + ": plan was created with fwi_buffers=0"); return 1; }
+    if (!p->factored || !p->fwi_done) { set_error(std::string(name) + ": call ust_fwi_loss_grad_lossy first"); return 1; }
+    if (!p->lossy) {
+        set_error(std::string(name) + ": the last evaluation was lossless (ust_fwi_loss_grad); use the lossless entry point or call "
+                  "ust_fwi_loss_grad_lossy first");
+        return 1;
+    }
+    if (!p->gn_lossy_ok) {
+        set_error(std::string(name) + ": the factors were replaced (ust_factor / ust_factor_lossy / ust_solve_helmholtz_host) after the "
+                  "last ust_fwi_loss_grad_lossy; call ust_fwi_loss_grad_lossy again");
+        return 1;
+    }
+    return 0;
+}
+
+template <typename R>
+static int linesearch_lossy_impl(ust_plan* p, const void* sd, const void* sd_kappa, double* out2, cudaStream_t st) {
+    const Geom& g = p->g;
+    UST_TRY(check_lossy_state(p, "ust_ncg_linesearch_lossy"));
+    UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    UST_CUDA(cudaMemcpyAsync(p->vk_in, sd_kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    const long long key = 1000LL * p->nfreq_cur + 800;
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_, true); }));
+    UST_CUDA(cudaMemcpyAsync(out2, p->d_scal + 2, 2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+template <typename R>
+static int gn_hvp_lossy_impl(ust_plan* p, const void* v, const void* v_kappa, void* hv, void* hv_kappa, double* jv2, void* jv,
+                             cudaStream_t st) {
+    const Geom& g = p->g;
+    UST_TRY(check_lossy_state(p, "ust_fwi_gn_hvp_lossy"));
+    UST_CUDA(cudaMemcpyAsync(p->v_in, v, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    UST_CUDA(cudaMemcpyAsync(p->vk_in, v_kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    const long long key = 1000LL * p->nfreq_cur + 900;
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_, true); }));
+    UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+    UST_CUDA(cudaMemcpyAsync(hv_kappa, p->hv_kappa_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     UST_CUDA(cudaMemcpyAsync(jv2, p->d_scal + 6, sizeof(double), cudaMemcpyDeviceToDevice, st));
     if (jv) UST_CUDA(cudaMemcpyAsync(jv, p->drec, (size_t)p->nfreq_cur * p->nt * p->nm * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
     return 0;
@@ -1112,6 +1169,8 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
         rc |= dev_alloc(p, &p->hv_out, g.N * p->rsz);
         rc |= dev_alloc(p, &p->kappa_in, g.N * p->rsz);
         rc |= dev_alloc(p, &p->grad_kappa_out, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->vk_in, g.N * p->rsz);
+        rc |= dev_alloc(p, &p->hv_kappa_out, g.N * p->rsz);
     }
     if (const char* e = getenv("UST_NO_GRAPHS")) p->use_graphs = atoi(e) == 0;
     if (const char* e = getenv("UST_NO_PDL")) ust::g_use_pdl = atoi(e) == 0;
@@ -1178,7 +1237,8 @@ int ust_plan_destroy(ust_plan* p) {
     for (void* q : ptrs)
         if (q) cudaFree(q);
     drop_graphs(p);
-    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in, p->v_in, p->hv_out, p->drec, p->kappa_in, p->grad_kappa_out})
+    for (void* q : {p->slow_in, p->rec_in, p->grad_out, p->sd_in, p->v_in, p->hv_out, p->drec, p->kappa_in, p->grad_kappa_out,
+                     p->vk_in, p->hv_kappa_out})
         if (q) cudaFree(q);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
     if (p->ev_out) cudaEventDestroy(p->ev_out);
@@ -1240,7 +1300,7 @@ int ust_plan_set_acquisition(ust_plan* p, int nt, const int32_t* src_lin, int ne
     UST_CUDA(cudaDeviceSynchronize());
     drop_graphs(p);
     p->fwi_done = false;
-    p->gn_ok = false;
+    p->gn_ok = p->gn_lossy_ok = false;
     for (int** q : {&p->src_lin, &p->rx_lin, &p->mask})
         if (*q) { cudaFree(*q); *q = nullptr; }
     if (p->rec_in) { cudaFree(p->rec_in); p->rec_in = nullptr; }
@@ -1395,6 +1455,27 @@ int ust_fwi_gn_hvp(ust_plan* p, const void* v_dev, void* hv_dev, double* jv2_dev
     if (!v_dev || !hv_dev || !jv2_dev) { set_error("ust_fwi_gn_hvp: null argument"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
     return DISPATCH(p, gn_hvp_impl, p, v_dev, hv_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
+}
+
+int ust_ncg_linesearch_lossy(ust_plan* p, const void* sd_s_dev, const void* sd_kappa_dev, double* out2_dev, void* stream) {
+    UST_TRY(check_plan(p));
+    if (!sd_s_dev || !sd_kappa_dev || !out2_dev) {
+        set_error("ust_ncg_linesearch_lossy: null argument (sd_kappa_dev is required)");
+        return 1;
+    }
+    UST_CUDA(cudaSetDevice(p->d.device));
+    return DISPATCH(p, linesearch_lossy_impl, p, sd_s_dev, sd_kappa_dev, out2_dev, (cudaStream_t)stream);
+}
+
+int ust_fwi_gn_hvp_lossy(ust_plan* p, const void* v_s_dev, const void* v_kappa_dev, void* hv_s_dev, void* hv_kappa_dev,
+                         double* jv2_dev, void* jv_dev, void* stream) {
+    UST_TRY(check_plan(p));
+    if (!v_s_dev || !v_kappa_dev || !hv_s_dev || !hv_kappa_dev || !jv2_dev) {
+        set_error("ust_fwi_gn_hvp_lossy: null argument (v_kappa_dev and hv_kappa_dev are required)");
+        return 1;
+    }
+    UST_CUDA(cudaSetDevice(p->d.device));
+    return DISPATCH(p, gn_hvp_lossy_impl, p, v_s_dev, v_kappa_dev, hv_s_dev, hv_kappa_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
 }
 
 int ust_get_bde(ust_plan* p, double* out) {

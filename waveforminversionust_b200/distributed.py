@@ -129,6 +129,20 @@ class ShardedFWI:
             grad = torch.zeros((2,) + tuple(slow_dev.shape), dtype=slow_dev.dtype, device=slow_dev.device)
         return allreduce_loss_grad(loss, grad, self.group)
 
+    def gn_hvp_lossy_device(self, v_s_dev, v_k_dev):
+        """Joint Gauss-Newton product at the point of the last ``loss_grad_lossy_device``: this rank's part
+        (``HelmholtzPlan.gn_hvp_lossy``: its frequencies or its transmitters) and one all-reduce of the packed
+        ``[hv_s, hv_kappa, jv2]``.  Returns ``(hv (2, Ny, Nx), jv2 (0-d float64 tensor))``."""
+        torch = self.torch
+        if len(self.local) and len(self.local_tx):
+            hv, jv2 = self.plan.gn_hvp_lossy(v_s_dev, v_k_dev)
+            jv2 = jv2[0]
+        else:
+            jv2 = torch.zeros((), dtype=torch.float64, device=v_s_dev.device)
+            hv = torch.zeros((2,) + tuple(v_s_dev.shape), dtype=v_s_dev.dtype, device=v_s_dev.device)
+        jv2, hv = allreduce_loss_grad(jv2, hv, self.group)
+        return hv, jv2
+
     def local_rec(self, rec_all):
         """This rank's part of the full observed data ``rec_all`` (nfreq, Nt, E): its frequencies (all transmitters) or its
         transmitters (all frequencies)."""
@@ -226,3 +240,29 @@ def run_lbfgs_joint_sharded(eng, rec_local_dev, c_init, kappa_init=0.0, kappa_sc
                                    geom.L_PML, geom.mask_indices, kappa_init=kappa_init, kappa_scale=kappa_scale, maxiter=maxiter,
                                    tol=tol, history_size=history_size, dtype=plan.dtype, history=history, loss_grad=loss_grad,
                                    pert_scale=pert_scale)
+
+
+def run_gauss_newton_joint_sharded(eng, rec_local_dev, c_init, Niter, kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, cg_iters=8,
+                                   cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None):
+    """``api.gauss_newton_joint_fwi`` on a sharded engine: every rank runs the same joint driver on the all-reduced
+    ``loss_grad_lossy_device`` and ``gn_hvp_lossy_device``, so the ranks take identical steps.  Returns ``(c, kappa)`` (Ny, Nx)
+    NumPy arrays (identical on every rank)."""
+    import torch
+    from . import api
+    geom, plan = eng.geom, eng.plan
+    dv = torch.device(f"cuda:{eng.device}")
+
+    def loss_grad(x):
+        x = x.to(dv, plan.treal)
+        loss, grad = eng.loss_grad_lossy_device(x[0].contiguous(), x[1].contiguous(), rec_local_dev)
+        return float(loss), grad
+
+    def hvp(v):
+        v = v.to(dv, plan.treal)
+        return eng.gn_hvp_lossy_device(v[0].contiguous(), v[1].contiguous())[0]
+
+    return api.gauss_newton_joint_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init,
+                                      eng.freqs, Niter, geom.a0, geom.L_PML, geom.mask_indices, kappa_init=kappa_init,
+                                      kappa_scale=kappa_scale, pert_scale=pert_scale, cg_iters=cg_iters, cg_tol=cg_tol,
+                                      damping=damping, max_backtracks=max_backtracks, dtype=plan.dtype, device=eng.device,
+                                      history=history, loss_grad=loss_grad, hvp=hvp)

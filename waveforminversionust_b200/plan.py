@@ -210,6 +210,34 @@ class HelmholtzPlan:
                                          C.c_void_p(jvt.data_ptr()) if jv else None, _stream_ptr(self.device)), "ust_fwi_gn_hvp")
         return (hv, jv2, jvt) if jv else (hv, jv2)
 
+    def ncg_linesearch_lossy(self, sd_s, sd_k):
+        """Line-search scalars ``[num, den]`` (2-element float64 tensor) of the joint direction ``[sd_s, sd_k]`` on the state of
+        the last ``fwi_loss_grad_lossy`` (``ust_ncg_linesearch_lossy``)."""
+        torch = _torch()
+        self._check_tensor(sd_s, self.treal, self.nx * self.ny)
+        self._check_tensor(sd_k, self.treal, self.nx * self.ny)
+        out = torch.empty(2, dtype=torch.float64, device=sd_s.device)
+        _lib.check(self.L.ust_ncg_linesearch_lossy(self.h, C.c_void_p(sd_s.data_ptr()), C.c_void_p(sd_k.data_ptr()),
+                                                   C.c_void_p(out.data_ptr()), _stream_ptr(self.device)), "ust_ncg_linesearch_lossy")
+        return out
+
+    def gn_hvp_lossy(self, v_s, v_k, jv=False):
+        """Joint Gauss-Newton product on the state of the last ``fwi_loss_grad_lossy``: ``v_s``, ``v_k`` (ny, nx) real CUDA
+        tensors -> ``(hv, jv2[, jv])`` with ``hv = Re(J^H J v)`` (2, ny, nx) = [s, kappa] blocks, ``jv2 = sum |J v|^2``
+        (1-element float64 tensor) and, when ``jv``, ``J v`` at the kept receivers (nfreq, nt, nm) complex
+        (``ust_fwi_gn_hvp_lossy``)."""
+        torch = _torch()
+        self._check_tensor(v_s, self.treal, self.nx * self.ny)
+        self._check_tensor(v_k, self.treal, self.nx * self.ny)
+        hv = torch.empty((2, self.ny, self.nx), dtype=self.treal, device=v_s.device)
+        jv2 = torch.empty(1, dtype=torch.float64, device=v_s.device)
+        jvt = torch.empty((getattr(self, "nfreq", 1), self.nt, getattr(self, "nm", 0)), dtype=self.tcplx, device=v_s.device) if jv else None
+        _lib.check(self.L.ust_fwi_gn_hvp_lossy(self.h, C.c_void_p(v_s.data_ptr()), C.c_void_p(v_k.data_ptr()),
+                                               C.c_void_p(hv[0].data_ptr()), C.c_void_p(hv[1].data_ptr()), C.c_void_p(jv2.data_ptr()),
+                                               C.c_void_p(jvt.data_ptr()) if jv else None, _stream_ptr(self.device)),
+                   "ust_fwi_gn_hvp_lossy")
+        return (hv, jv2, jvt) if jv else (hv, jv2)
+
     # -- host-buffer entry points (NumPy; no torch needed) ------------------------------------
     def solve_helmholtz_host(self, vel, src, f, adjoint=False, bde=None, refactor=True):
         vel = None if vel is None else np.ascontiguousarray(np.asarray(vel, dtype=self.real))
