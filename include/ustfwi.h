@@ -145,8 +145,8 @@ int ust_fwi_loss_grad_lossy_host(ust_plan* plan, const void* slow_host, const vo
  * perturbation solve with RHS -VIRT*sd on the existing factors, gather at the receivers and return
  * the two line-search scalars  num = Re<dREC, REC_DATA-REC_SIM>, den = Re<dREC,dREC>
  * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles.
- * Fails while the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad);
- * ust_ncg_linesearch_lossy is the line search of the lossy model. */
+ * Fails if ust_factor, ust_factor_lossy or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and
+ * after a lossy evaluation (ust_fwi_loss_grad_lossy); ust_ncg_linesearch_lossy is the line search of the lossy model. */
 int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, void* stream);
 
 /* Gauss-Newton Hessian-vector product of the joint objective on the factors, forward fields and source estimates of the last
@@ -155,9 +155,8 @@ int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, voi
  * jv_dev: (nfreq, nt, nm) complex J v at the kept receivers (mask order), or NULL.  Overwrites the adjoint wavefield.
  * J is the linearisation the gradient uses (virtual source 2 w^2 s alpha u without the stencil's mass weights and the PML
  * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).
- * Fails if ust_factor or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and while the plan holds
- * a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy since the last ust_fwi_loss_grad); ust_fwi_gn_hvp_lossy is the
- * product of the lossy model. */
+ * Fails if ust_factor, ust_factor_lossy or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and
+ * after a lossy evaluation (ust_fwi_loss_grad_lossy); ust_fwi_gn_hvp_lossy is the product of the lossy model. */
 int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream);
 
 /* Lossy twins of ust_ncg_linesearch and ust_fwi_gn_hvp for the joint (s, kappa) problem, valid only on the state of the last

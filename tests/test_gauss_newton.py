@@ -288,6 +288,17 @@ def test_plan_state(torch_):
     close = lambda x, y: bool(torch_.all(torch_.abs(x - y) <= 1e-13 * torch_.abs(y)))
     assert torch_.equal(a[0], b[0]) and close(a[1], b[1])
     assert close(plan.ncg_linesearch(vt), nd0)
+    # replaced factors: the line search refuses, after a factorisation and after a refactorising host solve; the next
+    # evaluation makes it run again
+    rt1 = rt.to(plan.tcplx).reshape(1, plan.nt, plan.nelem).contiguous()
+    replace = (lambda: plan.factor(torch_.as_tensor(c0.astype(np.float32)).cuda(), [f]),
+               lambda: plan.solve_helmholtz_host(c0.astype(np.float32), np.zeros((48, 48, 1), np.complex64), f, refactor=True))
+    for r in replace:
+        r()
+        with pytest.raises(_lib.UstError, match="replaced"):
+            plan.ncg_linesearch(vt)
+        plan.fwi_loss_grad(st, rt1, [f], bde=bde)
+        assert close(plan.ncg_linesearch(vt), nd0)
     # replaced factors: the product refuses ...
     plan.factor(torch_.as_tensor(c0.astype(np.float32)).cuda(), [f])
     with pytest.raises(_lib.UstError, match="replaced"):

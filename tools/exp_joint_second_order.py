@@ -66,7 +66,7 @@ def main():
              f"# start: c = 1480 m/s (error {c_err(np.full((n, n), 1480.0)):.3f} m/s), kappa = 0 (error {k_err(np.zeros((n, n))):.4f} dB/(cm MHz))"]
     results = {}
     for name in ("a_ncg", "b_gauss_newton", "c_lbfgs"):
-        lg0, ls0, hvp0 = api._joint_callables(*dargs[:7], freqs, *tail, "c64", None, "python", 0, "auto")
+        lg0, ls0, hvp0 = api._gpu_callables(True, *dargs[:7], freqs, *tail, "c64", None, "python", 0, "auto")
         trace, count = [], {"products": 0, "linesearches": 0}
         t0 = [0.0]
 

@@ -181,18 +181,8 @@ def fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, i
     With ``f`` of length Nf and ``REC_DATA`` of shape (Nf, Nt, E) the joint objective sum_f loss_f is
     returned.  Usable as ``jaxopt.LBFGS(fun, value_and_grad=True)`` / ``scipy.optimize.minimize(jac=True)``.
     """
-    dev = _device_of(params, REC_DATA)
-    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
-    if _is_torch(params) and params.is_cuda:
-        rec = REC_DATA.to(plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
-        slow = params.to(plan.treal).reshape(plan.ny, plan.nx).contiguous()
-        loss, grad = plan.fwi_loss_grad(slow, rec, freqs, bde=bde)
-        plan._eval_key = _eval_key(params, REC_DATA, freqs, bde)
-        return loss[0], grad.reshape(params.shape)
-    p = _to_np(params)
-    loss, grad = plan.fwi_loss_grad_host(p.reshape(plan.ny, plan.nx), _to_np(REC_DATA), freqs, bde=bde)
-    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde)
-    return loss, grad.reshape(p.shape)
+    return _loss_function(False, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil,
+                          engine)
 
 
 def fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
@@ -202,21 +192,30 @@ def fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_incl
     ([dloss/ds, dloss/dkappa]).  The other arguments and the loss are those of ``fwi_loss_function``; the gradients use the
     same linearisation (source estimates held fixed, DESIGN.md section 7d).  The ``value_and_grad`` contract of
     ``fwi_loss_function``: torch CUDA in -> torch out (device buffers), NumPy in -> NumPy out (host buffers)."""
+    return _loss_function(True, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil,
+                          engine)
+
+
+def _loss_function(lossy, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil, engine):
+    """The body of ``fwi_loss_function`` (``lossy``: of ``fwi_joint_loss_function``, ``params`` = [s, kappa])."""
     dev = _device_of(params, REC_DATA)
     plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
-    if tuple(params.shape) != (2, plan.ny, plan.nx):
+    if lossy and tuple(params.shape) != (2, plan.ny, plan.nx):
         raise ValueError(f"params must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa]")
     if _is_torch(params) and params.is_cuda:
         import torch
         rec = REC_DATA.to(plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
         p = params.to(plan.treal)
-        loss, gs, gk = plan.fwi_loss_grad_lossy(p[0].contiguous(), p[1].contiguous(), rec, freqs, bde=bde)
-        plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy=True)
-        return loss[0], torch.stack([gs, gk])
-    p = np.asarray(_to_np(params), dtype=plan.real)
-    loss, gs, gk = plan.fwi_loss_grad_lossy_host(p[0], p[1], _to_np(REC_DATA), freqs, bde=bde)
-    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy=True)
-    return loss, np.stack([gs, gk])
+        maps = (p[0].contiguous(), p[1].contiguous()) if lossy else (p.reshape(plan.ny, plan.nx).contiguous(), None)
+        loss, *grads = plan._loss_grad(*maps, rec, freqs, bde)
+        loss, grad, shape = loss[0], torch.stack(grads) if lossy else grads[0], params.shape
+    else:
+        p = np.asarray(_to_np(params), dtype=plan.real)
+        maps = (p[0], p[1]) if lossy else (p.reshape(plan.ny, plan.nx), None)
+        loss, *grads = plan._loss_grad_host(*maps, _to_np(REC_DATA), freqs, bde, None)
+        grad, shape = np.stack(grads) if lossy else grads[0], p.shape
+    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy)
+    return loss, grad.reshape(shape)
 
 
 def _eval_key(params, REC_DATA, freqs, bde, lossy=False):
@@ -258,19 +257,8 @@ def fwi_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_
     A product costs two all-source sweeps on the factorisation the last evaluation left on the plan; when the last
     ``fwi_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)``, the evaluation runs first.
     """
-    import torch
-    dev = _device_of(params, REC_DATA, v)
-    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
-    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde)):
-        fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
-                          dtype=dtype, bde=bde, stencil=stencil, engine=engine)
-    shape = tuple(params.shape) if hasattr(params, "shape") else np.shape(params)
-    if _is_torch(v) and v.is_cuda:
-        hv, _ = plan.gn_hvp(v.detach().to(plan.treal).reshape(plan.ny, plan.nx).contiguous())
-        return hv.reshape(shape)
-    vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real).reshape(plan.ny, plan.nx))).to(f"cuda:{plan.device}")
-    hv, _ = plan.gn_hvp(vt)
-    return hv.cpu().numpy().reshape(shape)
+    return _gauss_newton_product(False, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
+                                 num_elements, dtype, bde, stencil, engine)
 
 
 def fwi_joint_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
@@ -288,21 +276,32 @@ def fwi_joint_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PM
     ``fwi_joint_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)`` (or the last evaluation was lossless),
     the evaluation runs first.
     """
+    return _gauss_newton_product(True, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
+                                 num_elements, dtype, bde, stencil, engine)
+
+
+def _gauss_newton_product(lossy, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
+                          num_elements, dtype, bde, stencil, engine):
+    """The body of ``fwi_gauss_newton_product`` (``lossy``: of ``fwi_joint_gauss_newton_product``)."""
     import torch
     dev = _device_of(params, REC_DATA, v)
     plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
-    if tuple(v.shape) != (2, plan.ny, plan.nx):
+    if lossy and tuple(v.shape) != (2, plan.ny, plan.nx):
         raise ValueError(f"v must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa] directions")
-    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde, lossy=True)):
-        fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
-                                dtype=dtype, bde=bde, stencil=stencil, engine=engine)
-    if _is_torch(v) and v.is_cuda:
+    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde, lossy)):
+        # looked up at call time: tests record the evaluation points by replacing these module functions
+        evaluate = fwi_joint_loss_function if lossy else fwi_loss_function
+        evaluate(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements, dtype=dtype,
+                 bde=bde, stencil=stencil, engine=engine)
+    on_device = _is_torch(v) and v.is_cuda
+    if on_device:
         vt = v.detach().to(plan.treal)
-        hv, _ = plan.gn_hvp_lossy(vt[0].contiguous(), vt[1].contiguous())
-        return hv
-    vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real))).to(f"cuda:{plan.device}")
-    hv, _ = plan.gn_hvp_lossy(vt[0].contiguous(), vt[1].contiguous())
-    return hv.cpu().numpy()
+    else:
+        vt = torch.as_tensor(np.ascontiguousarray(np.asarray(_to_np(v), dtype=plan.real))).to(f"cuda:{plan.device}")
+    dirs = (vt[0].contiguous(), vt[1].contiguous()) if lossy else (vt.reshape(plan.ny, plan.nx).contiguous(), None)
+    hv, _ = plan._gn_hvp(*dirs, False)
+    hv = hv.reshape(np.shape(params))
+    return hv if on_device else hv.cpu().numpy()
 
 
 def nonlinear_conjugate_gradient(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter,
@@ -373,34 +372,57 @@ def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, 
     ``loss_grad(slow_2d) -> (loss, grad_2d)`` replaces the objective (the parity test drives the same optimiser with the
     oracle's); ``history`` receives ``(loss, params.copy())`` of every evaluation.
     """
-    from scipy.optimize import minimize
     ny, nx = _to_np(yi).size, _to_np(xi).size
     num_elements = int(SRC.shape[2]) if SRC is not None else 0  # unused when ``loss_grad`` is injected
     c0 = np.asarray(_to_np(c_init), dtype=np.float64)
     s0 = 1.0 / float(c0.mean())
     real = np.float32 if dtype == "c64" else np.float64
-    state = {"loss0": None}
     if loss_grad is None:
         def loss_grad(slow):
             return fwi_loss_function(slow.astype(real), xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
                                      num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine)
 
+    slow, = _lbfgs_blocks(loss_grad, [_slowness_block(c0, s0, pert_scale, ny, nx)], ny, nx, maxiter, tol, history_size, history)
+    return 1.0 / slow
+
+
+def _slowness_block(c0, s0, pert_scale, ny, nx):
+    """The slowness block of the L-BFGS drivers: ``s = (1 + pert_scale p) s0``, starting at ``1 / c0``."""
+    p0 = ((np.ones((ny, nx)) / (c0 * s0) - 1.0) / pert_scale).ravel()
+    return (lambda p: (1.0 + pert_scale * p) * s0), s0 * pert_scale, p0, None
+
+
+def _lbfgs_blocks(loss_grad, blocks, ny, nx, maxiter, tol, history_size, history):
+    """SciPy's L-BFGS-B on a model of one (Ny, Nx) map or a stack of several, each non-dimensionalised on its own: block
+    ``(to_model, dmodel_dp, p0, lower_bound)`` maps its part ``p`` of the unknown to its map ``to_model(p)``, starts at ``p0``
+    and is bounded below by ``lower_bound`` (None: unbounded).  The objective is ``loss / loss(start)``.  ``history``
+    receives ``(loss, model.copy())`` of every evaluation.  Returns the final maps."""
+    from scipy.optimize import minimize
+    n = ny * nx
+    state = {"loss0": None}
+
+    def maps(p):
+        return [to_model(p[i * n:(i + 1) * n].reshape(ny, nx)) for i, (to_model, _, _, _) in enumerate(blocks)]
+
     def fun(p):
-        slow = (1.0 + pert_scale * p.reshape(ny, nx)) * s0
-        loss, grad = loss_grad(slow)
-        if np.shape(grad) != slow.shape:
-            raise ValueError("loss_grad must return a gradient with the shape of its argument")
+        m = maps(p)
+        model = m[0] if len(m) == 1 else np.stack(m)
+        loss, grad = loss_grad(model)
+        if np.shape(grad) != model.shape:
+            raise ValueError(f"loss_grad must return a gradient with the shape of its argument {model.shape}")
         if state["loss0"] is None:
             state["loss0"] = float(loss)
         if history is not None:
-            history.append((float(loss), slow.copy()))
+            history.append((float(loss), model.copy()))
         scale = 1.0 / state["loss0"]
-        return float(loss) * scale, np.asarray(grad, dtype=np.float64).ravel() * (s0 * pert_scale * scale)
+        g = np.asarray(grad, dtype=np.float64).reshape(len(blocks), n)
+        return float(loss) * scale, np.concatenate([g[i] * (dmodel_dp * scale) for i, (_, dmodel_dp, _, _) in enumerate(blocks)])
 
-    p0 = ((np.ones((ny, nx)) / (c0 * s0) - 1.0) / pert_scale).ravel()
-    res = minimize(fun, p0, jac=True, method="L-BFGS-B", options=dict(maxiter=int(maxiter), maxcor=int(history_size), gtol=float(tol)))
-    final_slow = (1.0 + pert_scale * res.x.reshape(ny, nx)) * s0
-    return 1.0 / final_slow
+    p0 = np.concatenate([b[2] for b in blocks])
+    bounds = None if all(b[3] is None for b in blocks) else [(b[3], None) for b in blocks for _ in range(n)]
+    res = minimize(fun, p0, jac=True, method="L-BFGS-B", bounds=bounds,
+                   options=dict(maxiter=int(maxiter), maxcor=int(history_size), gtol=float(tol)))
+    return maps(res.x)
 
 
 def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, L_PML, mask_indices, *, kappa_init=0.0,
@@ -418,7 +440,6 @@ def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f
     parity test drives the same optimiser with the oracle's); ``history`` receives ``(loss, params.copy())`` of every
     evaluation.
     """
-    from scipy.optimize import minimize
     from .geometry import db_cm_mhz_to_kappa
     ny, nx = _to_np(yi).size, _to_np(xi).size
     num_elements = int(SRC.shape[2]) if SRC is not None else 0  # unused when ``loss_grad`` is injected
@@ -426,34 +447,15 @@ def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f
     s0 = 1.0 / float(c0.mean())
     ks = float(db_cm_mhz_to_kappa(0.5) if kappa_scale is None else kappa_scale)
     real = np.float32 if dtype == "c64" else np.float64
-    state = {"loss0": None}
     if loss_grad is None:
         def loss_grad(params):
             return fwi_joint_loss_function(params.astype(real), xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab,
                                            mask_indices, num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine)
 
-    n = ny * nx
-
-    def fun(p):
-        params = np.stack([(1.0 + pert_scale * p[:n].reshape(ny, nx)) * s0, ks * p[n:].reshape(ny, nx)])
-        loss, grad = loss_grad(params)
-        if np.shape(grad) != params.shape:
-            raise ValueError("loss_grad must return a gradient with the shape of its argument (2, Ny, Nx)")
-        if state["loss0"] is None:
-            state["loss0"] = float(loss)
-        if history is not None:
-            history.append((float(loss), params.copy()))
-        scale = 1.0 / state["loss0"]
-        g = np.asarray(grad, dtype=np.float64)
-        return float(loss) * scale, np.concatenate([g[0].ravel() * (s0 * pert_scale * scale), g[1].ravel() * (ks * scale)])
-
-    p0 = np.concatenate([((np.ones((ny, nx)) / (c0 * s0) - 1.0) / pert_scale).ravel(),
-                         (np.asarray(_to_np(kappa_init), dtype=np.float64) * np.ones((ny, nx)) / ks).ravel()])
-    bounds = [(None, None)] * n + [(0.0, None)] * n
-    res = minimize(fun, p0, jac=True, method="L-BFGS-B", bounds=bounds,
-                   options=dict(maxiter=int(maxiter), maxcor=int(history_size), gtol=float(tol)))
-    final_slow = (1.0 + pert_scale * res.x[:n].reshape(ny, nx)) * s0
-    return 1.0 / final_slow, ks * res.x[n:].reshape(ny, nx)
+    kappa_block = (lambda p: ks * p), ks, (np.asarray(_to_np(kappa_init), dtype=np.float64) * np.ones((ny, nx)) / ks).ravel(), 0.0
+    slow, kappa = _lbfgs_blocks(loss_grad, [_slowness_block(c0, s0, pert_scale, ny, nx), kappa_block], ny, nx, maxiter, tol,
+                                history_size, history)
+    return 1.0 / slow, kappa
 
 
 def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
@@ -479,22 +481,8 @@ def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or hvp is None:
-        freqs = np.atleast_1d(np.asarray(_to_np(f), dtype=np.float64)).ravel()
-        dv = torch.device(f"cuda:{device}")
-        real = torch.float32 if dtype == "c64" else torch.float64
-        rec = torch.as_tensor(_to_np(REC_DATA)).to(dv).reshape(freqs.size, len(_to_np(tx_include)), -1).contiguous()
-        state = {}
-        fargs = (xi, yi, rec, SRC, freqs, a0, L_PML, tx_include, ind_matlab, mask_indices, numElements)
-        kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine)
-
-        def loss_grad(slow):
-            state["slow"] = slow.to(dv, real).contiguous()
-            loss, grad = fwi_loss_function(state["slow"], *fargs, **kw)
-            return float(loss), grad
-
-        def hvp(v):
-            return fwi_gauss_newton_product(state["slow"], v.to(dv, real).contiguous(), *fargs, **kw)
-
+        loss_grad, _, hvp = _gpu_callables(False, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
+                                           mask_indices, dtype, bde, stencil, device, engine)
     c0 = np.asarray(_to_np(c_init), dtype=np.float64) * np.ones((ny, nx))
     s = _gauss_newton_loop(torch.as_tensor(1.0 / c0), loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history,
                            slow_of=lambda x: x)
@@ -598,10 +586,10 @@ def _project_kappa(x):
     return torch.stack([x[0], torch.clamp(x[1], min=0.0)]), int(neg.sum())
 
 
-def _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices, dtype, bde, stencil,
-                     device, engine):
-    """GPU objective of the joint drivers: loss_grad(x), the lossy line search and the lossy product at the point of the last
-    loss_grad call, on (2, Ny, Nx) float64 torch models."""
+def _gpu_callables(lossy, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices, dtype, bde,
+                   stencil, device, engine):
+    """GPU objective of the drivers on float64 torch models, (Ny, Nx) slowness maps or, ``lossy``, (2, Ny, Nx) = [s, kappa]:
+    loss_grad(x), and the line search and the Gauss-Newton product at the point of the last loss_grad call."""
     import torch
     freqs = np.atleast_1d(np.asarray(_to_np(f), dtype=np.float64)).ravel()
     dv = torch.device(f"cuda:{device}")
@@ -611,19 +599,21 @@ def _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
     fargs = (xi, yi, rec, SRC, freqs, a0, L_PML, tx_include, ind_matlab, mask_indices, numElements)
     kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine)
 
+    # the module functions are looked up at call time: tests record the evaluation points by replacing them
     def loss_grad(x):
         state["x"] = x.to(dv, real).contiguous()
-        loss, grad = fwi_joint_loss_function(state["x"], *fargs, **kw)
+        loss, grad = (fwi_joint_loss_function if lossy else fwi_loss_function)(state["x"], *fargs, **kw)
         return float(loss), grad
 
     def linesearch(sd):
         plan, _ = _fwi_plan(xi, yi, rec, SRC, freqs, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine)
         sdt = sd.to(dv, real)
-        nd = plan.ncg_linesearch_lossy(sdt[0].contiguous(), sdt[1].contiguous())
+        nd = plan._linesearch(*((sdt[0].contiguous(), sdt[1].contiguous()) if lossy else (sdt.contiguous(), None)))
         return float(nd[0]), float(nd[1])
 
     def hvp(v):
-        return fwi_joint_gauss_newton_product(state["x"], v.to(dv, real).contiguous(), *fargs, **kw)
+        product = fwi_joint_gauss_newton_product if lossy else fwi_gauss_newton_product
+        return product(state["x"], v.to(dv, real).contiguous(), *fargs, **kw)
 
     return loss_grad, linesearch, hvp
 
@@ -648,8 +638,8 @@ def nonlinear_conjugate_gradient_joint(xi, yi, numElements, REC_DATA, SRC, tx_in
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or linesearch is None:
-        loss_grad, linesearch, _ = _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
-                                                    mask_indices, dtype, bde, stencil, device, engine)
+        loss_grad, linesearch, _ = _gpu_callables(True, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
+                                                  mask_indices, dtype, bde, stencil, device, engine)
     x, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
     dot = lambda a, b: float(torch.sum(a * b))
     d = gprev = None
@@ -697,8 +687,8 @@ def gauss_newton_joint_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or hvp is None:
-        loss_grad, _, hvp = _joint_callables(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices,
-                                             dtype, bde, stencil, device, engine)
+        loss_grad, _, hvp = _gpu_callables(True, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
+                                           mask_indices, dtype, bde, stencil, device, engine)
     x0, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
     x = _gauss_newton_loop(x0, loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history, slow_of=lambda x: x[0],
                            scale=D, project=_project_kappa)
@@ -808,11 +798,25 @@ def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
     """
     if method not in ("ncg", "gn"):
         raise ValueError("method must be 'ncg' or 'gn'")
+
+    def stage(vel, rec, f, h):
+        if method == "gn":
+            return gauss_newton_fwi(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML, mask_indices,
+                                    dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+        return nonlinear_conjugate_gradient(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML,
+                                            mask_indices, dtype=dtype, stencil=stencil, device=device, history=h,
+                                            return_fields=False, engine=engine)[0]
+
+    return _continuation(REC_DATA, f, stages, history, c_init, stage)
+
+
+def _continuation(REC_DATA, f, stages, history, model, stage):
+    """The stage loop of the continuation drivers: ``model = stage(model, REC_DATA[idx], f[idx], h)`` for every stage ``idx``,
+    with ``h`` the stage's history list (None without ``history``).  Returns the final model."""
     f = np.asarray(_to_np(f), dtype=np.float64).ravel()
     rec = _to_np(REC_DATA)
     if rec.ndim != 3 or rec.shape[0] != f.size:
         raise ValueError("REC_DATA must be (Nf, Nt, E) with Nf == len(f)")
-    vel = c_init
     prev = None
     for st in stages:
         idx = np.asarray(st, dtype=np.int64).ravel()
@@ -820,16 +824,10 @@ def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
             clear_plans()  # a plan is sized for its number of frequencies; do not keep two factor stores alive
         prev = idx.size
         h = [] if history is not None else None
-        if method == "gn":
-            vel = gauss_newton_fwi(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter, a0, L_PML,
-                                   mask_indices, dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
-        else:
-            vel, _, _, _, _ = nonlinear_conjugate_gradient(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter,
-                                                           a0, L_PML, mask_indices, dtype=dtype, stencil=stencil, device=device,
-                                                           history=h, return_fields=False, engine=engine)
+        model = stage(model, rec[idx], f[idx], h)
         if history is not None:
             history.append(h)
-    return vel
+    return model
 
 
 def joint_frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, stages, Niter, a0, L_PML,
@@ -843,25 +841,14 @@ def joint_frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include,
     """
     if method not in ("ncg", "gn", "lbfgs"):
         raise ValueError("method must be 'ncg', 'gn' or 'lbfgs'")
-    f = np.asarray(_to_np(f), dtype=np.float64).ravel()
-    rec = _to_np(REC_DATA)
-    if rec.ndim != 3 or rec.shape[0] != f.size:
-        raise ValueError("REC_DATA must be (Nf, Nt, E) with Nf == len(f)")
-    vel, kap = c_init, kappa_init
-    prev = None
-    for st in stages:
-        idx = np.asarray(st, dtype=np.int64).ravel()
-        if prev is not None and prev != idx.size:
-            clear_plans()  # a plan is sized for its number of frequencies; do not keep two factor stores alive
-        prev = idx.size
-        h = [] if history is not None else None
+
+    def stage(model, rec, f, h):
+        vel, kap = model
         if method == "lbfgs":
-            vel, kap = run_lbfgs_joint_fwi(xi, yi, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], a0, L_PML, mask_indices,
-                                           kappa_init=kap, maxiter=Niter, dtype=dtype, stencil=stencil, engine=engine, history=h)
-        else:
-            drv = gauss_newton_joint_fwi if method == "gn" else nonlinear_conjugate_gradient_joint
-            vel, kap = drv(xi, yi, numElements, rec[idx], SRC, tx_include, ind_matlab, vel, f[idx], Niter, a0, L_PML, mask_indices,
-                           kappa_init=kap, dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
-        if history is not None:
-            history.append(h)
-    return vel, kap
+            return run_lbfgs_joint_fwi(xi, yi, rec, SRC, tx_include, ind_matlab, vel, f, a0, L_PML, mask_indices, kappa_init=kap,
+                                       maxiter=Niter, dtype=dtype, stencil=stencil, engine=engine, history=h)
+        drv = gauss_newton_joint_fwi if method == "gn" else nonlinear_conjugate_gradient_joint
+        return drv(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML, mask_indices, kappa_init=kap,
+                   dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+
+    return _continuation(REC_DATA, f, stages, history, (c_init, kappa_init), stage)

@@ -84,12 +84,12 @@ struct ust_plan {
     void *kappa_in = nullptr, *grad_kappa_out = nullptr;       // lossy evaluation: attenuation slowness, its gradient
     void *kappa_h2d = nullptr, *grad_kappa_d2h = nullptr;      // staging of ust_fwi_loss_grad_lossy_host
     void *vk_in = nullptr, *hv_kappa_out = nullptr;  // lossy line search / product: kappa part of the direction, of H_GN v
-    bool fwi_done = false;
-    // the factors and fields are those of a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy): the line search and the
-    // Gauss-Newton product, whose virtual source assumes a real slowness, refuse until a lossless ust_fwi_loss_grad
-    bool lossy = false;
-    bool gn_ok = false;  // the factors, fields and source estimates are those of the last ust_fwi_loss_grad (ust_fwi_gn_hvp)
-    bool gn_lossy_ok = false;  // ... of the last ust_fwi_loss_grad_lossy (ust_ncg_linesearch_lossy, ust_fwi_gn_hvp_lossy)
+    // the last evaluation (ust_fwi_loss_grad[_lossy]), whose forward fields, source estimates and inputs the line search
+    // and the Gauss-Newton product reuse (check_eval)
+    enum EvalKind { EVAL_NONE, EVAL_LOSSLESS, EVAL_LOSSY };
+    EvalKind eval_kind = EVAL_NONE;  // cleared by ust_plan_set_acquisition
+    bool factored_since_eval = false;  // factor_impl ran after it: the factors no longer belong to its fields
+    bool factors_lossy = false;        // the current factors are those of a lossy model
     bool use_graphs = true;  // UST_NO_GRAPHS=1 disables
     struct GraphEntry { cudaGraphExec_t exec = nullptr; long long launches = 0; };
     std::map<long long, GraphEntry> graphs;
@@ -484,9 +484,9 @@ static int factor_enqueue(ust_plan* p, const void* vel_dev, int nfreq, bool has_
 template <typename R>
 static int factor_impl(ust_plan* p, const void* vel_dev, int nfreq, const double* freqs, const double* bde, cudaStream_t st,
                        const void* kappa_dev = nullptr) {
-    p->gn_ok = p->gn_lossy_ok = false;  // the factors no longer belong to the forward fields of the last evaluation
+    p->factored_since_eval = true;
+    p->factors_lossy = kappa_dev != nullptr;
     UST_TRY(upload_params(p, nfreq, freqs, bde, st));
-    if (kappa_dev) p->lossy = true;
     return factor_enqueue<R>(p, vel_dev, nfreq, bde != nullptr, st, kappa_dev);
 }
 
@@ -664,7 +664,7 @@ __global__ void recip_kernel(const R* __restrict__ in, R* __restrict__ out, long
 // adjoint sweeps as its own chain; the groups meet again at the gradient, which sums over all frequencies.
 // lossy: also reads p->kappa_in (sigma^2 assembly) and writes p->grad_kappa_out; everything between assembly and gradient is the same.
 template <typename R>
-static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bool lossy = false) {
+static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bool lossy) {
     const Geom& g = p->g;
     const int nt = p->nt;
     const size_t stride = (size_t)g.N * nt;
@@ -738,7 +738,7 @@ static int pert_rhs_groups(ust_plan* p, const std::vector<Group>& gs, const void
 // perturbation solve + line-search scalars, device work only: reads p->sd_in (lossy: also p->kappa_in and p->vk_in), writes
 // p->d_scal[2..3]
 template <typename R>
-static int linesearch_enqueue(ust_plan* p, cudaStream_t st, bool lossy = false) {
+static int linesearch_enqueue(ust_plan* p, cudaStream_t st, bool lossy) {
     const Geom& g = p->g;
     const int nt = p->nt, nfreq = p->nfreq_cur;
     const size_t stride = (size_t)g.N * nt;
@@ -768,7 +768,7 @@ static int linesearch_enqueue(ust_plan* p, cudaStream_t st, bool lossy = false) 
 // lossy: the complex-slowness RHS from v = [p->v_in, p->vk_in], and gradient_kernel<R, true> on p->slow_in / p->kappa_in writes
 // both halves of J^H (J v): p->hv_out and p->hv_kappa_out.
 template <typename R>
-static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st, bool lossy = false) {
+static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st, bool lossy) {
     const Geom& g = p->g;
     const int nt = p->nt, nfreq = p->nfreq_cur;
     const size_t stride = (size_t)g.N * nt;
@@ -869,101 +869,71 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     // lossless evaluation 0/1, line search 500, Gauss-Newton product 600, lossy evaluation 700/701, lossy line search 800,
     // lossy Gauss-Newton product 900
     const long long key = 1000LL * nfreq + (lossy ? 700 : 0) + (has_bde ? 1 : 0);
-    p->gn_ok = p->gn_lossy_ok = false;
+    p->factored_since_eval = true;  // until this evaluation completes, the factors belong to no evaluation
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_, lossy); }));
     p->nfreq_cur = nfreq;
     p->factored = true;
     UST_CUDA(cudaMemcpyAsync(loss_dev, p->d_scal, sizeof(double), cudaMemcpyDeviceToDevice, st));
     UST_CUDA(cudaMemcpyAsync(grad_dev, p->grad_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(grad_kappa_dev, p->grad_kappa_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    p->fwi_done = true;
-    p->lossy = lossy;
-    p->gn_ok = !lossy;
-    p->gn_lossy_ok = lossy;
+    p->eval_kind = lossy ? ust_plan::EVAL_LOSSY : ust_plan::EVAL_LOSSLESS;
+    p->factored_since_eval = false;
+    p->factors_lossy = lossy;
     if (p->trace) return dump_update_trace(p, st);
     return 0;
 }
 
-template <typename R>
-static int linesearch_impl(ust_plan* p, const void* sd, double* out2, cudaStream_t st) {
-    const Geom& g = p->g;
-    if (!p->factored || !p->fwi_done) { set_error("ust_ncg_linesearch: call ust_fwi_loss_grad first"); return 1; }
-    if (p->lossy) {
-        set_error("ust_ncg_linesearch: the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy) and the line search "
-                  "assumes a real slowness; call ust_fwi_loss_grad first");
+// The line search and the Gauss-Newton product run on the factors, forward fields, source estimates and inputs of the last
+// evaluation: only when it was of their own kind (the lossless entry points' virtual source assumes a real slowness) and no
+// factorisation has replaced its factors since.
+static int check_eval(const ust_plan* p, const char* name, bool lossy) {
+    const std::string n(name);
+    const char* want = lossy ? "ust_fwi_loss_grad_lossy" : "ust_fwi_loss_grad";
+    if (!p->U) { set_error(n + ": plan was created with fwi_buffers=0"); return 1; }
+    if (!p->factored || p->eval_kind == ust_plan::EVAL_NONE) { set_error(n + ": call " + want + " first"); return 1; }
+    const bool last_lossy = p->eval_kind == ust_plan::EVAL_LOSSY;
+    if (p->factored_since_eval) {
+        set_error(n + ": the factors were replaced (" + (p->factors_lossy ? "ust_factor_lossy" : "ust_factor / ust_solve_helmholtz_host") +
+                  ") after the last " + (last_lossy ? "ust_fwi_loss_grad_lossy" : "ust_fwi_loss_grad") + "; call " + want + " again");
         return 1;
     }
-    UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + 500;
-    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_); }));
+    if (last_lossy != lossy) {
+        set_error(n + (lossy ? ": the last evaluation was lossless (ust_fwi_loss_grad); use the lossless entry point or call "
+                               "ust_fwi_loss_grad_lossy first"
+                             : ": the last evaluation was lossy (ust_fwi_loss_grad_lossy) and this entry point assumes a real "
+                               "slowness; use the lossy entry point or call ust_fwi_loss_grad first"));
+        return 1;
+    }
+    return 0;
+}
+
+// sd_kappa != nullptr: the line search of the joint direction [sd, sd_kappa] on a lossy evaluation (ust_ncg_linesearch_lossy)
+template <typename R>
+static int linesearch_impl(ust_plan* p, const void* sd, const void* sd_kappa, double* out2, cudaStream_t st) {
+    const bool lossy = sd_kappa != nullptr;
+    UST_TRY(check_eval(p, lossy ? "ust_ncg_linesearch_lossy" : "ust_ncg_linesearch", lossy));
+    const size_t bytes = p->g.N * sizeof(R);
+    UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, bytes, cudaMemcpyDeviceToDevice, st));
+    if (lossy) UST_CUDA(cudaMemcpyAsync(p->vk_in, sd_kappa, bytes, cudaMemcpyDeviceToDevice, st));
+    const long long key = 1000LL * p->nfreq_cur + (lossy ? 800 : 500);
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_, lossy); }));
     UST_CUDA(cudaMemcpyAsync(out2, p->d_scal + 2, 2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
     return 0;
 }
 
+// v_kappa != nullptr: the joint product of [v, v_kappa] on a lossy evaluation, its kappa half into hv_kappa (ust_fwi_gn_hvp_lossy)
 template <typename R>
-static int gn_hvp_impl(ust_plan* p, const void* v, void* hv, double* jv2, void* jv, cudaStream_t st) {
-    const Geom& g = p->g;
-    if (!p->v_in) { set_error("ust_fwi_gn_hvp: plan was created with fwi_buffers=0"); return 1; }
-    if (!p->factored || !p->fwi_done) { set_error("ust_fwi_gn_hvp: call ust_fwi_loss_grad first"); return 1; }
-    if (p->lossy) {
-        set_error("ust_fwi_gn_hvp: the plan holds a lossy model (ust_factor_lossy / ust_fwi_loss_grad_lossy) and the product "
-                  "assumes a real slowness; call ust_fwi_loss_grad first");
-        return 1;
-    }
-    if (!p->gn_ok) {
-        set_error("ust_fwi_gn_hvp: the factors were replaced (ust_factor / ust_solve_helmholtz_host) after the last ust_fwi_loss_grad; "
-                  "call ust_fwi_loss_grad again");
-        return 1;
-    }
-    UST_CUDA(cudaMemcpyAsync(p->v_in, v, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + 600;
-    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_); }));
-    UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    UST_CUDA(cudaMemcpyAsync(jv2, p->d_scal + 6, sizeof(double), cudaMemcpyDeviceToDevice, st));
-    if (jv) UST_CUDA(cudaMemcpyAsync(jv, p->drec, (size_t)p->nfreq_cur * p->nt * p->nm * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
-    return 0;
-}
-
-// lossy twins of linesearch_impl / gn_hvp_impl: valid only on the state of the last ust_fwi_loss_grad_lossy
-static int check_lossy_state(ust_plan* p, const char* name) {
-    if (!p->vk_in) { set_error(std::string(name) + ": plan was created with fwi_buffers=0"); return 1; }
-    if (!p->factored || !p->fwi_done) { set_error(std::string(name) + ": call ust_fwi_loss_grad_lossy first"); return 1; }
-    if (!p->lossy) {
-        set_error(std::string(name) + ": the last evaluation was lossless (ust_fwi_loss_grad); use the lossless entry point or call "
-                  "ust_fwi_loss_grad_lossy first");
-        return 1;
-    }
-    if (!p->gn_lossy_ok) {
-        set_error(std::string(name) + ": the factors were replaced (ust_factor / ust_factor_lossy / ust_solve_helmholtz_host) after the "
-                  "last ust_fwi_loss_grad_lossy; call ust_fwi_loss_grad_lossy again");
-        return 1;
-    }
-    return 0;
-}
-
-template <typename R>
-static int linesearch_lossy_impl(ust_plan* p, const void* sd, const void* sd_kappa, double* out2, cudaStream_t st) {
-    const Geom& g = p->g;
-    UST_TRY(check_lossy_state(p, "ust_ncg_linesearch_lossy"));
-    UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    UST_CUDA(cudaMemcpyAsync(p->vk_in, sd_kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + 800;
-    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_, true); }));
-    UST_CUDA(cudaMemcpyAsync(out2, p->d_scal + 2, 2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
-    return 0;
-}
-
-template <typename R>
-static int gn_hvp_lossy_impl(ust_plan* p, const void* v, const void* v_kappa, void* hv, void* hv_kappa, double* jv2, void* jv,
-                             cudaStream_t st) {
-    const Geom& g = p->g;
-    UST_TRY(check_lossy_state(p, "ust_fwi_gn_hvp_lossy"));
-    UST_CUDA(cudaMemcpyAsync(p->v_in, v, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    UST_CUDA(cudaMemcpyAsync(p->vk_in, v_kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + 900;
-    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_, true); }));
-    UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
-    UST_CUDA(cudaMemcpyAsync(hv_kappa, p->hv_kappa_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
+static int gn_hvp_impl(ust_plan* p, const void* v, const void* v_kappa, void* hv, void* hv_kappa, double* jv2, void* jv,
+                       cudaStream_t st) {
+    const bool lossy = v_kappa != nullptr;
+    UST_TRY(check_eval(p, lossy ? "ust_fwi_gn_hvp_lossy" : "ust_fwi_gn_hvp", lossy));
+    const size_t bytes = p->g.N * sizeof(R);
+    UST_CUDA(cudaMemcpyAsync(p->v_in, v, bytes, cudaMemcpyDeviceToDevice, st));
+    if (lossy) UST_CUDA(cudaMemcpyAsync(p->vk_in, v_kappa, bytes, cudaMemcpyDeviceToDevice, st));
+    const long long key = 1000LL * p->nfreq_cur + (lossy ? 900 : 600);
+    UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_, lossy); }));
+    UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, bytes, cudaMemcpyDeviceToDevice, st));
+    if (lossy) UST_CUDA(cudaMemcpyAsync(hv_kappa, p->hv_kappa_out, bytes, cudaMemcpyDeviceToDevice, st));
     UST_CUDA(cudaMemcpyAsync(jv2, p->d_scal + 6, sizeof(double), cudaMemcpyDeviceToDevice, st));
     if (jv) UST_CUDA(cudaMemcpyAsync(jv, p->drec, (size_t)p->nfreq_cur * p->nt * p->nm * sizeof(cx<R>), cudaMemcpyDeviceToDevice, st));
     return 0;
@@ -1299,8 +1269,7 @@ int ust_plan_set_acquisition(ust_plan* p, int nt, const int32_t* src_lin, int ne
     UST_CUDA(cudaSetDevice(p->d.device));
     UST_CUDA(cudaDeviceSynchronize());
     drop_graphs(p);
-    p->fwi_done = false;
-    p->gn_ok = p->gn_lossy_ok = false;
+    p->eval_kind = ust_plan::EVAL_NONE;
     for (int** q : {&p->src_lin, &p->rx_lin, &p->mask})
         if (*q) { cudaFree(*q); *q = nullptr; }
     if (p->rec_in) { cudaFree(p->rec_in); p->rec_in = nullptr; }
@@ -1447,14 +1416,14 @@ int ust_ncg_linesearch(ust_plan* p, const void* sd_dev, double* out2_dev, void* 
     UST_TRY(check_plan(p));
     if (!sd_dev || !out2_dev) { set_error("ust_ncg_linesearch: null argument"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
-    return DISPATCH(p, linesearch_impl, p, sd_dev, out2_dev, (cudaStream_t)stream);
+    return DISPATCH(p, linesearch_impl, p, sd_dev, nullptr, out2_dev, (cudaStream_t)stream);
 }
 
 int ust_fwi_gn_hvp(ust_plan* p, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream) {
     UST_TRY(check_plan(p));
     if (!v_dev || !hv_dev || !jv2_dev) { set_error("ust_fwi_gn_hvp: null argument"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
-    return DISPATCH(p, gn_hvp_impl, p, v_dev, hv_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
+    return DISPATCH(p, gn_hvp_impl, p, v_dev, nullptr, hv_dev, nullptr, jv2_dev, jv_dev, (cudaStream_t)stream);
 }
 
 int ust_ncg_linesearch_lossy(ust_plan* p, const void* sd_s_dev, const void* sd_kappa_dev, double* out2_dev, void* stream) {
@@ -1464,7 +1433,7 @@ int ust_ncg_linesearch_lossy(ust_plan* p, const void* sd_s_dev, const void* sd_k
         return 1;
     }
     UST_CUDA(cudaSetDevice(p->d.device));
-    return DISPATCH(p, linesearch_lossy_impl, p, sd_s_dev, sd_kappa_dev, out2_dev, (cudaStream_t)stream);
+    return DISPATCH(p, linesearch_impl, p, sd_s_dev, sd_kappa_dev, out2_dev, (cudaStream_t)stream);
 }
 
 int ust_fwi_gn_hvp_lossy(ust_plan* p, const void* v_s_dev, const void* v_kappa_dev, void* hv_s_dev, void* hv_kappa_dev,
@@ -1475,7 +1444,7 @@ int ust_fwi_gn_hvp_lossy(ust_plan* p, const void* v_s_dev, const void* v_kappa_d
         return 1;
     }
     UST_CUDA(cudaSetDevice(p->d.device));
-    return DISPATCH(p, gn_hvp_lossy_impl, p, v_s_dev, v_kappa_dev, hv_s_dev, hv_kappa_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
+    return DISPATCH(p, gn_hvp_impl, p, v_s_dev, v_kappa_dev, hv_s_dev, hv_kappa_dev, jv2_dev, jv_dev, (cudaStream_t)stream);
 }
 
 int ust_get_bde(ust_plan* p, double* out) {
@@ -1506,7 +1475,7 @@ int ust_get_src_est(ust_plan* p, int ifreq, void* out_host) {
 
 int ust_residual_onehot(ust_plan* p, int ifreq, int t, double* out2_host) {
     UST_TRY(check_plan(p));
-    if (!p->fwi_done || !p->U) { set_error("ust_residual_onehot: call ust_fwi_loss_grad first"); return 1; }
+    if (p->eval_kind == ust_plan::EVAL_NONE || !p->U) { set_error("ust_residual_onehot: call ust_fwi_loss_grad first"); return 1; }
     if (ifreq < 0 || ifreq >= p->nfreq_cur || t < 0 || t >= p->nt || !out2_host) { set_error("ust_residual_onehot: bad arguments"); return 1; }
     UST_CUDA(cudaSetDevice(p->d.device));
     UST_CUDA(cudaDeviceSynchronize());

@@ -93,54 +93,44 @@ class ShardedFWI:
         self._rec_dev = torch.empty((max(len(self.local), 1), max(len(self.local_tx), 1), geom.num_elements),
                                     dtype=self.plan.tcplx, device=dv)
 
+    def _allreduced(self, evaluate, like, blocks):
+        """``evaluate() -> (scalar (1-element float64 tensor), result)`` on a rank that owns frequencies and transmitters,
+        zeros of ``like``'s shape (``blocks`` > 1: ``(blocks,) + like.shape``) on one that does not, then one all-reduce of
+        the packed ``[result, scalar]``.  Returns ``(scalar (0-d float64 tensor), result)``."""
+        torch = self.torch
+        if len(self.local) and len(self.local_tx):
+            scalar, result = evaluate()
+            scalar = scalar[0]
+        else:
+            scalar = torch.zeros((), dtype=torch.float64, device=like.device)
+            result = torch.zeros(((blocks,) if blocks > 1 else ()) + tuple(like.shape), dtype=like.dtype, device=like.device)
+        return allreduce_loss_grad(scalar, result, self.group)
+
     def loss_grad_device(self, slow_dev, rec_local_dev, bde=None):
         """Inputs already resident in HBM.  Returns all-reduced (loss (0-d float64 tensor), grad)."""
-        if len(self.local) and len(self.local_tx):
-            loss, grad = self.plan.fwi_loss_grad(slow_dev, rec_local_dev, self.local_freqs, bde=bde)
-            loss = loss[0]
-        else:
-            loss = self.torch.zeros((), dtype=self.torch.float64, device=slow_dev.device)
-            grad = self.torch.zeros_like(slow_dev)
-        return allreduce_loss_grad(loss, grad, self.group)
+        return self._allreduced(lambda: self.plan.fwi_loss_grad(slow_dev, rec_local_dev, self.local_freqs, bde=bde), slow_dev, 1)
 
     def gn_hvp_device(self, v_dev):
         """Gauss-Newton product of the joint objective at the point of the last ``loss_grad_device``: this rank's part
         (``HelmholtzPlan.gn_hvp``: its frequencies or its transmitters) and one all-reduce of the packed ``[hv, jv2]``.
         Returns ``(hv, jv2)`` with ``jv2 = sum |J v|^2`` (0-d float64 tensor)."""
-        if len(self.local) and len(self.local_tx):
-            hv, jv2 = self.plan.gn_hvp(v_dev)
-            jv2 = jv2[0]
-        else:
-            jv2 = self.torch.zeros((), dtype=self.torch.float64, device=v_dev.device)
-            hv = self.torch.zeros_like(v_dev)
-        jv2, hv = allreduce_loss_grad(jv2, hv, self.group)
+        jv2, hv = self._allreduced(lambda: self.plan.gn_hvp(v_dev)[::-1], v_dev, 1)
         return hv, jv2
 
     def loss_grad_lossy_device(self, slow_dev, kappa_dev, rec_local_dev, bde=None):
         """Joint sound-speed and attenuation evaluation (``HelmholtzPlan.fwi_loss_grad_lossy``) of this rank's frequencies or
         transmitters, and one all-reduce of the packed ``[grad_s, grad_kappa, loss]``.  Returns (loss (0-d float64 tensor),
         grad (2, Ny, Nx) = [grad_s, grad_kappa])."""
-        torch = self.torch
-        if len(self.local) and len(self.local_tx):
+        def evaluate():
             loss, gs, gk = self.plan.fwi_loss_grad_lossy(slow_dev, kappa_dev, rec_local_dev, self.local_freqs, bde=bde)
-            loss, grad = loss[0], torch.stack([gs, gk])
-        else:
-            loss = torch.zeros((), dtype=torch.float64, device=slow_dev.device)
-            grad = torch.zeros((2,) + tuple(slow_dev.shape), dtype=slow_dev.dtype, device=slow_dev.device)
-        return allreduce_loss_grad(loss, grad, self.group)
+            return loss, self.torch.stack([gs, gk])
+        return self._allreduced(evaluate, slow_dev, 2)
 
     def gn_hvp_lossy_device(self, v_s_dev, v_k_dev):
         """Joint Gauss-Newton product at the point of the last ``loss_grad_lossy_device``: this rank's part
         (``HelmholtzPlan.gn_hvp_lossy``: its frequencies or its transmitters) and one all-reduce of the packed
         ``[hv_s, hv_kappa, jv2]``.  Returns ``(hv (2, Ny, Nx), jv2 (0-d float64 tensor))``."""
-        torch = self.torch
-        if len(self.local) and len(self.local_tx):
-            hv, jv2 = self.plan.gn_hvp_lossy(v_s_dev, v_k_dev)
-            jv2 = jv2[0]
-        else:
-            jv2 = torch.zeros((), dtype=torch.float64, device=v_s_dev.device)
-            hv = torch.zeros((2,) + tuple(v_s_dev.shape), dtype=v_s_dev.dtype, device=v_s_dev.device)
-        jv2, hv = allreduce_loss_grad(jv2, hv, self.group)
+        jv2, hv = self._allreduced(lambda: self.plan.gn_hvp_lossy(v_s_dev, v_k_dev)[::-1], v_s_dev, 2)
         return hv, jv2
 
     def local_rec(self, rec_all):
@@ -178,22 +168,41 @@ class ShardedFWI:
         self.plan.close()
 
 
+def _engine_callables(eng, rec_local_dev, lossy):
+    """The objective of the ``api`` drivers on a sharded engine, on (Ny, Nx) slowness maps or, ``lossy``, (2, Ny, Nx) =
+    [s, kappa] models: ``loss_grad(x)`` and ``hvp(v)`` (at the point of the last ``loss_grad``) on float64 torch tensors, and
+    ``loss_grad_np(x)`` on NumPy arrays for the L-BFGS drivers."""
+    import torch
+    plan = eng.plan
+    dv = torch.device(f"cuda:{eng.device}")
+
+    def split(x):
+        x = x.to(dv, plan.treal)
+        return (x[0].contiguous(), x[1].contiguous()) if lossy else (x.contiguous(),)
+
+    def loss_grad(x):
+        loss, grad = (eng.loss_grad_lossy_device if lossy else eng.loss_grad_device)(*split(x), rec_local_dev)
+        return float(loss), grad
+
+    def hvp(v):
+        return (eng.gn_hvp_lossy_device if lossy else eng.gn_hvp_device)(*split(v))[0]
+
+    def loss_grad_np(x):
+        loss, grad = loss_grad(torch.as_tensor(np.ascontiguousarray(x.astype(plan.real))))
+        return loss, grad.to(torch.float64).cpu().numpy()
+
+    return loss_grad, hvp, loss_grad_np
+
+
 def run_lbfgs_sharded(eng, rec_local_dev, c_init, maxiter=1, tol=1e-5, history_size=10, history=None, pert_scale=1e-2):
     """``run_lbfgs_fwi`` (``fwi_loss_function.py:106-132``) on a sharded engine -- BASELINE configs[4]: multi-frequency L-BFGS on
     several GPUs.  Every rank runs the same L-BFGS driver (``api.run_lbfgs_fwi``) on the all-reduced joint (loss, grad), which
     NCCL delivers bit-identically to all ranks, so the ranks take identical steps without any further exchange.
     ``rec_local_dev``: this rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound
     speed (Ny, Nx) as a NumPy array (identical on every rank)."""
-    import torch
     from . import api
     geom, plan = eng.geom, eng.plan
-    dv = torch.device(f"cuda:{eng.device}")
-
-    def loss_grad(slow):
-        s = torch.as_tensor(np.ascontiguousarray(slow.astype(plan.real))).to(dv)
-        loss, grad = eng.loss_grad_device(s, rec_local_dev)
-        return float(loss), grad.to(torch.float64).cpu().numpy()
-
+    loss_grad = _engine_callables(eng, rec_local_dev, False)[2]
     return api.run_lbfgs_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0, geom.L_PML,
                              geom.mask_indices, maxiter=maxiter, tol=tol, history_size=history_size, dtype=plan.dtype,
                              history=history, loss_grad=loss_grad, pert_scale=pert_scale)
@@ -203,18 +212,9 @@ def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_t
     """``api.gauss_newton_fwi`` on a sharded engine: every rank runs the same driver on the all-reduced (loss, grad) and
     products, which NCCL delivers bit-identically to all ranks, so the ranks take identical steps.  ``rec_local_dev``: this
     rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound speed (Ny, Nx)."""
-    import torch
     from . import api
     geom, plan = eng.geom, eng.plan
-    dv = torch.device(f"cuda:{eng.device}")
-
-    def loss_grad(slow):
-        loss, grad = eng.loss_grad_device(slow.to(dv, plan.treal).contiguous(), rec_local_dev)
-        return float(loss), grad
-
-    def hvp(v):
-        return eng.gn_hvp_device(v.to(dv, plan.treal).contiguous())[0]
-
+    loss_grad, hvp, _ = _engine_callables(eng, rec_local_dev, False)
     return api.gauss_newton_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs,
                                 Niter, geom.a0, geom.L_PML, geom.mask_indices, cg_iters=cg_iters, cg_tol=cg_tol, damping=damping,
                                 max_backtracks=max_backtracks, dtype=plan.dtype, device=eng.device, history=history,
@@ -226,16 +226,9 @@ def run_lbfgs_joint_sharded(eng, rec_local_dev, c_init, kappa_init=0.0, kappa_sc
     """``api.run_lbfgs_joint_fwi`` on a sharded engine: every rank runs the same joint L-BFGS driver on the all-reduced
     ``(loss, [grad_s, grad_kappa])`` of ``ShardedFWI.loss_grad_lossy_device``, so the ranks take identical steps.  Returns
     ``(c, kappa)`` (Ny, Nx) NumPy arrays (identical on every rank)."""
-    import torch
     from . import api
     geom, plan = eng.geom, eng.plan
-    dv = torch.device(f"cuda:{eng.device}")
-
-    def loss_grad(params):
-        p = torch.as_tensor(np.ascontiguousarray(params.astype(plan.real))).to(dv)
-        loss, grad = eng.loss_grad_lossy_device(p[0].contiguous(), p[1].contiguous(), rec_local_dev)
-        return float(loss), grad.to(torch.float64).cpu().numpy()
-
+    loss_grad = _engine_callables(eng, rec_local_dev, True)[2]
     return api.run_lbfgs_joint_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0,
                                    geom.L_PML, geom.mask_indices, kappa_init=kappa_init, kappa_scale=kappa_scale, maxiter=maxiter,
                                    tol=tol, history_size=history_size, dtype=plan.dtype, history=history, loss_grad=loss_grad,
@@ -247,20 +240,9 @@ def run_gauss_newton_joint_sharded(eng, rec_local_dev, c_init, Niter, kappa_init
     """``api.gauss_newton_joint_fwi`` on a sharded engine: every rank runs the same joint driver on the all-reduced
     ``loss_grad_lossy_device`` and ``gn_hvp_lossy_device``, so the ranks take identical steps.  Returns ``(c, kappa)`` (Ny, Nx)
     NumPy arrays (identical on every rank)."""
-    import torch
     from . import api
     geom, plan = eng.geom, eng.plan
-    dv = torch.device(f"cuda:{eng.device}")
-
-    def loss_grad(x):
-        x = x.to(dv, plan.treal)
-        loss, grad = eng.loss_grad_lossy_device(x[0].contiguous(), x[1].contiguous(), rec_local_dev)
-        return float(loss), grad
-
-    def hvp(v):
-        v = v.to(dv, plan.treal)
-        return eng.gn_hvp_lossy_device(v[0].contiguous(), v[1].contiguous())[0]
-
+    loss_grad, hvp, _ = _engine_callables(eng, rec_local_dev, True)
     return api.gauss_newton_joint_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init,
                                       eng.freqs, Niter, geom.a0, geom.L_PML, geom.mask_indices, kappa_init=kappa_init,
                                       kappa_scale=kappa_scale, pert_scale=pert_scale, cg_iters=cg_iters, cg_tol=cg_tol,

@@ -25,6 +25,10 @@ def _pi(a):
     return a.ctypes.data_as(C.POINTER(C.c_int32))
 
 
+def _ptr(t):
+    return C.c_void_p(t.data_ptr())
+
+
 def _torch():
     import torch
     return torch
@@ -149,94 +153,88 @@ class HelmholtzPlan:
                                     _stream_ptr(self.device)), "ust_solve")
         return rhs
 
+    def _evaluated(self, nfreq):
+        self.nfreq = nfreq
+        self._factor_key = None  # the plan now holds the factors of this evaluation, not api.solve_helmholtz's
+        self._eval_key = None  # api.fwi_loss_function records its inputs after this call
+
+    def _freqs_bde(self, freqs, bde):
+        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
+        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
+        return fr, b
+
+    def _loss_grad(self, slow, kappa, rec, freqs, bde):
+        """(loss, grad) on device tensors, or (loss, grad_s, grad_kappa) of the lossy medium when ``kappa`` is given."""
+        torch = _torch()
+        fr, b = self._freqs_bde(freqs, bde)
+        maps = [slow] if kappa is None else [slow, kappa]
+        for t in maps:
+            self._check_tensor(t, self.treal, self.nx * self.ny)
+        self._check_tensor(rec, self.tcplx, fr.size * self.nt * self.nelem)
+        loss = torch.empty(1, dtype=torch.float64, device=slow.device)
+        grads = [torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device) for _ in maps]
+        name = "ust_fwi_loss_grad" if kappa is None else "ust_fwi_loss_grad_lossy"
+        _lib.check(getattr(self.L, name)(self.h, *map(_ptr, maps), _ptr(rec), fr.size, _pd(fr), _pd(b), _ptr(loss),
+                                         *map(_ptr, grads), _stream_ptr(self.device)), name)
+        self._evaluated(fr.size)
+        return (loss, *grads)
+
     def fwi_loss_grad(self, slow, rec, freqs, bde=None):
         """Fused (loss, grad) on device tensors.  slow (ny,nx) real; rec (nfreq, nt, nelem) complex."""
-        torch = _torch()
-        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
-        self._check_tensor(slow, self.treal, self.nx * self.ny)
-        self._check_tensor(rec, self.tcplx, fr.size * self.nt * self.nelem)
-        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
-        loss = torch.empty(1, dtype=torch.float64, device=slow.device)
-        grad = torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device)
-        _lib.check(self.L.ust_fwi_loss_grad(self.h, C.c_void_p(slow.data_ptr()), C.c_void_p(rec.data_ptr()), fr.size,
-                                            _pd(fr), _pd(b), C.c_void_p(loss.data_ptr()), C.c_void_p(grad.data_ptr()),
-                                            _stream_ptr(self.device)), "ust_fwi_loss_grad")
-        self.nfreq = fr.size
-        self._factor_key = None  # the plan now holds the factors of (slow, freqs), not api.solve_helmholtz's
-        self._eval_key = None  # api.fwi_loss_function records its inputs after this call
-        self._keep = (slow, rec)  # ust_ncg_linesearch reads them again
-        return loss, grad
+        return self._loss_grad(slow, None, rec, freqs, bde)
 
     def fwi_loss_grad_lossy(self, slow, kappa, rec, freqs, bde=None):
         """Fused (loss, grad_s, grad_kappa) of a lossy medium on device tensors (``ust_fwi_loss_grad_lossy``): slow and kappa
         (ny, nx) real, rec (nfreq, nt, nelem) complex.  Afterwards ``ncg_linesearch`` and ``gn_hvp`` refuse until the next
         ``fwi_loss_grad``."""
+        return self._loss_grad(slow, kappa, rec, freqs, bde)
+
+    def _linesearch(self, sd, sd_k):
+        """Line-search scalars [num, den] of ``sd`` (lossy: of the joint direction [sd, sd_k])."""
         torch = _torch()
-        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
-        self._check_tensor(slow, self.treal, self.nx * self.ny)
-        self._check_tensor(kappa, self.treal, self.nx * self.ny)
-        self._check_tensor(rec, self.tcplx, fr.size * self.nt * self.nelem)
-        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
-        loss = torch.empty(1, dtype=torch.float64, device=slow.device)
-        grad_s = torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device)
-        grad_k = torch.empty((self.ny, self.nx), dtype=self.treal, device=slow.device)
-        _lib.check(self.L.ust_fwi_loss_grad_lossy(self.h, C.c_void_p(slow.data_ptr()), C.c_void_p(kappa.data_ptr()),
-                                                  C.c_void_p(rec.data_ptr()), fr.size, _pd(fr), _pd(b), C.c_void_p(loss.data_ptr()),
-                                                  C.c_void_p(grad_s.data_ptr()), C.c_void_p(grad_k.data_ptr()),
-                                                  _stream_ptr(self.device)), "ust_fwi_loss_grad_lossy")
-        self.nfreq = fr.size
-        self._factor_key = None
-        self._eval_key = None
-        return loss, grad_s, grad_k
+        dirs = [sd] if sd_k is None else [sd, sd_k]
+        for t in dirs:
+            self._check_tensor(t, self.treal, self.nx * self.ny)
+        out = torch.empty(2, dtype=torch.float64, device=sd.device)
+        name = "ust_ncg_linesearch" if sd_k is None else "ust_ncg_linesearch_lossy"
+        _lib.check(getattr(self.L, name)(self.h, *map(_ptr, dirs), _ptr(out), _stream_ptr(self.device)), name)
+        return out
 
     def ncg_linesearch(self, sd):
+        return self._linesearch(sd, None)
+
+    def ncg_linesearch_lossy(self, sd_s, sd_k):
+        """Line-search scalars ``[num, den]`` (2-element float64 tensor) of the joint direction ``[sd_s, sd_k]`` on the state of
+        the last ``fwi_loss_grad_lossy`` (``ust_ncg_linesearch_lossy``)."""
+        return self._linesearch(sd_s, sd_k)
+
+    def _gn_hvp(self, v, v_k, jv):
+        """Gauss-Newton product of ``v`` (lossy: of the joint direction [v, v_k], hv of shape (2, ny, nx))."""
         torch = _torch()
-        self._check_tensor(sd, self.treal, self.nx * self.ny)
-        out = torch.empty(2, dtype=torch.float64, device=sd.device)
-        _lib.check(self.L.ust_ncg_linesearch(self.h, C.c_void_p(sd.data_ptr()), C.c_void_p(out.data_ptr()),
-                                             _stream_ptr(self.device)), "ust_ncg_linesearch")
-        return out
+        dirs = [v] if v_k is None else [v, v_k]
+        for t in dirs:
+            self._check_tensor(t, self.treal, self.nx * self.ny)
+        hv = torch.empty((self.ny, self.nx) if v_k is None else (2, self.ny, self.nx), dtype=self.treal, device=v.device)
+        jv2 = torch.empty(1, dtype=torch.float64, device=v.device)
+        jvt = torch.empty((getattr(self, "nfreq", 1), self.nt, getattr(self, "nm", 0)), dtype=self.tcplx, device=v.device) if jv else None
+        name = "ust_fwi_gn_hvp" if v_k is None else "ust_fwi_gn_hvp_lossy"
+        hvs = [hv] if v_k is None else [hv[0], hv[1]]
+        _lib.check(getattr(self.L, name)(self.h, *map(_ptr, dirs), *map(_ptr, hvs), _ptr(jv2), _ptr(jvt) if jv else None,
+                                         _stream_ptr(self.device)), name)
+        return (hv, jv2, jvt) if jv else (hv, jv2)
 
     def gn_hvp(self, v, jv=False):
         """Gauss-Newton product on the state of the last ``fwi_loss_grad`` (no factorisation): ``v`` (ny, nx) real CUDA
         tensor -> ``(hv, jv2[, jv])`` with ``hv = Re(J^H J v)`` (ny, nx), ``jv2 = sum |J v|^2`` (1-element float64 tensor)
         and, when ``jv``, ``J v`` at the kept receivers (nfreq, nt, nm) complex (``ust_fwi_gn_hvp``)."""
-        torch = _torch()
-        self._check_tensor(v, self.treal, self.nx * self.ny)
-        hv = torch.empty((self.ny, self.nx), dtype=self.treal, device=v.device)
-        jv2 = torch.empty(1, dtype=torch.float64, device=v.device)
-        jvt = torch.empty((getattr(self, "nfreq", 1), self.nt, getattr(self, "nm", 0)), dtype=self.tcplx, device=v.device) if jv else None
-        _lib.check(self.L.ust_fwi_gn_hvp(self.h, C.c_void_p(v.data_ptr()), C.c_void_p(hv.data_ptr()), C.c_void_p(jv2.data_ptr()),
-                                         C.c_void_p(jvt.data_ptr()) if jv else None, _stream_ptr(self.device)), "ust_fwi_gn_hvp")
-        return (hv, jv2, jvt) if jv else (hv, jv2)
-
-    def ncg_linesearch_lossy(self, sd_s, sd_k):
-        """Line-search scalars ``[num, den]`` (2-element float64 tensor) of the joint direction ``[sd_s, sd_k]`` on the state of
-        the last ``fwi_loss_grad_lossy`` (``ust_ncg_linesearch_lossy``)."""
-        torch = _torch()
-        self._check_tensor(sd_s, self.treal, self.nx * self.ny)
-        self._check_tensor(sd_k, self.treal, self.nx * self.ny)
-        out = torch.empty(2, dtype=torch.float64, device=sd_s.device)
-        _lib.check(self.L.ust_ncg_linesearch_lossy(self.h, C.c_void_p(sd_s.data_ptr()), C.c_void_p(sd_k.data_ptr()),
-                                                   C.c_void_p(out.data_ptr()), _stream_ptr(self.device)), "ust_ncg_linesearch_lossy")
-        return out
+        return self._gn_hvp(v, None, jv)
 
     def gn_hvp_lossy(self, v_s, v_k, jv=False):
         """Joint Gauss-Newton product on the state of the last ``fwi_loss_grad_lossy``: ``v_s``, ``v_k`` (ny, nx) real CUDA
         tensors -> ``(hv, jv2[, jv])`` with ``hv = Re(J^H J v)`` (2, ny, nx) = [s, kappa] blocks, ``jv2 = sum |J v|^2``
         (1-element float64 tensor) and, when ``jv``, ``J v`` at the kept receivers (nfreq, nt, nm) complex
         (``ust_fwi_gn_hvp_lossy``)."""
-        torch = _torch()
-        self._check_tensor(v_s, self.treal, self.nx * self.ny)
-        self._check_tensor(v_k, self.treal, self.nx * self.ny)
-        hv = torch.empty((2, self.ny, self.nx), dtype=self.treal, device=v_s.device)
-        jv2 = torch.empty(1, dtype=torch.float64, device=v_s.device)
-        jvt = torch.empty((getattr(self, "nfreq", 1), self.nt, getattr(self, "nm", 0)), dtype=self.tcplx, device=v_s.device) if jv else None
-        _lib.check(self.L.ust_fwi_gn_hvp_lossy(self.h, C.c_void_p(v_s.data_ptr()), C.c_void_p(v_k.data_ptr()),
-                                               C.c_void_p(hv[0].data_ptr()), C.c_void_p(hv[1].data_ptr()), C.c_void_p(jv2.data_ptr()),
-                                               C.c_void_p(jvt.data_ptr()) if jv else None, _stream_ptr(self.device)),
-                   "ust_fwi_gn_hvp_lossy")
-        return (hv, jv2, jvt) if jv else (hv, jv2)
+        return self._gn_hvp(v_s, v_k, jv)
 
     # -- host-buffer entry points (NumPy; no torch needed) ------------------------------------
     def solve_helmholtz_host(self, vel, src, f, adjoint=False, bde=None, refactor=True):
@@ -253,46 +251,37 @@ class HelmholtzPlan:
             "ust_solve_helmholtz_host")
         return out
 
-    def fwi_loss_grad_host(self, slow, rec, freqs, bde=None, out_grad=None):
-        """slow (ny,nx) real host array, rec (nfreq, nt, nelem) complex host array (pinned or pageable)."""
-        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
-        slow = np.ascontiguousarray(np.asarray(slow, dtype=self.real))
+    def _loss_grad_host(self, slow, kappa, rec, freqs, bde, out_grad):
+        """(loss, grad) on host arrays, or (loss, grad_s, grad_kappa) of the lossy medium when ``kappa`` is given.
+        ``out_grad``: the gradient array to fill, (ny, nx) or, lossy, (2, ny, nx); None allocates."""
+        fr, b = self._freqs_bde(freqs, bde)
+        maps = [np.ascontiguousarray(np.asarray(m, dtype=self.real)) for m in ([slow] if kappa is None else [slow, kappa])]
         rec = np.ascontiguousarray(np.asarray(rec).astype(self.cplx, copy=False))
         if rec.size != fr.size * self.nt * self.nelem:
             raise ValueError("REC_DATA has the wrong shape for (nfreq, nt, nelem)")
-        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
-        grad = out_grad if out_grad is not None else np.empty((self.ny, self.nx), dtype=self.real)
+        if any(m.size != self.nx * self.ny for m in maps):
+            raise ValueError("slowness and kappa must have ny * nx entries" if kappa is not None else "slowness must have ny * nx entries")
+        if out_grad is None:
+            grads = [np.empty((self.ny, self.nx), dtype=self.real) for _ in maps]
+        elif out_grad.dtype != self.real or out_grad.size != len(maps) * self.nx * self.ny or not out_grad.flags.c_contiguous:
+            raise ValueError(f"out_grad must be a C-contiguous {np.dtype(self.real)} array of {len(maps)} * ny * nx entries")
+        else:
+            grads = [out_grad] if kappa is None else list(out_grad.reshape(2, self.ny, self.nx))
         loss = C.c_double(0.0)
-        _lib.check(self.L.ust_fwi_loss_grad_host(self.h, slow.ctypes.data_as(C.c_void_p), rec.ctypes.data_as(C.c_void_p),
-                                                 fr.size, _pd(fr), _pd(b), C.byref(loss), grad.ctypes.data_as(C.c_void_p)),
-                   "ust_fwi_loss_grad_host")
-        self.nfreq = fr.size
-        self._factor_key = None
-        self._eval_key = None
-        return loss.value, grad
+        name = "ust_fwi_loss_grad_host" if kappa is None else "ust_fwi_loss_grad_lossy_host"
+        _lib.check(getattr(self.L, name)(self.h, *(m.ctypes.data_as(C.c_void_p) for m in maps), rec.ctypes.data_as(C.c_void_p),
+                                         fr.size, _pd(fr), _pd(b), C.byref(loss), *(g.ctypes.data_as(C.c_void_p) for g in grads)),
+                   name)
+        self._evaluated(fr.size)
+        return (loss.value, *grads)
+
+    def fwi_loss_grad_host(self, slow, rec, freqs, bde=None, out_grad=None):
+        """slow (ny,nx) real host array, rec (nfreq, nt, nelem) complex host array (pinned or pageable)."""
+        return self._loss_grad_host(slow, None, rec, freqs, bde, out_grad)
 
     def fwi_loss_grad_lossy_host(self, slow, kappa, rec, freqs, bde=None):
         """Host twin of ``fwi_loss_grad_lossy`` (``ust_fwi_loss_grad_lossy_host``): NumPy in, ``(loss, grad_s, grad_kappa)`` out."""
-        fr = np.ascontiguousarray(np.atleast_1d(np.asarray(freqs, dtype=np.float64)))
-        slow = np.ascontiguousarray(np.asarray(slow, dtype=self.real))
-        kappa = np.ascontiguousarray(np.asarray(kappa, dtype=self.real))
-        rec = np.ascontiguousarray(np.asarray(rec).astype(self.cplx, copy=False))
-        if rec.size != fr.size * self.nt * self.nelem:
-            raise ValueError("REC_DATA has the wrong shape for (nfreq, nt, nelem)")
-        if slow.size != self.nx * self.ny or kappa.size != self.nx * self.ny:
-            raise ValueError("slowness and kappa must have ny * nx entries")
-        b = None if bde is None else np.ascontiguousarray(np.asarray(bde, dtype=np.float64).reshape(fr.size, 3))
-        grad_s = np.empty((self.ny, self.nx), dtype=self.real)
-        grad_k = np.empty((self.ny, self.nx), dtype=self.real)
-        loss = C.c_double(0.0)
-        _lib.check(self.L.ust_fwi_loss_grad_lossy_host(self.h, slow.ctypes.data_as(C.c_void_p), kappa.ctypes.data_as(C.c_void_p),
-                                                       rec.ctypes.data_as(C.c_void_p), fr.size, _pd(fr), _pd(b), C.byref(loss),
-                                                       grad_s.ctypes.data_as(C.c_void_p), grad_k.ctypes.data_as(C.c_void_p)),
-                   "ust_fwi_loss_grad_lossy_host")
-        self.nfreq = fr.size
-        self._factor_key = None
-        self._eval_key = None
-        return loss.value, grad_s, grad_k
+        return self._loss_grad_host(slow, kappa, rec, freqs, bde, None)
 
     # -- introspection ---------------------------------------------------------------------
     def bde(self):
