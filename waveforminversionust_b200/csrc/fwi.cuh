@@ -53,6 +53,11 @@ struct RecvArgs {
     const cx<R>* rec;  // [nfreq][nt][nelem] observed data
     const int* rx_lin; // [nelem] row-major node of every element
     const int* mask;   // [nt][nm]
+    // [nt][nm] receivers that snap to one node: next kept receiver (mask order) on the same node, nm if none, stored as
+    // -1 - next when j is not the first on its node.  The first adds the residuals of all of them, in that order, and stores
+    // the sum once, so the adjoint source is the derivative of the loss (which counts every kept receiver) and is
+    // deterministic.  Without shared nodes every entry is nm and each receiver stores its own residual.
+    const int* rx_next;
     cx<R>* src_est;    // [nfreq][nt]
     double* loss;      // scalar accumulator
     int nt, nm, nelem;
@@ -81,6 +86,7 @@ __global__ void __launch_bounds__(256) receiver_kernel(RecvArgs<R> a) {
     if (threadIdx.x == 0) a.src_est[(size_t)f * a.nt + t] = cx<R>((R)ar, (R)ai);
     const cx<R> alpha((R)ar, (R)ai);
     cx<R>* Lf = a.Lam + (size_t)f * a.stride_f;
+    const int* nx = a.rx_next + (size_t)t * a.nm;
     double l2[1] = {0};
     for (int j = threadIdx.x; j < a.nm; j += blockDim.x) {
         int e = mk[j];
@@ -89,7 +95,10 @@ __global__ void __launch_bounds__(256) receiver_kernel(RecvArgs<R> a) {
         cx<R> ob = recf[e];
         cx<R> d = sim - ob;
         l2[0] += (double)d.re * d.re + (double)d.im * d.im;
-        Lf[o] = d;  // adjoint source (nonlinearcg.py:248-254)
+        int k = nx[j];
+        if (k < 0) continue;  // a receiver before this one on the same node stores the sum
+        for (; k < a.nm; k = -1 - nx[k]) d = d + (sim - recf[mk[k]]);
+        Lf[o] = d;  // adjoint source (nonlinearcg.py:248-254; summed over receivers sharing the node)
     }
     block_sum<1>(l2, sh);
     if (threadIdx.x == 0) atomicAdd(a.loss, 0.5 * l2[0]);
@@ -283,6 +292,7 @@ struct GnRecvArgs {
     size_t stride_f;
     const int* rx_lin;
     const int* mask;
+    const int* rx_next; // [nt][nm] receivers sharing a node (RecvArgs::rx_next)
     cx<R>* drec;        // [nfreq][nt][nm]
     double* jv2;
     int nt, nm;
@@ -305,14 +315,22 @@ __global__ void __launch_bounds__(256) gn_receiver_kernel(GnRecvArgs<R> a) {
     if (threadIdx.x == 0) atomicAdd(a.jv2, s[0]);
 }
 
-// J v as the adjoint source: the same stores as receiver_kernel's Lf[o] = d, so that J^H is the adjoint the gradient uses
+// J v as the adjoint source: the same stores as receiver_kernel's Lf[o] = d (one sum per node, in mask order), so that J^H is
+// the adjoint of J and the one the gradient uses
 template <typename R>
 __global__ void __launch_bounds__(256) gn_scatter_kernel(GnRecvArgs<R> a) {
     const int t = blockIdx.x, f = blockIdx.y;
     cx<R>* Lf = a.Lam + (size_t)f * a.stride_f;
     const int* mk = a.mask + (size_t)t * a.nm;
+    const int* nx = a.rx_next + (size_t)t * a.nm;
     const cx<R>* d_in = a.drec + ((size_t)f * a.nt + t) * a.nm;
-    for (int j = threadIdx.x; j < a.nm; j += blockDim.x) Lf[(size_t)a.rx_lin[mk[j]] * a.nt + t] = d_in[j];
+    for (int j = threadIdx.x; j < a.nm; j += blockDim.x) {
+        int k = nx[j];
+        if (k < 0) continue;
+        cx<R> d = d_in[j];
+        for (; k < a.nm; k = -1 - nx[k]) d = d + d_in[k];
+        Lf[(size_t)a.rx_lin[mk[j]] * a.nt + t] = d;
+    }
 }
 
 // Residual of one forward column: r = H u_t - e_src(t) on the interior nodes, from the nine coefficient planes (what

@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <map>
 #include <mutex>
+#include <unordered_map>
 #include <vector>
 
 #include "assemble.cuh"
@@ -75,6 +76,7 @@ struct ust_plan {
     void *vel = nullptr, *U = nullptr, *Lam = nullptr, *src_est = nullptr, *Xh = nullptr;
     void *slow_h2d = nullptr, *rec_h2d = nullptr, *grad_d2h = nullptr;
     int *src_lin = nullptr, *rx_lin = nullptr, *mask = nullptr;
+    int* rx_next = nullptr;  // [nt][nm] kept receivers sharing a node, chained in mask order (fwi.cuh RecvArgs::rx_next)
     int nt = 0, nelem = 0, nm = 0;
     bool onehot_ok = false;            // first_row / last_row valid (<= 8 column tiles)
     short first_row[8], last_row[8];   // per 128-column tile: smallest / largest interior block row holding a source
@@ -616,6 +618,10 @@ static int solve_impl(ust_plan* p, int ifreq, void* X, int nrhs, int adjoint, cu
     if (ifreq < 0 || ifreq >= p->nfreq_cur) { set_error("ust_solve: ifreq out of range"); return 1; }
     if (nrhs < 1 || nrhs > p->d.max_nrhs) { set_error("ust_solve: nrhs exceeds plan max_nrhs"); return 1; }
     UST_TRY(ring_fix<R>(p, ifreq, (cx<R>*)X, nrhs, adjoint, true, st));
+    // a stand-alone solve is one frequency on one chain: the split-K choice of its sweeps (sweep_step) depends on this solve
+    // alone, not on how many frequencies the plan's last factorisation or evaluation had
+    p->eval_nfreq = 1;
+    p->active_groups = 1;
     const std::vector<Group> one = {{ifreq, 1, st}};
     UST_TRY(sweeps_groups<R>(p, one, (cx<R>*)X, 0, nrhs, adjoint));
     UST_TRY(ring_fix<R>(p, ifreq, (cx<R>*)X, nrhs, adjoint, false, st));
@@ -691,7 +697,7 @@ static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bo
         RecvArgs<R> ra;
         ra.U = (const cx<R>*)p->U + (size_t)q.f0 * stride; ra.Lam = (cx<R>*)p->Lam + (size_t)q.f0 * stride; ra.stride_f = stride;
         ra.rec = (const cx<R>*)p->rec_in + (size_t)q.f0 * nt * p->nelem;
-        ra.rx_lin = p->rx_lin; ra.mask = p->mask; ra.src_est = (cx<R>*)p->src_est + (size_t)q.f0 * nt; ra.loss = loss_dev;
+        ra.rx_lin = p->rx_lin; ra.mask = p->mask; ra.rx_next = p->rx_next; ra.src_est = (cx<R>*)p->src_est + (size_t)q.f0 * nt; ra.loss = loss_dev;
         ra.nt = nt; ra.nm = p->nm; ra.nelem = p->nelem;
         ProfScope ps(p, PC_RECEIVER, q.st);
         receiver_kernel<R><<<dim3(nt, q.nf), 256, 0, q.st>>>(ra);
@@ -781,7 +787,7 @@ static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st, bool lossy) {
     for (const Group& q : gs) {
         GnRecvArgs<R> ra;
         ra.Pert = (const cx<R>*)p->Lam + (size_t)q.f0 * stride; ra.Lam = (cx<R>*)p->Lam + (size_t)q.f0 * stride; ra.stride_f = stride;
-        ra.rx_lin = p->rx_lin; ra.mask = p->mask; ra.drec = (cx<R>*)p->drec + (size_t)q.f0 * nt * p->nm; ra.jv2 = jv2;
+        ra.rx_lin = p->rx_lin; ra.mask = p->mask; ra.rx_next = p->rx_next; ra.drec = (cx<R>*)p->drec + (size_t)q.f0 * nt * p->nm; ra.jv2 = jv2;
         ra.nt = nt; ra.nm = p->nm;
         {
             ProfScope ps(p, PC_RECEIVER, q.st);
@@ -1202,7 +1208,7 @@ int ust_plan_destroy(ust_plan* p) {
     cudaSetDevice(p->d.device);
     cudaDeviceSynchronize();
     void* ptrs[] = {p->exn, p->rexh, p->eyn, p->reyh, p->d_vminmax, p->d_freqs, p->d_bde, p->d_scal, p->d_status, p->d_invv2, p->d_sig2, p->planes,
-                    p->T, p->scratch, p->W, p->pbuf, p->Tp, p->Wp, p->Rp, p->Cp, p->Xp, p->Pp, p->Rs, p->gj_flags, p->snap, p->vel, p->U, p->Lam, p->src_est, p->Xh, p->src_lin, p->rx_lin, p->mask,
+                    p->T, p->scratch, p->W, p->pbuf, p->Tp, p->Wp, p->Rp, p->Cp, p->Xp, p->Pp, p->Rs, p->gj_flags, p->snap, p->vel, p->U, p->Lam, p->src_est, p->Xh, p->src_lin, p->rx_lin, p->mask, p->rx_next,
                     p->slow_h2d, p->rec_h2d, p->grad_d2h, p->kappa_h2d, p->grad_kappa_d2h};
     for (void* q : ptrs)
         if (q) cudaFree(q);
@@ -1270,7 +1276,7 @@ int ust_plan_set_acquisition(ust_plan* p, int nt, const int32_t* src_lin, int ne
     UST_CUDA(cudaDeviceSynchronize());
     drop_graphs(p);
     p->eval_kind = ust_plan::EVAL_NONE;
-    for (int** q : {&p->src_lin, &p->rx_lin, &p->mask})
+    for (int** q : {&p->src_lin, &p->rx_lin, &p->mask, &p->rx_next})
         if (*q) { cudaFree(*q); *q = nullptr; }
     if (p->rec_in) { cudaFree(p->rec_in); p->rec_in = nullptr; }
     if (p->rec_h2d) { cudaFree(p->rec_h2d); p->rec_h2d = nullptr; }  // sized by nt * nelem: regrown by the next host call
@@ -1283,6 +1289,28 @@ int ust_plan_set_acquisition(ust_plan* p, int nt, const int32_t* src_lin, int ne
     UST_CUDA(cudaMemcpy(p->src_lin, src_lin, nt * sizeof(int), cudaMemcpyHostToDevice));
     UST_CUDA(cudaMemcpy(p->rx_lin, rx_lin, nelem * sizeof(int), cudaMemcpyHostToDevice));
     UST_CUDA(cudaMemcpy(p->mask, mask, (size_t)nt * nm * sizeof(int), cudaMemcpyHostToDevice));
+    // Kept receivers of one transmitter that snap to the same node: the adjoint source there is the sum of their residuals,
+    // added in mask order by the first of them (receiver_kernel, gn_scatter_kernel).  Entry j holds the next such receiver
+    // (nm: none), stored as -1 - next when j is not the first on its node.
+    {
+        std::vector<int> next((size_t)nt * nm, nm);
+        std::unordered_map<int, int> last;  // node -> last kept receiver seen on it
+        for (int t = 0; t < nt; ++t) {
+            int* nx = next.data() + (size_t)t * nm;
+            const int* mk = mask + (size_t)t * nm;
+            last.clear();
+            for (int j = 0; j < nm; ++j) {
+                auto it = last.find(rx_lin[mk[j]]);
+                if (it == last.end()) { last.emplace(rx_lin[mk[j]], j); continue; }
+                const int i = it->second;  // previous receiver on this node: link it to j, keep its own first / not-first sign
+                nx[i] = nx[i] >= 0 ? j : -1 - j;
+                nx[j] = -1 - nm;
+                it->second = j;
+            }
+        }
+        UST_CUDA(cudaMalloc((void**)&p->rx_next, next.size() * sizeof(int)));
+        UST_CUDA(cudaMemcpy(p->rx_next, next.data(), next.size() * sizeof(int), cudaMemcpyHostToDevice));
+    }
     p->nt = nt; p->nelem = nelem; p->nm = nm; p->acq_set = true;
     p->onehot_ok = cdiv_i(nt, 128) <= 8;
     for (int i = 0; i < 8; ++i) { p->first_row[i] = 32767; p->last_row[i] = -1; }

@@ -19,7 +19,9 @@ class RingGeometry:
     yi: np.ndarray  # (Ny,) grid y coordinates
     x_idx: np.ndarray  # (E,) grid column of each element
     y_idx: np.ndarray  # (E,) grid row of each element
-    ind_matlab: np.ndarray  # (E,) x_idx*Nxi + y_idx                    fwi_script.py:68
+    # (E,) x_idx*Ny + y_idx: the column-major (order='F') index of a (Ny, Nx) field, which api._acquisition decodes.  The
+    # reference writes x_idx*Nxi + y_idx (fwi_script.py:68), which is the same only on square grids.
+    ind_matlab: np.ndarray
     tx_include: np.ndarray  # (Nt,) transmitting elements               fwi_script.py:35
     mask_indices: np.ndarray  # (Nt, Nm) receivers kept per transmitter fwi_script.py:79-85
     num_elements: int
