@@ -627,11 +627,10 @@ def test_sharded_engine_parts_sum_to_the_whole(torch_, shard):
 
 
 def test_pivot_schedules_are_bit_identical(torch_, monkeypatch):
-    """Four schedules of a Gauss-Jordan pivot step -- pivot inversions as separate launches (UST_NO_LOOKAHEAD=1), look-ahead pivot
-    CTAs riding on the update launch (the default), the deep look-ahead kernel on a side stream (UST_DEEP=1) and riding pivot
-    CTAs plus the next row panel as trailing CTAs of the same launch (UST_FUSE_RP=1, in-launch flags) -- form every block with
-    the arithmetic of the tile that owns it: gradient and source estimates must agree to the bit (grids with 2, 3 and 6 pivot
-    blocks; the first case runs two launch chains with programmatic dependent launch, the others one chain without)."""
+    """Two schedules of a Gauss-Jordan pivot step -- pivot inversions as separate launches (UST_NO_LOOKAHEAD=1) and look-ahead
+    pivot CTAs riding on the update launch (the default) -- form every block with the arithmetic of the tile that owns it:
+    gradient and source estimates must agree to the bit (grids with 2, 3 and 6 pivot blocks; the first case runs two launch
+    chains with programmatic dependent launch, the others one chain without)."""
     import waveforminversionust_b200 as w
     for n, nelem, nf in ((100, 16, 8), (140, 24, 3), (330, 16, 2)):
         geom, f0, vel_true = small_case(n, nelem)
@@ -640,9 +639,8 @@ def test_pivot_schedules_are_bit_identical(torch_, monkeypatch):
         slow = np.full((n, n), 1 / 1485.0, dtype=np.float32)
         args = (geom.dense_src(), freqs, geom.a0, geom.L_PML, geom.tx_include, geom.ind_matlab, geom.mask_indices, geom.num_elements)
         out = {}
-        for name, env in (("separate", {"UST_NO_LOOKAHEAD": "1"}), ("riding", {}), ("deep", {"UST_DEEP": "1"}), ("fused", {"UST_FUSE_RP": "1"})):
-            for k in ("UST_NO_LOOKAHEAD", "UST_DEEP", "UST_FUSE_RP"):
-                monkeypatch.delenv(k, raising=False)
+        for name, env in (("separate", {"UST_NO_LOOKAHEAD": "1"}), ("riding", {})):
+            monkeypatch.delenv("UST_NO_LOOKAHEAD", raising=False)
             for k, v in env.items():
                 monkeypatch.setenv(k, v)
             w.clear_plans()
@@ -654,34 +652,9 @@ def test_pivot_schedules_are_bit_identical(torch_, monkeypatch):
                 if rep:
                     assert np.array_equal(res[1], out[name][1])
                 out[name] = res
-        for name in ("riding", "deep", "fused"):
-            assert np.array_equal(out[name][1], out["separate"][1]) and np.array_equal(out[name][2], out["separate"][2]), (n, name)
-            assert abs(out[name][0] - out["separate"][0]) <= 1e-13 * abs(out["separate"][0])
-    for k in ("UST_NO_LOOKAHEAD", "UST_DEEP", "UST_FUSE_RP"):
-        monkeypatch.delenv(k, raising=False)
-    w.clear_plans()
-
-
-def test_two_level_gauss_jordan_variant(torch_, monkeypatch):
-    """UST_GJ2=1 selects the two-level blocked Gauss-Jordan (outer block 128: row panel a, block row b, row panel b, block row a,
-    one rank-128 update of all other rows per pair of pivot blocks).  Opt-in (not faster, DESIGN.md 6b), but it must stay
-    correct: wavefields against the complex128 oracle on grids with 2, 4 and 6 pivot blocks (the last one padded)."""
-    import waveforminversionust_b200 as w
-    monkeypatch.setenv("UST_GJ2", "1")
-    w.clear_plans()
-    for n, nrhs in ((100, 6), (200, 9), (330, 5)):
-        geom, f, vel = small_case(n)
-        bde = bde_for(geom, vel, f)
-        rng = np.random.default_rng(n)
-        src = (rng.standard_normal((n, n, nrhs)) + 1j * rng.standard_normal((n, n, nrhs))).astype(np.complex64)
-        src[0] = 0; src[-1] = 0; src[:, 0] = 0; src[:, -1] = 0
-        velr = vel.astype(np.float32)
-        fac = oh.HelmholtzFactor(geom.xi, geom.yi, velr.astype(np.float64), f, geom.a0, geom.L_PML, "c128", bde=bde)
-        for adjoint in (False, True):
-            got = w.solve_helmholtz(geom.xi, geom.yi, velr, src, f, geom.a0, geom.L_PML, adjoint, dtype="c64", bde=bde)
-            err = rel(got[1:-1, 1:-1], fac.solve(src.astype(np.complex128), adjoint)[1:-1, 1:-1])
-            print(f"two-level Gauss-Jordan n={n} adjoint={adjoint}: {err:.3e}")
-            assert err < WV_TOL["c64"]
+        assert np.array_equal(out["riding"][1], out["separate"][1]) and np.array_equal(out["riding"][2], out["separate"][2]), n
+        assert abs(out["riding"][0] - out["separate"][0]) <= 1e-13 * abs(out["separate"][0])
+    monkeypatch.delenv("UST_NO_LOOKAHEAD", raising=False)
     w.clear_plans()
 
 

@@ -36,11 +36,6 @@ print("ctas", len(first), "kernel span", max(max(t[:17]) for _, _, t in first), 
 print("%5s %4s " % ("cta", "sm") + " ".join("%8s" % n for n in names))
 for b, sm, t in first[:: max(1, len(first) // 48)]:
     print("%5d %4d " % (b, sm) + " ".join("%8d" % x for x in t[:17]))
-rp = [r_ for r_ in first if 900 <= r_[0] < 1000]
-if rp:
-    print("fused row-panel CTAs (rows 900 + index): 'pivdone' column = time the CTA became resident, 'enter' = flags seen")
-    for b, sm, t in rp[:: max(1, len(rp) // 12)]:
-        print("%5d %4d " % (b, sm) + " ".join("%8d" % x for x in t[:17]))
 piv = [r_ for r_ in first if r_[0] >= 1000]
 if piv:
     print("look-ahead pivot CTAs (rows 1000 + chain): formed = 'staged', inversion done = 'pivdone'")

@@ -16,10 +16,7 @@ python bench.py --config cfg4 --steps 2 --warmup 1 --no-cpu-baseline > $O/bench_
 python bench.py --nfreq 2 --no-cpu-baseline > $O/bench_f2_$R.json 2> $O/bench_f2_$R.err
 python bench.py --nfreq 4 --no-cpu-baseline > $O/bench_f4_$R.json 2> $O/bench_f4_$R.err
 python bench.py --nfreq 8 --no-cpu-baseline > $O/bench_f8_$R.json 2> $O/bench_f8_$R.err
-UST_DEEP=1 python bench.py --no-cpu-baseline > $O/bench_deep_$R.json 2> $O/bench_deep_$R.err
-UST_FUSE_RP=1 python bench.py --no-cpu-baseline > $O/bench_fused_$R.json 2> $O/bench_fused_$R.err
 python bench.py --dtype c128 --nfreq 4 --no-cpu-baseline > $O/bench_c128_$R.json 2> $O/bench_c128_$R.err
-UST_GJ2=1 python bench.py --no-cpu-baseline > $O/bench_gj2_$R.json 2> $O/bench_gj2_$R.err
 python bench.py --groups 1 --no-cpu-baseline > $O/bench_g1_$R.json 2> $O/bench_g1_$R.err
 python tools/exp_update_trace.py > $O/exp_update_trace_$R.log 2>&1
 python tools/exp_update_trace.py --nfreq 2 > $O/exp_update_trace_f2_$R.log 2>&1

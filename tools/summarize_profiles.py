@@ -134,7 +134,7 @@ copy(f"exp_accuracy_{R}.log", f"exp_accuracy_{R}.txt",
 copy(f"pytest_gpu_{R}.log", f"pytest_gpu_{R}.txt", "# python -m pytest tests -m gpu -q -s on one B200\n")
 copy(f"smoke_{R}.log", f"smoke_{R}.txt")
 copy(f"gpu_{R}.txt", f"gpu_{R}.txt")
-for tag in ("bench", "bench_final", "bench_simt", "bench_ref", "bench_cfg2", "bench_cfg4", "bench_cfg4_c128", "bench_f2", "bench_f4", "bench_f8", "bench_deep", "bench_fused", "bench_c128", "bench_gj2", "bench_g1",
+for tag in ("bench", "bench_final", "bench_simt", "bench_ref", "bench_cfg2", "bench_cfg4", "bench_cfg4_c128", "bench_f2", "bench_f4", "bench_f8", "bench_c128", "bench_g1",
             "bench_2gpu_strong", "bench_2gpu_cfg4", "bench_4gpu_strong", "bench_8gpu_strong", "cfg5_8gpu", "cpu_baseline"):
     s = os.path.join(O, f"{tag}_{R}.json")
     if os.path.exists(s):

@@ -92,7 +92,6 @@ struct AsmArgs {
     double h, gr;  // grid step, anisotropy ratio dy/dx
     int stencil;   // 0 python (clamped out-of-bounds gathers), 1 matlab
     int nfreq;
-    int exp;       // timing experiment (UST_EXP & 8): store constants only -- what the store pattern alone costs
 };
 
 // 1 / v^2 per node in float64, once per model (every frequency and every one of a node's nine neighbours reuses it: the
@@ -231,12 +230,6 @@ __global__ void __launch_bounds__(256, 4) assemble_kernel(AsmArgs a, const doubl
     if (x >= Nx) return;
     const size_t pl = (size_t)Nx * Ny;
     cx<R>* out0 = planes + (size_t)y * Nx + x;
-    if (a.exp) {
-        for (int fi = 0; fi < a.nfreq; ++fi)
-#pragma unroll
-            for (int p = 0; p < 9; ++p) out0[((size_t)fi * 9 + p) * pl] = cx<R>((R)fc[fi][p], (R)0);
-        return;
-    }
     if (x == 0 || y == 0 || x == Nx - 1 || y == Ny - 1) {
         for (int fi = 0; fi < a.nfreq; ++fi)
 #pragma unroll

@@ -38,9 +38,7 @@ struct FactorArgs {
     uint16_t* Cp;         // [2][nbmax][6][nP/8][8][8][8] A planes of the column panel X_:,k (nP x 64), ping-pong on k
     uint16_t* Pp;         // [nbmax][6][8][8][8][8] A planes of the pivot-block inverse P (64 x 64)
     uint16_t* Tp;         // [nfreq*M][6][nP/8][nP/8][8][8] A planes of the finished block inverses
-    size_t rp_stride;     // elements per batch entry of Xp (and of Rp in the classic scheme): B planes of 64 rows
-    size_t rp2_stride;    // two-level scheme: elements per batch entry of Rp, B planes of 128 rows ([R_a; R_b], 8 k-chunks per column tile)
-    int kb;               // outer block of the Gauss-Jordan inversion: 64 = classic, 128 = two-level (gj2 kernels below)
+    size_t rp_stride;     // elements per batch entry of Xp and Rp: B planes of 64 rows
     int nbmax;            // batch capacity (2 * max_freq)
     int gj_drain;         // drain period (chunks) of the leading accumulator in the K = 64 Gauss-Jordan GEMMs
     int inplace;          // TMA-fed engine: X^(k) is updated in place in its T slot (no ping-pong: the batch stays L2 resident)
@@ -48,13 +46,6 @@ struct FactorArgs {
     unsigned long long* trace;  // debugging (UST_TC2_TRACE_UPDATE=step,k): [1024][16] phase timestamps of the update CTAs
     int trace_step, trace_k;
     int prefetch_cin;     // update kernel: L2 prefetch of the X tile at CTA start
-    int deep;             // deep look-ahead (tc2_gj_pivot_deep_kernel on a side stream)
-    int pp;               // Pp and snap are ping-ponged on the pivot index, the snapshots are taken by the update tiles (deep / fused modes)
-    int fuse;             // row panel k+1 runs as trailing CTAs of update launch k (in-launch flags); Rp is ping-ponged on the pivot index
-    int* flags;           // [2][GJ_MAXBLK][nbmax]: [0] = P_k written (set by the pivot CTA), [1] = finished tiles of pivot block row k
-    uint16_t* Rs;         // [nbmax] B planes (layout of Rp) private to the deep look-ahead pivot CTAs: their own copy of R_k[:, k+1]
-    int exp;              // timing experiments only (UST_EXP bit mask, results are WRONG when set): 1 = look-ahead pivot CTAs skip the
-                          // inversion, 2 = they exit at once, 4 = row-panel launches skipped (host side)
     // Frequency groups run as independent launch chains on separate streams: a launch covers the chains of the
     // frequencies [f0, f0 + nbatch / 2) (PH_MID: nbatch); blockIdx.z is local to the group, zb0 + z indexes the per-chain
     // work buffers (Rp, Xp, Cp, Pp, snap, pbuf, scratch) and f0 + chain_freq() the per-frequency arrays.
@@ -83,20 +74,6 @@ __device__ __forceinline__ cx<R>* gj_buffer(const FactorArgs<R>& a, int z, int f
     const bool k_even = (k & 1) == 0;
     const bool slot_holds_even = (nblk & 1) == 0;  // X^{(nblk)} must land in the T slot
     return (k_even == slot_holds_even) ? slot : scr;
-}
-
-constexpr int GJ_MAXBLK = 64;  // pivot blocks per matrix the in-launch flags are sized for (nP <= 4096)
-__device__ __forceinline__ int* gj_flag(const FactorArgs<float>& a, int kind, int k, int z) {
-    return a.flags + ((size_t)(kind * GJ_MAXBLK + k) * a.nbmax + a.zb0 + z);
-}
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-template <typename R>
-__device__ __forceinline__ uint16_t* gj_rp(const FactorArgs<R>& a, int k, int z) {  // B planes of row panel R_k
-    return a.Rp + ((size_t)(a.fuse ? (k & 1) * a.nbmax : 0) + a.zb0 + z) * a.rp_stride;
 }
 
 // One CTA (16 x 16 threads) = one TS x TS tile of S.  Thread (tx, ty) owns rows a0 + PT*ty .. + PT-1 (contiguous) and
@@ -132,10 +109,6 @@ __global__ void __launch_bounds__(256, sizeof(R) == 4 ? 3 : 2) schur_kernel(Fact
     if (row < 0) return;
     const int freq = (a.f0 + chain_freq(a.phase, z)), dir = chain_dir(a.phase, z);
     const int tx = threadIdx.x, ty = threadIdx.y, tid = ty * 16 + tx;
-    if constexpr (sizeof(R) == 4) {
-        // fused row panels: the in-launch flags of this chain's pivot steps start from zero for every block row
-        if (a.fuse && bx == 0 && by == 0 && tid < 2 * GJ_MAXBLK) a.flags[(size_t)tid * a.nbmax + a.zb0 + z] = 0;
-    }
     const int b0 = bx * TS, a0 = by * TS;
     const int nI = a.g.nI, nP = a.g.nP, M = a.g.M;
     const size_t pl = (size_t)a.g.Nx * a.g.Ny;
@@ -596,7 +569,7 @@ __device__ __forceinline__ void gj_pivot_blocked(const FactorArgs<float>& a, int
     }
 }
 
-// stand-alone form: the block is fetched from X^(k) in global memory first (pivot launches without look-ahead, k = 0 launch)
+// stand-alone form: the block is fetched from X^(k) in global memory first (pivot launches without look-ahead)
 __device__ __forceinline__ void gj_pivot_blocked_global(const FactorArgs<float>& a, int k, int z, unsigned char* smem_raw, int tid) {
     const int row = chain_row(a.g, a.phase, z, a.step);
     if (row < 0) return;
@@ -938,40 +911,19 @@ __device__ __forceinline__ void gj_colsplit_body(const FactorArgs<float>& a, int
     }
 }
 
-// k = 0 preparation of the TMA-fed engine in ONE launch: CTA role by blockIdx.x --
+// k = 0 preparation of the TMA-fed engine in ONE launch (pivot block 0 is inverted by the Schur launch): CTA role by blockIdx.x --
 //   [0, nrow)            B planes of the pivot block row 0 (gj_rowsplit, 128 columns per CTA)
 //   [nrow, nrow + ncol)  A planes of block column 0 (gj_colsplit, 32 rows per CTA)
-//   nrow + ncol          inversion of pivot block 0 (runs beside the two splits instead of after them)
-// grid = (nrow + ncol + 1, 1, nbatch), 256 threads, dynamic smem = gj_pivot_smem.
+// grid = (nrow + ncol, 1, nbatch), 256 threads.
 __device__ __forceinline__ void gj_rowsplit_body(const FactorArgs<float>& a, int k, int z, int tn, int r);
-__device__ __forceinline__ void gj_colsplit_body(const FactorArgs<float>& a, int k, int z, int bx, int tid);
-__global__ void __launch_bounds__(256) gj_k0_kernel(FactorArgs<float> a, int nrow, int ncol, int snap11) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
+__global__ void __launch_bounds__(256) gj_k0_kernel(FactorArgs<float> a, int nrow) {
     pdl_trigger();
     pdl_wait();
     const int z = blockIdx.z, bx = blockIdx.x;
     if (bx < nrow) {
         if (threadIdx.x < 128) gj_rowsplit_body(a, 0, z, bx, threadIdx.x);
-    } else if (bx < nrow + ncol) {
-        gj_colsplit_body(a, 0, z, bx - nrow, threadIdx.x);
-    } else if (snap11 && bx == nrow + ncol) {
-        // deep look-ahead: copy of X^(0)_{11} for the pivot CTA that inverts P_1 beside row panel 0 and update 0
-        const int row = chain_row(a.g, a.phase, z, a.step);
-        if (row < 0) return;
-        const int freq = a.f0 + chain_freq(a.phase, z), nP = a.g.nP;
-        const cx<float>* __restrict__ Xc = gj_buffer(a, z, freq, row, 0);
-        cx<float>* __restrict__ S = a.snap + ((size_t)a.nbmax + a.zb0 + z) * GJ_NB * GJ_NB;
-        constexpr int PER = GJ_NB * GJ_NB / 2 / 256;
-        float4 v[PER];
-#pragma unroll
-        for (int j = 0; j < PER; ++j) {
-            const int w = threadIdx.x + 256 * j, r = w >> 5, c2 = w & 31;
-            v[j] = *reinterpret_cast<const float4*>(Xc + (size_t)(GJ_NB + r) * nP + GJ_NB + 2 * c2);
-        }
-#pragma unroll
-        for (int j = 0; j < PER; ++j) reinterpret_cast<float4*>(S)[threadIdx.x + 256 * j] = v[j];
     } else {
-        gj_pivot_blocked_global(a, 0, z, smem_raw, threadIdx.x);
+        gj_colsplit_body(a, 0, z, bx - nrow, threadIdx.x);
     }
 }
 
@@ -1022,31 +974,9 @@ __device__ __forceinline__ void gj_emit_a(const FactorArgs<float>& a, tc2::Tc2Ti
     }
 }
 
-// one 64 x 64 tile (block column `ntile`) of row panel k
-__device__ __forceinline__ void gj_rowpanel_tile(const FactorArgs<float>& a, int k, int z, int row, int freq, int ntile, float bias_fix,
-                                                 const CUtensorMap* pmap, unsigned char* tc2_smem, unsigned long long* trace = nullptr) {
-    const int nP = a.g.nP;
-    tc2::Tc2Tile t;
-    tc2::tile_no_emit(t);
-    t.bplanes = a.Xp + ((size_t)(k & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;
-    t.amat = (a.pp ? (k & 1) * a.nbmax : 0) + a.zb0 + z;
-    t.Cin = nullptr; t.ldcin = nP;
-    t.Cout = gj_buffer(a, z, freq, row, k + 1) + (size_t)k * GJ_NB * nP; t.ldc = nP;
-    t.M = GJ_NB; t.N = nP; t.K = GJ_NB; t.Mstore = GJ_NB;
-    t.m0 = 0; t.n0 = ntile * tc2::TNH;
-    t.mask_lo = 0; t.mask_hi = 0; t.skip_lo = 0; t.skip_hi = 0;
-    t.sgn = 1.f;
-    t.bias_fix = bias_fix;
-    t.drain_every = a.gj_drain;
-    t.eb_planes = gj_rp(a, k, z); t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0;
-    gj_emit_a(a, t, z, freq, row, k, k * GJ_NB);
-    t.trace = trace;
-    tc2::cgemm_tile_h(t, pmap, tc2_smem);
-}
-
 // TMA-fed tensor-core row panel: R = P * Xtilde_k,: -> block row k of X' (FP32), B planes of R for the update and the
-// rows of the next column panel that lie in block row k.  grid = (ceil(nP/128), 1, nbatch), 576 threads.
-// 128 x 64 tiles on the two-CTAs-per-SM form of the engine (gemm_tc2h.cuh): grid = (nP/64 [+1 snapshot CTA], 1, nbatch), 256 threads.
+// rows of the next column panel that lie in block row k.  One 64 x 64 tile (block column blockIdx.x) per CTA on the
+// two-CTAs-per-SM form of the engine (gemm_tc2h.cuh): grid = (nP/64 [+1 snapshot CTA], 1, nbatch), 256 threads.
 __global__ void __launch_bounds__(tc2::NUM_THREADS_H, 2)
 tc2_gj_rowpanel_kernel(FactorArgs<float> a, int k, float bias_fix, const __grid_constant__ CUtensorMap pmap) {
     extern __shared__ __align__(1024) unsigned char tc2_smem[];
@@ -1077,23 +1007,30 @@ tc2_gj_rowpanel_kernel(FactorArgs<float> a, int k, float bias_fix, const __grid_
         for (int j = 0; j < PER; ++j) reinterpret_cast<float4*>(S)[threadIdx.x + 256 * j] = v[j];
         return;
     }
-    gj_rowpanel_tile(a, k, z, row, freq, blockIdx.x, bias_fix, &pmap, tc2_smem);
+    tc2::Tc2Tile t;
+    tc2::tile_no_emit(t);
+    t.bplanes = a.Xp + ((size_t)(k & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;
+    t.amat = a.zb0 + z;
+    t.Cin = nullptr; t.ldcin = nP;
+    t.Cout = gj_buffer(a, z, freq, row, k + 1) + (size_t)k * GJ_NB * nP; t.ldc = nP;
+    t.M = GJ_NB; t.N = nP; t.K = GJ_NB; t.Mstore = GJ_NB;
+    t.m0 = 0; t.n0 = blockIdx.x * TW;
+    t.mask_lo = 0; t.mask_hi = 0; t.skip_lo = 0; t.skip_hi = 0;
+    t.sgn = 1.f;
+    t.bias_fix = bias_fix;
+    t.drain_every = a.gj_drain;
+    t.eb_planes = a.Rp + (size_t)(a.zb0 + z) * a.rp_stride; t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0;
+    gj_emit_a(a, t, z, freq, row, k, k * GJ_NB);
+    tc2::cgemm_tile_h(t, &pmap, tc2_smem);
 }
 
 // TMA-fed tensor-core update: X' = Xtilde - X_:,k R over the whole matrix except the pivot block row; the epilogue also
 // emits the next pivot block row (B planes) and the next column panel (A planes), or the finished inverse.
-// 128 x 64 tiles, two CTAs per SM (gemm_tc2h.cuh), 256 threads, 1-D grid of up to three CTA roles:
+// 128 x 64 tiles, two CTAs per SM (gemm_tc2h.cuh), 256 threads, 1-D grid of up to two CTA roles:
 //   [nbatch look-ahead pivot CTAs]  (pivot_next)  form and invert pivot block k+1 beside the tiles
 //   [nbatch * ceil(nP/128) * nP/64 tile CTAs]
-//   [nbatch * nP/64 row-panel CTAs] (rp_next, "fused" schedule)  row panel k+1 = P_{k+1} X~_{k+1,:} inside THIS launch: they wait
-//       on in-launch flags for P_{k+1} (pivot CTA of their chain) and for the nP/64 tiles of the 128-row tile row that holds
-//       block row k+1 (numbered first), so a pivot step is one launch instead of two and the row panel runs in the update's
-//       tail round instead of after it.  What a row-panel CTA overwrites is dead by then: block row k+1 of X (its tiles are
-//       done), rows of block row k+1 in the column-panel planes two steps ahead (= the buffer of column panel k, whose rows
-//       are only read by those tiles and by the pivot CTA), and the OTHER row-panel plane buffer (Rp ping-pong).
 __global__ void __launch_bounds__(tc2::NUM_THREADS_H, 2)
-tc2_gj_update_kernel(FactorArgs<float> a, int k, float bias_fix, int pivot_next, int rp_next, const __grid_constant__ CUtensorMap cmap,
-                     const __grid_constant__ CUtensorMap pmap) {
+tc2_gj_update_kernel(FactorArgs<float> a, int k, float bias_fix, int pivot_next, const __grid_constant__ CUtensorMap cmap) {
     extern __shared__ __align__(1024) unsigned char tc2_smem[];
     constexpr int TW = tc2::TNH;
     // With pivot_next the first nbatch CTAs are look-ahead pivot CTAs: CTA z forms and inverts the NEXT pivot
@@ -1103,115 +1040,57 @@ tc2_gj_update_kernel(FactorArgs<float> a, int k, float bias_fix, int pivot_next,
     int bid = blockIdx.x;
     if (pivot_next) {
         if (bid < a.nbatch) {
-            {
-                // The next pivot block is formed by the SAME tensor-core arithmetic as the update tile that owns it (same
-                // operand planes, chunking, draining): a 128 x 64 product whose Cin is the snapshot of X^(k)_{k+1,k+1}
-                // and whose result stays in shared memory.  Forming it with FP32 FMAs from the snapshot instead is more
-                // accurate per entry but no longer consistent with the rest of block row k+1, and costs a factor 1.4 in
-                // the wavefield error at 512^2 (tools/exp_accuracy.py: 9.5e-6 vs 6.7e-6).
-                static_assert(tc2::CH_LD == GJ_NB + 1, "pivot body reads the staged tile with row stride GJ_NB + 1");
-                const int z = bid, kb = k + 1, nP = a.g.nP;
-                const int row = chain_row(a.g, a.phase, z, a.step);
-                if (row < 0 || (a.exp & 2)) {
-                    if (row >= 0 && rp_next && threadIdx.x == 0) atomicExch(gj_flag(a, 0, kb, z), 1);  // timing experiments: do not strand the row-panel CTAs
-                    pdl_wait();
-                    return;
-                }
-                tc2::Tc2Tile t;
-                tc2::tile_no_emit(t);
-                t.bplanes = gj_rp(a, k, z);
-                t.amat = (k & 1) * a.nbmax + a.zb0 + z;
-                const cx<float>* S1 = a.snap + ((size_t)(a.pp ? (kb & 1) * a.nbmax : 0) + a.zb0 + z) * GJ_NB * GJ_NB;  // X^(k)_{k+1,k+1}
-                t.Cin = S1 - (size_t)(kb * GJ_NB) * GJ_NB - kb * GJ_NB; t.ldcin = GJ_NB;
-                t.Cout = nullptr; t.ldc = nP; t.keep = 1;
-                t.M = nP; t.N = nP; t.K = GJ_NB; t.Mstore = nP;
-                t.m0 = (kb >> 1) * tc2::TM; t.n0 = kb * GJ_NB;
-                t.mask_lo = 0; t.mask_hi = 0;
-                t.skip_lo = (kb ^ 1) * GJ_NB; t.skip_hi = t.skip_lo + GJ_NB;  // the sibling block of the 128-row tile is not needed
-                t.sgn = -1.f; t.bias_fix = bias_fix; t.drain_every = a.gj_drain;
-                const bool traced = a.trace && a.step == a.trace_step && k == a.trace_k && z < 24;
-                if (traced) {  // debugging: pivot CTAs use trace rows 1000 + z, their end-of-inversion stamp goes to column 17
-                    t.trace = a.trace + 16 * (1000 + z);
-                    if (threadIdx.x == 0) { unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); a.trace[16 * 1024 + 1000 + z] = smid; }
-                }
-                tc2::cgemm_tile_h(t, &cmap, tc2_smem);
-                __syncthreads();
-                if (a.exp & 1) {
-                    if (rp_next && threadIdx.x == 0) atomicExch(gj_flag(a, 0, kb, z), 1);
-                    return;
-                }
-                unsigned char* smem_al = tc2_smem + ((128u - (tc::smem_u32(tc2_smem) & 127u)) & 127u);
-                // the staged 128 x 65 tile holds the block (rows 64 (kb & 1) ..): invert it where it lies, scratch behind the tile
-                cx<float>* blk = reinterpret_cast<cx<float>*>(smem_al) + (size_t)(kb & 1) * GJ_NB * tc2::CH_LD;
-                cx<float>* scr = reinterpret_cast<cx<float>*>(smem_al) + (size_t)tc2::TM * tc2::CH_LD;
-                static_assert((size_t)tc2::TM * tc2::CH_LD * sizeof(cx<float>) + gj_pivot2_scratch_bytes <= (size_t)tc2::STAGES_H * tc2::STAGE_H,
-                              "pivot scratch must fit behind the staging tile inside the operand ring");
-                FactorArgs<float> a2 = a;
-                if (a.pp) a2.Pp = a.Pp + (size_t)(kb & 1) * a.nbmax * tc2::NPL_A * GJ_NB * GJ_NB;
-                gj_pivot_blocked(a2, z, blk, scr, threadIdx.x, traced ? a.trace + 18 * 1024 + 16 * z : nullptr);
-                if (traced && threadIdx.x == 0) a.trace[17 * 1024 + 1000 + z] = tc2::gtime();
-                if (rp_next) {  // P_{k+1} is out: release the row-panel CTAs of this chain
-                    __threadfence();
-                    __syncthreads();
-                    if (threadIdx.x == 0) atomicExch(gj_flag(a, 0, kb, z), 1);
-                }
+            // The next pivot block is formed by the SAME tensor-core arithmetic as the update tile that owns it (same
+            // operand planes, chunking, draining): a 128 x 64 product whose Cin is the snapshot of X^(k)_{k+1,k+1}
+            // and whose result stays in shared memory.  Forming it with FP32 FMAs from the snapshot instead is more
+            // accurate per entry but no longer consistent with the rest of block row k+1, and costs a factor 1.4 in
+            // the wavefield error at 512^2 (tools/exp_accuracy.py: 9.5e-6 vs 6.7e-6).
+            static_assert(tc2::CH_LD == GJ_NB + 1, "pivot body reads the staged tile with row stride GJ_NB + 1");
+            const int z = bid, kb = k + 1, nP = a.g.nP;
+            const int row = chain_row(a.g, a.phase, z, a.step);
+            if (row < 0) { pdl_wait(); return; }
+            tc2::Tc2Tile t;
+            tc2::tile_no_emit(t);
+            t.bplanes = a.Rp + (size_t)(a.zb0 + z) * a.rp_stride;
+            t.amat = (k & 1) * a.nbmax + a.zb0 + z;
+            const cx<float>* S1 = a.snap + (size_t)(a.zb0 + z) * GJ_NB * GJ_NB;  // X^(k)_{k+1,k+1}
+            t.Cin = S1 - (size_t)(kb * GJ_NB) * GJ_NB - kb * GJ_NB; t.ldcin = GJ_NB;
+            t.Cout = nullptr; t.ldc = nP; t.keep = 1;
+            t.M = nP; t.N = nP; t.K = GJ_NB; t.Mstore = nP;
+            t.m0 = (kb >> 1) * tc2::TM; t.n0 = kb * GJ_NB;
+            t.mask_lo = 0; t.mask_hi = 0;
+            t.skip_lo = (kb ^ 1) * GJ_NB; t.skip_hi = t.skip_lo + GJ_NB;  // the sibling block of the 128-row tile is not needed
+            t.sgn = -1.f; t.bias_fix = bias_fix; t.drain_every = a.gj_drain;
+            const bool traced = a.trace && a.step == a.trace_step && k == a.trace_k && z < 24;
+            if (traced) {  // debugging: pivot CTAs use trace rows 1000 + z, their end-of-inversion stamp goes to column 17
+                t.trace = a.trace + 16 * (1000 + z);
+                if (threadIdx.x == 0) { unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); a.trace[16 * 1024 + 1000 + z] = smid; }
             }
+            tc2::cgemm_tile_h(t, &cmap, tc2_smem);
+            __syncthreads();
+            unsigned char* smem_al = tc2_smem + ((128u - (tc::smem_u32(tc2_smem) & 127u)) & 127u);
+            // the staged 128 x 65 tile holds the block (rows 64 (kb & 1) ..): invert it where it lies, scratch behind the tile
+            cx<float>* blk = reinterpret_cast<cx<float>*>(smem_al) + (size_t)(kb & 1) * GJ_NB * tc2::CH_LD;
+            cx<float>* scr = reinterpret_cast<cx<float>*>(smem_al) + (size_t)tc2::TM * tc2::CH_LD;
+            static_assert((size_t)tc2::TM * tc2::CH_LD * sizeof(cx<float>) + gj_pivot2_scratch_bytes <= (size_t)tc2::STAGES_H * tc2::STAGE_H,
+                          "pivot scratch must fit behind the staging tile inside the operand ring");
+            gj_pivot_blocked(a, z, blk, scr, threadIdx.x, traced ? a.trace + 18 * 1024 + 16 * z : nullptr);
+            if (traced && threadIdx.x == 0) a.trace[17 * 1024 + 1000 + z] = tc2::gtime();
             return;
         }
         bid -= a.nbatch;
     }
     const int nP = a.g.nP, nblk = nP / GJ_NB;
     const int tiles_m = (nP + tc2::TM - 1) / tc2::TM, tiles = (nP + TW - 1) / TW;
-    const int ntile_ctas = a.nbatch * tiles_m * tiles;
-    if (bid >= ntile_ctas) {
-        // ---- fused row panel k+1 ----
-        const int idx = bid - ntile_ctas, z = idx / tiles, ntile = idx % tiles, kn = k + 1;
-        const int row = chain_row(a.g, a.phase, z, a.step);
-        if (row < 0) { pdl_wait(); return; }
-        const int freq = a.f0 + chain_freq(a.phase, z);
-        // debugging (UST_TC2_TRACE_UPDATE): row-panel CTAs use trace rows 900 + idx, column 17 = the time they became resident
-        const bool traced = a.trace && a.step == a.trace_step && k == a.trace_k && idx < 96;
-        if (traced && threadIdx.x == 0) {
-            unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            a.trace[16 * 1024 + 900 + idx] = smid; a.trace[17 * 1024 + 900 + idx] = tc2::gtime();
-        }
-        // The flags of this block row were zeroed by its Schur launch.  With programmatic dependent launch this CTA can be resident
-        // before that launch has even passed its own wait (Schur -> k = 0 -> row panel 0 -> this launch all trigger at entry) and
-        // would then see the previous block row's flags: wait for the preceding launch (transitively: for the zeroing) first.
-        pdl_wait();
-        if (threadIdx.x == 0) {
-            const int* fp = gj_flag(a, 0, kn, z);
-            const int* fc = gj_flag(a, 1, kn, z);
-            unsigned spins = 0;
-            while (ld_acquire_gpu(fp) == 0 || ld_acquire_gpu(fc) < tiles) {
-                __nanosleep(100);
-                if (++spins > (1u << 22)) __trap();  // a protocol bug becomes a launch failure instead of a hang
-            }
-        }
-        __syncthreads();
-        // what the producers wrote with ordinary stores is read below by bulk / tensor copies (async proxy)
-        asm volatile("fence.proxy.async;" ::: "memory");
-        gj_rowpanel_tile(a, kn, z, row, freq, ntile, bias_fix, &pmap, tc2_smem, traced ? a.trace + 16 * (900 + idx) : nullptr);
-        return;
-    }
-    // tile CTAs: with fused row panels the tile row that holds pivot block row k+1 comes first, for all chains
-    int z, mt, nt;
-    const int first = (k + 1) >> 1;
-    if (rp_next) {
-        const int mt_local = bid / (a.nbatch * tiles), rem = bid % (a.nbatch * tiles);
-        z = rem / tiles; nt = rem % tiles;
-        mt = mt_local == 0 ? first : (mt_local <= first ? mt_local - 1 : mt_local);
-    } else {
-        z = bid / (tiles_m * tiles);
-        const int rem = bid % (tiles_m * tiles);
-        mt = rem / tiles; nt = rem % tiles;
-    }
+    const int z = bid / (tiles_m * tiles);
+    const int rem = bid % (tiles_m * tiles);
+    const int mt = rem / tiles, nt = rem % tiles;
     const int row = chain_row(a.g, a.phase, z, a.step);
     if (row < 0) { pdl_wait(); return; }
     const int freq = (a.f0 + chain_freq(a.phase, z));
     tc2::Tc2Tile t;
     tc2::tile_no_emit(t);
-    t.bplanes = gj_rp(a, k, z);
+    t.bplanes = a.Rp + (size_t)(a.zb0 + z) * a.rp_stride;
     t.amat = (k & 1) * a.nbmax + a.zb0 + z;
     t.Cin = gj_buffer(a, z, freq, row, k); t.ldcin = nP;
     t.Cout = gj_buffer(a, z, freq, row, k + 1); t.ldc = nP;
@@ -1232,317 +1111,6 @@ tc2_gj_update_kernel(FactorArgs<float> a, int k, float bias_fix, int pivot_next,
         if (threadIdx.x == 0) { unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); a.trace[16 * 1024 + bid] = smid; }
     }
     t.prefetch_cin = a.prefetch_cin;
-    // ping-pong schedules: the tile that owns X^(k+1)_{k+2,k+2} leaves a copy for the pivot CTA that forms P_{k+2} (the
-    // block is overwritten in place by the launch that needs the copy)
-    const int kk = k + 2;
-    const bool snap_next = a.pp && kk < nblk && t.m0 == (kk >> 1) * tc2::TM && t.n0 == kk * GJ_NB;
-    if (snap_next) t.keep = 1;
-    tc2::cgemm_tile_h(t, &cmap, tc2_smem);
-    if (snap_next) {
-        __syncthreads();
-        unsigned char* smem_al = tc2_smem + ((128u - (tc::smem_u32(tc2_smem) & 127u)) & 127u);
-        const cx<float>* blk = reinterpret_cast<const cx<float>*>(smem_al) + (size_t)(kk & 1) * GJ_NB * tc2::CH_LD;
-        cx<float>* __restrict__ S = a.snap + ((size_t)(kk & 1) * a.nbmax + a.zb0 + z) * GJ_NB * GJ_NB;
-#pragma unroll
-        for (int j = 0; j < GJ_NB * GJ_NB / tc2::NUM_THREADS_H; ++j) {
-            const int e = threadIdx.x + tc2::NUM_THREADS_H * j;
-            S[e] = blk[(e >> 6) * tc2::CH_LD + (e & 63)];
-        }
-    }
-    if (rp_next && mt == first) {  // a tile of the row that holds pivot block row k+1 is out (X, its B planes, its column-panel planes)
-        __threadfence();
-        __syncthreads();
-        if (threadIdx.x == 0) atomicAdd(gj_flag(a, 1, k + 1, z), 1);
-    }
-}
-
-// Deep look-ahead pivot kernel: P_j = inv(X^(j)_jj) for j >= 1, one CTA per chain, launched on a side stream as soon as
-// update j-2 has finished (j = 1: after the k = 0 preparation), i.e. BEFORE row panel j-1 -- it runs beside row panel j-1 and
-// update j-1 and is only awaited by row panel j, so the latency-bound 64 x 64 inversion is off the launch chain's critical path
-// (measured bound, tools/exp_bounds.py: a free pivot inversion is worth 53 of 297 ms at the benchmark batch).  What it needs
-// exists after update j-2: P_{j-1} (Pp, ping-pong), the pivot block row j-1 (Xp) and column panel j-1 (Cp) as planes, and the
-// snapshot of X^(j-1)_jj.  It forms the block with the arithmetic of the kernels that own it, so the result is bit-identical
-// to the schedule without look-ahead:
-//   1. R_{j-1}[:, j] = P_{j-1} X~_{j-1,j}      the row-panel tile of block column j (same operands, chunks, draining), emitted as
-//                                               B planes into the CTA's private buffer Rs
-//   2. X^(j)_jj = X^(j-1)_jj - X_{j,j-1} R_{j-1}[:, j]    the update tile that owns the block (Cin = snapshot), kept in shared memory
-//   3. blocked Gauss-Jordan inversion in shared memory, P_j out as A planes (Pp slot j & 1)
-// grid = nbatch CTAs, 256 threads, dynamic smem = SMEM_BYTES_H.
-__global__ void __launch_bounds__(tc2::NUM_THREADS_H, 2)
-tc2_gj_pivot_deep_kernel(FactorArgs<float> a, int j, float bias_fix, const __grid_constant__ CUtensorMap pmap, const __grid_constant__ CUtensorMap cmap) {
-    extern __shared__ __align__(1024) unsigned char tc2_smem[];
-    static_assert(tc2::CH_LD == GJ_NB + 1, "the pivot inversion reads the staged tile with row stride GJ_NB + 1");
-    pdl_trigger();
-    const int z = blockIdx.x, k = j - 1, nP = a.g.nP;
-    const int row = chain_row(a.g, a.phase, z, a.step);
-    if (row < 0) { pdl_wait(); return; }
-    uint16_t* Rs = a.Rs + (size_t)(a.zb0 + z) * a.rp_stride;
-    {
-        tc2::Tc2Tile t;
-        tc2::tile_no_emit(t);
-        t.bplanes = a.Xp + ((size_t)(k & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;
-        t.amat = (k & 1) * a.nbmax + a.zb0 + z;
-        t.Cin = nullptr; t.ldcin = nP;
-        t.Cout = nullptr; t.ldc = nP;
-        t.M = GJ_NB; t.N = nP; t.K = GJ_NB; t.Mstore = GJ_NB;
-        t.m0 = 0; t.n0 = j * GJ_NB;
-        t.mask_lo = 0; t.mask_hi = 0; t.skip_lo = 0; t.skip_hi = 0;
-        t.sgn = 1.f; t.bias_fix = bias_fix; t.drain_every = a.gj_drain;
-        t.eb_planes = Rs; t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0;
-        t.tmem_hold = 2;
-        tc2::cgemm_tile_h(t, &pmap, tc2_smem);
-    }
-    // the planes just written with ordinary stores are read back by bulk copies (async proxy) of the same CTA
-    __threadfence();
-    asm volatile("fence.proxy.async;" ::: "memory");
-    __syncthreads();
-    tc2::engine_h_release(tc2_smem);
-    {
-        tc2::Tc2Tile t;
-        tc2::tile_no_emit(t);
-        t.bplanes = Rs;
-        t.amat = (k & 1) * a.nbmax + a.zb0 + z;
-        const cx<float>* S1 = a.snap + ((size_t)(j & 1) * a.nbmax + a.zb0 + z) * GJ_NB * GJ_NB;  // X^(k)_{jj}
-        t.Cin = S1 - (size_t)(j * GJ_NB) * GJ_NB - j * GJ_NB; t.ldcin = GJ_NB;
-        t.Cout = nullptr; t.ldc = nP; t.keep = 1;
-        t.M = nP; t.N = nP; t.K = GJ_NB; t.Mstore = nP;
-        t.m0 = (j >> 1) * tc2::TM; t.n0 = j * GJ_NB;
-        t.mask_lo = 0; t.mask_hi = 0;
-        t.skip_lo = (j ^ 1) * GJ_NB; t.skip_hi = t.skip_lo + GJ_NB;  // the sibling block of the 128-row tile is not needed
-        t.sgn = -1.f; t.bias_fix = bias_fix; t.drain_every = a.gj_drain;
-        t.tmem_hold = 1;
-        tc2::cgemm_tile_h(t, &cmap, tc2_smem);
-    }
-    __syncthreads();
-    unsigned char* smem_al = tc2_smem + ((128u - (tc::smem_u32(tc2_smem) & 127u)) & 127u);
-    cx<float>* blk = reinterpret_cast<cx<float>*>(smem_al) + (size_t)(j & 1) * GJ_NB * tc2::CH_LD;
-    cx<float>* scr = reinterpret_cast<cx<float>*>(smem_al) + (size_t)tc2::TM * tc2::CH_LD;
-    FactorArgs<float> a2 = a;
-    a2.Pp = a.Pp + (size_t)(j & 1) * a.nbmax * tc2::NPL_A * GJ_NB * GJ_NB;
-    gj_pivot_blocked(a2, z, blk, scr, threadIdx.x);
-}
-
-// ---------------------------------------------------------------------------------------------
-// Two-level blocked Gauss-Jordan (outer block 128 = two pivot blocks a = 2K, b = 2K + 1).  OPT-IN (UST_GJ2=1): measured
-// equal to the classic scheme at the benchmark batch and slower for small batches (DESIGN.md section 6b).
-//
-// A rank-64 update visits every 128 x 64 tile of X once per pivot block: ~12 us of CTA life for 1.6 us of tensor work, and the
-// whole launch is bound by CTA slots.  Two consecutive pivot steps commute into ONE rank-128 update of all other block rows,
-//     X_i <- X~_i - [X_ia X_ib] [R_a'; R_b]          (i not in {a, b};  X_ia, X_ib taken BEFORE either step),
-// if the 128-row panel is finished first:
-//     R_a  = P_a X~_a,:                         row panel a                    (tc2_gj2_rowpanel_kernel, k = a)
-//     X_b,: <- X~_b,: - X_ba R_a                block row b only ("MINI"), look-ahead inversion of P_b rides on the launch
-//     R_b  = P_b X~_b,:                         row panel b                    (tc2_gj2_rowpanel_kernel, k = b)
-//     R_a' = R_a - R_ab R_b                     block row a only ("FIXA"; R_ab = R_a[:, b] is row a of column panel b)
-// so every tile outside the panel is visited half as often with twice the K (8 k-chunks per visit instead of 4).
-// Operand planes: Cp = A planes of the 128-wide column panel [X_:,a X_:,b] of outer step K (ping-pong on K; the 64-wide
-// halves are K-slices, Tc2Tile::a_k0), Rp = B planes of the 128-row panel [R_a'; R_b] (chunks 0-3 / 4-7, Tc2Tile::b_chunk0),
-// Xp = B planes of the 64-row pivot block row (ping-pong on the pivot step).  Every finished row emits its entries of the
-// NEXT outer step's column panel (or, after the last outer step, the inverse itself as the sweeps' A planes).
-// ---------------------------------------------------------------------------------------------
-constexpr int GJ_KB = 128;
-enum Gj2Mode { GJ2_MINI = 0, GJ2_FIXA = 1, GJ2_TRAIL = 2 };
-
-__device__ __forceinline__ uint16_t* gj2_cp(const FactorArgs<float>& a, int K, int z) {
-    return a.Cp + ((size_t)(K & 1) * a.nbmax + a.zb0 + z) * tc2::NPL_A * (size_t)a.g.nP * GJ_KB;
-}
-// finished rows -> next outer step's column panel, or after the last outer step the inverse planes
-__device__ __forceinline__ void gj2_emit_next(const FactorArgs<float>& a, tc2::Tc2Tile& t, int z, int freq, int row, int K, int row_off) {
-    const int nP = a.g.nP, nouter = nP / GJ_KB;
-    t.ea_row_off = row_off;
-    if (K + 1 < nouter) {
-        t.ea_planes = gj2_cp(a, K + 1, z);
-        t.ea_plane_elems = (unsigned)(nP * GJ_KB); t.ea_nbc = GJ_KB / 8;
-        t.ea_n_lo = (K + 1) * GJ_KB; t.ea_n_hi = (K + 2) * GJ_KB; t.ea_col_off = (K + 1) * GJ_KB;
-        t.ea_zero_from = 0x7fffffff;
-    } else {
-        const size_t mat = (size_t)freq * a.g.M + row;
-        t.ea_planes = a.Tp + mat * (size_t)tc2::NPL_A * nP * nP;
-        t.ea_plane_elems = (unsigned)(nP * nP); t.ea_nbc = nP / 8;
-        t.ea_n_lo = 0; t.ea_n_hi = nP; t.ea_col_off = 0;
-        t.ea_zero_from = a.g.nI;
-    }
-}
-
-// Column panel 0 (nP x 128, FP32) -> A planes.  grid.x = nP / 16 CTAs of 256 threads: thread = (block row I, block column J, row r).
-__device__ __forceinline__ void gj2_colsplit_body(const FactorArgs<float>& a, int z, int bx, int tid) {
-    const int row = chain_row(a.g, a.phase, z, a.step);
-    if (row < 0) return;
-    const int freq = a.f0 + chain_freq(a.phase, z);
-    const int nP = a.g.nP;
-    const cx<float>* __restrict__ Xc = gj_buffer(a, z, freq, row, 0);
-    const int I = bx * 2 + (tid >> 7), J = (tid >> 3) & 15, r = tid & 7;
-    const int rr = I * 8 + r;
-    if (rr >= nP) return;
-    const cx<float>* src = Xc + (size_t)rr * nP + J * 8;
-    float re[8], im[8];
-#pragma unroll
-    for (int c = 0; c < 8; ++c) { cx<float> v = src[c]; re[c] = v.re; im[c] = v.im; }
-    const size_t plane = (size_t)nP * GJ_KB;
-    tc2::store_a8(gj2_cp(a, 0, z) + ((size_t)I * (GJ_KB / 8) + J) * 64 + r * 8, plane, re, im);
-}
-
-// k = 0 preparation of the two-level scheme: [0, nrow) B planes of pivot block row 0, [nrow, nrow + ncol) A planes of the
-// first 128-wide column panel, nrow + ncol: inversion of pivot block 0 (only when the Schur launch does not carry it).
-__global__ void __launch_bounds__(256) gj2_k0_kernel(FactorArgs<float> a, int nrow, int ncol) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    pdl_trigger();
-    pdl_wait();
-    const int z = blockIdx.z, bx = blockIdx.x;
-    if (bx < nrow) {
-        if (threadIdx.x < 128) gj_rowsplit_body(a, 0, z, bx, threadIdx.x);
-    } else if (bx < nrow + ncol) {
-        gj2_colsplit_body(a, z, bx - nrow, threadIdx.x);
-    } else {
-        gj_pivot_blocked_global(a, 0, z, smem_raw, threadIdx.x);
-    }
-}
-
-// Row panel of pivot step k (two-level scheme): R_k = P_k X~_k,: -> block row k of X, B planes of R_k into its half of Rp,
-// and the entries of block row k that later panels need: k even (a): R_a[:, b] -> row a of the CURRENT column panel's second
-// half (the A operand of FIXA); k odd (b): row b of the NEXT outer step's column panel / of the inverse.
-// grid = (nP / 64 [+ 1 snapshot CTA], 1, nbatch), 256 threads.
-__global__ void __launch_bounds__(tc2::NUM_THREADS_H, 2)
-tc2_gj2_rowpanel_kernel(FactorArgs<float> a, int k, float bias_fix, const __grid_constant__ CUtensorMap pmap) {
-    extern __shared__ __align__(1024) unsigned char tc2_smem[];
-    constexpr int TW = tc2::TNH;
-    pdl_trigger();
-    const int z = blockIdx.z;
-    const int row = chain_row(a.g, a.phase, z, a.step);
-    if (row < 0) { pdl_wait(); return; }
-    const int freq = a.f0 + chain_freq(a.phase, z);
-    const int nP = a.g.nP, K = k >> 1;
-    if (blockIdx.x * TW >= nP) {
-        // snapshot of X_{k+1,k+1}: the Cin of the look-ahead pivot CTA of the next update launch (which overwrites it in place)
-        pdl_wait();
-        const cx<float>* __restrict__ Xc = gj_buffer(a, z, freq, row, k);
-        cx<float>* __restrict__ S = a.snap + (size_t)(a.zb0 + z) * GJ_NB * GJ_NB;
-        const int k1 = (k + 1) * GJ_NB;
-        constexpr int PER = GJ_NB * GJ_NB / 2 / 256;
-        float4 v[PER];
-#pragma unroll
-        for (int j = 0; j < PER; ++j) {
-            const int w = threadIdx.x + 256 * j, r = w >> 5, c2 = w & 31;
-            v[j] = *reinterpret_cast<const float4*>(Xc + (size_t)(k1 + r) * nP + k1 + 2 * c2);
-        }
-#pragma unroll
-        for (int j = 0; j < PER; ++j) reinterpret_cast<float4*>(S)[threadIdx.x + 256 * j] = v[j];
-        return;
-    }
-    tc2::Tc2Tile t;
-    tc2::tile_no_emit(t);
-    t.bplanes = a.Xp + ((size_t)(k & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;
-    t.amat = a.zb0 + z;
-    t.Cin = nullptr; t.ldcin = nP;
-    t.Cout = gj_buffer(a, z, freq, row, k) + (size_t)k * GJ_NB * nP; t.ldc = nP;
-    t.M = GJ_NB; t.N = nP; t.K = GJ_NB; t.Mstore = GJ_NB;
-    t.m0 = 0; t.n0 = blockIdx.x * TW;
-    t.mask_lo = 0; t.mask_hi = 0; t.skip_lo = 0; t.skip_hi = 0;
-    t.sgn = 1.f;
-    t.bias_fix = bias_fix;
-    t.drain_every = a.gj_drain;
-    t.eb_planes = a.Rp + (size_t)(a.zb0 + z) * a.rp2_stride; t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0;
-    t.eb_chunks = GJ_KB / tc2::KC; t.eb_chunk0 = (k & 1) * (GJ_NB / tc2::KC);
-    if ((k & 1) == 0) {
-        t.ea_row_off = k * GJ_NB;
-        t.ea_planes = gj2_cp(a, K, z);
-        t.ea_plane_elems = (unsigned)(nP * GJ_KB); t.ea_nbc = GJ_KB / 8;
-        t.ea_n_lo = (k + 1) * GJ_NB; t.ea_n_hi = (k + 2) * GJ_NB; t.ea_col_off = k * GJ_NB;
-        t.ea_zero_from = 0x7fffffff;
-    } else {
-        gj2_emit_next(a, t, z, freq, row, K, k * GJ_NB);
-    }
-    tc2::cgemm_tile_h(t, &pmap, tc2_smem);
-}
-
-// The three update launches of an outer step (see the header of this section).  1-D grid: [nbatch look-ahead pivot CTAs
-// (MINI: P_b, TRAIL: P_{a+2})] + nbatch * (m-tiles of the mode) * (nP / 64) tile CTAs, 256 threads.
-__global__ void __launch_bounds__(tc2::NUM_THREADS_H, 2)
-tc2_gj2_update_kernel(FactorArgs<float> a, int k, int mode, float bias_fix, int pivot_next, const __grid_constant__ CUtensorMap cmap) {
-    extern __shared__ __align__(1024) unsigned char tc2_smem[];
-    constexpr int TW = tc2::TNH;
-    pdl_trigger();
-    const int nP = a.g.nP, nblk = nP / GJ_NB, K = k >> 1;
-    const int ka = 2 * K, kbk = 2 * K + 1;  // the two pivot blocks of this outer step
-    int bid = blockIdx.x;
-    if (pivot_next) {
-        if (bid < a.nbatch) {
-            // look-ahead pivot CTA: forms the next pivot block with the arithmetic of the tile that owns it (same planes, chunks,
-            // draining; Cin = the snapshot taken by the preceding row-panel launch) and inverts it in shared memory
-            static_assert(tc2::CH_LD == GJ_NB + 1, "the pivot inversion reads the staged tile with row stride GJ_NB + 1");
-            const int z = bid, kn = mode == GJ2_MINI ? k + 1 : ka + 2;
-            const int row = chain_row(a.g, a.phase, z, a.step);
-            if (row < 0 || (a.exp & 2)) { pdl_wait(); return; }
-            tc2::Tc2Tile t;
-            tc2::tile_no_emit(t);
-            t.bplanes = a.Rp + (size_t)(a.zb0 + z) * a.rp2_stride;
-            t.b_chunks = GJ_KB / tc2::KC; t.b_chunk0 = 0;
-            t.amat = (K & 1) * a.nbmax + a.zb0 + z; t.a_k0 = 0;
-            const cx<float>* S1 = a.snap + (size_t)(a.zb0 + z) * GJ_NB * GJ_NB;
-            t.Cin = S1 - (size_t)(kn * GJ_NB) * GJ_NB - kn * GJ_NB; t.ldcin = GJ_NB;
-            t.Cout = nullptr; t.ldc = nP; t.keep = 1;
-            t.M = nP; t.N = nP; t.K = mode == GJ2_MINI ? GJ_NB : GJ_KB; t.Mstore = nP;
-            t.m0 = (kn >> 1) * tc2::TM; t.n0 = kn * GJ_NB;
-            t.mask_lo = 0; t.mask_hi = 0;
-            t.skip_lo = (kn ^ 1) * GJ_NB; t.skip_hi = t.skip_lo + GJ_NB;  // the sibling block of the 128-row tile is not needed
-            t.sgn = -1.f; t.bias_fix = bias_fix; t.drain_every = a.gj_drain;
-            tc2::cgemm_tile_h(t, &cmap, tc2_smem);
-            __syncthreads();
-            if (a.exp & 1) return;
-            unsigned char* smem_al = tc2_smem + ((128u - (tc::smem_u32(tc2_smem) & 127u)) & 127u);
-            cx<float>* blk = reinterpret_cast<cx<float>*>(smem_al) + (size_t)(kn & 1) * GJ_NB * tc2::CH_LD;
-            cx<float>* scr = reinterpret_cast<cx<float>*>(smem_al) + (size_t)tc2::TM * tc2::CH_LD;
-            gj_pivot_blocked(a, z, blk, scr, threadIdx.x);
-            return;
-        }
-        bid -= a.nbatch;
-    }
-    const int tiles = nP / TW, tiles_m = nP / tc2::TM;
-    const int mt_count = mode == GJ2_TRAIL ? tiles_m - 1 : 1;
-    const int z = bid / (mt_count * tiles), rem = bid % (mt_count * tiles);
-    const int row = chain_row(a.g, a.phase, z, a.step);
-    if (row < 0) { pdl_wait(); return; }
-    const int freq = a.f0 + chain_freq(a.phase, z);
-    int mt = rem / tiles;
-    if (mode == GJ2_TRAIL) mt += (mt >= K) ? 1 : 0;  // every 128-row tile but the panel's own
-    else mt = K;
-    tc2::Tc2Tile t;
-    tc2::tile_no_emit(t);
-    t.bplanes = a.Rp + (size_t)(a.zb0 + z) * a.rp2_stride;
-    t.b_chunks = GJ_KB / tc2::KC;
-    t.amat = (K & 1) * a.nbmax + a.zb0 + z;
-    t.Cin = gj_buffer(a, z, freq, row, k); t.ldcin = nP;
-    t.Cout = gj_buffer(a, z, freq, row, k + 1); t.ldc = nP;
-    t.M = nP; t.N = nP; t.Mstore = nP;
-    t.m0 = mt * tc2::TM; t.n0 = (rem % tiles) * TW;
-    t.sgn = -1.f;
-    t.bias_fix = bias_fix;
-    t.drain_every = a.gj_drain;
-    t.prefetch_cin = a.prefetch_cin;
-    if (mode == GJ2_MINI) {          // block row b: X_b,: <- X~_b,: - X_ba R_a
-        t.K = GJ_NB; t.a_k0 = 0; t.b_chunk0 = 0;
-        t.mask_lo = ka * GJ_NB; t.mask_hi = (ka + 1) * GJ_NB;
-        t.skip_lo = ka * GJ_NB; t.skip_hi = (ka + 1) * GJ_NB;
-        t.eb_planes = a.Xp + ((size_t)(kbk & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;   // pivot block row b for its row panel
-        t.eb_m_lo = kbk * GJ_NB; t.eb_id_lo = kbk * GJ_NB; t.eb_id_hi = (kbk + 1) * GJ_NB;
-    } else if (mode == GJ2_FIXA) {   // block row a: R_a' = R_a - R_ab R_b
-        t.K = GJ_NB; t.a_k0 = GJ_NB; t.b_chunk0 = GJ_NB / tc2::KC;
-        t.mask_lo = kbk * GJ_NB; t.mask_hi = (kbk + 1) * GJ_NB;
-        t.skip_lo = kbk * GJ_NB; t.skip_hi = (kbk + 1) * GJ_NB;
-        t.eb_planes = a.Rp + (size_t)(a.zb0 + z) * a.rp2_stride;                         // R_a' replaces R_a in the 128-row panel
-        t.eb_chunks = GJ_KB / tc2::KC; t.eb_chunk0 = 0;
-        t.eb_m_lo = ka * GJ_NB; t.eb_id_lo = 0; t.eb_id_hi = 0;
-        gj2_emit_next(a, t, z, freq, row, K, 0);
-    } else {                         // every other block row: rank-128 update
-        t.K = GJ_KB; t.a_k0 = 0; t.b_chunk0 = 0;
-        t.mask_lo = ka * GJ_NB; t.mask_hi = (ka + 2) * GJ_NB;
-        t.skip_lo = 0; t.skip_hi = 0;
-        if (ka + 2 < nblk) {
-            t.eb_planes = a.Xp + ((size_t)((ka + 2) & 1) * a.nbmax + a.zb0 + z) * a.rp_stride;  // next pivot block row a'
-            t.eb_m_lo = (ka + 2) * GJ_NB; t.eb_id_lo = (ka + 2) * GJ_NB; t.eb_id_hi = (ka + 3) * GJ_NB;
-        }
-        gj2_emit_next(a, t, z, freq, row, K, 0);
-    }
     tc2::cgemm_tile_h(t, &cmap, tc2_smem);
 }
 

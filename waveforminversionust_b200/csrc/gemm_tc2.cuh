@@ -222,15 +222,6 @@ struct Tc2Tile {
     int prefetch_cin;              // L2 prefetch of the Cin tile when the CTA starts
     int keep;                      // 128 x 64 form: leave the finished tile (Cin + sgn*A*B, live rows) in the shared-memory staging
                                    // tile [128][65] at the 128-byte aligned base of the dynamic shared memory; Cout may be null
-    // 128 x 64 form, operands that are a K-slice of wider plane buffers (two-level Gauss-Jordan: 128-wide column panels and
-    // 128-row row panels whose 64-wide halves are separate operands):
-    int a_k0;                      // first K index of the A operand inside its planes (multiple of 16)
-    int b_chunks, b_chunk0;        // k-chunks per 128-column tile in `bplanes` (0 = K/16) and the first chunk of this operand
-    int eb_chunks, eb_chunk0;      // same for the emitted B planes (0 = 64/16: a 64-row buffer)
-    // 128 x 64 form, a CTA that runs two products back to back (deep look-ahead pivot CTAs): tensor memory is allocated once -- a CTA
-    // may not allocate again after relinquishing its permit --: bit 1 = keep the allocation at the end (first product),
-    // bit 0 = reuse the allocation of the previous product (its address is still in the shared-memory slot)
-    int tmem_hold;
     // 128 x 128 form launched as clusters of two or four CTAs (split K): CTA rank r computes its share of the k-chunks, all stage
     // their partial tile, rank 0 adds the others' through distributed shared memory (in rank order) and writes the result (no
     // emission in this mode).
@@ -239,8 +230,7 @@ struct Tc2Tile {
 };
 __host__ __device__ __forceinline__ void tile_no_emit(Tc2Tile& t) {
     t.ea_planes = nullptr; t.ea_plane_elems = 0; t.ea_nbc = 0; t.ea_n_lo = 0; t.ea_n_hi = 0; t.ea_col_off = 0; t.ea_row_off = 0;
-    t.drain_every = 1; t.ea_zero_from = 0x7fffffff; t.eb_planes = nullptr; t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0; t.trace = nullptr; t.prefetch_cin = 0; t.keep = 0;
-    t.a_k0 = 0; t.b_chunks = 0; t.b_chunk0 = 0; t.eb_chunks = 0; t.eb_chunk0 = 0; t.tmem_hold = 0; t.ksplit = 0;
+    t.drain_every = 1; t.ea_zero_from = 0x7fffffff; t.eb_planes = nullptr; t.eb_m_lo = 0; t.eb_id_lo = 0; t.eb_id_hi = 0; t.trace = nullptr; t.prefetch_cin = 0; t.keep = 0; t.ksplit = 0;
 }
 
 static_assert(sizeof(Tc2Tile) <= 384, "tile descriptor must fit in its shared-memory slot");

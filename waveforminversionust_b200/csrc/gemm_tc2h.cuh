@@ -35,18 +35,6 @@ static_assert(2 * (SMEM_BYTES_H + 1024) <= 227 * 1024, "two CTAs per SM");
 constexpr uint32_t TMEM_COLS_H = 256;                       // D1 = cols [0,128), D2 = cols [128,256)
 constexpr uint32_t IDESC_N64 = IDESC_BASE | ((64u >> 3) << 17);
 
-// A CTA that runs cgemm_tile_h a second time must give the mbarrier words back first (initialising a live mbarrier object is
-// undefined).  Call after every thread has left the first product.
-__device__ __forceinline__ void engine_h_release(unsigned char* smem_raw) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const uint32_t smem_base = (smem_u32(smem_raw) + 127u) & ~127u;
-        const uint32_t bar_base = smem_base + STAGES_H * STAGE_H;
-        for (int i = 0; i < 2 * STAGES_H + 3; ++i) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(bar_base + 8u * i) : "memory");
-    }
-    __syncthreads();
-}
-
 __device__ __forceinline__ void cgemm_tile_h(const Tc2Tile& t_in, const CUtensorMap* amap, unsigned char* smem_raw) {
     typedef cx<float> C;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -75,10 +63,8 @@ __device__ __forceinline__ void cgemm_tile_h(const Tc2Tile& t_in, const CUtensor
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         }
         __syncwarp();
-        if (!(t_in.tmem_hold & 1)) {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS_H) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(TMEM_COLS_H) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -91,15 +77,14 @@ __device__ __forceinline__ void cgemm_tile_h(const Tc2Tile& t_in, const CUtensor
     const int D = t.drain_every < 1 ? 1 : (t.drain_every > nk ? nk : t.drain_every);  // D1 is drained every D chunks
 
     // B source of this 64-column half: chunk c of the 128-column tile tn, plane p: re rows at +2048*half, im rows at +4096+2048*half
-    const int bch = t.b_chunks > 0 ? t.b_chunks : nk;
-    const unsigned char* bsrc = reinterpret_cast<const unsigned char*>(t.bplanes) + ((size_t)(t.n0 / TN) * bch + t.b_chunk0) * B_STAGE + ((t.n0 % TN) / TNH) * 2048;
-    const int am0 = t.m0, amat = t.amat, ak0 = t.a_k0;
+    const unsigned char* bsrc = reinterpret_cast<const unsigned char*>(t.bplanes) + (size_t)(t.n0 / TN) * nk * B_STAGE + ((t.n0 % TN) / TNH) * 2048;
+    const int am0 = t.m0, amat = t.amat;
     // one chunk = 1 tensor copy (A) + 6 bulk copies (B), issued warp-convergently by warp 0 (one elected lane)
     auto load_chunk = [&](int c) {
         const int s = c % STAGES_H;
         const uint32_t sa = smem_base + s * STAGE_H, sb = sa + A_STAGE;
         mbar_expect_tx_e(full_bar(s), STAGE_H);
-        tma_load_5d_e(sa, amap, full_bar(s), 0, (ak0 + c * KC) >> 3, am0 >> 3, 0, amat);  // box {64, 2, 16, 6, 1}
+        tma_load_5d_e(sa, amap, full_bar(s), 0, (c * KC) >> 3, am0 >> 3, 0, amat);  // box {64, 2, 16, 6, 1}
         const unsigned char* bc = bsrc + (size_t)c * B_STAGE;
 #pragma unroll
         for (int p = 0; p < NPL_B; ++p) {
@@ -230,7 +215,7 @@ __device__ __forceinline__ void cgemm_tile_h(const Tc2Tile& t_in, const CUtensor
     if (warp == 3) TC2_TRACE(11);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (warp == 2 && !(t_in.tmem_hold & 2)) {  // the accumulators are in shared memory: give the TMEM columns back early (the co-resident CTA may be waiting)
+    if (warp == 2) {  // the accumulators are in shared memory: give the TMEM columns back early (the co-resident CTA may be waiting)
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(TMEM_COLS_H) : "memory");
     }
@@ -311,8 +296,7 @@ __device__ __forceinline__ void cgemm_tile_h(const Tc2Tile& t_in, const CUtensor
                     if (n >= tl.N) v = cxzero<float>();
                     re[c] = v.re; im[c] = v.im;
                 }
-                const int ech = tl.eb_chunks > 0 ? tl.eb_chunks : 64 / KC;
-                uint16_t* chunk = tl.eb_planes + ((size_t)(n / TN) * ech + tl.eb_chunk0 + (kg >> 1)) * (B_STAGE / 2);
+                uint16_t* chunk = tl.eb_planes + ((size_t)(n / TN) * (64 / KC) + (kg >> 1)) * (B_STAGE / 2);
                 store_b8(chunk, n % TN, kg & 1, re, im);
             }
         }

@@ -45,19 +45,14 @@ struct ust_plan {
     int ngroups = 2;
     cudaStream_t side[MAX_GROUPS] = {};
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS] = {};
-    // deep look-ahead of the Gauss-Jordan pivot inversions: one high-priority side stream per group, forked / joined with events
-    bool deep = false;    // UST_DEEP=0 selects the pivot CTAs riding on the update launches
+    // complex128 look-ahead of the Gauss-Jordan pivot inversions: one high-priority side stream per group, forked / joined with events
     cudaStream_t pivst[MAX_GROUPS] = {};
     cudaEvent_t ev_upd[MAX_GROUPS] = {}, ev_piv[MAX_GROUPS][2] = {};
-    uint16_t* Rs = nullptr;  // private B planes of the deep look-ahead pivot CTAs
-    bool fuse = false;       // row panel k+1 as trailing CTAs of update launch k (UST_FUSE_RP=0 disables)
-    int* gj_flags = nullptr; // in-launch flags of the fused row panels
     uint16_t *Tp = nullptr, *Wp = nullptr;  // bf16 operand planes of the TC2 engine
     void* snap = nullptr;
     uint16_t *Rp = nullptr, *Cp = nullptr, *Xp = nullptr, *Pp = nullptr;  // panel / pivot planes of the TC2 Gauss-Jordan kernels
-    size_t rp_stride = 0, rp2_stride = 0;
-    bool gj2 = false;  // two-level Gauss-Jordan (outer block 128): UST_GJ2=0 selects the classic rank-64 scheme
-    CUtensorMap cmaps[2], cmaps2[2], pmaps[2];
+    size_t rp_stride = 0;
+    CUtensorMap cmaps[2], pmaps[2];
     size_t wp_stride = 0;
     int kpad = 0;
     int gj_drain = 1, sweep_drain = 1;  // drain periods of the leading accumulator (UST_TC2_GJ_DRAIN / UST_TC2_SWEEP_DRAIN)
@@ -101,13 +96,11 @@ struct ust_plan {
     cudaStream_t own_stream = nullptr;
     unsigned long long* trace = nullptr;  // UST_TC2_TRACE_UPDATE=step,k: in-situ phase timestamps of one update launch
     int trace_step = -1, trace_k = -1;
-    bool schur_pivot0 = true;  // pivot block 0 inverted by the Schur CTA that computes it (UST_NO_SCHUR_PIVOT=1: by the k = 0 launch)
     int pdl_min_batch = 8;  // programmatic dependent launch only when the launch chains in flight carry more matrices than this in total
                             // (UST_PDL_MIN_BATCH; measured: 4 frequencies on one chain 145 vs 153 ms without / with, 8 frequencies on two chains 181 vs 177)
     int active_groups = 1;
     int eval_nfreq = 1;     // frequencies of the evaluation being enqueued (all groups)
     int ksplit_ok = 2;      // largest split-K cluster of the sweep GEMM (UST_KSPLIT = 1 (off), 2 or 4; measured at 2 frequencies: 43.2 / 33.7 / 40.7 ms of sweep GEMM)
-    int exp = 0;  // UST_EXP: timing experiments (factor.cuh FactorArgs::exp); results are wrong when set
     bool lookahead = true;  // next pivot block inverted by extra CTAs of the update launch (UST_NO_LOOKAHEAD=1 disables)
     // optional per-kernel-class device timing (ust_profile): event pairs around every launch
     bool prof = false;
@@ -218,113 +211,53 @@ static int gj_invert_batch(ust_plan* p, int phase, int step, int f0, int nf, cud
                           (long long)nbatch * p->active_groups * cdiv_i(g.nP, tc2::TM) * (g.nP / tc2::TNH) > 2LL * p->num_sms;
     a.planes = (const cx<R>*)p->planes; a.T = (cx<R>*)p->T; a.scratch = (cx<R>*)p->scratch; a.pbuf = (cx<R>*)p->pbuf; a.status = p->d_status;
     a.Rp = p->Rp; a.Cp = p->Cp; a.Xp = p->Xp; a.Pp = p->Pp; a.Tp = p->Tp; a.rp_stride = p->rp_stride; a.nbmax = 2 * p->d.max_freq;
-    a.rp2_stride = p->rp2_stride; a.kb = p->gj2 ? GJ_KB : GJ_NB;
     a.inplace = p->use_tc2 ? 1 : 0; a.gj_drain = p->gj_drain; a.snap = (cx<R>*)p->snap;
     a.trace = p->trace; a.trace_step = p->trace_step; a.trace_k = p->trace_k;
-    a.prefetch_cin = p->prefetch_cin; a.exp = p->exp;
-    a.deep = (p->deep && g.nP / GJ_NB > 1) ? 1 : 0; a.Rs = p->Rs;
-    a.fuse = (p->fuse && !p->deep && p->lookahead && g.nP / GJ_NB > 1 && g.nP / GJ_NB <= GJ_MAXBLK) ? 1 : 0;
-    a.pp = (a.deep || a.fuse) ? 1 : 0; a.flags = p->gj_flags;
+    a.prefetch_cin = p->prefetch_cin;
     const int nblk = g.nP / GJ_NB;
     {
         dim3 grid(cdiv_i(g.nP, SchurTile<R>::TS), cdiv_i(g.nP, SchurTile<R>::TS), nbatch), block(16, 16);
         // TMA-fed engine: the CTA of tile (0, 0) also inverts it (= pivot block 0) and emits P_0
-        const int pivot0 = (sizeof(R) == 4 && p->use_tc2 && p->schur_pivot0) ? 1 : 0;
+        const int pivot0 = (sizeof(R) == 4 && p->use_tc2) ? 1 : 0;
         ProfScope ps(p, PC_SCHUR, st);
         UST_CUDA(launch_pdl(schur_kernel<R>, grid, block, pivot0 ? gj_pivot2_scratch_bytes : 0, st, a, pivot0));
         UST_LAUNCH_CHECK();
     }
     const size_t smem = gj_rowpanel_smem<R>();
     if constexpr (sizeof(R) == 4) {
-        if (p->use_tc2 && p->gj2) {
-            // two-level scheme (factor.cuh, "Two-level blocked Gauss-Jordan"): per outer step of two pivot blocks a, b:
-            //   row panel a | MINI (block row b) + look-ahead P_b | row panel b | FIXA (block row a) | TRAIL (rank 128) + look-ahead P_a'
-            {
-                ProfScope ps(p, PC_GJ_K0, st);
-                const int nrow = cdiv_i(g.nP, tc2::TN), ncol = g.nP / 16;
-                UST_CUDA(launch_pdl(gj2_k0_kernel, dim3(nrow + ncol + (p->schur_pivot0 ? 0 : 1), 1, nbatch), dim3(256), gj_pivot2_smem_bytes, st, a, nrow, ncol));
-            }
-            UST_LAUNCH_CHECK();
-            const int tiles_h = g.nP / tc2::TNH, tiles_m = g.nP / tc2::TM;
-            auto rowpanel = [&](int k) -> int {
-                if (p->exp & 4) return 0;
-                ProfScope ps(p, PC_GJ_ROWPANEL, st);
-                const int snap_cta = (k + 1 < nblk) ? 1 : 0;
-                UST_CUDA(launch_pdl(tc2_gj2_rowpanel_kernel, dim3(tiles_h + snap_cta, 1, nbatch), dim3(tc2::NUM_THREADS_H), tc2::SMEM_BYTES_H, st, a, k, p->bias_fix, p->pmaps[0]));
-                UST_LAUNCH_CHECK();
-                return 0;
-            };
-            auto update = [&](int k, int mode, int mt_count, int pivot_next) -> int {
-                // profile classes: TRAIL = gj_update, MINI = gj_panel, FIXA = gj_pivot (the classic scheme's meanings of the last two do not occur here)
-                ProfScope ps(p, mode == GJ2_TRAIL ? PC_GJ_UPDATE : (mode == GJ2_MINI ? PC_GJ_PANEL : PC_GJ_PIVOT), st);
-                UST_CUDA(launch_pdl(tc2_gj2_update_kernel, dim3(nbatch * mt_count * tiles_h + (pivot_next ? nbatch : 0)), dim3(tc2::NUM_THREADS_H),
-                                    tc2::SMEM_BYTES_H, st, a, k, mode, p->bias_fix, pivot_next, p->cmaps2[0]));
-                UST_LAUNCH_CHECK();
-                return 0;
-            };
-            for (int K = 0; K < nblk / 2; ++K) {
-                const int ka = 2 * K, kbk = ka + 1;
-                UST_TRY(rowpanel(ka));
-                UST_TRY(update(ka, GJ2_MINI, 1, 1));
-                UST_TRY(rowpanel(kbk));
-                UST_TRY(update(kbk, GJ2_FIXA, 1, 0));
-                if (tiles_m > 1) UST_TRY(update(ka, GJ2_TRAIL, tiles_m - 1, ka + 2 < nblk ? 1 : 0));
-            }
-            return 0;
-        }
         if (p->use_tc2) {
             // everything GEMM-shaped on the TMA-fed tensor-core engine; operands travel between the kernels as bf16 planes
-            const bool deep = a.deep != 0;
             {
-                // block row 0 -> B planes, block column 0 -> A planes, pivot block 0 inverted: one launch, three CTA roles
-                // (deep look-ahead: a fourth one copies X^(0)_11 for the pivot CTA of P_1)
+                // block row 0 -> B planes, block column 0 -> A planes: one launch, two CTA roles
                 ProfScope ps(p, PC_GJ_K0, st);
                 const int nrow = cdiv_i(g.nP, tc2::TN), ncol = nblk > 1 ? cdiv_i(g.nP, 32) : 0;
-                UST_CUDA(launch_pdl(gj_k0_kernel, dim3(nrow + ncol + (a.pp ? 1 : 0) + (p->schur_pivot0 ? 0 : 1), 1, nbatch), dim3(256), gj_pivot2_smem_bytes, st, a, nrow, ncol, a.pp));
+                UST_CUDA(launch_pdl(gj_k0_kernel, dim3(nrow + ncol, 1, nbatch), dim3(256), 0, st, a, nrow));
             }
             UST_LAUNCH_CHECK();
-            const bool la = p->lookahead && nblk > 1 && !deep;
+            const bool la = p->lookahead && nblk > 1;
             const int tiles = cdiv_i(g.nP, tc2::TN), tiles_h = cdiv_i(g.nP, tc2::TNH);
-            cudaStream_t ps_st = p->pivst[gidx];
-            // deep look-ahead: P_j (j >= 1) is inverted on the side stream beside row panel j-1 and update j-1; it starts when
-            // update j-2 (j = 1: the k = 0 preparation) is done and is awaited by row panel j only
-            auto pivot_deep = [&](int j) -> int {
-                UST_CUDA(cudaEventRecord(p->ev_upd[gidx], st));
-                UST_CUDA(cudaStreamWaitEvent(ps_st, p->ev_upd[gidx], 0));
-                {
-                    ProfScope p1(p, PC_GJ_PIVOT, ps_st);
-                    UST_CUDA(launch_pdl(tc2_gj_pivot_deep_kernel, dim3(nbatch), dim3(tc2::NUM_THREADS_H), tc2::SMEM_BYTES_H, ps_st, a, j, p->bias_fix, p->pmaps[0], p->cmaps[0]));
-                }
-                UST_LAUNCH_CHECK();
-                UST_CUDA(cudaEventRecord(p->ev_piv[gidx][j & 1], ps_st));
-                return 0;
-            };
-            if (deep) UST_TRY(pivot_deep(1));
             for (int k = 0; k < nblk; ++k) {
                 {
                     ProfScope ps(p, PC_GJ_PANEL, st);
-                    if (k > 0 && !la && !deep) {  // otherwise P_k came from the k = 0 launch / the look-ahead CTAs of the previous update launch
+                    if (k > 0 && !la) {  // otherwise P_k came from the Schur launch / the look-ahead CTAs of the previous update launch
                         ProfScope p1(p, PC_GJ_PIVOT, st);
                         UST_CUDA(launch_pdl(gj_pivot_kernel<R>, dim3(1, 1, nbatch), dim3(256), gj_pivot2_smem_bytes, st, a, k, 0));
                         UST_LAUNCH_CHECK();
                     }
-                    if (k > 0 && deep) UST_CUDA(cudaStreamWaitEvent(st, p->ev_piv[gidx][k & 1], 0));
-                    if (!(p->exp & 4) && (!a.fuse || k == 0)) {  // fused schedule: row panel k >= 1 ran inside update launch k-1
+                    {
                         ProfScope p2(p, PC_GJ_ROWPANEL, st);
-                        const int snap_cta = (la && !a.pp && k + 1 < nblk) ? 1 : 0;
+                        const int snap_cta = (la && k + 1 < nblk) ? 1 : 0;
                         UST_CUDA(launch_pdl(tc2_gj_rowpanel_kernel, dim3(tiles_h + snap_cta, 1, nbatch), dim3(tc2::NUM_THREADS_H), tc2::SMEM_BYTES_H, st, a, k, p->bias_fix, p->pmaps[0]));
                     }
                     UST_LAUNCH_CHECK();
                 }
                 if (nblk > 1) {
                     const int pivot_next = (la && k + 1 < nblk) ? 1 : 0;
-                    const int rp_next = (a.fuse && k + 1 < nblk && !(p->exp & 4)) ? 1 : 0;
                     ProfScope ps(p, PC_GJ_UPDATE, st);
-                    UST_CUDA(launch_pdl(tc2_gj_update_kernel, dim3(nbatch * tiles * tiles_h + (pivot_next ? nbatch : 0) + (rp_next ? nbatch * tiles_h : 0)), dim3(tc2::NUM_THREADS_H),
-                                        tc2::SMEM_BYTES_H, st, a, k, p->bias_fix, pivot_next, rp_next, p->cmaps[0], p->pmaps[0]));
+                    UST_CUDA(launch_pdl(tc2_gj_update_kernel, dim3(nbatch * tiles * tiles_h + (pivot_next ? nbatch : 0)), dim3(tc2::NUM_THREADS_H),
+                                        tc2::SMEM_BYTES_H, st, a, k, p->bias_fix, pivot_next, p->cmaps[0]));
                     UST_LAUNCH_CHECK();
                 }
-                if (deep && k + 2 < nblk) UST_TRY(pivot_deep(k + 2));
             }
             return 0;
         }
@@ -446,7 +379,7 @@ template <typename R>
 static int factor_groups(ust_plan* p, const void* vel_dev, const std::vector<Group>& gs, bool lossy = false) {
     const Geom& g = p->g;
     AsmArgs aa;
-    aa.g = g; aa.h = p->h; aa.gr = p->gr; aa.stencil = p->d.stencil; aa.exp = (p->exp & 8) ? 1 : 0;
+    aa.g = g; aa.h = p->h; aa.gr = p->gr; aa.stencil = p->d.stencil;
     for (const Group& q : gs)
         for (int c0 = 0; c0 < q.nf; c0 += ASM_MAXF) {
             const int f0 = q.f0 + c0;
@@ -949,7 +882,6 @@ template <typename R>
 static int set_kernel_attrs() {
     UST_CUDA(cudaFuncSetAttribute(gj_pivot_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)std::max(gj_pivot_smem<R>(), sizeof(R) == 4 ? gj_pivot2_smem_bytes : gj_pivot_f64_smem_bytes)));
-    if (sizeof(R) == 4) UST_CUDA(cudaFuncSetAttribute(gj_k0_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gj_pivot2_smem_bytes));
     // static tiles (38 KB) + the dynamic scratch of the blocked pivot-0 inversion exceed the 48 KB a kernel gets without opting in
     if (sizeof(R) == 4) UST_CUDA(cudaFuncSetAttribute(schur_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gj_pivot2_scratch_bytes));
 
@@ -959,10 +891,6 @@ static int set_kernel_attrs() {
         UST_CUDA(cudaFuncSetAttribute(tc2_sweep_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES));
         UST_CUDA(cudaFuncSetAttribute(tc2_gj_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
         UST_CUDA(cudaFuncSetAttribute(tc2_gj_rowpanel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
-        UST_CUDA(cudaFuncSetAttribute(tc2_gj_pivot_deep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
-        UST_CUDA(cudaFuncSetAttribute(tc2_gj2_rowpanel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
-        UST_CUDA(cudaFuncSetAttribute(tc2_gj2_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
-        UST_CUDA(cudaFuncSetAttribute(gj2_k0_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gj_pivot2_smem_bytes));
         UST_CUDA(cudaFuncSetAttribute(tc2h_test_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES_H));
         UST_CUDA(cudaFuncSetAttribute(tc2_test_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES));
         UST_CUDA(cudaFuncSetAttribute(tc2_test_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc2::SMEM_BYTES));
@@ -1056,25 +984,6 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
     Geom& g = p->g;
     g.Nx = d->nx; g.Ny = d->ny; g.nI = d->nx - 2; g.M = d->ny - 2;
     g.nP = ((g.nI + GJ_NB - 1) / GJ_NB) * GJ_NB;
-    const bool want_tc2 = d->dtype == UST_C64 && (d->engine == UST_ENGINE_TC2 || d->engine == UST_ENGINE_AUTO);
-    // Two-level scheme: measured equal to the classic rank-64 scheme at the benchmark batch (296 vs 293 ms) and slower for small
-    // batches (cfg4, one frequency: 705 vs 633 ms) -- both are bound by the chain pivot inversion -> row panel, which it does not
-    // shorten (DESIGN.md section 6b) -- so it is opt-in.
-    p->gj2 = false;
-    if (const char* e = getenv("UST_GJ2")) p->gj2 = want_tc2 && atoi(e) != 0;
-    if (const char* e = getenv("UST_NO_LOOKAHEAD")) { if (atoi(e) != 0) p->gj2 = false; }  // the two-level scheme is built on the look-ahead pivots
-    if (p->gj2) g.nP = ((g.nI + GJ_KB - 1) / GJ_KB) * GJ_KB;  // outer block 128: pairs of pivot blocks
-    // deep look-ahead of the pivot inversions (classic scheme on the TMA-fed engine): built, bit-identical, and measured SLOWER
-    // than the pivot CTAs riding on the update launch (16 frequencies 321 vs 289 ms, 2 frequencies 137 vs 134 ms: the pivot kernel --
-    // two tile products + the inversion, 54 us alone, 88 us beside the tile CTAs -- is a serial chain of its own), so opt-in
-    p->deep = false;
-    if (const char* e = getenv("UST_DEEP")) p->deep = want_tc2 && !p->gj2 && atoi(e) != 0;
-    // row panel k+1 as trailing CTAs of update launch k (in-launch flags): built, bit-identical, and measured slower than two launches
-    // (16 frequencies 296 vs 284 ms, 2 frequencies 141 vs 134 ms: replayed from a graph a launch boundary costs ~1.5 us, the flag
-    // hand-over 2.5 us), so opt-in
-    p->fuse = false;
-    if (const char* e = getenv("UST_FUSE_RP")) p->fuse = want_tc2 && !p->gj2 && atoi(e) != 0;
-    if (const char* e = getenv("UST_NO_LOOKAHEAD")) { if (atoi(e) != 0) p->deep = false; }
     g.mid = g.M / 2;
     g.N = (long long)d->nx * d->ny;
     // AUTO = the TMA-fed tcgen05 engine for complex64 (FP32-accurate products, leading terms accumulated in FP32 registers);
@@ -1119,20 +1028,14 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
         if (!rc && cudaMemset(p->Wp, 0, wp_bytes) != cudaSuccess) rc = 1;
         if (!rc) rc = tc2::make_aplane_maps(p->Tp, g.nP, (long long)d->max_freq * g.M, p->amaps);
         p->rp_stride = tc2::bplanes_elems(GJ_NB, g.nP);
-        p->rp2_stride = tc2::bplanes_elems(GJ_KB, g.nP);
         const size_t nbmax = (size_t)2 * d->max_freq;
-        const int cpw = p->gj2 ? GJ_KB : GJ_NB;  // width of the column-panel planes
-        rc |= dev_alloc(p, (void**)&p->Rp, (p->gj2 ? 1 : 2) * nbmax * (p->gj2 ? p->rp2_stride : p->rp_stride) * sizeof(uint16_t));  // classic scheme: ping-pong on the pivot index (fused row panels)
-        rc |= dev_alloc(p, (void**)&p->gj_flags, 2 * GJ_MAXBLK * nbmax * sizeof(int));
-        if (!rc && cudaMemset(p->gj_flags, 0, 2 * GJ_MAXBLK * nbmax * sizeof(int)) != cudaSuccess) rc = 1;
+        rc |= dev_alloc(p, (void**)&p->Rp, nbmax * p->rp_stride * sizeof(uint16_t));
         rc |= dev_alloc(p, (void**)&p->Xp, 2 * nbmax * p->rp_stride * sizeof(uint16_t));
-        rc |= dev_alloc(p, (void**)&p->Cp, 2 * nbmax * tc2::NPL_A * g.nP * cpw * sizeof(uint16_t));
-        rc |= dev_alloc(p, (void**)&p->Pp, 2 * nbmax * tc2::NPL_A * GJ_NB * GJ_NB * sizeof(uint16_t));  // ping-pong on the pivot index (deep look-ahead)
-        rc |= dev_alloc(p, &p->snap, 2 * nbmax * GJ_NB * GJ_NB * p->csz);
-        if (p->deep) rc |= dev_alloc(p, (void**)&p->Rs, nbmax * p->rp_stride * sizeof(uint16_t));
-        if (!rc && !p->gj2) rc = tc2::make_aplane_maps(p->Cp, g.nP, GJ_NB, (long long)(2 * nbmax), p->cmaps);
-        if (!rc && p->gj2) rc = tc2::make_aplane_maps(p->Cp, g.nP, GJ_KB, (long long)(2 * nbmax), p->cmaps2);
-        if (!rc) rc = tc2::make_aplane_maps(p->Pp, GJ_NB, GJ_NB, (long long)(2 * nbmax), p->pmaps);
+        rc |= dev_alloc(p, (void**)&p->Cp, 2 * nbmax * tc2::NPL_A * g.nP * GJ_NB * sizeof(uint16_t));
+        rc |= dev_alloc(p, (void**)&p->Pp, nbmax * tc2::NPL_A * GJ_NB * GJ_NB * sizeof(uint16_t));
+        rc |= dev_alloc(p, &p->snap, nbmax * GJ_NB * GJ_NB * p->csz);
+        if (!rc) rc = tc2::make_aplane_maps(p->Cp, g.nP, GJ_NB, (long long)(2 * nbmax), p->cmaps);
+        if (!rc) rc = tc2::make_aplane_maps(p->Pp, GJ_NB, GJ_NB, (long long)nbmax, p->pmaps);
     }
     if (d->fwi_buffers) {
         rc |= dev_alloc(p, &p->U, (size_t)d->max_freq * g.N * d->max_nrhs * p->csz);
@@ -1170,7 +1073,7 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
             set_error("ust_plan_create: group stream / event creation failed");
             rc = 1;
         }
-    if (!rc && (p->deep || d->dtype == UST_C128)) {
+    if (!rc && d->dtype == UST_C128) {
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);  // hi = numerically lowest = highest priority
         for (int i = 0; i < ust_plan::MAX_GROUPS && !rc; ++i)
@@ -1183,8 +1086,6 @@ int ust_plan_create(const ust_plan_desc* d, ust_plan** out) {
             }
     }
     if (const char* e = getenv("UST_NO_LOOKAHEAD")) p->lookahead = atoi(e) == 0;
-    if (const char* e = getenv("UST_NO_SCHUR_PIVOT")) p->schur_pivot0 = atoi(e) == 0;
-    if (const char* e = getenv("UST_EXP")) p->exp = atoi(e);
     if (const char* e = getenv("UST_PDL_MIN_BATCH")) p->pdl_min_batch = atoi(e);
     if (const char* e = getenv("UST_KSPLIT")) p->ksplit_ok = atoi(e);
     if (const char* e = getenv("UST_TC2_TRACE_UPDATE")) {
@@ -1208,7 +1109,7 @@ int ust_plan_destroy(ust_plan* p) {
     cudaSetDevice(p->d.device);
     cudaDeviceSynchronize();
     void* ptrs[] = {p->exn, p->rexh, p->eyn, p->reyh, p->d_vminmax, p->d_freqs, p->d_bde, p->d_scal, p->d_status, p->d_invv2, p->d_sig2, p->planes,
-                    p->T, p->scratch, p->W, p->pbuf, p->Tp, p->Wp, p->Rp, p->Cp, p->Xp, p->Pp, p->Rs, p->gj_flags, p->snap, p->vel, p->U, p->Lam, p->src_est, p->Xh, p->src_lin, p->rx_lin, p->mask, p->rx_next,
+                    p->T, p->scratch, p->W, p->pbuf, p->Tp, p->Wp, p->Rp, p->Cp, p->Xp, p->Pp, p->snap, p->vel, p->U, p->Lam, p->src_est, p->Xh, p->src_lin, p->rx_lin, p->mask, p->rx_next,
                     p->slow_h2d, p->rec_h2d, p->grad_d2h, p->kappa_h2d, p->grad_kappa_d2h};
     for (void* q : ptrs)
         if (q) cudaFree(q);
