@@ -69,6 +69,20 @@ size_t ust_plan_device_bytes(const ust_plan* plan);
  * the reference handles one frequency at a time (fwi_script.py:24). */
 int ust_plan_set_groups(ust_plan* plan, int ngroups);
 
+/* Linearisation J behind the gradient, the NCG line search and the Gauss-Newton product (DESIGN.md section 7f).
+ *   UST_GRAD_REFERENCE (the default): the reference's virtual source 2 w^2 sigma alpha u (nonlinearcg.py:258), which leaves out
+ *     the stencil's mass weights and the PML factor, so the gradient is not the exact derivative of the loss.
+ *   UST_GRAD_DISCRETE: the exact derivative of the discrete forward map at fixed stencil weights (b, d, e): the virtual source
+ *     is the 9-point mass stencil (1-d-e, d/4, e/4) applied to C 2 w^2 sigma dsigma alpha u, with C = e_x e_y, and zero on the
+ *     Dirichlet ring.  (b, d, e) are held fixed as the reference treats them, also when they follow min/max(vel); their
+ *     dependence on the model is not differentiated.
+ * The mode governs ust_fwi_loss_grad[_host], ust_fwi_loss_grad_lossy[_host], ust_ncg_linesearch[_lossy] and
+ * ust_fwi_gn_hvp[_lossy]; solves, factorisations, ust_residual_onehot and ust_idtft do not depend on it.  Every evaluation records
+ * the mode it ran with; a line search or product whose plan mode differs from it fails until the next evaluation.  Changing the
+ * mode leaves the results of earlier calls as they are.  Any other mode is an error. */
+enum { UST_GRAD_REFERENCE = 0, UST_GRAD_DISCRETE = 1 };
+int ust_plan_set_gradient(ust_plan* plan, int mode);
+
 /* Grid + PML: x (nx doubles), y (ny doubles) host arrays, a0, L_PML as in
  * solve_helmholtz.py:22-60 (h = mean(diff(x)), g = mean(diff(y))/h, half-grid PML profiles). */
 int ust_plan_set_grid(ust_plan* plan, const double* x_host, const double* y_host, double a0, double L_pml);
@@ -110,7 +124,8 @@ int ust_solve_helmholtz_host(ust_plan* plan, const void* vel_host, const void* s
 
 /* Fused (loss, grad) of fwi_loss_function.py:29-103 + nonlinearcg.py:243-265 summed over nfreq
  * frequencies: factor, all-source forward sweeps (one-hot sources), source-strength estimate, residual,
- * loss, adjoint sweeps on the same factors, gradient w.r.t. slowness.
+ * loss, adjoint sweeps on the same factors, gradient w.r.t. slowness.  The gradient is Re(J^H residual) with J of the plan's
+ * gradient mode (ust_plan_set_gradient); the loss does not depend on the mode.
  *   slow_dev   (ny, nx) real slowness (params of fwi_loss_function.py:49)
  *   rec_dev    (nfreq, nt, nelem) complex observed data REC_DATA per frequency
  *   loss_dev   one double (sum over frequencies of 0.5*sum|rec_sim-rec_obs|^2)
@@ -120,7 +135,7 @@ int ust_fwi_loss_grad(ust_plan* plan, const void* slow_dev, const void* rec_dev,
                       void* stream);
 
 /* Same, HOST buffers in and out (pinned staging inside): the reference-facing call that bench.py's
- * "e2e" times. */
+ * "e2e" times.  Follows the plan's gradient mode. */
 int ust_fwi_loss_grad_host(ust_plan* plan, const void* slow_host, const void* rec_host, int nfreq,
                            const double* freqs_host, const double* bde_host, double* loss_host,
                            void* grad_host);
@@ -131,12 +146,14 @@ int ust_fwi_loss_grad_host(ust_plan* plan, const void* slow_host, const void* re
  *   grad_s = s A - kappa B,   grad_kappa = -s B - kappa A      (kappa = 0: grad_s is ust_fwi_loss_grad's gradient, bit for bit)
  *   slow_dev, kappa_dev (ny, nx) real; kappa_dev is required.  grad_s_dev, grad_kappa_dev (ny, nx) real, overwritten.
  * After it, ust_ncg_linesearch and ust_fwi_gn_hvp refuse (their virtual source assumes a real slowness) until the next
- * ust_fwi_loss_grad; their lossy twins ust_ncg_linesearch_lossy and ust_fwi_gn_hvp_lossy run on its state instead. */
+ * ust_fwi_loss_grad; their lossy twins ust_ncg_linesearch_lossy and ust_fwi_gn_hvp_lossy run on its state instead.
+ * In the discrete gradient mode z_f carries the mass stencil and the PML factor: z_j = conj(C_j) sum_t conj(alpha_t u_tj)
+ * (W lambda_t)_j, with W the 9-point mass weights restricted to interior rows (ust_plan_set_gradient). */
 int ust_fwi_loss_grad_lossy(ust_plan* plan, const void* slow_dev, const void* kappa_dev, const void* rec_dev, int nfreq,
                             const double* freqs_host, const double* bde_host, double* loss_dev, void* grad_s_dev,
                             void* grad_kappa_dev, void* stream);
 
-/* Same, HOST buffers in and out (the twin of ust_fwi_loss_grad_host). */
+/* Same, HOST buffers in and out (the twin of ust_fwi_loss_grad_host).  Follows the plan's gradient mode. */
 int ust_fwi_loss_grad_lossy_host(ust_plan* plan, const void* slow_host, const void* kappa_host, const void* rec_host, int nfreq,
                                  const double* freqs_host, const double* bde_host, double* loss_host, void* grad_s_host,
                                  void* grad_kappa_host);
@@ -146,7 +163,8 @@ int ust_fwi_loss_grad_lossy_host(ust_plan* plan, const void* slow_host, const vo
  * the two line-search scalars  num = Re<dREC, REC_DATA-REC_SIM>, den = Re<dREC,dREC>
  * (compute_step_size, nonlinearcg.py:22-32) summed over frequencies.  out2_dev: two doubles.
  * Fails if ust_factor, ust_factor_lossy or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and
- * after a lossy evaluation (ust_fwi_loss_grad_lossy); ust_ncg_linesearch_lossy is the line search of the lossy model. */
+ * after a lossy evaluation (ust_fwi_loss_grad_lossy); ust_ncg_linesearch_lossy is the line search of the lossy model.
+ * The perturbation RHS is that of the plan's gradient mode; fails when it differs from the mode of that evaluation. */
 int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, void* stream);
 
 /* Gauss-Newton Hessian-vector product of the joint objective on the factors, forward fields and source estimates of the last
@@ -154,7 +172,9 @@ int ust_ncg_linesearch(ust_plan* plan, const void* sd_dev, double* out2_dev, voi
  * nonlinearcg.py:258,279 (alpha fixed).  v_dev, hv_dev: (ny, nx) real.  jv2_dev: one double, sum |J v|^2 (= <v, hv>).
  * jv_dev: (nfreq, nt, nm) complex J v at the kept receivers (mask order), or NULL.  Overwrites the adjoint wavefield.
  * J is the linearisation the gradient uses (virtual source 2 w^2 s alpha u without the stencil's mass weights and the PML
- * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).
+ * factor), not the exact derivative of the discrete forward map; the gradient equals Re(J^H (alpha P u - rec_obs)).  In the
+ * discrete gradient mode (ust_plan_set_gradient) J is that exact derivative at fixed (b, d, e); either way J is the one the
+ * evaluation's gradient used, and a plan mode that differs from the evaluation's fails.
  * Fails if ust_factor, ust_factor_lossy or ust_solve_helmholtz_host replaced the factors after that ust_fwi_loss_grad, and
  * after a lossy evaluation (ust_fwi_loss_grad_lossy); ust_fwi_gn_hvp_lossy is the product of the lossy model. */
 int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_dev, void* jv_dev, void* stream);
@@ -169,7 +189,9 @@ int ust_fwi_gn_hvp(ust_plan* plan, const void* v_dev, void* hv_dev, double* jv2_
  * hv_s / jv2 / jv equal those of the lossless entry points on the same slowness, bit for bit.
  *   ust_ncg_linesearch_lossy: out2_dev = {num = Re<J sd, REC_DATA - REC_SIM>, den = |J sd|^2} (= -<sd, grad> and |J sd|^2).
  *   ust_fwi_gn_hvp_lossy:     hv_s_dev, hv_kappa_dev (ny, nx) real = Re(J^H J v); jv2_dev = sum |J v|^2 (= <v, hv>);
- *                             jv_dev (nfreq, nt, nm) complex J v at the kept receivers, or NULL. */
+ *                             jv_dev (nfreq, nt, nm) complex J v at the kept receivers, or NULL.
+ * In the discrete gradient mode the virtual source carries the mass stencil and the PML factor (ust_plan_set_gradient); both
+ * fail when the plan's mode differs from the mode of the last evaluation. */
 int ust_ncg_linesearch_lossy(ust_plan* plan, const void* sd_s_dev, const void* sd_kappa_dev, double* out2_dev, void* stream);
 int ust_fwi_gn_hvp_lossy(ust_plan* plan, const void* v_s_dev, const void* v_kappa_dev, void* hv_s_dev, void* hv_kappa_dev,
                          double* jv2_dev, void* jv_dev /* (nfreq, nt, nm) complex or NULL */, void* stream);

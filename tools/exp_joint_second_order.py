@@ -11,7 +11,10 @@ gets the same budget of objective evaluations (one factorisation each):
 Reported per run, per evaluation: wall time since the start (with a device synchronise), loss, sound-speed RMS error (m/s) and
 attenuation RMS error (dB/(cm MHz)) over the disc r < 100 mm, and the products / line searches so far.
 
-    python tools/exp_joint_second_order.py --out DIR [--evals 40]     -> DIR/exp_joint_second_order.txt
+``--gradient discrete`` runs all three on the exact derivative of the discrete loss (DESIGN.md section 7f) instead of the
+reference's linearisation.
+
+    python tools/exp_joint_second_order.py --out DIR [--evals 40] [--gradient reference|discrete]  -> DIR/exp_joint_second_order.txt
 """
 import argparse
 import os
@@ -32,6 +35,7 @@ def main():
     ap.add_argument("--n", type=int, default=256)
     ap.add_argument("--evals", type=int, default=40)
     ap.add_argument("--cg-iters", type=int, default=4)
+    ap.add_argument("--gradient", default="reference", choices=["reference", "discrete"])
     a = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -58,7 +62,7 @@ def main():
     dargs = (geom.xi, geom.yi, geom.num_elements, rec, src1, geom.tx_include, geom.ind_matlab, 1480.0, freqs)
     tail = (geom.a0, geom.L_PML, geom.mask_indices)
     lines = [f"# tools/exp_joint_second_order.py: {n}x{n} grid, 256-element ring, frequencies {[round(f / 1e3, 1) for f in freqs]} kHz, "
-             f"complex64, budget {a.evals} evaluations (factorisations) per run, Gauss-Newton cg_iters = {a.cg_iters}",
+             f"complex64, budget {a.evals} evaluations (factorisations) per run, Gauss-Newton cg_iters = {a.cg_iters}, gradient {a.gradient}",
              f"# card: {card()}",
              f"# truth: sound speed {vel_true[inside].min():.1f}..{vel_true[inside].max():.1f} m/s, attenuation "
              f"{G.kappa_to_db_cm_mhz(kappa_true[inside]).min():.3f}..{G.kappa_to_db_cm_mhz(kappa_true[inside]).max():.3f} dB/(cm MHz); "
@@ -66,7 +70,8 @@ def main():
              f"# start: c = 1480 m/s (error {c_err(np.full((n, n), 1480.0)):.3f} m/s), kappa = 0 (error {k_err(np.zeros((n, n))):.4f} dB/(cm MHz))"]
     results = {}
     for name in ("a_ncg", "b_gauss_newton", "c_lbfgs"):
-        lg0, ls0, hvp0 = api._gpu_callables(True, *dargs[:7], freqs, *tail, "c64", None, "python", 0, "auto")
+        lg0, ls0, hvp0 = api._gpu_callables(True, *dargs[:7], freqs, *tail, "c64", None, "python", 0, "auto",
+                                                gradient=a.gradient)
         trace, count = [], {"products": 0, "linesearches": 0}
         t0 = [0.0]
 

@@ -14,7 +14,7 @@ _LIB = None
 
 EXPORTS = [
     "ust_last_error", "ust_version", "ust_plan_create", "ust_plan_destroy", "ust_plan_device_bytes",
-    "ust_plan_set_groups", "ust_plan_set_grid", "ust_plan_set_acquisition", "ust_factor", "ust_factor_lossy", "ust_solve",
+    "ust_plan_set_groups", "ust_plan_set_gradient", "ust_plan_set_grid", "ust_plan_set_acquisition", "ust_factor", "ust_factor_lossy", "ust_solve",
     "ust_solve_helmholtz_host", "ust_fwi_loss_grad", "ust_fwi_loss_grad_host", "ust_fwi_loss_grad_lossy", "ust_fwi_loss_grad_lossy_host", "ust_ncg_linesearch", "ust_fwi_gn_hvp",
     "ust_ncg_linesearch_lossy", "ust_fwi_gn_hvp_lossy", "ust_get_bde", "ust_get_planes",
     "ust_get_src_est", "ust_get_wavefield", "ust_get_adjoint_wavefield", "ust_get_status",
@@ -52,6 +52,7 @@ def lib():
     L.ust_plan_device_bytes.argtypes = [vp]
     L.ust_plan_device_bytes.restype = C.c_size_t
     L.ust_plan_set_groups.argtypes = [vp, i]
+    L.ust_plan_set_gradient.argtypes = [vp, i]
     L.ust_plan_set_grid.argtypes = [vp, pd, pd, d, d]
     L.ust_plan_set_acquisition.argtypes = [vp, i, pi, i, pi, i, pi]
     L.ust_factor.argtypes = [vp, vp, i, pd, pd, vp]

@@ -20,6 +20,10 @@ Attenuation (not in the reference): ``kappa`` (attenuation slowness, s/m) makes 
 invert sound speed and attenuation together (DESIGN.md section 7d); ``fwi_joint_gauss_newton_product``,
 ``nonlinear_conjugate_gradient_joint``, ``gauss_newton_joint_fwi`` and ``joint_frequency_continuation`` add the joint
 Gauss-Newton product, NCG and truncated Gauss-Newton (section 7e).
+
+Exact derivative (not in the reference): ``gradient="discrete"`` on every gradient-based function and driver builds the
+gradient, the line search and the Gauss-Newton product from the exact derivative of the discrete forward map at fixed stencil
+weights instead of the reference's virtual source (DESIGN.md section 7f).  The default ``"reference"`` keeps the reference's.
 """
 from __future__ import annotations
 
@@ -162,7 +166,10 @@ class OneHotSources:
         self.shape = tuple(shape)
 
 
-def _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine="auto"):
+def _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine="auto",
+              gradient="reference"):
+    """The cached plan of this problem with its grid, acquisition and gradient mode set.  Plans are shared, so the mode is set
+    on every call rather than left from an earlier one."""
     xh, yh = _to_np(xi).astype(np.float64).ravel(), _to_np(yi).astype(np.float64).ravel()
     nx, ny = xh.size, yh.size
     freqs = np.atleast_1d(np.asarray(_to_np(f), dtype=np.float64)).ravel()
@@ -170,36 +177,42 @@ def _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dty
     plan = get_plan(nx, ny, dtype, device, freqs.size, src_lin.size, stencil, True, engine)
     plan.set_grid(xh, yh, float(a0), float(L_PML))
     plan.set_acquisition(src_lin, rx_lin, mask)
+    plan.set_gradient(gradient)
     return plan, freqs
 
 
 def fwi_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                      num_elements, *, dtype="c64", bde=None, stencil="python", engine="auto"):
+                      num_elements, *, dtype="c64", bde=None, stencil="python", engine="auto", gradient="reference"):
     """(loss, grad): loss of fwi_loss_function.py:29-103 and the adjoint-state gradient with respect to
     the slowness ``params`` (nonlinearcg.py:243-265), ``grad.shape == params.shape``.
+
+    ``gradient``: ``"reference"`` builds the gradient from the reference's virtual source ``2 w^2 s alpha u``;
+    ``"discrete"`` from the exact derivative of the discrete forward map at fixed stencil weights (the 9-point mass stencil
+    and the PML factor, DESIGN.md section 7f), so that it is the derivative of the returned loss.  The loss is the same.
 
     With ``f`` of length Nf and ``REC_DATA`` of shape (Nf, Nt, E) the joint objective sum_f loss_f is
     returned.  Usable as ``jaxopt.LBFGS(fun, value_and_grad=True)`` / ``scipy.optimize.minimize(jac=True)``.
     """
     return _loss_function(False, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil,
-                          engine)
+                          engine, gradient)
 
 
 def fwi_joint_loss_function(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
-                            *, dtype="c64", bde=None, stencil="python", engine="auto"):
+                            *, dtype="c64", bde=None, stencil="python", engine="auto", gradient="reference"):
     """(loss, grad) of the joint sound-speed and attenuation problem: ``params`` is (2, Ny, Nx) = [slowness s (s/m),
     attenuation slowness kappa (s/m)] of the complex slowness ``s - i kappa``, and ``grad`` has ``params``' shape
     ([dloss/ds, dloss/dkappa]).  The other arguments and the loss are those of ``fwi_loss_function``; the gradients use the
-    same linearisation (source estimates held fixed, DESIGN.md section 7d).  The ``value_and_grad`` contract of
+    same linearisation (source estimates held fixed, DESIGN.md section 7d) and ``gradient`` mode.  The ``value_and_grad`` contract of
     ``fwi_loss_function``: torch CUDA in -> torch out (device buffers), NumPy in -> NumPy out (host buffers)."""
     return _loss_function(True, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil,
-                          engine)
+                          engine, gradient)
 
 
-def _loss_function(lossy, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil, engine):
+def _loss_function(lossy, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, bde, stencil, engine,
+                   gradient):
     """The body of ``fwi_loss_function`` (``lossy``: of ``fwi_joint_loss_function``, ``params`` = [s, kappa])."""
     dev = _device_of(params, REC_DATA)
-    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine, gradient)
     if lossy and tuple(params.shape) != (2, plan.ny, plan.nx):
         raise ValueError(f"params must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa]")
     if _is_torch(params) and params.is_cuda:
@@ -214,15 +227,16 @@ def _loss_function(lossy, params, xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matla
         maps = (p[0], p[1]) if lossy else (p.reshape(plan.ny, plan.nx), None)
         loss, *grads = plan._loss_grad_host(*maps, _to_np(REC_DATA), freqs, bde, None)
         grad, shape = np.stack(grads) if lossy else grads[0], p.shape
-    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy)
+    plan._eval_key = _eval_key(params, REC_DATA, freqs, bde, lossy, gradient)
     return loss, grad.reshape(shape)
 
 
-def _eval_key(params, REC_DATA, freqs, bde, lossy=False):
+def _eval_key(params, REC_DATA, freqs, bde, lossy=False, gradient="reference"):
     """What identifies an evaluation's state on the plan: device inputs are kept as copies (compared on the device), host
-    inputs as a hash.  The key of a lossy evaluation is tagged, so that it never matches a lossless one."""
+    inputs as a hash.  The key of a lossy evaluation is tagged, so that it never matches a lossless one, and so is the key of
+    the discrete gradient mode, so that an evaluation in one mode is never reused for a product in the other."""
     b = None if bde is None else np.asarray(bde, dtype=np.float64)
-    tag = "-lossy" if lossy else ""
+    tag = ("-lossy" if lossy else "") + ("-discrete" if gradient == "discrete" else "")
     if _is_torch(params) and params.is_cuda:
         rec = REC_DATA.detach().clone() if _is_torch(REC_DATA) else _fingerprint(np.asarray(REC_DATA))
         return ("dev" + tag, params.detach().clone(), rec, _fingerprint(freqs, b))
@@ -245,24 +259,26 @@ def _same_eval(a, b):
 
 
 def fwi_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements,
-                             *, dtype="c64", bde=None, stencil="python", engine="auto"):
+                             *, dtype="c64", bde=None, stencil="python", engine="auto", gradient="reference"):
     """Gauss-Newton Hessian-vector product ``H_GN v = Re(J^H J v)`` of the objective of ``fwi_loss_function`` at slowness
     ``params``, returned with ``params``' shape (NumPy in, NumPy out; a CUDA tensor ``v`` gives a CUDA tensor).
 
     ``J`` is the linearisation the gradient is built from (``nonlinearcg.py:258,279``): the perturbation solve with virtual
     source ``-2 w^2 s alpha u v``, gathered at the kept receivers, with the source estimates ``alpha`` held fixed, so that the
     gradient is ``Re(J^H residual)``.  The virtual source leaves out the stencil's mass weights and the PML factor, as the
-    reference does: ``J`` is not the exact derivative of the discrete forward map (DESIGN.md section 7c).
+    reference does: ``J`` is not the exact derivative of the discrete forward map (DESIGN.md section 7c).  With
+    ``gradient="discrete"`` it is, at fixed stencil weights (section 7f), and the gradient of
+    ``fwi_loss_function(..., gradient="discrete")`` is ``Re(J^H residual)`` of that ``J``.
 
     A product costs two all-source sweeps on the factorisation the last evaluation left on the plan; when the last
     ``fwi_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)``, the evaluation runs first.
     """
     return _gauss_newton_product(False, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                                 num_elements, dtype, bde, stencil, engine)
+                                 num_elements, dtype, bde, stencil, engine, gradient)
 
 
 def fwi_joint_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                                   num_elements, *, dtype="c64", bde=None, stencil="python", engine="auto"):
+                                   num_elements, *, dtype="c64", bde=None, stencil="python", engine="auto", gradient="reference"):
     """Gauss-Newton product ``H_GN v = Re(J^H J v)`` of the joint objective of ``fwi_joint_loss_function``: ``params`` and
     ``v`` are (2, Ny, Nx) = [slowness, kappa] blocks, and so is the result (NumPy in, NumPy out; a CUDA tensor ``v`` gives a
     CUDA tensor).
@@ -270,29 +286,29 @@ def fwi_joint_gauss_newton_product(params, v, xi, yi, REC_DATA, SRC, f, a0, L_PM
     With the complex slowness ``sigma = s - i kappa`` and the source estimates held fixed, ``J [v_s; v_kappa]`` is the
     perturbation solve with virtual source ``-2 w^2 sigma alpha u (v_s - i v_kappa)`` gathered at the kept receivers, the
     linearisation the joint gradient is built from (DESIGN.md section 7e).  Because ``J_kappa = -i J_s``, the blocks satisfy
-    ``H_kk = H_ss`` and ``H_ks = -H_sk``.
+    ``H_kk = H_ss`` and ``H_ks = -H_sk``; both hold in the ``gradient="discrete"`` mode too (section 7f).
 
     A product costs two all-source sweeps on the factorisation the last evaluation left on the plan; when the last
     ``fwi_joint_loss_function`` on this plan had other ``(params, REC_DATA, f, bde)`` (or the last evaluation was lossless),
     the evaluation runs first.
     """
     return _gauss_newton_product(True, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                                 num_elements, dtype, bde, stencil, engine)
+                                 num_elements, dtype, bde, stencil, engine, gradient)
 
 
 def _gauss_newton_product(lossy, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                          num_elements, dtype, bde, stencil, engine):
+                          num_elements, dtype, bde, stencil, engine, gradient):
     """The body of ``fwi_gauss_newton_product`` (``lossy``: of ``fwi_joint_gauss_newton_product``)."""
     import torch
     dev = _device_of(params, REC_DATA, v)
-    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, dev, engine, gradient)
     if lossy and tuple(v.shape) != (2, plan.ny, plan.nx):
         raise ValueError(f"v must have shape (2, {plan.ny}, {plan.nx}) = [slowness, kappa] directions")
-    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde, lossy)):
+    if not _same_eval(plan._eval_key, _eval_key(params, REC_DATA, freqs, bde, lossy, gradient)):
         # looked up at call time: tests record the evaluation points by replacing these module functions
         evaluate = fwi_joint_loss_function if lossy else fwi_loss_function
         evaluate(params, xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices, num_elements, dtype=dtype,
-                 bde=bde, stencil=stencil, engine=engine)
+                 bde=bde, stencil=stencil, engine=engine, gradient=gradient)
     on_device = _is_torch(v) and v.is_cuda
     if on_device:
         vt = v.detach().to(plan.treal)
@@ -306,17 +322,19 @@ def _gauss_newton_product(lossy, params, v, xi, yi, REC_DATA, SRC, f, a0, L_PML,
 
 def nonlinear_conjugate_gradient(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter,
                                  a0, L_PML, mask_indices, *, dtype="c64", bde=None, stencil="python",
-                                 device=0, history=None, return_fields=True, engine="auto"):
+                                 device=0, history=None, return_fields=True, engine="auto", gradient="reference"):
     """The reference's NCG loop (nonlinearcg.py:41-180 / 184-308: Hestenes-Stiefel beta, forced to 0 at
     the first iteration; linearised exact step) on the GPU path: per iteration one factorisation,
     forward + adjoint + perturbation sweeps, all on device.
 
     Returns (VEL, sd, grad, ADJ_WV, WV) as NumPy arrays like the reference; ADJ_WV / WV (each
     (Ny, Nx, Nt) complex, WV scaled by the source estimates, nonlinearcg.py:227) are only materialised
-    when ``return_fields`` and refer to the last iteration / first frequency.
+    when ``return_fields`` and refer to the last iteration / first frequency.  ``gradient``: the gradient and line-search
+    linearisation, ``"reference"`` or ``"discrete"`` (``fwi_loss_function``).
     """
     import torch
-    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine)
+    plan, freqs = _fwi_plan(xi, yi, REC_DATA, SRC, f, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine,
+                            gradient)
     dv = torch.device(f"cuda:{device}")
     ny, nx = plan.ny, plan.nx
     rec = torch.as_tensor(_to_np(REC_DATA)).to(device=dv, dtype=plan.tcplx).reshape(freqs.size, plan.nt, plan.nelem).contiguous()
@@ -356,7 +374,7 @@ nonlinear_conjugate_gradient_vectorized = nonlinear_conjugate_gradient
 
 def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, L_PML, mask_indices, *, maxiter=1, tol=1e-5,
                   history_size=10, dtype="c64", bde=None, stencil="python", engine="auto", history=None, loss_grad=None,
-                  pert_scale=1e-2):
+                  pert_scale=1e-2, gradient="reference"):
     """``run_lbfgs_fwi`` of the reference (``fwi_loss_function.py:106-132``): L-BFGS on the slowness map, returning the
     final sound speed ``(Ny, Nx)``.  The reference wires ``jaxopt.LBFGS(fun=loss_fn, maxiter=1, tol=1e-5)`` around a
     loss-only function (which JAX cannot differentiate through ``pure_callback``); here the objective is this package's
@@ -370,7 +388,8 @@ def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, 
     ``loss / loss(s0)``; ``tol`` applies to the projected gradient of that scaled problem.
 
     ``loss_grad(slow_2d) -> (loss, grad_2d)`` replaces the objective (the parity test drives the same optimiser with the
-    oracle's); ``history`` receives ``(loss, params.copy())`` of every evaluation.
+    oracle's); ``history`` receives ``(loss, params.copy())`` of every evaluation.  ``gradient`` is the gradient mode of
+    ``fwi_loss_function``.
     """
     ny, nx = _to_np(yi).size, _to_np(xi).size
     num_elements = int(SRC.shape[2]) if SRC is not None else 0  # unused when ``loss_grad`` is injected
@@ -380,7 +399,7 @@ def run_lbfgs_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, 
     if loss_grad is None:
         def loss_grad(slow):
             return fwi_loss_function(slow.astype(real), xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab, mask_indices,
-                                     num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+                                     num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine, gradient=gradient)
 
     slow, = _lbfgs_blocks(loss_grad, [_slowness_block(c0, s0, pert_scale, ny, nx)], ny, nx, maxiter, tol, history_size, history)
     return 1.0 / slow
@@ -427,7 +446,7 @@ def _lbfgs_blocks(loss_grad, blocks, ny, nx, maxiter, tol, history_size, history
 
 def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, a0, L_PML, mask_indices, *, kappa_init=0.0,
                         kappa_scale=None, maxiter=1, tol=1e-5, history_size=10, dtype="c64", bde=None, stencil="python",
-                        engine="auto", history=None, loss_grad=None, pert_scale=1e-2):
+                        engine="auto", history=None, loss_grad=None, pert_scale=1e-2, gradient="reference"):
     """L-BFGS on sound speed and attenuation together (``fwi_joint_loss_function``); returns ``(c, kappa)``, both (Ny, Nx).
 
     SciPy's L-BFGS-B with the bound ``kappa >= 0``, on the problem non-dimensionalised per block: the slowness as in
@@ -438,7 +457,7 @@ def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f
 
     ``loss_grad(params) -> (loss, grad)`` with ``params`` (2, Ny, Nx) float64 = [slowness, kappa] replaces the objective (the
     parity test drives the same optimiser with the oracle's); ``history`` receives ``(loss, params.copy())`` of every
-    evaluation.
+    evaluation.  ``gradient`` is the gradient mode of ``fwi_joint_loss_function``.
     """
     from .geometry import db_cm_mhz_to_kappa
     ny, nx = _to_np(yi).size, _to_np(xi).size
@@ -450,7 +469,8 @@ def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f
     if loss_grad is None:
         def loss_grad(params):
             return fwi_joint_loss_function(params.astype(real), xi, yi, REC_DATA, SRC, f, a0, L_PML, tx_include, ind_matlab,
-                                           mask_indices, num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+                                           mask_indices, num_elements, dtype=dtype, bde=bde, stencil=stencil, engine=engine,
+                                           gradient=gradient)
 
     kappa_block = (lambda p: ks * p), ks, (np.asarray(_to_np(kappa_init), dtype=np.float64) * np.ones((ny, nx)) / ks).ravel(), 0.0
     slow, kappa = _lbfgs_blocks(loss_grad, [_slowness_block(c0, s0, pert_scale, ny, nx), kappa_block], ny, nx, maxiter, tol,
@@ -460,7 +480,7 @@ def run_lbfgs_joint_fwi(xi, yi, REC_DATA, SRC, tx_include, ind_matlab, c_init, f
 
 def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
                      cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, dtype="c64", bde=None, stencil="python", device=0,
-                     engine="auto", history=None, loss_grad=None, hvp=None):
+                     engine="auto", history=None, loss_grad=None, hvp=None, gradient="reference"):
     """Truncated Gauss-Newton FWI on the slowness, with the arguments of ``nonlinear_conjugate_gradient``; returns the sound
     speed (Ny, Nx) as a NumPy array.
 
@@ -477,12 +497,14 @@ def gauss_newton_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab,
     algebra is float64 torch on the device of the first gradient.  ``history`` (a list) receives one dict per outer
     iteration: loss, CG iterations, the quadratic-model value ``q(p_k) = <g,p_k>/2 - <p_k,r_k>/2`` of every CG iterate, mu,
     the accepted step, cumulative evaluation and product counts, the velocity range, and ``stop`` when the driver stops.
+    ``gradient``: the linearisation of the gradient and the products, ``"reference"`` or ``"discrete"``
+    (``fwi_gauss_newton_product``).
     """
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or hvp is None:
         loss_grad, _, hvp = _gpu_callables(False, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
-                                           mask_indices, dtype, bde, stencil, device, engine)
+                                           mask_indices, dtype, bde, stencil, device, engine, gradient)
     c0 = np.asarray(_to_np(c_init), dtype=np.float64) * np.ones((ny, nx))
     s = _gauss_newton_loop(torch.as_tensor(1.0 / c0), loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history,
                            slow_of=lambda x: x)
@@ -587,7 +609,7 @@ def _project_kappa(x):
 
 
 def _gpu_callables(lossy, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML, mask_indices, dtype, bde,
-                   stencil, device, engine):
+                   stencil, device, engine, gradient="reference"):
     """GPU objective of the drivers on float64 torch models, (Ny, Nx) slowness maps or, ``lossy``, (2, Ny, Nx) = [s, kappa]:
     loss_grad(x), and the line search and the Gauss-Newton product at the point of the last loss_grad call."""
     import torch
@@ -597,7 +619,7 @@ def _gpu_callables(lossy, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_ma
     rec = torch.as_tensor(_to_np(REC_DATA)).to(dv).reshape(freqs.size, len(_to_np(tx_include)), -1).contiguous()
     state = {}
     fargs = (xi, yi, rec, SRC, freqs, a0, L_PML, tx_include, ind_matlab, mask_indices, numElements)
-    kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine)
+    kw = dict(dtype=dtype, bde=bde, stencil=stencil, engine=engine, gradient=gradient)
 
     # the module functions are looked up at call time: tests record the evaluation points by replacing them
     def loss_grad(x):
@@ -606,7 +628,7 @@ def _gpu_callables(lossy, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_ma
         return float(loss), grad
 
     def linesearch(sd):
-        plan, _ = _fwi_plan(xi, yi, rec, SRC, freqs, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine)
+        plan, _ = _fwi_plan(xi, yi, rec, SRC, freqs, a0, L_PML, ind_matlab, mask_indices, dtype, stencil, device, engine, gradient)
         sdt = sd.to(dv, real)
         nd = plan._linesearch(*((sdt[0].contiguous(), sdt[1].contiguous()) if lossy else (sdt.contiguous(), None)))
         return float(nd[0]), float(nd[1])
@@ -621,7 +643,7 @@ def _gpu_callables(lossy, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_ma
 def nonlinear_conjugate_gradient_joint(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML,
                                        mask_indices, *, kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, dtype="c64", bde=None,
                                        stencil="python", device=0, engine="auto", history=None, loss_grad=None,
-                                       linesearch=None):
+                                       linesearch=None, gradient="reference"):
     """The reference's NCG loop (``nonlinear_conjugate_gradient``) on sound speed and attenuation together; returns ``(c,
     kappa)`` as NumPy (Ny, Nx) arrays.
 
@@ -634,12 +656,13 @@ def nonlinear_conjugate_gradient_joint(xi, yi, numElements, REC_DATA, SRC, tx_in
     ``loss_grad(x) -> (loss, grad)`` and ``linesearch(sd) -> (num, den)`` (at the point of the last ``loss_grad`` call)
     replace the GPU objective; they receive (2, Ny, Nx) float64 torch tensors = [slowness, kappa].  ``history`` (a list)
     receives one dict per iteration: loss, gradient norm, beta, step, velocity range, largest kappa and clipped nodes.
+    ``gradient`` is the linearisation of the gradient and the line search (``fwi_joint_loss_function``).
     """
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or linesearch is None:
         loss_grad, linesearch, _ = _gpu_callables(True, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
-                                                  mask_indices, dtype, bde, stencil, device, engine)
+                                                  mask_indices, dtype, bde, stencil, device, engine, gradient)
     x, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
     dot = lambda a, b: float(torch.sum(a * b))
     d = gprev = None
@@ -671,7 +694,7 @@ def nonlinear_conjugate_gradient_joint(xi, yi, numElements, REC_DATA, SRC, tx_in
 def gauss_newton_joint_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, Niter, a0, L_PML, mask_indices, *,
                            kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, cg_iters=8, cg_tol=1e-2, damping=0.0,
                            max_backtracks=4, dtype="c64", bde=None, stencil="python", device=0, engine="auto", history=None,
-                           loss_grad=None, hvp=None):
+                           loss_grad=None, hvp=None, gradient="reference"):
     """Truncated Gauss-Newton on sound speed and attenuation together; returns ``(c, kappa)`` as NumPy (Ny, Nx) arrays.
 
     The outer loop of ``gauss_newton_fwi`` on the block-scaled variables of ``run_lbfgs_joint_fwi`` (``D = diag(s0 pert_scale,
@@ -682,13 +705,14 @@ def gauss_newton_joint_fwi(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
 
     ``loss_grad(x) -> (loss, grad)`` and ``hvp(v) -> hv`` (at the point of the last ``loss_grad`` call) replace the GPU
     objective; they receive (2, Ny, Nx) float64 torch tensors = [slowness, kappa].  ``history`` receives the records of
-    ``gauss_newton_fwi`` plus ``clipped``, the number of kappa nodes clipped in the last trial.
+    ``gauss_newton_fwi`` plus ``clipped``, the number of kappa nodes clipped in the last trial.  ``gradient`` is the
+    linearisation of the gradient and the products (``fwi_joint_gauss_newton_product``).
     """
     import torch
     ny, nx = _to_np(yi).size, _to_np(xi).size
     if loss_grad is None or hvp is None:
         loss_grad, _, hvp = _gpu_callables(True, xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, f, a0, L_PML,
-                                           mask_indices, dtype, bde, stencil, device, engine)
+                                           mask_indices, dtype, bde, stencil, device, engine, gradient)
     x0, D = _joint_setup(ny, nx, c_init, kappa_init, kappa_scale, pert_scale)
     x = _gauss_newton_loop(x0, loss_grad, hvp, Niter, cg_iters, cg_tol, damping, max_backtracks, history, slow_of=lambda x: x[0],
                            scale=D, project=_project_kappa)
@@ -789,12 +813,13 @@ def continuation_stages(f, nstages):
 
 def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, stages, Niter,
                            a0, L_PML, mask_indices, *, dtype="c64", stencil="python", device=0, engine="auto", history=None,
-                           method="ncg"):
+                           method="ncg", gradient="reference"):
     """Multi-frequency FWI by frequency continuation: for every stage (an index array into ``f``, see
     ``continuation_stages``) ``Niter`` NCG iterations (``nonlinear_conjugate_gradient``; ``method="gn"``: ``Niter`` outer
     iterations of ``gauss_newton_fwi`` with its default settings) on the joint objective of that stage's frequencies, each
     stage starting from the sound speed the previous one ended with.  ``REC_DATA`` is (Nf, Nt, E).  Returns the final sound
-    speed (Ny, Nx); ``history`` (a list) receives one list of per-iteration records per stage.
+    speed (Ny, Nx); ``history`` (a list) receives one list of per-iteration records per stage.  ``gradient`` is passed to
+    the stage driver.
     """
     if method not in ("ncg", "gn"):
         raise ValueError("method must be 'ncg' or 'gn'")
@@ -802,10 +827,10 @@ def frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_m
     def stage(vel, rec, f, h):
         if method == "gn":
             return gauss_newton_fwi(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML, mask_indices,
-                                    dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+                                    dtype=dtype, stencil=stencil, device=device, engine=engine, history=h, gradient=gradient)
         return nonlinear_conjugate_gradient(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML,
                                             mask_indices, dtype=dtype, stencil=stencil, device=device, history=h,
-                                            return_fields=False, engine=engine)[0]
+                                            return_fields=False, engine=engine, gradient=gradient)[0]
 
     return _continuation(REC_DATA, f, stages, history, c_init, stage)
 
@@ -832,12 +857,12 @@ def _continuation(REC_DATA, f, stages, history, model, stage):
 
 def joint_frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include, ind_matlab, c_init, f, stages, Niter, a0, L_PML,
                                  mask_indices, *, kappa_init=0.0, dtype="c64", stencil="python", device=0, engine="auto",
-                                 history=None, method="ncg"):
+                                 history=None, method="ncg", gradient="reference"):
     """``frequency_continuation`` for sound speed and attenuation together: per stage ``Niter`` iterations of
     ``nonlinear_conjugate_gradient_joint`` (``method="ncg"``), outer iterations of ``gauss_newton_joint_fwi`` (``"gn"``) or
     L-BFGS-B iterations of ``run_lbfgs_joint_fwi`` (``"lbfgs"``), each with its default settings and each stage starting
     from the maps the previous one ended with.  Returns ``(c, kappa)``; ``history`` (a list) receives one list of records per
-    stage (for ``"lbfgs"``, ``(loss, params)`` of every evaluation).
+    stage (for ``"lbfgs"``, ``(loss, params)`` of every evaluation).  ``gradient`` is passed to the stage driver.
     """
     if method not in ("ncg", "gn", "lbfgs"):
         raise ValueError("method must be 'ncg', 'gn' or 'lbfgs'")
@@ -846,9 +871,9 @@ def joint_frequency_continuation(xi, yi, numElements, REC_DATA, SRC, tx_include,
         vel, kap = model
         if method == "lbfgs":
             return run_lbfgs_joint_fwi(xi, yi, rec, SRC, tx_include, ind_matlab, vel, f, a0, L_PML, mask_indices, kappa_init=kap,
-                                       maxiter=Niter, dtype=dtype, stencil=stencil, engine=engine, history=h)
+                                       maxiter=Niter, dtype=dtype, stencil=stencil, engine=engine, history=h, gradient=gradient)
         drv = gauss_newton_joint_fwi if method == "gn" else nonlinear_conjugate_gradient_joint
         return drv(xi, yi, numElements, rec, SRC, tx_include, ind_matlab, vel, f, Niter, a0, L_PML, mask_indices, kappa_init=kap,
-                   dtype=dtype, stencil=stencil, device=device, engine=engine, history=h)
+                   dtype=dtype, stencil=stencil, device=device, engine=engine, history=h, gradient=gradient)
 
     return _continuation(REC_DATA, f, stages, history, (c_init, kappa_init), stage)

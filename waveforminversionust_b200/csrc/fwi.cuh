@@ -6,6 +6,8 @@
 //                           one warp per pixel, warp-shuffle reduction     (nonlinearcg.py:258,264-265)
 //                           LOSSY: gradients w.r.t. s and kappa of the complex slowness s - i kappa (DESIGN.md section 7d)
 //   pert_rhs_kernel       : RHS of the perturbation solve  -VIRT * sd      (nonlinearcg.py:279-281)
+//   gradient_mass_kernel, pert_rhs_mass_kernel : the discrete gradient mode's gradient and perturbation RHS, with the
+//                           stencil's 9-point mass weights and the PML factor (DESIGN.md section 7f)
 //   linesearch_kernel     : dREC gather and the two step-size scalars      (nonlinearcg.py:22-28,284-298)
 //   gn_receiver_kernel    : Gauss-Newton product: J v = perturbation field at the kept receivers, and sum |J v|^2
 //   gn_scatter_kernel     : Gauss-Newton product: J v back at the receiver nodes as the adjoint source of J^H (J v)
@@ -239,6 +241,219 @@ __global__ void __launch_bounds__(256) pert_rhs_kernel(PertArgs<R> a) {
             R c = (R)(-2.0 * w * w * (double)a.slow[p] * (double)a.sd[p]);
             cx<R> v = a.src_est[(size_t)f * a.nt + t] * a.U[(size_t)f * a.stride_f + i];
             a.Out[(size_t)f * a.stride_f + i] = cx<R>(c * v.re, c * v.im);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Discrete gradient mode (UST_GRAD_DISCRETE, DESIGN.md section 7f): the exact derivative of the discrete forward map at fixed
+// stencil weights (b, d, e).  Interior row i of the operator holds the mass term sum_{j in N9(i)} w_ij C_j w^2 sigma_j^2 u_j with
+// w_ij = 1-d-e, d/4, e/4 at the centre, edge and corner offsets and C = e_x e_y; ring rows are identity rows.  So
+//   (dH u)_i = sum_j w_ij C_j 2 w^2 sigma_j dsigma_j u_j  (interior i, 0 on the ring),   J v = P H^-1(-dH alpha u),
+//   z_j = conj(C_j) sum_t conj(alpha_t u_tj) (W lambda_t)_j,  (W lambda)_j = sum_{i in N9(j), i interior} w_ij lambda_i,
+// and A, B, grad_s, grad_kappa follow from z as in gradient_kernel.  With w = delta and C = 1 this is the reference's J.
+// Both kernels give a warp a segment of MASS_SEG pixels of one grid row and slide a 3x3 window of source-units along it, so a
+// lane loads three new columns per pixel instead of nine (4.5 loads per pixel with the segment's halo columns).  Rows y-1 and
+// y+1 are loaded again by the warps of the neighbouring rows; whether L2 serves those loads is not established: the measured
+// time (DESIGN.md section 7f) is what they would cost from HBM.  A unit is what a lane loads in one step: two complex64
+// sources (16 B) or one complex.
+constexpr int MASS_SEG = 4;
+
+template <typename R>
+struct MassArgs {
+    const cx<R>* exn;   // [Nx] e_x at the nodes
+    const cx<R>* eyn;   // [Ny] e_y at the nodes
+    const double* bde;  // [nfreq][3] stencil weights of the launch's frequencies
+    int Nx, Ny;
+};
+
+template <typename R, int NS>
+struct alignas(NS * sizeof(cx<R>)) Unit { cx<R> c[NS]; };
+
+template <typename U>
+__device__ __forceinline__ U ld_stream(const U* p) {  // read-once stream: do not displace the fields the window re-reads
+    U r;
+    if constexpr (sizeof(U) == 16) { const float4 v = __ldcs(reinterpret_cast<const float4*>(p)); memcpy(&r, &v, 16); }
+    else { const float2 v = __ldcs(reinterpret_cast<const float2*>(p)); memcpy(&r, &v, 8); }
+    return r;
+}
+
+// unit k of the three rows y-1, y, y+1 at column x; zero where the node is not an interior row (keep_ring: where it is off the grid)
+template <typename R, int NS>
+__device__ __forceinline__ void mass_column(Unit<R, NS> (&col)[3], const cx<R>* F, const MassArgs<R>& m, int nt, int y, int x, int k,
+                                            bool keep_ring) {
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const int yy = y - 1 + r;
+        const bool ok = keep_ring ? (x >= 0 && x < m.Nx && yy >= 0 && yy < m.Ny) : (x > 0 && x < m.Nx - 1 && yy > 0 && yy < m.Ny - 1);
+        if (ok) col[r] = reinterpret_cast<const Unit<R, NS>*>(F + ((size_t)yy * m.Nx + x) * nt)[k];
+        else {
+#pragma unroll
+            for (int s = 0; s < NS; ++s) col[r].c[s] = cxzero<R>();
+        }
+    }
+}
+
+// (W f) at the centre of the window: c0 * centre + d4 * edges + e4 * corners
+template <typename R, int NS>
+__device__ __forceinline__ cx<R> mass_apply(int s, R c0, R d4, R e4, const Unit<R, NS> (&L)[3], const Unit<R, NS> (&M)[3],
+                                            const Unit<R, NS> (&Rt)[3]) {
+    const cx<R> edge = (M[0].c[s] + M[2].c[s]) + (L[1].c[s] + Rt[1].c[s]);
+    const cx<R> corner = (L[0].c[s] + L[2].c[s]) + (Rt[0].c[s] + Rt[2].c[s]);
+    return c0 * M[1].c[s] + d4 * edge + e4 * corner;
+}
+
+// Gradient of the discrete mode: one warp per MASS_SEG-pixel row segment, lanes over source-units; the per-pixel partials of
+// Re / Im z_f are folded into FP64 once per frequency, as in gradient_kernel.
+template <typename R, int NS, bool LOSSY>
+__global__ void __launch_bounds__(256) gradient_mass_kernel(GradArgs<R> a, MassArgs<R> m) {
+    typedef Unit<R, NS> V;
+    const int lane = threadIdx.x & 31;
+    const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+    const double PI = 3.14159265358979323846;
+    const int nseg = (m.Nx + MASS_SEG - 1) / MASS_SEG, nunits = a.nt / NS;
+    for (long long item = warp; item < (long long)m.Ny * nseg; item += nwarps) {
+        const int y = (int)(item / nseg), x0 = (int)(item % nseg) * MASS_SEG;
+        const int np = min(MASS_SEG, m.Nx - x0);
+        double tr[MASS_SEG], ti[MASS_SEG];
+#pragma unroll
+        for (int i = 0; i < MASS_SEG; ++i) tr[i] = ti[i] = 0.0;
+        for (int f = 0; f < a.nfreq; ++f) {
+            const cx<R>* u = a.U + (size_t)f * a.stride_f;
+            const cx<R>* l = a.Lam + (size_t)f * a.stride_f;
+            const V* al = reinterpret_cast<const V*>(a.src_est + (size_t)f * a.nt);
+            const double d = m.bde[3 * f + 1], e = m.bde[3 * f + 2];
+            const R c0 = (R)(1.0 - d - e), d4 = (R)(d * 0.25), e4 = (R)(e * 0.25);
+            R zr[MASS_SEG], zi[MASS_SEG];
+#pragma unroll
+            for (int i = 0; i < MASS_SEG; ++i) zr[i] = zi[i] = R(0);
+            for (int k = lane; k < nunits; k += 32) {
+                V L[3], M[3], Rt[3];
+                mass_column(L, l, m, a.nt, y, x0 - 1, k, false);
+                mass_column(M, l, m, a.nt, y, x0, k, false);
+                const V aa = al[k];
+#pragma unroll
+                for (int i = 0; i < MASS_SEG; ++i) {
+                    if (i < np) {
+                        mass_column(Rt, l, m, a.nt, y, x0 + i + 1, k, false);
+                        const V uu = ld_stream(reinterpret_cast<const V*>(u + ((size_t)y * m.Nx + x0 + i) * a.nt) + k);
+#pragma unroll
+                        for (int s = 0; s < NS; ++s) {
+                            const cx<R> au = aa.c[s] * uu.c[s], wl = mass_apply<R, NS>(s, c0, d4, e4, L, M, Rt);
+                            zr[i] += au.re * wl.re + au.im * wl.im;  // Re(conj(alpha u) W lambda)
+                            zi[i] += au.re * wl.im - au.im * wl.re;  // Im(conj(alpha u) W lambda)
+                        }
+#pragma unroll
+                        for (int r = 0; r < 3; ++r) { L[r] = M[r]; M[r] = Rt[r]; }
+                    }
+                }
+            }
+            const double w = 2.0 * PI * a.freqs[f], q = -2.0 * w * w;
+            const cx<R> ey = m.eyn[y];
+#pragma unroll
+            for (int i = 0; i < MASS_SEG; ++i) {
+                if (i < np) {
+                    const cx<R> ex = m.exn[x0 + i];
+                    const double cr = (double)ex.re * ey.re - (double)ex.im * ey.im, ci = (double)ex.re * ey.im + (double)ex.im * ey.re;
+                    tr[i] += q * (cr * zr[i] + ci * zi[i]);  // Re(conj(C) z)
+                    ti[i] += q * (cr * zi[i] - ci * zr[i]);  // Im(conj(C) z)
+                }
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < MASS_SEG; ++i) {
+            if (i < np) {
+                const double A = warp_sum(tr[i]), B = warp_sum(ti[i]);
+                const long long p = (long long)y * m.Nx + x0 + i;
+                if (lane == 0) {
+                    const double s = (double)a.slow[p];
+                    if constexpr (LOSSY) {
+                        const double k = (double)a.kappa[p];
+                        a.grad[p] = (R)(A * s - B * k);
+                        a.grad_kappa[p] = (R)(-s * B - k * A);
+                    } else {
+                        a.grad[p] = (R)(A * s);
+                    }
+                }
+            }
+        }
+    }
+}
+
+// Perturbation RHS of the discrete mode: Out_i = alpha_t sum_{j in N9(i)} w_ij c_j u_tj on interior rows, 0 on the ring, with
+// c_j = -2 w^2 C_j sigma_j dsigma_j formed in FP64 once per node and frequency into the warp's shared-memory tile.
+// grid = (blocks, nfreq); one warp per MASS_SEG-pixel row segment.  Two blocks per SM: unbounded, ptxas gives it 151-160
+// registers and one block (8 warps) per SM.
+template <typename R, int NS, bool LOSSY>
+__global__ void __launch_bounds__(256, 2) pert_rhs_mass_kernel(PertArgs<R> a, MassArgs<R> m) {
+    typedef Unit<R, NS> V;
+    __shared__ cx<R> coef_all[8][3][MASS_SEG + 2];
+    const int lane = threadIdx.x & 31;
+    cx<R> (*coef)[MASS_SEG + 2] = coef_all[threadIdx.x >> 5];
+    const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+    const double PI = 3.14159265358979323846;
+    const int f = blockIdx.y;
+    const double w = 2.0 * PI * a.freqs[f], q = -2.0 * w * w;
+    const double d = m.bde[3 * f + 1], e = m.bde[3 * f + 2];
+    const R c0 = (R)(1.0 - d - e), d4 = (R)(d * 0.25), e4 = (R)(e * 0.25);
+    const cx<R>* u = a.U + (size_t)f * a.stride_f;
+    cx<R>* out = a.Out + (size_t)f * a.stride_f;
+    const V* al = reinterpret_cast<const V*>(a.src_est + (size_t)f * a.nt);
+    const int nseg = (m.Nx + MASS_SEG - 1) / MASS_SEG, nunits = a.nt / NS;
+    for (long long item = warp; item < (long long)m.Ny * nseg; item += nwarps) {
+        const int y = (int)(item / nseg), x0 = (int)(item % nseg) * MASS_SEG;
+        const int np = min(MASS_SEG, m.Nx - x0);
+        __syncwarp();
+        if (lane < 3 * (MASS_SEG + 2)) {
+            const int r = lane / (MASS_SEG + 2), c = lane % (MASS_SEG + 2);
+            const int yy = y - 1 + r, xx = x0 - 1 + c;
+            double cr = 0.0, ci = 0.0;
+            if (yy >= 0 && yy < m.Ny && xx >= 0 && xx < m.Nx) {
+                const long long p = (long long)yy * m.Nx + xx;
+                const cx<R> ex = m.exn[xx], ey = m.eyn[yy];
+                const double Cr = (double)ex.re * ey.re - (double)ex.im * ey.im, Ci = (double)ex.re * ey.im + (double)ex.im * ey.re;
+                double gr = (double)a.slow[p] * (double)a.sd[p], gi = 0.0;  // sigma dsigma
+                if constexpr (LOSSY) {
+                    const double s = (double)a.slow[p], k = (double)a.kappa[p], ds = (double)a.sd[p], dk = (double)a.sd_kappa[p];
+                    gr = s * ds - k * dk;
+                    gi = -(s * dk + k * ds);
+                }
+                cr = q * (Cr * gr - Ci * gi);
+                ci = q * (Cr * gi + Ci * gr);
+            }
+            coef[r][c] = cx<R>((R)cr, (R)ci);
+        }
+        __syncwarp();
+        const bool ring_row = y == 0 || y == m.Ny - 1;
+        for (int k = lane; k < nunits; k += 32) {
+            V L[3], M[3], Rt[3];
+            mass_column(L, u, m, a.nt, y, x0 - 1, k, true);
+            mass_column(M, u, m, a.nt, y, x0, k, true);
+#pragma unroll
+            for (int r = 0; r < 3; ++r)
+#pragma unroll
+                for (int s = 0; s < NS; ++s) { L[r].c[s] = coef[r][0] * L[r].c[s]; M[r].c[s] = coef[r][1] * M[r].c[s]; }
+            const V aa = al[k];
+#pragma unroll
+            for (int i = 0; i < MASS_SEG; ++i) {
+                if (i < np) {
+                    mass_column(Rt, u, m, a.nt, y, x0 + i + 1, k, true);
+#pragma unroll
+                    for (int r = 0; r < 3; ++r)
+#pragma unroll
+                        for (int s = 0; s < NS; ++s) Rt[r].c[s] = coef[r][i + 2] * Rt[r].c[s];
+                    const int x = x0 + i;
+                    V o;
+#pragma unroll
+                    for (int s = 0; s < NS; ++s)
+                        o.c[s] = (ring_row || x == 0 || x == m.Nx - 1) ? cxzero<R>() : aa.c[s] * mass_apply<R, NS>(s, c0, d4, e4, L, M, Rt);
+                    reinterpret_cast<V*>(out + ((size_t)y * m.Nx + x) * a.nt)[k] = o;
+#pragma unroll
+                    for (int r = 0; r < 3; ++r) { L[r] = M[r]; M[r] = Rt[r]; }
+                }
+            }
         }
     }
 }

@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <map>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
 #include <vector>
 
@@ -87,6 +88,8 @@ struct ust_plan {
     EvalKind eval_kind = EVAL_NONE;  // cleared by ust_plan_set_acquisition
     bool factored_since_eval = false;  // factor_impl ran after it: the factors no longer belong to its fields
     bool factors_lossy = false;        // the current factors are those of a lossy model
+    int grad_mode = UST_GRAD_REFERENCE;  // ust_plan_set_gradient: linearisation of the evaluation, line search and product
+    int eval_grad_mode = UST_GRAD_REFERENCE;  // the mode the last evaluation ran with
     bool use_graphs = true;  // UST_NO_GRAPHS=1 disables
     struct GraphEntry { cudaGraphExec_t exec = nullptr; long long launches = 0; };
     std::map<long long, GraphEntry> graphs;
@@ -598,6 +601,47 @@ __global__ void recip_kernel(const R* __restrict__ in, R* __restrict__ out, long
     if (i < n) out[i] = R(1) / in[i];
 }
 
+// stencil weights and PML factors of the discrete gradient mode's kernels, for the frequencies from f0 on
+template <typename R>
+static MassArgs<R> mass_args(const ust_plan* p, int f0) {
+    MassArgs<R> m;
+    m.exn = (const cx<R>*)p->exn; m.eyn = (const cx<R>*)p->eyn; m.bde = p->d_bde + 3 * f0; m.Nx = p->g.Nx; m.Ny = p->g.Ny;
+    return m;
+}
+
+// Calls launch(NS) with the unit width of the discrete-mode kernels: complex64 lanes load two sources (16 B) when every pixel's
+// source row is 16-byte aligned (even nt), one otherwise; complex128 lanes load one.
+template <typename R, typename F>
+static void with_mass_unit(const ust_plan* p, F launch) {
+    if constexpr (sizeof(R) == 4) {
+        if ((p->nt & 1) == 0) { launch(std::integral_constant<int, 2>()); return; }
+    }
+    launch(std::integral_constant<int, 1>());
+}
+
+// Gradient over all frequencies of the evaluation into ga.grad (lossy: also ga.grad_kappa): gradient_kernel, or in the discrete
+// mode gradient_mass_kernel
+template <typename R>
+static int gradient_launch(ust_plan* p, const GradArgs<R>& ga, bool lossy, cudaStream_t st) {
+    const Geom& g = p->g;
+    ProfScope ps(p, PC_GRADIENT, st);
+    if (p->grad_mode == UST_GRAD_DISCRETE) {
+        const MassArgs<R> m = mass_args<R>(p, 0);
+        const long long items = (long long)g.Ny * cdiv_i(g.Nx, MASS_SEG);
+        const int blocks = (int)std::min<long long>((items + 7) / 8, (long long)p->num_sms * 8);
+        with_mass_unit<R>(p, [&](auto ns) {
+            if (lossy) gradient_mass_kernel<R, ns.value, true><<<blocks, 256, 0, st>>>(ga, m);
+            else gradient_mass_kernel<R, ns.value, false><<<blocks, 256, 0, st>>>(ga, m);
+        });
+    } else {
+        const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
+        if (lossy) gradient_kernel<R, true><<<blocks, 256, 0, st>>>(ga);
+        else gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
+    }
+    UST_LAUNCH_CHECK();
+    return 0;
+}
+
 // One joint (loss, grad) evaluation, device work only (CUDA-graph capturable): reads p->slow_in / p->rec_in, writes
 // p->d_scal[0] (loss) and p->grad_out.  Each frequency group runs assemble -> factor -> forward sweeps -> receivers ->
 // adjoint sweeps as its own chain; the groups meet again at the gradient, which sums over all frequencies.
@@ -646,14 +690,7 @@ static int fwi_enqueue(ust_plan* p, int nfreq, bool has_bde, cudaStream_t st, bo
     ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
     ga.freqs = p->d_freqs; ga.slow = (const R*)slow; ga.grad = (R*)p->grad_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
     ga.kappa = (const R*)p->kappa_in; ga.grad_kappa = (R*)p->grad_kappa_out;
-    const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
-    {
-        ProfScope ps(p, PC_GRADIENT, st);
-        if (lossy) gradient_kernel<R, true><<<blocks, 256, 0, st>>>(ga);
-        else gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
-    }
-    UST_LAUNCH_CHECK();
-    return 0;
+    return gradient_launch<R>(p, ga, lossy, st);
 }
 
 // RHS of the perturbation solve for every group, from the direction `dir` (and, lossy, its kappa part p->vk_in)
@@ -667,8 +704,19 @@ static int pert_rhs_groups(ust_plan* p, const std::vector<Group>& gs, const void
         pa.src_est = (const cx<R>*)p->src_est + (size_t)q.f0 * nt;
         pa.freqs = p->d_freqs + q.f0; pa.slow = (const R*)p->slow_in; pa.sd = (const R*)dir; pa.N = p->g.N; pa.nt = nt; pa.nfreq = q.nf;
         pa.kappa = (const R*)p->kappa_in; pa.sd_kappa = (const R*)p->vk_in;
-        if (lossy) pert_rhs_kernel<R, true><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
-        else pert_rhs_kernel<R, false><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+        if (p->grad_mode == UST_GRAD_DISCRETE) {  // profiled as "receiver" (the reference RHS is not profiled)
+            ProfScope ps(p, PC_RECEIVER, q.st);
+            const MassArgs<R> m = mass_args<R>(p, q.f0);
+            const long long items = (long long)p->g.Ny * cdiv_i(p->g.Nx, MASS_SEG);
+            const dim3 grid((unsigned)std::min<long long>((items + 7) / 8, (long long)p->num_sms * 8), q.nf);
+            with_mass_unit<R>(p, [&](auto ns) {
+                if (lossy) pert_rhs_mass_kernel<R, ns.value, true><<<grid, 256, 0, q.st>>>(pa, m);
+                else pert_rhs_mass_kernel<R, ns.value, false><<<grid, 256, 0, q.st>>>(pa, m);
+            });
+        } else {
+            if (lossy) pert_rhs_kernel<R, true><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+            else pert_rhs_kernel<R, false><<<dim3(p->num_sms * 4, q.nf), 256, 0, q.st>>>(pa);
+        }
         UST_LAUNCH_CHECK();
     }
     return 0;
@@ -742,14 +790,7 @@ static int gn_hvp_enqueue(ust_plan* p, cudaStream_t st, bool lossy) {
     ga.U = (const cx<R>*)p->U; ga.Lam = (const cx<R>*)p->Lam; ga.stride_f = stride; ga.src_est = (const cx<R>*)p->src_est;
     ga.freqs = p->d_freqs; ga.slow = (const R*)p->slow_in; ga.grad = (R*)p->hv_out; ga.N = g.N; ga.nt = nt; ga.nfreq = nfreq;
     ga.kappa = (const R*)p->kappa_in; ga.grad_kappa = (R*)p->hv_kappa_out;
-    const int blocks = (int)std::min<long long>((g.N + 7) / 8, (long long)p->num_sms * 8);
-    {
-        ProfScope ps(p, PC_GRADIENT, st);
-        if (lossy) gradient_kernel<R, true><<<blocks, 256, 0, st>>>(ga);
-        else gradient_kernel<R, false><<<blocks, 256, 0, st>>>(ga);
-    }
-    UST_LAUNCH_CHECK();
-    return 0;
+    return gradient_launch<R>(p, ga, lossy, st);
 }
 
 // Run `enqueue` on the caller's stream directly, or -- the normal case -- as a CUDA graph captured once per key and
@@ -790,6 +831,10 @@ static int run_graphed(ust_plan* p, long long key, cudaStream_t user, F enqueue)
     return 0;
 }
 
+// graph keys of the discrete gradient mode: every key below 1000 * nfreq + 1000 gains 50, which no reference key (0, 1, 500,
+// 600, 700, 701, 800, 900) reaches
+static long long grad_key_offset(const ust_plan* p) { return p->grad_mode == UST_GRAD_DISCRETE ? 50 : 0; }
+
 // kappa != nullptr: lossy evaluation (ust_fwi_loss_grad_lossy), gradient w.r.t. kappa into grad_kappa_dev
 template <typename R>
 static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, const double* freqs, const double* bde,
@@ -806,8 +851,8 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     if (lossy) UST_CUDA(cudaMemcpyAsync(p->kappa_in, kappa, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     const bool has_bde = bde != nullptr;
     // lossless evaluation 0/1, line search 500, Gauss-Newton product 600, lossy evaluation 700/701, lossy line search 800,
-    // lossy Gauss-Newton product 900
-    const long long key = 1000LL * nfreq + (lossy ? 700 : 0) + (has_bde ? 1 : 0);
+    // lossy Gauss-Newton product 900; the discrete gradient mode adds 50 to each (grad_key_offset)
+    const long long key = 1000LL * nfreq + (lossy ? 700 : 0) + (has_bde ? 1 : 0) + grad_key_offset(p);
     p->factored_since_eval = true;  // until this evaluation completes, the factors belong to no evaluation
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return fwi_enqueue<R>(p, nfreq, has_bde, s_, lossy); }));
     p->nfreq_cur = nfreq;
@@ -816,6 +861,7 @@ static int fwi_impl(ust_plan* p, const void* slow, const void* rec, int nfreq, c
     UST_CUDA(cudaMemcpyAsync(grad_dev, p->grad_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(grad_kappa_dev, p->grad_kappa_out, g.N * sizeof(R), cudaMemcpyDeviceToDevice, st));
     p->eval_kind = lossy ? ust_plan::EVAL_LOSSY : ust_plan::EVAL_LOSSLESS;
+    p->eval_grad_mode = p->grad_mode;
     p->factored_since_eval = false;
     p->factors_lossy = lossy;
     if (p->trace) return dump_update_trace(p, st);
@@ -836,6 +882,12 @@ static int check_eval(const ust_plan* p, const char* name, bool lossy) {
                   ") after the last " + (last_lossy ? "ust_fwi_loss_grad_lossy" : "ust_fwi_loss_grad") + "; call " + want + " again");
         return 1;
     }
+    if (p->eval_grad_mode != p->grad_mode) {
+        static const char* mode_name[2] = {"UST_GRAD_REFERENCE", "UST_GRAD_DISCRETE"};
+        set_error(n + ": the last evaluation ran in gradient mode " + mode_name[p->eval_grad_mode] + " and the plan is now in " +
+                  mode_name[p->grad_mode] + " (ust_plan_set_gradient); call " + want + " again");
+        return 1;
+    }
     if (last_lossy != lossy) {
         set_error(n + (lossy ? ": the last evaluation was lossless (ust_fwi_loss_grad); use the lossless entry point or call "
                                "ust_fwi_loss_grad_lossy first"
@@ -854,7 +906,7 @@ static int linesearch_impl(ust_plan* p, const void* sd, const void* sd_kappa, do
     const size_t bytes = p->g.N * sizeof(R);
     UST_CUDA(cudaMemcpyAsync(p->sd_in, sd, bytes, cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(p->vk_in, sd_kappa, bytes, cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + (lossy ? 800 : 500);
+    const long long key = 1000LL * p->nfreq_cur + (lossy ? 800 : 500) + grad_key_offset(p);
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return linesearch_enqueue<R>(p, s_, lossy); }));
     UST_CUDA(cudaMemcpyAsync(out2, p->d_scal + 2, 2 * sizeof(double), cudaMemcpyDeviceToDevice, st));
     return 0;
@@ -869,7 +921,7 @@ static int gn_hvp_impl(ust_plan* p, const void* v, const void* v_kappa, void* hv
     const size_t bytes = p->g.N * sizeof(R);
     UST_CUDA(cudaMemcpyAsync(p->v_in, v, bytes, cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(p->vk_in, v_kappa, bytes, cudaMemcpyDeviceToDevice, st));
-    const long long key = 1000LL * p->nfreq_cur + (lossy ? 900 : 600);
+    const long long key = 1000LL * p->nfreq_cur + (lossy ? 900 : 600) + grad_key_offset(p);
     UST_TRY(run_graphed(p, key, st, [&](cudaStream_t s_) { return gn_hvp_enqueue<R>(p, s_, lossy); }));
     UST_CUDA(cudaMemcpyAsync(hv, p->hv_out, bytes, cudaMemcpyDeviceToDevice, st));
     if (lossy) UST_CUDA(cudaMemcpyAsync(hv_kappa, p->hv_kappa_out, bytes, cudaMemcpyDeviceToDevice, st));
@@ -1146,6 +1198,16 @@ int ust_plan_set_groups(ust_plan* p, int ngroups) {
     UST_CUDA(cudaDeviceSynchronize());
     drop_graphs(p);  // the captured graphs bake the fork / join structure
     p->ngroups = ngroups;
+    return 0;
+}
+
+int ust_plan_set_gradient(ust_plan* p, int mode) {
+    UST_TRY(check_plan(p));
+    if (mode != UST_GRAD_REFERENCE && mode != UST_GRAD_DISCRETE) {
+        set_error("ust_plan_set_gradient: mode must be UST_GRAD_REFERENCE (0) or UST_GRAD_DISCRETE (1)");
+        return 1;
+    }
+    p->grad_mode = mode;  // the graphs of both modes stay: their keys differ (grad_key_offset)
     return 0;
 }
 

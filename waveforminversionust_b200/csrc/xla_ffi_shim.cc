@@ -7,6 +7,7 @@
 // present.  In this image it is compiled against a TEST DOUBLE of that header (tests/xla_ffi_stub/) and its handlers are
 // driven on the GPU by tests/test_ffi_shim.py, so the code below has met a compiler and run -- but not inside XLA.
 // Every handler only forwards device pointers + XLA's stream to the C ABI; there is no numerical code here.
+// Its plans keep the default gradient mode, UST_GRAD_REFERENCE: the discrete mode (ust_plan_set_gradient) is not exposed here.
 // The loss is returned as two float32 words (hi, lo with hi + lo = the float64 loss to ~1e-14): the reference runs JAX
 // with x64 disabled, where a float64 result buffer cannot exist.
 #include <cuda_runtime.h>

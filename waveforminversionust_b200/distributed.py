@@ -54,10 +54,11 @@ def allreduce_loss_grad(loss, grad, group=None):
 
 class ShardedFWI:
     """(loss, grad) of the joint objective over ``freqs`` with the frequencies sharded over the ranks of
-    the default process group.  One instance per rank / GPU."""
+    the default process group.  One instance per rank / GPU.  ``gradient`` (``"reference"`` or ``"discrete"``,
+    ``HelmholtzPlan.set_gradient``) is the linearisation of its gradients and Gauss-Newton products."""
 
     def __init__(self, geom, freqs, dtype="c64", device=0, stencil="python", rank=None, world=None, group=None,
-                 engine="auto", shard="freq"):
+                 engine="auto", shard="freq", *, gradient="reference"):
         import torch
         import torch.distributed as dist
         from .plan import HelmholtzPlan
@@ -85,6 +86,7 @@ class ShardedFWI:
                                   max_nrhs=max(len(self.local_tx), 1), device=device, stencil=stencil, fwi_buffers=True,
                                   engine=engine)
         self.plan.set_grid(geom.xi, geom.yi, geom.a0, geom.L_PML)
+        self.plan.set_gradient(gradient)
         rx_lin = (geom.y_idx * geom.Nx + geom.x_idx).astype(np.int32)
         if len(self.local_tx):
             self.plan.set_acquisition(geom.src_lin[self.local_tx], rx_lin, geom.mask_indices[self.local_tx])
@@ -194,13 +196,21 @@ def _engine_callables(eng, rec_local_dev, lossy):
     return loss_grad, hvp, loss_grad_np
 
 
-def run_lbfgs_sharded(eng, rec_local_dev, c_init, maxiter=1, tol=1e-5, history_size=10, history=None, pert_scale=1e-2):
+def _use_gradient(eng, gradient):
+    """``gradient`` None keeps the engine's mode; a mode name sets it on the engine's plan for this and later calls."""
+    if gradient is not None:
+        eng.plan.set_gradient(gradient)
+
+
+def run_lbfgs_sharded(eng, rec_local_dev, c_init, maxiter=1, tol=1e-5, history_size=10, history=None, pert_scale=1e-2, *,
+                      gradient=None):
     """``run_lbfgs_fwi`` (``fwi_loss_function.py:106-132``) on a sharded engine -- BASELINE configs[4]: multi-frequency L-BFGS on
     several GPUs.  Every rank runs the same L-BFGS driver (``api.run_lbfgs_fwi``) on the all-reduced joint (loss, grad), which
     NCCL delivers bit-identically to all ranks, so the ranks take identical steps without any further exchange.
     ``rec_local_dev``: this rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound
-    speed (Ny, Nx) as a NumPy array (identical on every rank)."""
+    speed (Ny, Nx) as a NumPy array (identical on every rank).  ``gradient``: the gradient mode (None: the engine's)."""
     from . import api
+    _use_gradient(eng, gradient)
     geom, plan = eng.geom, eng.plan
     loss_grad = _engine_callables(eng, rec_local_dev, False)[2]
     return api.run_lbfgs_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0, geom.L_PML,
@@ -208,11 +218,14 @@ def run_lbfgs_sharded(eng, rec_local_dev, c_init, maxiter=1, tol=1e-5, history_s
                              history=history, loss_grad=loss_grad, pert_scale=pert_scale)
 
 
-def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None):
+def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None,
+                             *, gradient=None):
     """``api.gauss_newton_fwi`` on a sharded engine: every rank runs the same driver on the all-reduced (loss, grad) and
     products, which NCCL delivers bit-identically to all ranks, so the ranks take identical steps.  ``rec_local_dev``: this
-    rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound speed (Ny, Nx)."""
+    rank's observed data on its device (``eng.local_rec`` of the full set).  Returns the final sound speed (Ny, Nx).
+    ``gradient``: the linearisation of the gradient and the products (None: the engine's)."""
     from . import api
+    _use_gradient(eng, gradient)
     geom, plan = eng.geom, eng.plan
     loss_grad, hvp, _ = _engine_callables(eng, rec_local_dev, False)
     return api.gauss_newton_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs,
@@ -222,11 +235,12 @@ def run_gauss_newton_sharded(eng, rec_local_dev, c_init, Niter, cg_iters=8, cg_t
 
 
 def run_lbfgs_joint_sharded(eng, rec_local_dev, c_init, kappa_init=0.0, kappa_scale=None, maxiter=1, tol=1e-5, history_size=10,
-                            history=None, pert_scale=1e-2):
+                            history=None, pert_scale=1e-2, *, gradient=None):
     """``api.run_lbfgs_joint_fwi`` on a sharded engine: every rank runs the same joint L-BFGS driver on the all-reduced
     ``(loss, [grad_s, grad_kappa])`` of ``ShardedFWI.loss_grad_lossy_device``, so the ranks take identical steps.  Returns
-    ``(c, kappa)`` (Ny, Nx) NumPy arrays (identical on every rank)."""
+    ``(c, kappa)`` (Ny, Nx) NumPy arrays (identical on every rank).  ``gradient``: the gradient mode (None: the engine's)."""
     from . import api
+    _use_gradient(eng, gradient)
     geom, plan = eng.geom, eng.plan
     loss_grad = _engine_callables(eng, rec_local_dev, True)[2]
     return api.run_lbfgs_joint_fwi(geom.xi, geom.yi, None, None, geom.tx_include, geom.ind_matlab, c_init, eng.freqs, geom.a0,
@@ -236,11 +250,13 @@ def run_lbfgs_joint_sharded(eng, rec_local_dev, c_init, kappa_init=0.0, kappa_sc
 
 
 def run_gauss_newton_joint_sharded(eng, rec_local_dev, c_init, Niter, kappa_init=0.0, kappa_scale=None, pert_scale=1e-2, cg_iters=8,
-                                   cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None):
+                                   cg_tol=1e-2, damping=0.0, max_backtracks=4, history=None, *, gradient=None):
     """``api.gauss_newton_joint_fwi`` on a sharded engine: every rank runs the same joint driver on the all-reduced
     ``loss_grad_lossy_device`` and ``gn_hvp_lossy_device``, so the ranks take identical steps.  Returns ``(c, kappa)`` (Ny, Nx)
-    NumPy arrays (identical on every rank)."""
+    NumPy arrays (identical on every rank).  ``gradient``: the linearisation of the gradient and the products (None: the
+    engine's)."""
     from . import api
+    _use_gradient(eng, gradient)
     geom, plan = eng.geom, eng.plan
     loss_grad, hvp, _ = _engine_callables(eng, rec_local_dev, True)
     return api.gauss_newton_joint_fwi(geom.xi, geom.yi, geom.num_elements, None, None, geom.tx_include, geom.ind_matlab, c_init,

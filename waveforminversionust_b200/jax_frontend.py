@@ -2,6 +2,9 @@
 (``Final_python/solve_helmholtz.py:85-93``) so that ``solve_helmholtz`` / ``fwi_loss_function`` stay traceable inside
 ``jax.jit`` / ``lax.scan`` (``nonlinearcg.py:172-174, 305-307``) / ``jaxopt.LBFGS``.
 
+Reference gradient only: the handlers' plans keep the default ``UST_GRAD_REFERENCE`` linearisation; the ``gradient="discrete"``
+mode of ``api`` (DESIGN.md section 7f) is not exposed through XLA.
+
 STATUS: ``csrc/xla_ffi_shim.cc`` binds the C ABI of libustfwi.so as two XLA FFI handlers.  JAX / jaxlib are not installable
 in the build image (no network), so here the shim is compiled against a test double of ``xla/ffi/api/ffi.h``
 (``build_ffi(stub=True)``, ``tests/xla_ffi_stub/``) and its handlers are driven on the GPU by ``tests/test_ffi_shim.py``;

@@ -13,6 +13,7 @@ from . import _lib
 DTYPES = {"c64": 0, "c128": 1}
 STENCILS = {"python": 0, "matlab": 1}
 ENGINES = {"auto": 0, "simt": 1, "tc2": 3}
+GRADIENTS = {"reference": 0, "discrete": 1}
 _NP_REAL = {"c64": np.float32, "c128": np.float64}
 _NP_CPLX = {"c64": np.complex64, "c128": np.complex128}
 
@@ -59,6 +60,7 @@ class HelmholtzPlan:
         self._acq_key = None
         self._factor_key = None
         self._eval_key = None  # inputs of the last fwi_loss_function on this plan (api.fwi_gauss_newton_product)
+        self.gradient = "reference"  # ust_plan_set_gradient's mode (set_gradient)
 
     def close(self):
         if getattr(self, "h", None):
@@ -78,6 +80,17 @@ class HelmholtzPlan:
     def set_groups(self, ngroups):
         """Number of independent launch chains (streams) the frequencies of one call are split into."""
         _lib.check(self.L.ust_plan_set_groups(self.h, int(ngroups)), "ust_plan_set_groups")
+
+    def set_gradient(self, mode):
+        """Linearisation behind the gradient, the line search and the Gauss-Newton product (``ust_plan_set_gradient``):
+        ``"reference"`` (the default) is the reference's virtual source ``2 w^2 sigma alpha u``; ``"discrete"`` adds the
+        stencil's 9-point mass weights and the PML factor, so that the gradient is the exact derivative of the discrete loss at
+        fixed stencil weights (DESIGN.md section 7f).  A line search or product refuses when the mode differs from the one the
+        last evaluation ran with."""
+        if mode not in GRADIENTS:
+            raise ValueError(f"gradient must be one of {sorted(GRADIENTS)}, got {mode!r}")
+        _lib.check(self.L.ust_plan_set_gradient(self.h, GRADIENTS[mode]), "ust_plan_set_gradient")
+        self.gradient = mode
 
     # -- setup ------------------------------------------------------------------------------
     def set_grid(self, x, y, a0, L_PML):
